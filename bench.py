@@ -231,6 +231,25 @@ def bind_to_gpu_local_cpus(local_rank: int):
     return info
 
 
+DUMP_READS = 65536  # 65 536 records of 105 values (plus read_index) in float64 stay under 64 MB
+
+
+def dump_outputs(out_dir: str, recs: np.ndarray, status: np.ndarray):
+    """What the last timed step handed its caller: every field of the adb_record array (as records_<field>.npy, one row
+    per read) and the per-minibatch status.  Runs with more than DUMP_READS reads keep a fixed, seeded sample of the
+    reads (read_index.npy), so two builds given the same arguments write comparable files."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.arange(len(recs))
+    if len(recs) > DUMP_READS:
+        idx = np.sort(np.random.default_rng(0).choice(len(recs), DUMP_READS, replace=False))
+    arrays = {"read_index": idx, "status": status}
+    for name in recs.dtype.names:
+        if name != "_reserved":
+            arrays["records_" + name] = recs[name][idx]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
 CLS_NAMES = ["global_select_pass", "global_select_small", "validate_hist_kernel", "llr_primary_kernel", "mvs_series_kernel + series_median_kernel",
              "cnn_conv_kernels", "cnn_pre_post | start_peak | svb16_decode", "handover_kernels"]
 
@@ -319,6 +338,8 @@ class Runner:
         rec_dev_host = records.cpu()
         n_pass = int(torch.frombuffer(rec_dev_host.numpy(), dtype=torch.int32).reshape(n, 128)[:, 0].sum().item())
         lost = int((status != 0).sum().item())
+        if args.dump_outputs and label == "main" and self.rank == 0:
+            dump_outputs(args.dump_outputs, rec_dev_host.numpy().view(_lib.RECORD_DTYPE), status.cpu().numpy())
         gsel_fallbacks = ctx.query("global_select_fallbacks") if flat["primary_method"] == 0 else 0
         val_handovers = ctx.query("validate_handovers")
 
@@ -508,6 +529,8 @@ def main():
                     help="for ncu launch lists: device-resident steps only")
     ap.add_argument("--stress", action="store_true",
                     help="BASELINE config 4: poly(A) lengths up to the preload limit, 10 %% of the reads ending early")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step of the main workload returned (records, status) to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     chem = args.chemistry.lower()

@@ -110,6 +110,22 @@ def build_scratch_package(force: bool = False) -> str:
     return root
 
 
+def kernel_available() -> bool:
+    """the reference's compiled _c_llr can be loaded: from its source, or prebuilt in oracle/_ref"""
+    return reference_present() or os.path.exists(ref_so_path())
+
+
+def load_c_llr():
+    """the reference's compiled _c_llr module (built first where the source is present)"""
+    import importlib.util
+
+    so = build_c_llr() if reference_present() else ref_so_path()
+    spec = importlib.util.spec_from_file_location("_c_llr", so)
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
 def import_reference():
     """Put the runnable copy on sys.path and return the reference's ``adapted`` package (built first where
     /root/reference exists; on the GPU box the prebuilt oracle/_ref/pkg is used as it is)."""

@@ -1,6 +1,7 @@
-"""Generate tests/golden/* by EXECUTING THE REFERENCE (TEST INFRASTRUCTURE; build container only).
+"""Generate tests/golden/* by EXECUTING THE REFERENCE (TEST INFRASTRUCTURE; needs the reference's source).
 
     python -m oracle.make_golden
+    python -m oracle.make_golden --checks [--from-oracle]   (the oracle-vs-reference tests' data, see write_checks)
 
 Inputs are seeded synthetic minibatches from adapted_b200.synth.make_reads; each golden file records the
 generator arguments and a sha256 of the generated ADC blob (so a drifting generator is detected instead
@@ -136,7 +137,87 @@ def reference_configs():
     return out
 
 
+CHECK_CASES = [
+    # the fresh seeds of tests/test_oracle_vs_reference.py: name, seam, chemistry, n, seed, generator kwargs
+    ("check_llr_rna002_101", "llr2", "rna002", 40, 101, {}),
+    ("check_llr_rna002_102", "llr2", "rna002", 40, 102, {"stress": True}),
+    ("check_cnn_rna004_201", "cnn", "rna004", 60, 201, {}),
+    ("check_cnn_rna004_202", "cnn", "rna004", 60, 202, {"short_frac": 0.3}),
+    ("check_cnn_rna004_203", "cnn", "rna004", 60, 203, {"stress": True}),
+    ("check_start_peak_rna004_301", "start_peak", "rna004", 40, 301, {}),
+    ("check_start_peak_rna004_302", "start_peak", "rna004", 40, 302, {"short_frac": 0.3}),
+]
+
+
+def write_checks(from_oracle: bool = False):
+    """tests/golden/check_*.json.gz and c_llr_calls.json.gz: what the reference returns for the inputs of
+    tests/test_oracle_vs_reference.py and tests/test_oracle_llr.py, which compare the oracle with them where no copy of
+    the reference is present.  Needs such a copy (its source, or a prebuilt oracle/_ref).  Only with from_oracle
+    (--from-oracle) are the oracle's own results recorded instead, and every file then says so in its "source"."""
+    from oracle import detect_ref
+    from tests import test_oracle_llr as t
+    from tests.golden_io import C_LLR_CALLS, KernelCalls, ORACLE_SOURCE, load_cnn_weights
+
+    logging.disable(logging.CRITICAL)
+    warnings.simplefilter("ignore")
+    live = (build_ref.reference_present() or build_ref.package_present()) and build_ref.kernel_available()
+    if not live and not from_oracle:
+        sys.exit("--checks runs the reference: build oracle/_ref from its source first (python -m oracle.build_ref); "
+                 "--from-oracle records the oracle's own results instead")
+    if live:
+        build_ref.import_reference()
+        from adapted.detect import combined
+        from adapted.detect.cnn import load_cnn_model
+
+        cfgs = reference_configs()
+        model = load_cnn_model(cfgs[("plain", "rna004")].cnn_boundaries.model_name)
+        kernel, source = build_ref.load_c_llr(), "KleistLab/ADAPTed v0.2.4 (executed)"
+    else:
+        from types import SimpleNamespace
+
+        from adapted_b200.config import get_chemistry_specific_config, start_peak_config
+
+        cfgs = {(v, c): (start_peak_config(c) if v == "start_peak" else get_chemistry_specific_config(c))
+                for v in ("plain", "start_peak") for c in ("rna002", "rna004")}
+        # the oracle's restatement under the names of the reference's _c_llr module
+        kernel = SimpleNamespace(c_llr_trace=detect_ref.llr_trace, c_llr_detect_adapter=detect_ref.llr_detect_adapter,
+                                 c_llr_detect_adapter_polya=detect_ref.llr_detect_adapter_polya,
+                                 c_llr_detect_adapter_polya_trace=detect_ref.llr_boundary_traces,
+                                 c_llr_boundary_traces=detect_ref.llr_boundary_traces)
+        source = ORACLE_SOURCE
+    for name, seam, chem, n, seed, kw in CHECK_CASES:
+        spc = cfgs[("start_peak" if seam == "start_peak" else "plain", chem)]
+        batch = make_reads(n, chem, spc.sig_preload_size, seed=seed, **kw)
+        x = batch.to_dense_pa()
+        if seam == "llr2":
+            res = (combined.combined_detect_llr2 if live else detect_ref.detect_llr2)(x, batch.full_lens, spc)
+        elif seam == "cnn":
+            res = combined.combined_detect_cnn(x.copy(), batch.full_lens, model, spc) if live else \
+                detect_ref.detect_cnn(x, batch.full_lens, load_cnn_weights(), spc)
+        else:
+            res = (combined.combined_detect_start_peak if live else detect_ref.detect_start_peak)(x, batch.full_lens, spc)
+        res = [r if isinstance(r, dict) else r.to_dict() for r in (res if isinstance(res, list) else [res])]
+        rec = dict(name=name, seam=seam, chemistry=chem, n=n, seed=seed, gen_kwargs=kw, m=int(spc.sig_preload_size),
+                   adc_sha256=hashlib.sha256(batch.adc.tobytes()).hexdigest(), config=config_as_dict(spc), source=source,
+                   results=[{k: _jsonable(v) for k, v in r.items()} for r in res])
+        with gzip.GzipFile(os.path.join(GOLDEN, name + ".json.gz"), "wb", mtime=0) as f:
+            f.write(json.dumps(rec).encode())
+    # the test functions themselves make the kernel calls, so the recorded arguments are exactly theirs
+    rec = KernelCalls(kernel)
+    for fn, params in ((t.test_full_trace_bit_identical, [(s,) for s in range(6)]),
+                       (t.test_early_stop_variants_bit_identical, [(s, k) for s in range(6) for k in (1, 2, 5)]),
+                       (t.test_degenerate_variances, [()]),
+                       (t.test_legacy_three_split_detectors_match_reference_kernel, [(s,) for s in range(4)])):
+        for p in params:
+            fn(rec, *p)
+    with gzip.GzipFile(C_LLR_CALLS, "wb", mtime=0) as f:
+        f.write(json.dumps(dict(source=source, calls=rec.calls)).encode())
+    print(f"{len(CHECK_CASES)} seam checks and {len(rec.calls)} kernel calls from {source}")
+
+
 def main():
+    if "--checks" in sys.argv:
+        return write_checks(from_oracle="--from-oracle" in sys.argv)
     if not build_ref.reference_present():
         sys.exit("needs /root/reference")
     build_ref.import_reference()

@@ -1,22 +1,10 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE_PRESENT = os.path.isfile("/root/reference/adapted/detect/_c_llr.pyx")
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run with -m gpu on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    skip_ref = pytest.mark.skip(reason="/root/reference not present on this machine")
-    for item in items:
-        if "reference" in item.keywords and not REFERENCE_PRESENT:
-            item.add_marker(skip_ref)
