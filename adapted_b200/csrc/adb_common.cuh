@@ -160,6 +160,13 @@ __device__ __forceinline__ uint32_t warp_max_u(uint32_t v) {
     return v;
 }
 
+// python slice clipping of [a, b) to [0, size)
+__device__ __forceinline__ void clip_seg(int &a, int &b, int size) {
+    a = min(max(a, 0), size);
+    b = min(max(b, 0), size);
+    if (b < a) b = a;
+}
+
 // in_range of adapted/detect/utils.py:16-26 on doubles (NaN -> false)
 __device__ __forceinline__ bool in_range_d(double v, const double r[2]) { return r[0] <= v && v <= r[1]; }
 

@@ -8,6 +8,7 @@
 #pragma once
 #include "adb_common.cuh"
 #include "adb_select.cuh"
+#include "adb_vcheck.cuh"
 
 #define ADB_MAX_MOVE_WINDOW 4096   // bottleneck window sizes accepted (any value up to the segment length works)
 #define ADB_MAX_MEAN_WINDOW 65536
@@ -72,13 +73,6 @@ __device__ void val_window_bounds(ValCtx &C) {
         C.wvmin = C.wvmax = 0.f;
         C.wkmin = C.wkmax = 0;
     }
-}
-
-// python slice clipping of [a, b) to [0, size)
-__device__ __forceinline__ void clip_seg(int &a, int &b, int size) {
-    a = min(max(a, 0), size);
-    b = min(max(b, 0), size);
-    if (b < a) b = a;
 }
 
 __device__ float seg_median(ValCtx &C, int a, int b) {
@@ -272,8 +266,7 @@ __device__ float seg_mean_exact_small(ValCtx &C, int a, int n) {
     __syncthreads();
     if (threadIdx.x == 0) {
         const ReadSrc &src = C.src;
-        float s = np_sum_f32([&](int i) { return src.pa(a + i); }, n);
-        ((float *)C.dtmp)[0] = __fdiv_rn(s, (float)n);
+        ((float *)C.dtmp)[0] = np_mean_f32([&](int i) { return src.pa(a + i); }, n);
     }
     __syncthreads();
     float r = ((float *)C.dtmp)[0];
@@ -301,8 +294,7 @@ __device__ float seg_var_exact_small(ValCtx &C, int a, int n) {
     float mean = seg_mean_exact_small(C, a, n);
     if (threadIdx.x == 0) {
         const ReadSrc &src = C.src;
-        float s = np_sum_f32([&](int i) { float d = __fsub_rn(src.pa(a + i), mean); return __fmul_rn(d, d); }, n);
-        ((float *)C.dtmp)[0] = __fdiv_rn(s, (float)n);
+        ((float *)C.dtmp)[0] = np_var_f32([&](int i) { return src.pa(a + i); }, n, mean);
     }
     __syncthreads();
     float r = ((float *)C.dtmp)[0];
@@ -984,14 +976,8 @@ __device__ MvsOut mvs_check(ValCtx &C, int ae, int pe, double mean_lo, double me
     const float shift32 = __fsub_rn(m_after, m_before);
     R.v[0] = (double)mean32; R.v[1] = (double)var32; R.v[2] = (double)med32; R.v[3] = lr; R.v[4] = (double)shift32;
     const double mr[2] = {mean_lo, mean_hi};
-    int mask = 0;
-    if (!in_range_d(R.v[0], mr)) mask |= 1;
-    if (!in_range_d(R.v[1], cfg.pA_var_range)) mask |= 2;
-    if (!in_range_d(R.v[2], cfg.polyA_med_range)) mask |= 4;
-    if (!in_range_d(R.v[3], cfg.polyA_local_range)) mask |= 8;
-    if (!in_range_d(R.v[4], cfg.median_shift_range)) mask |= 16;
-    R.fail_mask = mask;
-    R.ok = (mask == 0);
+    R.fail_mask = vc_mvs_mask(cfg, R.v, mr);
+    R.ok = (R.fail_mask == 0);
     return R;
 }
 
@@ -1147,16 +1133,10 @@ struct PrimaryBounds {
 __device__ void validate_boundaries_cta(ValCtx &C, const PrimaryBounds &B, int full_len, adb_record *rec) {
     const adb_config &cfg = *C.cfg;
     const int size = C.src.n;
-    int a_start = B.adapter_start, a_end = B.adapter_end, pe_best = B.polya_end;
-    bool success = true;
-    int fail = ADB_FAIL_NONE, fail_mask = 0;
-    uint32_t valid = ADB_V_FIELDS;
+    VcOut o = vc_out(B.adapter_start);
+    int a_end = B.adapter_end, pe_best = B.polya_end;
     float a_med = CUDART_NAN_F, a_mad = CUDART_NAN_F;
     bool have_amed = false;
-    double mvs_v[5] = {0, 0, 0, 0, 0};
-    double real_v[3] = {0, 0, 0};
-    double med_shift = 0.0;
-    int n_open = 0;
     int mvs_a_end = 0;
     bool polya_none = false;
     const int a_end0 = B.adapter_end;
@@ -1164,76 +1144,71 @@ __device__ void validate_boundaries_cta(ValCtx &C, const PrimaryBounds &B, int f
     bool lr0_ok = false; double lr0 = 0.0;
 
     if (a_end == 0) {
-        success = false; fail = ADB_FAIL_NO_ADAPTER;
+        o.success = false; o.fail = ADB_FAIL_NO_ADAPTER;
     } else {
         // the local range of real_range_check covers the same samples when the adapter is short and no open
         // pore moves its start: take it from the same histogram
-        int ca = a_start, cb = a_end;
+        int ca = o.a_start, cb = a_end;
         clip_seg(ca, cb, size);
         lr0_ok = cfg.real_signal_check && (cb - ca) <= cfg.max_obs_local_range;
-        const SegStats A0 = seg_stats(C, a_start, a_end, SS_MED | SS_MAD | (lr0_ok ? SS_LR : 0));
+        const SegStats A0 = seg_stats(C, o.a_start, a_end, SS_MED | SS_MAD | (lr0_ok ? SS_LR : 0));
         a_med = A0.med; a_mad = A0.mad; lr0 = A0.lr;
         have_amed = true;
     }
-    if (success && (a_mad != 0.0f) && !in_range_d((double)a_mad, cfg.adapter_mad_range)) {
-        success = false; fail = ADB_FAIL_ADAPTER_MAD;
+    if (o.success && (a_mad != 0.0f) && !in_range_d((double)a_mad, cfg.adapter_mad_range)) {
+        o.success = false; o.fail = ADB_FAIL_ADAPTER_MAD;
     }
-    const int a_start0 = a_start;
-    if (success && cfg.detect_open_pores) {
+    const int a_start0 = o.a_start;
+    if (o.success && cfg.detect_open_pores) {
         int last = 0;
-        n_open = open_pores_scan(C, a_start, a_end, rec, &last);
-        valid |= ADB_V_OPEN_PORES;
-        if (n_open > 0) {
-            a_start = last;
-            if (a_end - a_start < cfg.min_obs_adapter) { success = false; fail = ADB_FAIL_OPEN_PORE; }
+        o.n_open = open_pores_scan(C, o.a_start, a_end, rec, &last);
+        o.valid |= ADB_V_OPEN_PORES;
+        if (o.n_open > 0) {
+            o.a_start = last;
+            if (a_end - o.a_start < cfg.min_obs_adapter) { o.success = false; o.fail = ADB_FAIL_OPEN_PORE; }
         }
     }
-    if (success && cfg.real_signal_check) {
-        int a = a_start, b = a_end;
+    if (o.success && cfg.real_signal_check) {
+        int a = o.a_start, b = a_end;
         clip_seg(a, b, size);
         const int len = b - a;
         if (len < 2 * cfg.mean_window) {
-            success = false; fail = ADB_FAIL_REAL_RANGE;
+            o.success = false; o.fail = ADB_FAIL_REAL_RANGE;
         } else {
             float m0, m1;
             seg_mean_exact_pair(C, a, b - cfg.mean_window, cfg.mean_window, m0, m1);
-            real_v[0] = (double)m0; real_v[1] = (double)m1;
-            valid |= ADB_V_REAL_MEANS;
+            o.real[0] = (double)m0; o.real[1] = (double)m1;
+            o.valid |= ADB_V_REAL_MEANS;
             if (in_range_d((double)m0, cfg.mean_start_range) && in_range_d((double)m1, cfg.mean_end_range)) {
                 const int w = min(cfg.max_obs_local_range, len);
-                const double lr = (lr0_ok && a_start == a_start0 && w == len) ? lr0 : seg_stats(C, b - w, b, SS_MED | SS_LR).lr;
-                real_v[2] = lr;
-                valid |= ADB_V_REAL_RANGE;
-                if (!in_range_d(lr, cfg.local_range)) { success = false; fail = ADB_FAIL_REAL_RANGE; }
+                const double lr = (lr0_ok && o.a_start == a_start0 && w == len) ? lr0 : seg_stats(C, b - w, b, SS_MED | SS_LR).lr;
+                o.real[2] = lr;
+                o.valid |= ADB_V_REAL_RANGE;
+                if (!in_range_d(lr, cfg.local_range)) { o.success = false; o.fail = ADB_FAIL_REAL_RANGE; }
             } else {
-                success = false; fail = ADB_FAIL_REAL_RANGE;
+                o.success = false; o.fail = ADB_FAIL_REAL_RANGE;
             }
         }
     }
-    bool exception = false;
-    if (success && cfg.mvs_detect_check) {
+    if (o.success && cfg.mvs_detect_check) {
         if (pe_best == 0) {
-            success = false; fail = ADB_FAIL_NO_POLYA;
+            o.success = false; o.fail = ADB_FAIL_NO_POLYA;
         } else {
-            double mlo = cfg.pA_mean_range[0], mhi = cfg.pA_mean_range[1];
-            if (cfg.pA_mean_range_empty && !cfg.pA_mean_scale_range_empty) {
-                mlo = __dmul_rn(cfg.pA_mean_scale_range[0], (double)a_med);
-                mhi = __dmul_rn(cfg.pA_mean_scale_range[1], (double)a_med);
-            } else if (cfg.pA_mean_range_empty) {
-                exception = true; fail = ADB_FAIL_EXC_PA_MEAN_RANGE;
-            }
-            if (!exception && B.n_topk < 0) { exception = true; fail = ADB_FAIL_EXC_TOPK_NONE; }
-            if (!exception && cfg.mvs_detect_overwrite) {
+            double mr[2];
+            if (!vc_pa_mean_bounds(cfg, a_med, mr)) { o.exception = true; o.fail = ADB_FAIL_EXC_PA_MEAN_RANGE; }
+            else if (B.n_topk < 0) { o.exception = true; o.fail = ADB_FAIL_EXC_TOPK_NONE; }
+            const double mlo = mr[0], mhi = mr[1];
+            if (!o.exception && cfg.mvs_detect_overwrite) {
                 // combined.py:517-566.  The detection only depends on adapter_end, which changes on success only,
                 // and success ends the loop: every further candidate after a failure repeats the same evaluation.
                 if (B.n_topk > 0 && B.topk[0] != 0) {
                     const bool f64_bounds = cfg.pA_mean_range_empty != 0;
                     const MvsLocOut R = mvs_detect_at_loc(C, a_end, mlo, mhi, f64_bounds);
-                    for (int i = 0; i < 5; i++) mvs_v[i] = R.v[i];
+                    for (int i = 0; i < 5; i++) o.mvs[i] = R.v[i];
                     mvs_a_end = R.idx;
-                    valid |= ADB_V_MVS | ADB_V_MVS_ADAPTER_END;
+                    o.valid |= ADB_V_MVS | ADB_V_MVS_ADAPTER_END;
                     if (!R.ok) {
-                        success = false; fail = ADB_FAIL_MVS_NO_ADAPTER;
+                        o.success = false; o.fail = ADB_FAIL_MVS_NO_ADAPTER;
                     } else {
                         int pe = B.topk[0];
                         if (R.idx - a_end > 0) {
@@ -1242,14 +1217,14 @@ __device__ void validate_boundaries_cta(ValCtx &C, const PrimaryBounds &B, int f
                                 // polya_end_adjust and polya_truncated are None in v0.2.4, so polya_end becomes
                                 // trace_early_stop_pos -- None as well (combined.py:560-562)
                                 polya_none = true;
-                                valid |= ADB_V_TO_EARLY_STOP | ADB_V_POLYA_NONE;
+                                o.valid |= ADB_V_TO_EARLY_STOP | ADB_V_POLYA_NONE;
                             }
                         }
                         pe_best = pe;
                     }
                 }
             } else
-            if (!exception) {
+            if (!o.exception) {
                 // combined.py:464-566.  `success` is never set back to True, so once the first candidate fails the
                 // reference evaluates EVERY remaining non-zero candidate and ends with: the values of the LAST
                 // candidate, the fail reason of the last candidate that failed, polya_end = the first candidate.
@@ -1257,50 +1232,42 @@ __device__ void validate_boundaries_cta(ValCtx &C, const PrimaryBounds &B, int f
                 // candidate 0, then the last candidate, then -- only while those pass -- the ones before it.
                 int n_eval = 0;
                 while (n_eval < B.n_topk && B.topk[n_eval] != 0) n_eval++;
-                auto take_fail = [&](const MvsOut &R) {
-                    if (R.v[0] == 0.0) { fail = ADB_FAIL_MVS_NOT_ENOUGH; fail_mask = 0; }
-                    else { fail = ADB_FAIL_MVS_CHECKS; fail_mask = R.fail_mask; }
-                };
                 if (n_eval > 0) {
                     const int pe0 = B.topk[0];
                     const MvsOut R0 = mvs_check(C, a_end, pe0, mlo, mhi);
-                    for (int i = 0; i < 5; i++) mvs_v[i] = R0.v[i];
-                    valid |= ADB_V_MVS;
+                    for (int i = 0; i < 5; i++) o.mvs[i] = R0.v[i];
+                    o.valid |= ADB_V_MVS;
                     if (R0.ok || R0.v[0] != 0.0) { polya_med_cache = (float)R0.v[2]; polya_mad_cache = R0.polya_mad; polya_med_cache_pe = pe0; }
                     if (R0.ok) {
                         pe_best = pe0;
                     } else {
-                        success = false;
-                        take_fail(R0);
+                        o.success = false;
+                        vc_mvs_fail(R0.v[0], R0.fail_mask, o.fail, o.fail_mask);
                         bool fail_known = false;  // fail reason of the last failing candidate found?
                         for (int t = n_eval - 1; t >= 1 && !fail_known; t--) {
                             const MvsOut R = mvs_check(C, a_end, B.topk[t], mlo, mhi);
-                            if (t == n_eval - 1) for (int i = 0; i < 5; i++) mvs_v[i] = R.v[i];
-                            if (!R.ok) { take_fail(R); fail_known = true; }
+                            if (t == n_eval - 1) for (int i = 0; i < 5; i++) o.mvs[i] = R.v[i];
+                            if (!R.ok) { vc_mvs_fail(R.v[0], R.fail_mask, o.fail, o.fail_mask); fail_known = true; }
                         }
                     }
                 }
             }
         }
     }
-    if (!exception && success && cfg.detect_med_shift) {
+    if (!o.exception && o.success && cfg.detect_med_shift) {
         const int w = cfg.med_shift_window;
         const float m_after = seg_stats(C, a_end, min(a_end + w, full_len), SS_MED).med;
         const float m_before = seg_stats(C, max(a_end - w, 0), a_end, SS_MED).med;
-        const float sh = __fsub_rn(m_after, m_before);
-        med_shift = (double)sh;
-        valid |= ADB_V_MED_SHIFT;
-        if (!in_range_d(med_shift, cfg.med_shift_range)) { success = false; fail = ADB_FAIL_MED_SHIFT; }
+        o.med_shift = (double)__fsub_rn(m_after, m_before);
+        o.valid |= ADB_V_MED_SHIFT;
+        if (!in_range_d(o.med_shift, cfg.med_shift_range)) { o.success = false; o.fail = ADB_FAIL_MED_SHIFT; }
     }
-    if (exception) {
-        // combined.py:225-226 / 304-305 / 350-351: DetectResults(success=False, fail_reason=str(e)), all else None
-        if (threadIdx.x == 0) {
-            rec->success = 0; rec->fail_code = fail; rec->mvs_fail_mask = 0; rec->valid = 0;
-            rec->signal_len = full_len; rec->preloaded = min(full_len, size);
-        }
+    if (o.exception) {
+        if (threadIdx.x == 0) vc_write_exception(rec, o.fail, full_len, size);
         return;
     }
     // partition statistics (signal_partitions.py:65-96), with the updated adapter_start
+    const int a_start = o.a_start;
     double st[3][4];
     for (int p = 0; p < 3; p++) for (int q = 0; q < 4; q++) st[p][q] = 0.0;
     if (a_end > a_start) {
@@ -1311,7 +1278,7 @@ __device__ void validate_boundaries_cta(ValCtx &C, const PrimaryBounds &B, int f
             med = Q.med; mad = Q.mad;
         }
         st[0][2] = (double)med; st[0][3] = (double)mad;
-        valid |= ADB_V_ADAPTER_STATS;
+        o.valid |= ADB_V_ADAPTER_STATS;
     }
     if (polya_none) pe_best = 0;  // calc_partition_stats(…, None): no polya and no rna partition
     if (!polya_none && pe_best > a_end) {
@@ -1322,34 +1289,15 @@ __device__ void validate_boundaries_cta(ValCtx &C, const PrimaryBounds &B, int f
             med = Q.med; mad = Q.mad;
         }
         st[1][2] = (double)med; st[1][3] = (double)mad;
-        valid |= ADB_V_POLYA_STATS;
+        o.valid |= ADB_V_POLYA_STATS;
     }
     if (!polya_none && size > pe_best) {
         seg_mean_std(C, pe_best, size, st[2][0], st[2][1]);
         const SegStats Q = seg_stats(C, pe_best, size, SS_MED | SS_MAD);
         const float med = Q.med, mad = Q.mad;
         st[2][2] = (double)med; st[2][3] = (double)mad;
-        valid |= ADB_V_RNA_STATS;
+        o.valid |= ADB_V_RNA_STATS;
     }
-    if (threadIdx.x == 0) {
-        rec->success = success ? 1 : 0;
-        rec->fail_code = fail;
-        rec->mvs_fail_mask = fail_mask;
-        rec->valid = valid | (B.n_topk >= 0 ? ADB_V_CAND : 0);
-        rec->signal_len = full_len;
-        rec->preloaded = min(full_len, size);
-        rec->adapter_start = a_start;
-        rec->adapter_end = a_end;
-        rec->polya_end = pe_best;
-        rec->primary_adapter_end = B.adapter_end;
-        rec->primary_polya_end = B.polya_end;
-        rec->mvs_adapter_end = mvs_a_end;
-        rec->n_cand = max(B.n_topk, 0);
-        for (int t = 0; t < ADB_MAX_CAND; t++) rec->cand[t] = (t < B.n_topk) ? B.topk[t] : 0;
-        rec->n_open_pores = n_open;
-        for (int p = 0; p < 3; p++) for (int q = 0; q < 4; q++) rec->stats[p][q] = st[p][q];
-        for (int i = 0; i < 5; i++) rec->mvs[i] = mvs_v[i];
-        for (int i = 0; i < 3; i++) rec->real[i] = real_v[i];
-        rec->med_shift = med_shift;
-    }
+    if (threadIdx.x == 0)
+        vc_write_record(rec, o, st, full_len, size, a_end, pe_best, B.adapter_end, B.polya_end, mvs_a_end, B.n_topk, B.topk);
 }

@@ -1,6 +1,6 @@
 // validate_boundaries + per-segment statistics for int16 sources WITHOUT shared-memory atomics.
 //
-// Reference: adapted/detect/combined.py:358-631 (control flow as in adb_validate.cuh, SURVEY.md A.8).
+// Reference: adapted/detect/combined.py:358-631 (the checks and the record: adb_vcheck.cuh, SURVEY.md A.8).
 //
 // The histogram-based statistics of adb_validate.cuh are bound by the shared-memory atomic unit (~2 cycles per
 // sample and histogram, ncu: profiles/r1_validate_kernel_v3.txt).  Here every order statistic of a read is found by
@@ -14,9 +14,10 @@
 //            probing the middle candidate of the longer side.
 // Sums for mean / std are exact integer sums of the codes.  The float32 moving-statistics series (bottleneck
 // recurrences, mvs_series_kernel) are staged in shared memory and their medians found by bisection on the ordered
-// float bits.  Anything outside this path (float32 sources, codes outside [0, 0x7c00), no precomputed series, further
-// poly(A) candidates after a failed first one, the CNN path's hail-mary fallback) is left to validate_kernel, which
-// skips the reads flagged done here.
+// float bits.  The checks and the record are those of adb_vcheck.cuh.  Further poly(A) candidates after a failed first
+// one go to validate_cand_kernel (below); anything else outside this path (float32 sources, codes outside [0, 0x7c00),
+// no precomputed series, the CNN path's hail-mary fallback) is left to validate_kernel, which skips the reads flagged
+// done here.
 #pragma once
 #include <cuda_fp16.h>
 
@@ -24,6 +25,7 @@
 #include "adb_gsample.cuh"
 #include "adb_validate.cuh"
 #include "adb_series_median.cuh"
+#include "adb_vcheck.cuh"
 
 #define VF_THREADS 256
 #define VF_MAX_TASKS 12
@@ -71,6 +73,8 @@ struct VfScratch {  // shared memory
     float ftmp[8];
     double dtmp[8];
     uint32_t utmp[8];
+    VcStats st;    // what the counting passes hand over to the checks (adb_vcheck.cuh)
+    VcOut out;     // their outcome (validate_fast_kernel: thread 0 runs the checks)
 };
 
 struct VfRead {      // per-read constants (registers)
@@ -509,8 +513,7 @@ __device__ __forceinline__ void vf_mean_pair(const VfRead &R, VfScratch &S, int 
 }
 
 // exact integer sums of the codes of up to three segments [sa[i], sb[i]) (clipped; skipped unless on[i]) -> mean /
-// population std of the pA values in float64 (signal_partitions.py:91-92; numpy sums float32 pairwise -- the
-// contract for these statistics is 1e-5 relative).  CTA-wide.
+// population std of the pA values (vc_mean_std).  CTA-wide.
 __device__ void vf_mean_std3(const VfRead &R, VfScratch &S, const int sa[3], const int sb[3], const bool on[3],
                              double mean_out[3], double std_out[3]) {
     const int tid = threadIdx.x;
@@ -562,11 +565,7 @@ __device__ void vf_mean_std3(const VfRead &R, VfScratch &S, const int sa[3], con
     for (int sgm = 0; sgm < 3; sgm++) {
         const int n = na[sgm];
         if (n <= 0) { mean_out[sgm] = CUDART_NAN; std_out[sgm] = CUDART_NAN; continue; }
-        const double mk = (double)S.ltmp[2 * sgm] / n;
-        double vk = (double)S.ltmp[2 * sgm + 1] / n - mk * mk;
-        if (vk < 0) vk = 0;
-        mean_out[sgm] = (double)(float)((mk + (double)R.coff) * (double)R.cscale);
-        std_out[sgm] = (double)(float)(sqrt(vk) * fabs((double)R.cscale));
+        vc_mean_std(S.ltmp[2 * sgm], S.ltmp[2 * sgm + 1], n, R.coff, R.cscale, mean_out[sgm], std_out[sgm]);
     }
     __syncthreads();
 }
@@ -706,25 +705,6 @@ __device__ void vf_series_medians(VfScratch &S, const float *g0, int n0, const f
 }
 
 // ---- the kernel ----------------------------------------------------------------------------------------------------
-struct VfastArgs {
-    BatchDev B;
-    const int *given;           // [n_reads][given_stride] = adapter_end, polya_end(= topk[0]), topk[1..]
-    int given_stride;
-    int given_ntopk;            // entries per read when ntopk_per_read == nullptr (-1: None)
-    const int *ntopk_per_read;
-    int mode;                   // ADB_METHOD_*
-    int win_bytes;              // capacity of the staged window (bytes)
-    adb_record *out;
-    const int *batch_status;
-    const float *pre_var, *pre_mean;  // compact pools of precomputed moving statistics (mvs_series_kernel)
-    const long long *pre_off;
-    const int *pre_meta;
-    const float *series_med;    // [n_reads][2] medians of the two series of the row (series_median_kernel)
-    unsigned char *done;        // [n_reads], zeroed before the launch; 1 = record written by this kernel,
-                                // 2 = record written with the FIRST poly(A) candidate's outcome, further candidates pending
-    int cand_followup;          // 1: validate_cand_kernel runs behind this kernel (CNN path with several candidates)
-};
-
 __host__ __device__ inline size_t vfast_smem_bytes(int win_bytes) {
     return (((size_t)win_bytes + 48 + 15) & ~(size_t)15);  // dynamic part: the window; the scratch is static
 }
@@ -755,15 +735,16 @@ __device__ __forceinline__ void vf_rank_pair(const VfRead &R, VfScratch &S, int 
     if (two && !(c > k + 1)) v1 = vf_neighbour(R, S, a, b, v0, true);
 }
 
-// numpy median of the range of a finished rank task with k = (n - 1) / 2
-__device__ float vf_median_of(const VfRead &R, VfScratch &S, int q) {
-    if (q < 0) return CUDART_NAN_F;
-    const int n = S.task[q].b - S.task[q].a;
-    int v0, v1;
-    vf_rank_pair(R, S, q, (n & 1) == 0, v0, v1);
-    const float x0 = vf_pa(R, v0);
-    if (n & 1) return x0;
-    return __fdiv_rn(__fadd_rn(x0, vf_pa(R, v1)), 2.0f);
+// hand the order statistics of range q (finished rank task t; -1: empty range) over to the checks.  CTA-wide (uniform).
+__device__ void vf_put_ranks(const VfRead &R, VfScratch &S, int q, int t) {
+    int n = 0, v0 = 0, v1 = 0;
+    if (t >= 0) {
+        bool two;
+        n = S.task[t].b - S.task[t].a;
+        vc_rank(q, n, two);
+        vf_rank_pair(R, S, t, two, v0, v1);
+    }
+    if (threadIdx.x == 0) { S.st.n[q] = n; S.st.c0[q] = v0; S.st.c1[q] = v1; }
 }
 
 struct VfDevOut { float mad; };
@@ -832,37 +813,15 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_fast_kernel(VfastArgs 
     uint32_t phase = 0;
 
     for (int r = blockIdx.x; r < A.B.n_reads; r += gridDim.x) {
-        const int mb = r / A.B.batch_size;
         adb_record *rec = A.out + r;
         // generic-proxy accesses to the window memory of the previous read are ordered before the next bulk copy
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncthreads();
-        if (A.batch_status[mb] != ADB_OK) {  // minibatch lost (host raises): zero record
-            for (int w = tid; w < (int)(sizeof(adb_record) / 4); w += blockDim.x) ((uint32_t *)rec)[w] = 0;
-            if (tid == 0) A.done[r] = 1;
-            continue;
-        }
-        const ReadSrc gsrc = make_src(A.B, r);
-        if (!(gsrc.i16 != nullptr && gsrc.cscale > 0.0f && isfinite(gsrc.cscale) && isfinite(gsrc.coff))) continue;
-        const int full_len = A.B.full_lens[r];
-        const int size = gsrc.n;
-        const int *g = A.given + (size_t)r * A.given_stride;
-        const int a_end = g[0], pe_best = g[1];
-        const int n_topk = A.ntopk_per_read ? A.ntopk_per_read[r] : A.given_ntopk;
-        const int pe0 = (n_topk >= 1) ? g[1] : 0;
-        const int topk1 = (n_topk >= 2) ? g[2] : 0;
-        const int msw = cfg.median_shift_window;
-        const bool haveA = (a_end != 0);
-        const bool mvs_geom = cfg.mvs_detect_check && !(pe0 == 0 || a_end == 0 || pe0 < a_end || pe0 - a_end <= 2) &&
-                              !(size < a_end + msw);
-        const bool win_var = !(pe0 - a_end <= cfg.pA_var_window + 2), win_mean = !(pe0 - a_end <= cfg.pA_mean_window + 2);
-        float smed_var = 0.f, smed_mean = 0.f;  // medians of the two moving-statistics series (series_median_kernel)
-        if (mvs_geom && (win_var || win_mean)) {
-            const long long po = A.pre_off ? A.pre_off[r] : -1;
-            if (!(po >= 0 && A.pre_meta[2 * r] == a_end && A.pre_meta[2 * r + 1] == pe0)) continue;  // not precomputed
-            smed_var = A.series_med[2 * r];
-            smed_mean = A.series_med[2 * r + 1];
-        }
+        ReadSrc gsrc;
+        if (!vc_read_start(A, r, gsrc)) continue;
+        VcIn I;
+        if (!vc_inputs(A, cfg, r, gsrc, I)) continue;
+        const int size = I.size, a_end = I.a_end;
         // ---- stage the preload window in shared memory (TMA bulk copy) ----
         VfRead R;
         {
@@ -874,255 +833,82 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_fast_kernel(VfastArgs 
         if (size <= 0) continue;
         vf_minmax(R, S, R.kmin, R.kmax);
         if (R.kmin < 0 || R.kmax >= VF_KEY_LIMIT) continue;  // codes must read as non-negative finite halves
-        for (int w = tid; w < (int)(sizeof(adb_record) / 4); w += blockDim.x) ((uint32_t *)rec)[w] = 0;
+        vc_zero_record(rec);
 
         // ---- speculative inputs of the checks (SURVEY A.8), all from the staged window ----
         int n_open = 0, op_last = 0;
-        if (haveA && cfg.detect_open_pores) {
+        if (a_end != 0 && cfg.detect_open_pores) {
             int ok = 1;
             const int c200 = gsb_code_at(200.0f, false, R.coff, R.cscale, &ok);
             n_open = vf_open_pores(R, S, 0, a_end, c200, rec, &op_last);
         }
-        const int a_start1 = (n_open > 0) ? op_last : 0;
-        int ra = a_start1, rb = a_end;
-        clip_seg(ra, rb, size);
-        const int rlen = rb - ra;
-        const bool rr_geom = haveA && cfg.real_signal_check && rlen >= 2 * cfg.mean_window;
-        float rm0 = 0.f, rm1 = 0.f;
-        if (rr_geom) vf_mean_pair(R, S, ra, rb - cfg.mean_window, cfg.mean_window, rm0, rm1);
-        const int lrw = min(cfg.max_obs_local_range, rlen);
-        // np.percentile positions of the two local ranges
-        const int nLR = lrw;
-        const double vLR85 = __dmul_rn((double)(nLR - 1), 0.85), vLR15 = __dmul_rn((double)(nLR - 1), 0.15);
-        int pa_ = a_end, pb_ = pe0;
-        clip_seg(pa_, pb_, size);
-        const int nP = pb_ - pa_;
-        const double vP85 = __dmul_rn((double)(nP - 1), 0.85), vP15 = __dmul_rn((double)(nP - 1), 0.15);
+        const VcGeom G = vc_geometry(cfg, I, n_open, op_last);
+        if (G.rr_geom) {
+            float rm0, rm1;
+            vf_mean_pair(R, S, G.ra, G.ra + G.rlen - cfg.mean_window, cfg.mean_window, rm0, rm1);
+            if (tid == 0) { S.st.rm0 = rm0; S.st.rm1 = rm1; }
+        }
 
         // ---- round A: every rank ----
         int nt = 0, rot = 0;
         __syncthreads();
-        const int tA0 = haveA ? vf_add_rank(S, R, nt, rot, 0, a_end, 0) : -1;
-        const int tA1 = (haveA && a_start1 != 0) ? vf_add_rank(S, R, nt, rot, a_start1, a_end, 0) : -1;
-        const int tL15 = rr_geom ? vf_add_rank(S, R, nt, rot, rb - lrw, rb, (int)floor(vLR15)) : -1;
-        const int tL85 = rr_geom ? vf_add_rank(S, R, nt, rot, rb - lrw, rb, (int)floor(vLR85)) : -1;
-        const bool needP = mvs_geom || (pe_best > a_end);
-        const int tP = needP ? vf_add_rank(S, R, nt, rot, a_end, pe_best, 0) : -1;
-        const int tP15 = (mvs_geom && nP > 0) ? vf_add_rank(S, R, nt, rot, a_end, pe0, (int)floor(vP15)) : -1;
-        const int tP85 = (mvs_geom && nP > 0) ? vf_add_rank(S, R, nt, rot, a_end, pe0, (int)floor(vP85)) : -1;
-        const int tAF = mvs_geom ? vf_add_rank(S, R, nt, rot, a_end, min(a_end + msw, size), 0) : -1;
-        const int tBF = mvs_geom ? vf_add_rank(S, R, nt, rot, max(a_end - msw, 0), a_end, 0) : -1;
-        const int tR = (size > pe_best) ? vf_add_rank(S, R, nt, rot, pe_best, size, 0) : -1;
-        const bool ms_geom = cfg.detect_med_shift && haveA;
-        const int tMA = ms_geom ? vf_add_rank(S, R, nt, rot, a_end, min(a_end + cfg.med_shift_window, full_len), 0) : -1;
-        const int tMB = ms_geom ? vf_add_rank(S, R, nt, rot, max(a_end - cfg.med_shift_window, 0), a_end, 0) : -1;
-        __syncthreads();
-        if (tid < nt) {  // medians: rank (n - 1) / 2 (the percentile tasks carry their own rank)
-            VfTask &t = S.task[tid];
-            if (tid != tL15 && tid != tL85 && tid != tP15 && tid != tP85) t.k = (t.b - t.a - 1) / 2;
+        int tq[VC_NQ];
+#pragma unroll
+        for (int q = 0; q < VC_NQ; q++) {
+            const int n = G.qb[q] - G.qa[q];
+            bool two;
+            tq[q] = (n > 0) ? vf_add_rank(S, R, nt, rot, G.qa[q], G.qb[q], vc_rank(q, n, two)) : -1;
         }
         if (tid == 0) { S.ntask = nt; S.vtotal = rot; }
         vf_task_bounds(R, S);
         vf_run(R, S);
-        const float medA0 = vf_median_of(R, S, tA0), medA1 = vf_median_of(R, S, tA1);
-        const float medP = vf_median_of(R, S, tP), medR = vf_median_of(R, S, tR);
-        const float medAF = vf_median_of(R, S, tAF), medBF = vf_median_of(R, S, tBF);
-        const float medMA = vf_median_of(R, S, tMA), medMB = vf_median_of(R, S, tMB);
-        auto local_range = [&](int q15, int q85, int n, double v15, double v85) -> double {
-            if (q15 < 0 || q85 < 0) return CUDART_NAN;
-            const int l15 = (int)floor(v15), l85 = (int)floor(v85);
-            int a15, b15, a85, b85;
-            vf_rank_pair(R, S, q15, min(l15 + 1, n - 1) != l15, a15, b15);
-            vf_rank_pair(R, S, q85, min(l85 + 1, n - 1) != l85, a85, b85);
-            const double p85 = np_lerp_f32(vf_pa(R, a85), vf_pa(R, b85), __dsub_rn(v85, (double)l85));
-            const double p15 = np_lerp_f32(vf_pa(R, a15), vf_pa(R, b15), __dsub_rn(v15, (double)l15));
-            return __dsub_rn(p85, p15);
-        };
-        const double lrA = local_range(tL15, tL85, nLR, vLR15, vLR85);
-        const double lrP = local_range(tP15, tP85, nP, vP15, vP85);
+#pragma unroll
+        for (int q = 0; q < VC_NQ; q++) vf_put_ranks(R, S, q, tq[q]);
+        __syncthreads();
 
         // ---- round B: every MAD ----
-        int bmin[4] = {0, 0, 0, 0}, bmax[4] = {0, 0, 0, 0};
-        {
-            const int src[4] = {tA0, tA1, tP, tR};
-            for (int q = 0; q < 4; q++) if (src[q] >= 0) { bmin[q] = S.task[src[q]].smin; bmax[q] = S.task[src[q]].smax; }
-        }
+        const int msrc[4] = {VC_A0, VC_A1, VC_P, VC_R};
+        VfTask src[4];  // (the MAD tasks take the places of the rank tasks)
+#pragma unroll
+        for (int m = 0; m < 4; m++) if (tq[msrc[m]] >= 0) src[m] = S.task[tq[msrc[m]]];
+        int dq[4];
         nt = 0; rot = 0;
         __syncthreads();
-        const int dA0 = (tA0 >= 0) ? vf_add_mad(S, R, nt, rot, 0, a_end, medA0, bmin[0], bmax[0]) : -1;
-        const int dA1 = (tA1 >= 0) ? vf_add_mad(S, R, nt, rot, a_start1, a_end, medA1, bmin[1], bmax[1]) : -1;
-        const int dP = (tP >= 0) ? vf_add_mad(S, R, nt, rot, a_end, pe_best, medP, bmin[2], bmax[2]) : -1;
-        const int dR = (tR >= 0) ? vf_add_mad(S, R, nt, rot, pe_best, size, medR, bmin[3], bmax[3]) : -1;
+#pragma unroll
+        for (int m = 0; m < 4; m++) {
+            const VfTask &t = src[m];
+            dq[m] = (tq[msrc[m]] >= 0) ? vf_add_mad(S, R, nt, rot, t.a, t.b, vc_median(S.st, msrc[m], R.coff, R.cscale), t.smin, t.smax) : -1;
+        }
         __syncthreads();
         if (tid == 0) { S.ntask = nt; S.vtotal = rot; }
         vf_run(R, S);
-        const float madA0 = vf_mad_of(R, S, dA0), madA1 = vf_mad_of(R, S, dA1);
-        const float madP = vf_mad_of(R, S, dP), madR = vf_mad_of(R, S, dR);
-
-        // ---- the checks (combined.py:394-580), part 1: everything that decides adapter_start ----
-        int a_start = 0;
-        bool success = true;
-        int fail = ADB_FAIL_NONE, fail_mask = 0;
-        uint32_t valid = ADB_V_FIELDS;
-        double mvs_v[5] = {0, 0, 0, 0, 0}, real_v[3] = {0, 0, 0}, med_shift = 0.0;
-        int n_open_rep = 0;
-        if (a_end == 0) { success = false; fail = ADB_FAIL_NO_ADAPTER; }
-        if (success && (madA0 != 0.0f) && !in_range_d((double)madA0, cfg.adapter_mad_range)) { success = false; fail = ADB_FAIL_ADAPTER_MAD; }
-        if (success && cfg.detect_open_pores) {
-            n_open_rep = n_open;
-            valid |= ADB_V_OPEN_PORES;
-            if (n_open > 0) {
-                a_start = op_last;
-                if (a_end - a_start < cfg.min_obs_adapter) { success = false; fail = ADB_FAIL_OPEN_PORE; }
-            }
+#pragma unroll
+        for (int m = 0; m < 4; m++) {
+            const float mad = vf_mad_of(R, S, dq[m]);
+            if (tid == 0) S.st.mad[m] = mad;
         }
-        // partition sums (signal_partitions.py:65-96) while the window is still staged
+        __syncthreads();
+
+        if (tid == 0) {
+            vc_small_mean_var(I, reinterpret_cast<const int16_t *>(R.W16) + R.s0, S.st);
+            S.out = vc_checks(cfg, I, G, S.st, A.mode, A.cand_followup != 0);
+        }
+        __syncthreads();
+        if (S.out.defer) continue;  // (uniform) validate_kernel redoes this read from scratch
         double pmean[3], pstd[3];
-        {
-            const int sa[3] = {a_start, a_end, pe_best}, sb[3] = {a_end, pe_best, size};
-            const bool on[3] = {a_end > a_start, pe_best > a_end, size > pe_best};
+        if (!S.out.exception) {  // partition sums (signal_partitions.py:65-96) while the window is still staged
+            int sa[3], sb[3];
+            bool on[3];
+            for (int p = 0; p < 3; p++) on[p] = vc_partition(I, S.out, p, sa[p], sb[p]);
             vf_mean_std3(R, S, sa, sb, on, pmean, pstd);
         }
-        if (success && cfg.real_signal_check) {
-            if (rlen < 2 * cfg.mean_window) {
-                success = false; fail = ADB_FAIL_REAL_RANGE;
-            } else {
-                real_v[0] = (double)rm0; real_v[1] = (double)rm1;
-                valid |= ADB_V_REAL_MEANS;
-                if (in_range_d((double)rm0, cfg.mean_start_range) && in_range_d((double)rm1, cfg.mean_end_range)) {
-                    real_v[2] = lrA;
-                    valid |= ADB_V_REAL_RANGE;
-                    if (!in_range_d(lrA, cfg.local_range)) { success = false; fail = ADB_FAIL_REAL_RANGE; }
-                } else {
-                    success = false; fail = ADB_FAIL_REAL_RANGE;
-                }
-            }
-        }
-        bool exception = false, defer = false, need_mvs = false, followup = false;
-        double mlo = cfg.pA_mean_range[0], mhi = cfg.pA_mean_range[1];
-        if (success && cfg.mvs_detect_check) {
-            if (pe_best == 0) {
-                success = false; fail = ADB_FAIL_NO_POLYA;
-            } else {
-                if (cfg.pA_mean_range_empty && !cfg.pA_mean_scale_range_empty) {
-                    mlo = __dmul_rn(cfg.pA_mean_scale_range[0], (double)medA0);
-                    mhi = __dmul_rn(cfg.pA_mean_scale_range[1], (double)medA0);
-                } else if (cfg.pA_mean_range_empty) {
-                    exception = true; fail = ADB_FAIL_EXC_PA_MEAN_RANGE;
-                }
-                if (!exception && n_topk < 0) { exception = true; fail = ADB_FAIL_EXC_TOPK_NONE; }
-                need_mvs = !exception && n_topk >= 1 && pe0 != 0;
-            }
-        }
-        if (need_mvs) {
-            // first candidate (mvs.py:45-158); further candidates after a failure are left to validate_kernel
-            valid |= ADB_V_MVS;
-            bool ok = false;
-            if (mvs_geom) {
-                const int L = nP;
-                __syncthreads();
-                if (!win_var || !win_mean) {
-                    // exact numpy mean / variance of a short segment (one thread, pairwise order)
-                    if (tid == 0) {
-                        const uint16_t *p = R.W16 + R.s0 + pa_;
-                        const float co = R.coff, cs = R.cscale;
-                        const float mean = __fdiv_rn(np_sum_f32([&](int i) { return __fmul_rn(__fadd_rn((float)(int)p[i], co), cs); }, L), (float)L);
-                        S.ftmp[0] = mean;
-                        S.ftmp[1] = __fdiv_rn(np_sum_f32([&](int i) { const float d = __fsub_rn(__fmul_rn(__fadd_rn((float)(int)p[i], co), cs), mean); return __fmul_rn(d, d); }, L), (float)L);
-                    }
-                    __syncthreads();
-                }
-                const float small_mean = S.ftmp[0], small_var = S.ftmp[1];
-                __syncthreads();
-                const float var32 = win_var ? smed_var : small_var;
-                const float mean32 = win_mean ? smed_mean : small_mean;
-                const float shift32 = __fsub_rn(medAF, medBF);
-                mvs_v[0] = (double)mean32; mvs_v[1] = (double)var32; mvs_v[2] = (double)medP; mvs_v[3] = lrP; mvs_v[4] = (double)shift32;
-                const double mr[2] = {mlo, mhi};
-                int mask = 0;
-                if (!in_range_d(mvs_v[0], mr)) mask |= 1;
-                if (!in_range_d(mvs_v[1], cfg.pA_var_range)) mask |= 2;
-                if (!in_range_d(mvs_v[2], cfg.polyA_med_range)) mask |= 4;
-                if (!in_range_d(mvs_v[3], cfg.polyA_local_range)) mask |= 8;
-                if (!in_range_d(mvs_v[4], cfg.median_shift_range)) mask |= 16;
-                ok = (mask == 0);
-                if (!ok) {
-                    success = false;
-                    if (mvs_v[0] == 0.0) { fail = ADB_FAIL_MVS_NOT_ENOUGH; fail_mask = 0; }  // combined.py:492-495 keys on the value
-                    else { fail = ADB_FAIL_MVS_CHECKS; fail_mask = mask; }
-                }
-            } else {
-                success = false; fail = ADB_FAIL_MVS_NOT_ENOUGH; fail_mask = 0;
-            }
-            if (!ok && topk1 != 0) {
-                // the reference goes on to the next candidates (combined.py:464-515): their moving statistics are
-                // prefixes of one more series pass, so validate_cand_kernel finishes the read from this record
-                const bool fits = A.cand_followup != 0;  // (series beyond the window memory are bisected from the pools there)
-                if (fits) followup = true; else defer = true;
-            }
-        }
-        if (!exception && success && cfg.detect_med_shift) {
-            const float sh = __fsub_rn(medMA, medMB);
-            med_shift = (double)sh;
-            valid |= ADB_V_MED_SHIFT;
-            if (!in_range_d(med_shift, cfg.med_shift_range)) { success = false; fail = ADB_FAIL_MED_SHIFT; }
-        }
-        if (A.mode == ADB_METHOD_CNN && cfg.fallback_to_llr_short_reads && !exception && !success && a_end > 0 && pe_best > 0 &&
-            pe_best - a_end > 1000 && full_len < 2 * cfg.max_obs_adapter)
-            defer = true;  // "hail mary" LLR fallback (combined.py:251-301) lives in validate_kernel
-        if (defer) continue;  // (uniform) validate_kernel redoes this read from scratch
-        __syncthreads();
-        if (!(valid & ADB_V_OPEN_PORES) || exception) {
+        if (!(S.out.valid & ADB_V_OPEN_PORES) || S.out.exception) {
             if (tid < ADB_MAX_OPEN_PORES) rec->open_pores[tid] = 0;  // the scan was speculative
         }
-        if (exception) {
-            // combined.py:225-226 / 304-305 / 350-351: DetectResults(success=False, fail_reason=str(e)), all else None
-            if (tid == 0) {
-                rec->success = 0; rec->fail_code = fail; rec->mvs_fail_mask = 0; rec->valid = 0;
-                rec->signal_len = full_len; rec->preloaded = min(full_len, size);
-                A.done[r] = 1;
-            }
-            continue;
-        }
         if (tid == 0) {
-            double st[3][4];
-            for (int p = 0; p < 3; p++) for (int q = 0; q < 4; q++) st[p][q] = 0.0;
-            if (a_end > a_start) {
-                st[0][0] = pmean[0]; st[0][1] = pstd[0];
-                st[0][2] = (double)(a_start == 0 ? medA0 : medA1);
-                st[0][3] = (double)(a_start == 0 ? madA0 : madA1);
-                valid |= ADB_V_ADAPTER_STATS;
-            }
-            if (pe_best > a_end) {
-                st[1][0] = pmean[1]; st[1][1] = pstd[1]; st[1][2] = (double)medP; st[1][3] = (double)madP;
-                valid |= ADB_V_POLYA_STATS;
-            }
-            if (size > pe_best) {
-                st[2][0] = pmean[2]; st[2][1] = pstd[2]; st[2][2] = (double)medR; st[2][3] = (double)madR;
-                valid |= ADB_V_RNA_STATS;
-            }
-            rec->success = success ? 1 : 0;
-            rec->fail_code = fail;
-            rec->mvs_fail_mask = fail_mask;
-            rec->valid = valid | (n_topk >= 0 ? ADB_V_CAND : 0);
-            rec->signal_len = full_len;
-            rec->preloaded = min(full_len, size);
-            rec->adapter_start = a_start;
-            rec->adapter_end = a_end;
-            rec->polya_end = pe_best;
-            rec->primary_adapter_end = a_end;
-            rec->primary_polya_end = pe_best;
-            rec->mvs_adapter_end = 0;
-            rec->n_cand = max(n_topk, 0);
-            for (int t = 0; t < ADB_MAX_CAND; t++) rec->cand[t] = (t < n_topk) ? g[1 + t] : 0;
-            rec->n_open_pores = n_open_rep;
-            for (int p = 0; p < 3; p++) for (int q = 0; q < 4; q++) rec->stats[p][q] = st[p][q];
-            for (int i = 0; i < 5; i++) rec->mvs[i] = mvs_v[i];
-            for (int i = 0; i < 3; i++) rec->real[i] = real_v[i];
-            rec->med_shift = med_shift;
-            if (followup) *reinterpret_cast<float *>(rec->_reserved) = medA0;  // scales the mean range of the later candidates
+            vc_write_spec_record(rec, I, S.st, S.out, pmean, pstd);
             __threadfence();
-            A.done[r] = followup ? 2 : 1;
+            A.done[r] = S.out.followup ? 2 : 1;
         }
     }
 }
@@ -1165,11 +951,8 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_cand_kernel(VfastArgs 
         const bool have_rows = po >= 0 && A.pre_meta[2 * r] == a_end;
         const int row_pe = have_rows ? A.pre_meta[2 * r + 1] : 0;
         const float medA0 = *reinterpret_cast<const float *>(rec->_reserved);
-        double mlo = cfg.pA_mean_range[0], mhi = cfg.pA_mean_range[1];
-        if (cfg.pA_mean_range_empty && !cfg.pA_mean_scale_range_empty) {
-            mlo = __dmul_rn(cfg.pA_mean_scale_range[0], (double)medA0);
-            mhi = __dmul_rn(cfg.pA_mean_scale_range[1], (double)medA0);
-        }
+        double mr[2];
+        vc_pa_mean_bounds(cfg, medA0, mr);  // (empty bounds raised in validate_fast_kernel: no follow-up)
         double last_v[5] = {0, 0, 0, 0, 0};
         int fail = rec->fail_code, fail_mask = rec->mvs_fail_mask;  // the first candidate's, unless a later one failed
         bool bail = false, fail_known = false;
@@ -1196,60 +979,43 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_cand_kernel(VfastArgs 
                 const int nv = win_var ? nP - (cfg.pA_var_window - 1) : 0, nm = win_mean ? nP - (cfg.pA_mean_window - 1) : 0;
                 if ((win_var || win_mean) && !(have_rows && row_pe >= pe)) { bail = true; break; }
                 const bool big = (size_t)(((max(nv, 0) + 3) & ~3) + max(nm, 0)) * 4 > win_cap;  // series beyond the window memory
-                const double vP85 = __dmul_rn((double)(nP - 1), 0.85), vP15 = __dmul_rn((double)(nP - 1), 0.15);
                 int nt = 0, rot = 0;
                 __syncthreads();
-                const int tP = vf_add_rank(S, R, nt, rot, a_end, pe, 0);
-                const int tP15 = (nP > 0) ? vf_add_rank(S, R, nt, rot, a_end, pe, (int)floor(vP15)) : -1;
-                const int tP85 = (nP > 0) ? vf_add_rank(S, R, nt, rot, a_end, pe, (int)floor(vP85)) : -1;
-                const int tAF = vf_add_rank(S, R, nt, rot, a_end, min(a_end + msw, size), 0);
-                const int tBF = vf_add_rank(S, R, nt, rot, max(a_end - msw, 0), a_end, 0);
-                __syncthreads();
-                if (tid < nt && tid != tP15 && tid != tP85) { VfTask &q = S.task[tid]; q.k = (q.b - q.a - 1) / 2; }
+                const int cq[5] = {VC_P, VC_P15, VC_P85, VC_AF, VC_BF};
+                const int ca[5] = {a_end, a_end, a_end, a_end, max(a_end - msw, 0)};
+                const int cb[5] = {pe, pe, pe, min(a_end + msw, size), a_end};
+                int tq[5];
+#pragma unroll
+                for (int c = 0; c < 5; c++) {
+                    int a = ca[c], b = cb[c];
+                    clip_seg(a, b, size);
+                    bool two;
+                    tq[c] = (b > a) ? vf_add_rank(S, R, nt, rot, a, b, vc_rank(cq[c], b - a, two)) : -1;
+                }
                 if (tid == 0) { S.ntask = nt; S.vtotal = rot; }
                 vf_task_bounds(R, S);
                 vf_run(R, S);
-                const float medP = vf_median_of(R, S, tP), medAF = vf_median_of(R, S, tAF), medBF = vf_median_of(R, S, tBF);
-                double lrP = CUDART_NAN;
-                if (tP15 >= 0 && tP85 >= 0) {
-                    const int l15 = (int)floor(vP15), l85 = (int)floor(vP85);
-                    int a15, b15, a85, b85;
-                    vf_rank_pair(R, S, tP15, min(l15 + 1, nP - 1) != l15, a15, b15);
-                    vf_rank_pair(R, S, tP85, min(l85 + 1, nP - 1) != l85, a85, b85);
-                    const double p85 = np_lerp_f32(vf_pa(R, a85), vf_pa(R, b85), __dsub_rn(vP85, (double)l85));
-                    const double p15 = np_lerp_f32(vf_pa(R, a15), vf_pa(R, b15), __dsub_rn(vP15, (double)l15));
-                    lrP = __dsub_rn(p85, p15);
+#pragma unroll
+                for (int c = 0; c < 5; c++) vf_put_ranks(R, S, cq[c], tq[c]);
+                if ((!win_var || !win_mean) && tid == 0) {
+                    const int16_t *p = reinterpret_cast<const int16_t *>(R.W16) + R.s0 + pa_;
+                    auto x = [&](int i) { return gsb_pa(p[i], R.coff, R.cscale); };
+                    S.st.small_mean = np_mean_f32(x, nP);
+                    S.st.small_var = np_var_f32(x, nP, S.st.small_mean);
                 }
-                __syncthreads();
-                if (!win_var || !win_mean) {  // exact numpy mean / variance of a short segment (one thread, pairwise order)
-                    if (tid == 0) {
-                        const uint16_t *p = R.W16 + R.s0 + pa_;
-                        const float co = R.coff, cs = R.cscale;
-                        const float mean = __fdiv_rn(np_sum_f32([&](int i) { return __fmul_rn(__fadd_rn((float)(int)p[i], co), cs); }, nP), (float)nP);
-                        S.ftmp[0] = mean;
-                        S.ftmp[1] = __fdiv_rn(np_sum_f32([&](int i) { const float d = __fsub_rn(__fmul_rn(__fadd_rn((float)(int)p[i], co), cs), mean); return __fmul_rn(d, d); }, nP), (float)nP);
-                    }
-                    __syncthreads();
-                }
-                const float small_mean = S.ftmp[0], small_var = S.ftmp[1];
                 __syncthreads();
                 float smed[2] = {0.f, 0.f};
                 if (big) vf_series_medians<false>(S, A.pre_var + po, max(nv, 0), A.pre_mean + po, max(nm, 0), (uint32_t *)winbuf, smed);
                 else if (nv > 0 || nm > 0) vf_series_medians<true>(S, A.pre_var + po, max(nv, 0), A.pre_mean + po, max(nm, 0), (uint32_t *)winbuf, smed);
-                v[0] = (double)(win_mean ? smed[1] : small_mean);
-                v[1] = (double)(win_var ? smed[0] : small_var);
-                v[2] = (double)medP; v[3] = lrP; v[4] = (double)__fsub_rn(medAF, medBF);
-                const double mr[2] = {mlo, mhi};
-                int mask = 0;
-                if (!in_range_d(v[0], mr)) mask |= 1;
-                if (!in_range_d(v[1], cfg.pA_var_range)) mask |= 2;
-                if (!in_range_d(v[2], cfg.polyA_med_range)) mask |= 4;
-                if (!in_range_d(v[3], cfg.polyA_local_range)) mask |= 8;
-                if (!in_range_d(v[4], cfg.median_shift_range)) mask |= 16;
+                v[0] = (double)(win_mean ? smed[1] : S.st.small_mean);
+                v[1] = (double)(win_var ? smed[0] : S.st.small_var);
+                v[2] = (double)vc_median(S.st, VC_P, R.coff, R.cscale);
+                v[3] = vc_local_range(S.st, VC_P15, VC_P85, R.coff, R.cscale);
+                v[4] = (double)__fsub_rn(vc_median(S.st, VC_AF, R.coff, R.cscale), vc_median(S.st, VC_BF, R.coff, R.cscale));
+                const int mask = vc_mvs_mask(cfg, v, mr);
                 ok = (mask == 0);
                 if (!ok) {
-                    if (v[0] == 0.0) { fail = ADB_FAIL_MVS_NOT_ENOUGH; fail_mask = 0; }
-                    else { fail = ADB_FAIL_MVS_CHECKS; fail_mask = mask; }
+                    vc_mvs_fail(v[0], mask, fail, fail_mask);
                     fail_known = true;
                 }
             } else {  // the early return of mean_var_shift_polyA_check: zeros, "not enough signal"

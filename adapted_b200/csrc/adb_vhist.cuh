@@ -1,6 +1,6 @@
 // validate_boundaries + per-segment statistics for int16 sources from HISTOGRAMS BUILT ON THE TENSOR CORES.
 //
-// Reference: adapted/detect/combined.py:358-631 (control flow and checks as in adb_vfast.cuh / adb_validate.cuh).
+// Reference: adapted/detect/combined.py:358-631 (the checks and the record: adb_vcheck.cuh, shared with adb_vfast.cuh).
 //
 // Every order statistic the reference asks for (medians, MADs, p15 / p85 of up to a dozen sample ranges of a read) is
 // a function of the histogram of the ADC codes of the range.  Shared-memory atomics build such a histogram at 2 cycles
@@ -28,7 +28,7 @@
 //
 // Codes outside [base, base + 1023] (base = the code of 25 pA: the range covers 25 .. 205 pA at a typical calibration)
 // fall into the end bins; a read is handed to validate_kernel (same results) whenever an answer or a decisive probe
-// touches an end bin that holds such codes.  Also handed over: what validate_fast_kernel hands over.
+// touches an end bin that holds such codes.  Also handed over: what validate_fast_kernel hands over (the same checks).
 #pragma once
 #include "adb_cnn_tc.cuh"
 #include "adb_vfast.cuh"
@@ -48,7 +48,6 @@
 #define VH_ARENA (VH_ARENA_TILES > VH_ARENA_CUM ? VH_ARENA_TILES : VH_ARENA_CUM)
 // instruction descriptor: D = f32, A = B = e4m3 (0), K-major, N = 16, M = VH_M
 #define VH_IDESC ((1u << 4) | ((16u >> 3) << 17) | (((unsigned)VH_M >> 4) << 24))
-#define VH_NQ 12
 #define VH_OP_WORDS 512                    // open-pore scan: 16 384 samples of adapter at most
 
 #ifdef ADB_VH_STATS
@@ -102,8 +101,7 @@ struct VhShared {
     int np;
     int n_low, n_high;                 // samples of the read below base / above base + 2047
     int unsettled;                     // an answer or a probe touched an end bin holding such samples
-    int qv0[VH_NQ], qv1[VH_NQ], qn[VH_NQ];  // rank queries: codes at rank k and k + 1, samples of the range
-    float mad[4];
+    VcIn in;                           // the read's inputs, for the checks (kept out of registers through the pass)
     int mfp[4][2];                     // first passing candidate of the right / left side of the four MAD ranges
     uint32_t hitw[VH_OP_WORDS];        // vh_open_pores: bit i = sample i of the aligned window is an open-pore sample
     unsigned long long psum[VH_MAX_PIECES][2];  // per piece: sum of (code - base), sum of (code - base)^2 (exact)
@@ -394,36 +392,15 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
     uint32_t phase = 0;  // parity of this warp's barrier
 
     for (int r = blockIdx.x; r < A.B.n_reads; r += gridDim.x) {
-        const int mb = r / A.B.batch_size;
         adb_record *rec = A.out + r;
         __syncthreads();
-        if (A.batch_status[mb] != ADB_OK) {  // minibatch lost (host raises): zero record
-            for (int w = tid; w < (int)(sizeof(adb_record) / 4); w += blockDim.x) ((uint32_t *)rec)[w] = 0;
-            if (tid == 0) A.done[r] = 1;
-            continue;
-        }
-        const ReadSrc gsrc = make_src(A.B, r);
-        if (!(gsrc.i16 != nullptr && gsrc.cscale > 0.0f && isfinite(gsrc.cscale) && isfinite(gsrc.coff))) continue;
-        const int full_len = A.B.full_lens[r];
-        const int size = gsrc.n;
-        const int *g = A.given + (size_t)r * A.given_stride;
-        const int a_end = g[0], pe_best = g[1];
-        const int n_topk = A.ntopk_per_read ? A.ntopk_per_read[r] : A.given_ntopk;
-        const int pe0 = (n_topk >= 1) ? g[1] : 0;
-        const int topk1 = (n_topk >= 2) ? g[2] : 0;
-        const int msw = cfg.median_shift_window;
-        const bool haveA = (a_end != 0);
-        const bool mvs_geom = cfg.mvs_detect_check && !(pe0 == 0 || a_end == 0 || pe0 < a_end || pe0 - a_end <= 2) &&
-                              !(size < a_end + msw);
-        const bool win_var = !(pe0 - a_end <= cfg.pA_var_window + 2), win_mean = !(pe0 - a_end <= cfg.pA_mean_window + 2);
-        float smed_var = 0.f, smed_mean = 0.f;  // medians of the two moving-statistics series (series_median_kernel)
-        if (mvs_geom && (win_var || win_mean)) {
-            const long long po = A.pre_off ? A.pre_off[r] : -1;
-            if (!(po >= 0 && A.pre_meta[2 * r] == a_end && A.pre_meta[2 * r + 1] == pe0)) continue;  // not precomputed
-            smed_var = A.series_med[2 * r];
-            smed_mean = A.series_med[2 * r + 1];
-        }
+        ReadSrc gsrc;
+        if (!vc_read_start(A, r, gsrc)) continue;
+        VcIn I;
+        if (!vc_inputs(A, cfg, r, gsrc, I)) continue;
+        const int size = I.size, a_end = I.a_end;
         if (size <= 0) continue;
+        if (tid == 0) H.in = I;
         // the window stays in global memory: the helpers take a 16-byte aligned base + the index of sample 0
         VfRead R;
         R.W16 = reinterpret_cast<const uint16_t *>((uintptr_t)gsrc.i16 & ~(uintptr_t)15);
@@ -445,7 +422,7 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
         int cok = 1;
         const int base = gsb_code_at(VH_M == 128 ? -20.0f : 25.0f, false, R.coff, R.cscale, &cok);
         if (!cok) continue;
-        for (int w = tid; w < (int)(sizeof(adb_record) / 4); w += blockDim.x) ((uint32_t *)rec)[w] = 0;
+        vc_zero_record(rec);
 #ifdef ADB_VH_STATS
         long long vh_t0 = clock64();
         if (tid == 0) atomicAdd(&vh_dbg[0], 1ull);
@@ -453,7 +430,7 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
 
         // ---- speculative inputs of the checks (SURVEY A.8) ----
         int n_open = 0, op_last = 0;
-        if (haveA && cfg.detect_open_pores) {
+        if (a_end != 0 && cfg.detect_open_pores) {
             int ok = 1;
             const int c200 = gsb_code_at(200.0f, false, R.coff, R.cscale, &ok);
             int ob = a_end;
@@ -461,41 +438,14 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
             if (ob + 16 > 32 * VH_OP_WORDS) continue;  // (uniform) adapter longer than the scan's bit mask: validate_kernel
             n_open = vh_open_pores(R, H, ob, c200, rec, &op_last);
         }
-        const int a_start1 = (n_open > 0) ? op_last : 0;
-        int ra = a_start1, rb = a_end;
-        clip_seg(ra, rb, size);
-        const int rlen = rb - ra;
-        const bool rr_geom = haveA && cfg.real_signal_check && rlen >= 2 * cfg.mean_window;
-        float rm0 = 0.f, rm1 = 0.f;
-        if (rr_geom) vf_mean_pair_t<int16_t>(W, R.coff, R.cscale, S, ra, rb - cfg.mean_window, cfg.mean_window, rm0, rm1);
-        const int lrw = min(cfg.max_obs_local_range, rlen);
-        const int nLR = lrw;
-        const double vLR85 = __dmul_rn((double)(nLR - 1), 0.85), vLR15 = __dmul_rn((double)(nLR - 1), 0.15);
-        int pa_ = a_end, pb_ = pe0;
-        clip_seg(pa_, pb_, size);
-        const int nP = pb_ - pa_;
-        const double vP85 = __dmul_rn((double)(nP - 1), 0.85), vP15 = __dmul_rn((double)(nP - 1), 0.15);
-        const bool needP = mvs_geom || (pe_best > a_end);
-        const bool ms_geom = cfg.detect_med_shift && haveA;
+        const VcGeom G = vc_geometry(cfg, I, n_open, op_last);
+        if (G.rr_geom) {
+            float rm0, rm1;
+            vf_mean_pair_t<int16_t>(W, R.coff, R.cscale, S, G.ra, G.ra + G.rlen - cfg.mean_window, cfg.mean_window, rm0, rm1);
+            if (tid == 0) { S.st.rm0 = rm0; S.st.rm1 = rm1; }
+        }
 
         VH_T(1);
-        // ---- the sample ranges of the statistics (query q works on [qa[q], qb[q]); empty: not wanted) ----
-        int qa[VH_NQ], qb[VH_NQ];
-#pragma unroll
-        for (int q = 0; q < VH_NQ; q++) { qa[q] = 0; qb[q] = 0; }
-        if (haveA) { qa[0] = 0; qb[0] = a_end; }                                              // adapter from 0
-        if (haveA && a_start1 != 0) { qa[1] = a_start1; qb[1] = a_end; }                      // adapter behind the open pore
-        if (rr_geom) { qa[2] = rb - lrw; qb[2] = rb; qa[3] = rb - lrw; qb[3] = rb; }          // local range: p15, p85
-        if (needP) { qa[4] = a_end; qb[4] = pe_best; }                                        // poly(A)
-        if (mvs_geom && nP > 0) { qa[5] = a_end; qb[5] = pe0; qa[6] = a_end; qb[6] = pe0; }   // its p15, p85
-        if (mvs_geom) { qa[7] = a_end; qb[7] = min(a_end + msw, size); qa[8] = max(a_end - msw, 0); qb[8] = a_end; }
-        if (size > pe_best) { qa[9] = pe_best; qb[9] = size; }                                // the rest
-        if (ms_geom) {
-            qa[10] = a_end; qb[10] = min(a_end + cfg.med_shift_window, full_len);
-            qa[11] = max(a_end - cfg.med_shift_window, 0); qb[11] = a_end;
-        }
-#pragma unroll
-        for (int q = 0; q < VH_NQ; q++) clip_seg(qa[q], qb[q], size);
         __syncthreads();
         if (warp == 0) {
             // cut points = the distinct range ends, sorted: lane l holds one end (lanes 24 / 25: 0 and size), its place is
@@ -503,8 +453,8 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
             int v = (lane == 25) ? size : 0;
             bool on = lane == 24 || lane == 25;
 #pragma unroll
-            for (int q = 0; q < VH_NQ; q++) {
-                if ((lane >> 1) == q) { v = (lane & 1) ? qb[q] : qa[q]; on = qb[q] > qa[q]; }
+            for (int q = 0; q < VC_NQ; q++) {
+                if ((lane >> 1) == q) { v = (lane & 1) ? G.qb[q] : G.qa[q]; on = G.qb[q] > G.qa[q]; }
             }
             const unsigned onm = __ballot_sync(ADB_FULL, on);
             bool first = on;
@@ -658,51 +608,42 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
         // ---- the statistics: rank query q on warp q % 8 (32-way searches), then the four MADs on warps 0..3 ----
         {
             const int n_low = H.n_low, n_high = H.n_high;
-            for (int qq = warp; qq < VH_NQ; qq += VH_WARPS) {
+            for (int qq = warp; qq < VC_NQ; qq += VH_WARPS) {
                 int a = 0, b = 0;
 #pragma unroll
-                for (int q = 0; q < VH_NQ; q++) if (qq == q) { a = qa[q]; b = qb[q]; }
+                for (int q = 0; q < VC_NQ; q++) if (qq == q) { a = G.qa[q]; b = G.qb[q]; }
                 int v0 = 0, v1 = 0;
                 const int n = b - a;
                 if (n > 0) {
                     const VhRange q = vh_range(H, a, b, size);
-                    int k = (n - 1) / 2;
-                    bool two = (n & 1) == 0;
-                    if (qq == 2 || qq == 3 || qq == 5 || qq == 6) {  // np.percentile: floor of the virtual index
-                        const double vv = (qq == 2) ? vLR15 : (qq == 3) ? vLR85 : (qq == 5) ? vP15 : vP85;
-                        k = (int)floor(vv);
-                        two = min(k + 1, n - 1) != k;
-                    }
+                    bool two;
+                    const int k = vc_rank(qq, n, two);
                     const int x0 = vh_wselect(cum, q.p0, q.p1, k);
                     const int x1 = two ? vh_wselect(cum, q.p0, q.p1, k + 1) : x0;
                     if (((x0 <= 0 || x1 <= 0) && n_low > 0) || ((x0 >= VH_BINS - 1 || x1 >= VH_BINS - 1) && n_high > 0)) H.unsettled = 1;
                     v0 = x0 + base;
                     v1 = x1 + base;
                 }
-                if (lane == 0) { H.qv0[qq] = v0; H.qv1[qq] = v1; H.qn[qq] = n; }
+                if (lane == 0) { S.st.c0[qq] = v0; S.st.c1[qq] = v1; S.st.n[qq] = n; }
             }
         }
         __syncthreads();
         // the four MADs (ranges 0, 1, 4, 9): warp w searches the right side of range w & 3 (w < 4) or its left side
         {
             const int t = warp & 3;
-            const int src = (t == 0) ? 0 : (t == 1) ? 1 : (t == 2) ? 4 : 9;
+            const int src = (t == 0) ? VC_A0 : (t == 1) ? VC_A1 : (t == 2) ? VC_P : VC_R;
             int a = 0, b = 0;
 #pragma unroll
-            for (int q = 0; q < VH_NQ; q++) if (src == q) { a = qa[q]; b = qb[q]; }
+            for (int q = 0; q < VC_NQ; q++) if (src == q) { a = G.qa[q]; b = G.qb[q]; }
             const int n = b - a;
-            float med = CUDART_NAN_F;
-            if (n > 0) {
-                const float x0 = vf_pa(R, H.qv0[src]);
-                med = (n & 1) ? x0 : __fdiv_rn(__fadd_rn(x0, vf_pa(R, H.qv1[src])), 2.0f);
-            }
+            const float med = vc_median(S.st, src, R.coff, R.cscale);
             const bool live = n > 0 && med == med;
             const VhMad M(R, H, cum, vh_range(H, a, b, size), base, max(n, 1), live ? med : 0.0f);
             if (live) { const int f = M.first_pass(warp < 4); if (lane == 0) H.mfp[t][warp >> 2] = f; }
             __syncthreads();
             if (warp < 4) {
                 const float mad = live ? M.finish(H.mfp[t][0], H.mfp[t][1]) : CUDART_NAN_F;
-                if (lane == 0) H.mad[t] = mad;
+                if (lane == 0) S.st.mad[t] = mad;
             }
         }
         __syncthreads();
@@ -714,213 +655,44 @@ __global__ void __launch_bounds__(VF_THREADS, 4) validate_hist_kernel(VfastArgs 
         VH_T(6);
         if (unsettled) continue;  // (uniform) codes outside the histogram range matter: validate_kernel
 
-        // ---- the checks (combined.py:394-580), as in validate_fast_kernel, on warp 0 only ----
+        // ---- the checks (adb_vcheck.cuh) on warp 0 only ----
         // (scalar work, much of it float64: run redundantly on all eight warps it takes issue slots and instruction
         // fetch from the other CTAs of the SM -- measured 14.0 -> 13.3 ms per 100k RNA002 reads; the other warps wait at
         // the top of the loop)
-        if (warp == 0) do {
-            auto median_of = [&](int q) -> float {
-                const int n = H.qn[q];
-                if (n <= 0) return CUDART_NAN_F;
-                const float x0 = vf_pa(R, H.qv0[q]);
-                if (n & 1) return x0;
-                return __fdiv_rn(__fadd_rn(x0, vf_pa(R, H.qv1[q])), 2.0f);
-            };
-            const float medA0 = median_of(0), medA1 = median_of(1), medP = median_of(4), medR = median_of(9);
-            const float medAF = median_of(7), medBF = median_of(8), medMA = median_of(10), medMB = median_of(11);
-            auto local_range = [&](int q15, int q85, double v15, double v85) -> double {
-                if (H.qn[q15] <= 0 || H.qn[q85] <= 0) return CUDART_NAN;
-                const int l15 = (int)floor(v15), l85 = (int)floor(v85);
-                const double p85 = np_lerp_f32(vf_pa(R, H.qv0[q85]), vf_pa(R, H.qv1[q85]), __dsub_rn(v85, (double)l85));
-                const double p15 = np_lerp_f32(vf_pa(R, H.qv0[q15]), vf_pa(R, H.qv1[q15]), __dsub_rn(v15, (double)l15));
-                return __dsub_rn(p85, p15);
-            };
-            const double lrA = local_range(2, 3, vLR15, vLR85);
-            const double lrP = local_range(5, 6, vP15, vP85);
-            const float madA0 = H.mad[0], madA1 = H.mad[1], madP = H.mad[2], madR = H.mad[3];
-            int a_start = 0;
-            bool success = true;
-            int fail = ADB_FAIL_NONE, fail_mask = 0;
-            uint32_t valid = ADB_V_FIELDS;
-            double mvs_v[5] = {0, 0, 0, 0, 0}, real_v[3] = {0, 0, 0}, med_shift = 0.0;
-            int n_open_rep = 0;
-            if (a_end == 0) { success = false; fail = ADB_FAIL_NO_ADAPTER; }
-            if (success && (madA0 != 0.0f) && !in_range_d((double)madA0, cfg.adapter_mad_range)) { success = false; fail = ADB_FAIL_ADAPTER_MAD; }
-            if (success && cfg.detect_open_pores) {
-                n_open_rep = n_open;
-                valid |= ADB_V_OPEN_PORES;
-                if (n_open > 0) {
-                    a_start = op_last;
-                    if (a_end - a_start < cfg.min_obs_adapter) { success = false; fail = ADB_FAIL_OPEN_PORE; }
-                }
-            }
-            // partition mean / std (signal_partitions.py:91-92) from the exact per-piece sums of the pass above: the same
-            // integers and the same float64 formulas as vf_mean_std3
-            double pmean[3], pstd[3];
-            {
-                const int sa[3] = {a_start, a_end, pe_best}, sb[3] = {a_end, pe_best, size};
-                const bool on[3] = {a_end > a_start, pe_best > a_end, size > pe_best};
-                // (three lanes, one partition each)
+        if (warp == 0) {
+            if (lane == 0) vc_small_mean_var(H.in, W, S.st);
+            __syncwarp();
+            const VcOut o = vc_checks(cfg, H.in, G, S.st, A.mode, A.cand_followup != 0);
+            if (!o.defer) {  // (else validate_kernel redoes this read from scratch)
+                // partition mean / std (S.dtmp[0..2] / [3..5]) from the exact per-piece sums of the pass above (three
+                // lanes, one partition each)
                 __syncwarp();
-                if (tid < 3) {
-                    const int sgm = tid;
-                    int a = sa[sgm], b = sb[sgm];
-                    clip_seg(a, b, size);
-                    const int n = on[sgm] ? b - a : 0;
+                if (lane < 3) {
+                    int a, b;
                     double pm = CUDART_NAN, ps = CUDART_NAN;
+                    vc_partition(H.in, o, lane, a, b);
+                    clip_seg(a, b, size);
+                    const int n = b - a;
                     if (n > 0) {
                         const VhRange q = vh_range(H, a, b, size);
                         long long d1 = 0, d2 = 0;
                         for (int p = q.p0; p < q.p1; p++) { d1 += (long long)H.psum[p][0]; d2 += (long long)H.psum[p][1]; }
                         const long long s1 = d1 + (long long)n * base;                                   // sum of the codes
                         const long long s2 = d2 + 2ll * base * d1 + (long long)n * base * (long long)base;  // sum of their squares
-                        const double mk = (double)s1 / n;
-                        double vk = (double)s2 / n - mk * mk;
-                        if (vk < 0) vk = 0;
-                        pm = (double)(float)((mk + (double)R.coff) * (double)R.cscale);
-                        ps = (double)(float)(sqrt(vk) * fabs((double)R.cscale));
+                        vc_mean_std(s1, s2, n, R.coff, R.cscale, pm, ps);
                     }
-                    S.dtmp[sgm] = pm; S.dtmp[3 + sgm] = ps;
+                    S.dtmp[lane] = pm; S.dtmp[3 + lane] = ps;
                 }
                 __syncwarp();
-                for (int sgm = 0; sgm < 3; sgm++) { pmean[sgm] = S.dtmp[sgm]; pstd[sgm] = S.dtmp[3 + sgm]; }
-            }
-            if (success && cfg.real_signal_check) {
-                if (rlen < 2 * cfg.mean_window) {
-                    success = false; fail = ADB_FAIL_REAL_RANGE;
-                } else {
-                    real_v[0] = (double)rm0; real_v[1] = (double)rm1;
-                    valid |= ADB_V_REAL_MEANS;
-                    if (in_range_d((double)rm0, cfg.mean_start_range) && in_range_d((double)rm1, cfg.mean_end_range)) {
-                        real_v[2] = lrA;
-                        valid |= ADB_V_REAL_RANGE;
-                        if (!in_range_d(lrA, cfg.local_range)) { success = false; fail = ADB_FAIL_REAL_RANGE; }
-                    } else {
-                        success = false; fail = ADB_FAIL_REAL_RANGE;
-                    }
+                if (!(o.valid & ADB_V_OPEN_PORES) || o.exception) {
+                    for (int i = lane; i < ADB_MAX_OPEN_PORES; i += 32) rec->open_pores[i] = 0;  // the scan was speculative
                 }
-            }
-            bool exception = false, defer = false, need_mvs = false, followup = false;
-            double mlo = cfg.pA_mean_range[0], mhi = cfg.pA_mean_range[1];
-            if (success && cfg.mvs_detect_check) {
-                if (pe_best == 0) {
-                    success = false; fail = ADB_FAIL_NO_POLYA;
-                } else {
-                    if (cfg.pA_mean_range_empty && !cfg.pA_mean_scale_range_empty) {
-                        mlo = __dmul_rn(cfg.pA_mean_scale_range[0], (double)medA0);
-                        mhi = __dmul_rn(cfg.pA_mean_scale_range[1], (double)medA0);
-                    } else if (cfg.pA_mean_range_empty) {
-                        exception = true; fail = ADB_FAIL_EXC_PA_MEAN_RANGE;
-                    }
-                    if (!exception && n_topk < 0) { exception = true; fail = ADB_FAIL_EXC_TOPK_NONE; }
-                    need_mvs = !exception && n_topk >= 1 && pe0 != 0;
-                }
-            }
-            if (need_mvs) {
-                valid |= ADB_V_MVS;
-                bool ok = false;
-                if (mvs_geom) {
-                    const int L = nP;
-                    __syncwarp();
-                    if (!win_var || !win_mean) {
-                        // exact numpy mean / variance of a short segment (one thread, pairwise order)
-                        if (tid == 0) {
-                            const int16_t *p = W + pa_;
-                            const float co = R.coff, cs = R.cscale;
-                            const float mean = __fdiv_rn(np_sum_f32([&](int i) { return __fmul_rn(__fadd_rn((float)(int)p[i], co), cs); }, L), (float)L);
-                            S.ftmp[0] = mean;
-                            S.ftmp[1] = __fdiv_rn(np_sum_f32([&](int i) { const float d = __fsub_rn(__fmul_rn(__fadd_rn((float)(int)p[i], co), cs), mean); return __fmul_rn(d, d); }, L), (float)L);
-                        }
-                        __syncwarp();
-                    }
-                    const float small_mean = S.ftmp[0], small_var = S.ftmp[1];
-                    __syncwarp();
-                    const float var32 = win_var ? smed_var : small_var;
-                    const float mean32 = win_mean ? smed_mean : small_mean;
-                    const float shift32 = __fsub_rn(medAF, medBF);
-                    mvs_v[0] = (double)mean32; mvs_v[1] = (double)var32; mvs_v[2] = (double)medP; mvs_v[3] = lrP; mvs_v[4] = (double)shift32;
-                    const double mr[2] = {mlo, mhi};
-                    int mask = 0;
-                    if (!in_range_d(mvs_v[0], mr)) mask |= 1;
-                    if (!in_range_d(mvs_v[1], cfg.pA_var_range)) mask |= 2;
-                    if (!in_range_d(mvs_v[2], cfg.polyA_med_range)) mask |= 4;
-                    if (!in_range_d(mvs_v[3], cfg.polyA_local_range)) mask |= 8;
-                    if (!in_range_d(mvs_v[4], cfg.median_shift_range)) mask |= 16;
-                    ok = (mask == 0);
-                    if (!ok) {
-                        success = false;
-                        if (mvs_v[0] == 0.0) { fail = ADB_FAIL_MVS_NOT_ENOUGH; fail_mask = 0; }  // combined.py:492-495 keys on the value
-                        else { fail = ADB_FAIL_MVS_CHECKS; fail_mask = mask; }
-                    }
-                } else {
-                    success = false; fail = ADB_FAIL_MVS_NOT_ENOUGH; fail_mask = 0;
-                }
-                if (!ok && topk1 != 0) {
-                    if (A.cand_followup != 0) followup = true; else defer = true;
-                }
-            }
-            if (!exception && success && cfg.detect_med_shift) {
-                const float sh = __fsub_rn(medMA, medMB);
-                med_shift = (double)sh;
-                valid |= ADB_V_MED_SHIFT;
-                if (!in_range_d(med_shift, cfg.med_shift_range)) { success = false; fail = ADB_FAIL_MED_SHIFT; }
-            }
-            if (A.mode == ADB_METHOD_CNN && cfg.fallback_to_llr_short_reads && !exception && !success && a_end > 0 && pe_best > 0 &&
-                pe_best - a_end > 1000 && full_len < 2 * cfg.max_obs_adapter)
-                defer = true;  // "hail mary" LLR fallback (combined.py:251-301) lives in validate_kernel
-            if (defer) break;       // (uniform) validate_kernel redoes this read from scratch
-            __syncwarp();
-            if (!(valid & ADB_V_OPEN_PORES) || exception) {
-                for (int i = lane; i < ADB_MAX_OPEN_PORES; i += 32) rec->open_pores[i] = 0;  // the scan was speculative
-            }
-            if (exception) {
                 if (tid == 0) {
-                    rec->success = 0; rec->fail_code = fail; rec->mvs_fail_mask = 0; rec->valid = 0;
-                    rec->signal_len = full_len; rec->preloaded = min(full_len, size);
-                    A.done[r] = 1;
+                    vc_write_spec_record(rec, H.in, S.st, o, S.dtmp, S.dtmp + 3);
+                    A.done[r] = o.followup ? 2 : 1;  // (read by the kernels launched behind this one: no fence needed)
                 }
-                break;
             }
-            if (tid == 0) {
-                double st[3][4];
-                for (int p = 0; p < 3; p++) for (int q = 0; q < 4; q++) st[p][q] = 0.0;
-                if (a_end > a_start) {
-                    st[0][0] = pmean[0]; st[0][1] = pstd[0];
-                    st[0][2] = (double)(a_start == 0 ? medA0 : medA1);
-                    st[0][3] = (double)(a_start == 0 ? madA0 : madA1);
-                    valid |= ADB_V_ADAPTER_STATS;
-                }
-                if (pe_best > a_end) {
-                    st[1][0] = pmean[1]; st[1][1] = pstd[1]; st[1][2] = (double)medP; st[1][3] = (double)madP;
-                    valid |= ADB_V_POLYA_STATS;
-                }
-                if (size > pe_best) {
-                    st[2][0] = pmean[2]; st[2][1] = pstd[2]; st[2][2] = (double)medR; st[2][3] = (double)madR;
-                    valid |= ADB_V_RNA_STATS;
-                }
-                rec->success = success ? 1 : 0;
-                rec->fail_code = fail;
-                rec->mvs_fail_mask = fail_mask;
-                rec->valid = valid | (n_topk >= 0 ? ADB_V_CAND : 0);
-                rec->signal_len = full_len;
-                rec->preloaded = min(full_len, size);
-                rec->adapter_start = a_start;
-                rec->adapter_end = a_end;
-                rec->polya_end = pe_best;
-                rec->primary_adapter_end = a_end;
-                rec->primary_polya_end = pe_best;
-                rec->mvs_adapter_end = 0;
-                rec->n_cand = max(n_topk, 0);
-                for (int t = 0; t < ADB_MAX_CAND; t++) rec->cand[t] = (t < n_topk) ? g[1 + t] : 0;
-                rec->n_open_pores = n_open_rep;
-                for (int p = 0; p < 3; p++) for (int q = 0; q < 4; q++) rec->stats[p][q] = st[p][q];
-                for (int i = 0; i < 5; i++) rec->mvs[i] = mvs_v[i];
-                for (int i = 0; i < 3; i++) rec->real[i] = real_v[i];
-                rec->med_shift = med_shift;
-                if (followup) *reinterpret_cast<float *>(rec->_reserved) = medA0;  // scales the mean range of the later candidates
-                A.done[r] = followup ? 2 : 1;  // (read by the kernels launched behind this one: no fence needed)
-            }
-        } while (0);
+        }
         VH_T(7);
     }
     __syncthreads();

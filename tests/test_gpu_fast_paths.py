@@ -37,9 +37,16 @@ def _oracle_llr(b, spc, mbs):
     return out
 
 
-@pytest.mark.parametrize("seed,kw", [(601, {}), (602, {"stress": True}), (603, {"short_frac": 0.3})])
-def test_llr_fast_and_general_validate_agree_with_oracle(seed, kw):
+@pytest.mark.parametrize("seed,kw,cfg", [(601, {}, {}), (602, {"stress": True}, {}), (603, {"short_frac": 0.3}, {}),
+                                         # the MVS check and the median-shift check together: validate_fast_kernel is the
+                                         # production path (validate_hist_kernel has too few accumulators for their ranges)
+                                         (604, {}, {"med_shift": {"detect_med_shift": True}})],
+                         ids=["601-kw0", "602-kw1", "603-kw2", "604-med_shift"])
+def test_llr_fast_and_general_validate_agree_with_oracle(seed, kw, cfg):
     spc = get_chemistry_specific_config("rna002")
+    for group, fields in cfg.items():
+        for k, v in fields.items():
+            setattr(getattr(spc, group), k, v)
     b = make_reads(200, "rna002", spc.sig_preload_size, seed=seed, **kw)
     if kw.get("short_frac"):
         # keep the minibatch alive: the reference loses it on an empty downscaled row (SURVEY A.11)
