@@ -15,4 +15,8 @@ def __getattr__(name):
         from . import detect
 
         return getattr(detect, name)
+    if name == "StreamSession":
+        from .stream import StreamSession
+
+        return StreamSession
     raise AttributeError(name)

@@ -154,6 +154,12 @@ def load() -> C.CDLL:
     L.adb_cnn_scores_host.argtypes = [vp, vp, C.c_int32, C.c_int32, vp, vp]
     L.adb_mvs_stream_detect_host.argtypes = [vp, C.POINTER(AdbBatch), C.POINTER(AdbStreamConfig), vp]
     L.adb_mvs_stream_detect_host.restype = ip
+    L.adb_stream_session_create.argtypes = [vp, C.POINTER(AdbStreamConfig), C.c_int32, C.c_int32, C.POINTER(vp)]
+    L.adb_stream_session_create.restype = ip
+    L.adb_stream_session_destroy.argtypes = [vp]
+    L.adb_stream_session_destroy.restype = None
+    L.adb_stream_session_push.argtypes = [vp, C.c_int32, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.adb_stream_session_push.restype = ip
     L.adb_format_csv.argtypes = [vp, vp, C.c_int32, vp, C.c_int32, C.c_char_p, C.c_int32, vp, C.c_int64]
     L.adb_format_csv.restype = C.c_int64
     L.adb_format_csv_ex.argtypes = [vp, vp, C.c_int32, vp, C.c_int32, C.c_char_p, C.c_int32, vp, vp, vp, vp, C.c_int64]

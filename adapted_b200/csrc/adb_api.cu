@@ -7,6 +7,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -20,6 +21,7 @@
 #include "adb_read_kernel.cuh"
 #include "adb_cnn.cuh"
 #include "adb_stream.cuh"
+#include "adb_stream_session.cuh"
 #include "adb_cnn_tc.cuh"
 #include "adb_vhist.cuh"
 #include "adb_start_peak.cuh"
@@ -830,17 +832,23 @@ extern "C" int adb_global_med_mad_host(adb_ctx *ctx, const adb_batch *batch, int
 }
 
 // ---- streaming poly(A) detector (row f4) ----------------------------------------------------------------------------
-extern "C" int adb_mvs_stream_detect_host(adb_ctx *ctx, const adb_batch *batch, const adb_stream_config *cfg,
-                                          int32_t *polya_start) {
-    if (!ctx || !cfg || !polya_start) { set_err("null argument"); return ADB_ERR_ARG; }
-    int rc = check_batch(batch);
-    if (rc) return rc;
+static int check_stream_config(const adb_stream_config *cfg) {
     if (cfg->pA_mean_window < 1 || cfg->pA_var_window < 1 || cfg->pA_mean_window > ADB_MAX_MOVE_WINDOW ||
         cfg->pA_var_window > ADB_MAX_MOVE_WINDOW || cfg->min_obs_adapter < 0 || cfg->search_increment_step < 1 ||
         cfg->polyA_window < 1 || cfg->median_shift_window < 1) {
         set_err("streaming config outside the supported range");
         return ADB_ERR_UNSUPPORTED;
     }
+    return ADB_OK;
+}
+
+extern "C" int adb_mvs_stream_detect_host(adb_ctx *ctx, const adb_batch *batch, const adb_stream_config *cfg,
+                                          int32_t *polya_start) {
+    if (!ctx || !cfg || !polya_start) { set_err("null argument"); return ADB_ERR_ARG; }
+    int rc = check_batch(batch);
+    if (rc) return rc;
+    rc = check_stream_config(cfg);
+    if (rc) return rc;
     CUDA_TRY(cudaSetDevice(ctx->device));
     if (batch->n_reads == 0) return ADB_OK;
     cudaStream_t st = ctx->stream;
@@ -866,6 +874,172 @@ extern "C" int adb_mvs_stream_detect_host(adb_ctx *ctx, const adb_batch *batch, 
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(polya_start, A.out, sizeof(int32_t) * (size_t)A.B.n_reads, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
+    return ADB_OK;
+}
+
+// ---- read-until sessions of the streaming detector (adb_stream_session.cuh) ---------------------------------------
+struct adb_stream_session {
+    adb_ctx *ctx = nullptr;
+    adb_stream_config cfg;
+    int n_slots = 0, max_samples = 0, mask_words = 0;
+    DevBuf slots, cache, mask, stage;  // stage: one push's entries, chunks and answers
+    void *pin = nullptr;               // pinned mirror of `stage`
+    size_t pin_cap = 0;
+    // host mirror per slot: samples cached, a read was started, last answer, settled; stamp: duplicate check of a push
+    std::vector<int32_t> n, result, stamp;
+    std::vector<uint8_t> live, settled;
+    int32_t push_id = 0;
+};
+
+extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
+                                         int32_t max_samples, adb_stream_session **out) {
+    if (!ctx || !cfg || !out) { set_err("null argument"); return ADB_ERR_ARG; }
+    *out = nullptr;
+    if (n_slots < 1 || max_samples < 1) { set_err("n_slots and max_samples must be positive"); return ADB_ERR_ARG; }
+    int rc = check_stream_config(cfg);
+    if (rc) return rc;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    adb_stream_session *s = new adb_stream_session();
+    s->ctx = ctx;
+    s->cfg = *cfg;
+    s->n_slots = n_slots;
+    s->max_samples = max_samples;
+    s->mask_words = (max_samples + 31) / 32;
+    s->n.assign(n_slots, 0);
+    s->result.assign(n_slots, 0);
+    s->stamp.assign(n_slots, 0);
+    s->live.assign(n_slots, 0);
+    s->settled.assign(n_slots, 0);
+    if (s->slots.ensure(sizeof(SessSlot) * (size_t)n_slots) || s->cache.ensure(sizeof(int16_t) * (size_t)n_slots * max_samples) ||
+        s->mask.ensure(sizeof(uint32_t) * (size_t)n_slots * s->mask_words)) {
+        adb_stream_session_destroy(s);
+        set_err("cudaMalloc stream session arena");
+        return ADB_ERR_CUDA;
+    }
+    if (cudaMemsetAsync(s->slots.p, 0, sizeof(SessSlot) * (size_t)n_slots, ctx->stream) != cudaSuccess ||
+        cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+        adb_stream_session_destroy(s);
+        set_err("cudaMemset stream session state");
+        return ADB_ERR_CUDA;
+    }
+    *out = s;
+    return ADB_OK;
+}
+
+extern "C" void adb_stream_session_destroy(adb_stream_session *s) {
+    if (!s) return;
+    cudaSetDevice(s->ctx->device);
+    s->slots.release();
+    s->cache.release();
+    s->mask.release();
+    s->stage.release();
+    if (s->pin) cudaFreeHost(s->pin);
+    delete s;
+}
+
+extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                                       const int16_t *adc, const uint8_t *reset, const float *calib_offset,
+                                       const float *calib_scale, int32_t *polya_start, uint8_t *settled) {
+    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (n == 0) return ADB_OK;
+    if (!slots || !chunk_offsets || !polya_start || !settled) { set_err("null argument"); return ADB_ERR_ARG; }
+    if (chunk_offsets[0] < 0) { set_err("chunk_offsets must be non-negative"); return ADB_ERR_ARG; }
+    for (int k = 0; k < n; k++)
+        if (chunk_offsets[k + 1] < chunk_offsets[k]) { set_err("chunk_offsets must be non-decreasing"); return ADB_ERR_ARG; }
+    if (chunk_offsets[n] > chunk_offsets[0] && !adc) { set_err("null adc with non-empty chunks"); return ADB_ERR_ARG; }
+    // validate the whole push before any state changes: a refused push leaves the session as it was
+    if (++s->push_id == 0x7fffffff) { std::fill(s->stamp.begin(), s->stamp.end(), 0); s->push_id = 1; }
+    for (int k = 0; k < n; k++) {
+        const int sl = slots[k];
+        if (sl < 0 || sl >= s->n_slots) { set_err("slot out of range"); return ADB_ERR_ARG; }
+        if (s->stamp[sl] == s->push_id) { set_err("the same slot twice in one push"); return ADB_ERR_ARG; }
+        s->stamp[sl] = s->push_id;
+        if (reset && reset[k]) {
+            if (!calib_offset || !calib_scale) { set_err("a reset needs calib_offset and calib_scale"); return ADB_ERR_ARG; }
+            if (!std::isfinite(calib_scale[k]) || !(calib_scale[k] > 0.f) || !std::isfinite(calib_offset[k])) {
+                set_err("calibration scale must be finite and positive, offset finite");
+                return ADB_ERR_ARG;
+            }
+        } else if (!s->live[sl]) {
+            set_err("append to a slot that was never reset");
+            return ADB_ERR_ARG;
+        }
+    }
+    // entries that reach the device: resets and slots whose answer is not final; chunks are clipped at max_samples
+    std::vector<SessEntry> ent;
+    std::vector<int> ent_k;
+    ent.reserve(n);
+    int64_t total = 0;
+    for (int k = 0; k < n; k++) {
+        const int sl = slots[k];
+        const bool rs = reset && reset[k];
+        if (!rs && s->settled[sl]) continue;
+        SessEntry E;
+        E.slot = sl;
+        E.reset = rs ? 1 : 0;
+        const int64_t have = rs ? 0 : s->n[sl];
+        E.len = (int32_t)std::min<int64_t>(chunk_offsets[k + 1] - chunk_offsets[k], s->max_samples - have);
+        E._pad = 0;
+        E.src = total;
+        E.coff = rs ? calib_offset[k] : 0.f;
+        E.cscale = rs ? calib_scale[k] : 0.f;
+        total += E.len;
+        ent.push_back(E);
+        ent_k.push_back(k);
+    }
+    const int ne = (int)ent.size();
+    if (ne > 0) {
+        const size_t ent_bytes = (sizeof(SessEntry) * (size_t)ne + 15) & ~(size_t)15;
+        const size_t blob_bytes = ((size_t)total * sizeof(int16_t) + 15) & ~(size_t)15;
+        const size_t in_bytes = ent_bytes + blob_bytes, bytes = in_bytes + sizeof(int32_t) * 2 * (size_t)ne;
+        CUDA_TRY(cudaSetDevice(s->ctx->device));
+        if (bytes > s->pin_cap) {
+            if (s->pin) cudaFreeHost(s->pin);
+            s->pin = nullptr;
+            s->pin_cap = 0;
+            const size_t want = bytes + bytes / 4;
+            CUDA_TRY(cudaHostAlloc(&s->pin, want, cudaHostAllocDefault));
+            s->pin_cap = want;
+        }
+        if (s->stage.ensure(bytes)) { set_err("cudaMalloc stream session staging"); return ADB_ERR_CUDA; }
+        unsigned char *hp = (unsigned char *)s->pin;
+        memcpy(hp, ent.data(), sizeof(SessEntry) * (size_t)ne);
+        int16_t *hb = (int16_t *)(hp + ent_bytes);
+        for (int q = 0; q < ne; q++)
+            if (ent[q].len > 0) memcpy(hb + ent[q].src, adc + chunk_offsets[ent_k[q]], sizeof(int16_t) * (size_t)ent[q].len);
+        cudaStream_t st = s->ctx->stream;
+        CUDA_TRY(cudaMemcpyAsync(s->stage.p, hp, in_bytes, cudaMemcpyHostToDevice, st));
+        unsigned char *dp = (unsigned char *)s->stage.p;
+        SessArgs A;
+        A.slots = (SessSlot *)s->slots.p;
+        A.cache = (int16_t *)s->cache.p;
+        A.mask = (uint32_t *)s->mask.p;
+        A.ent = (const SessEntry *)dp;
+        A.blob = (const int16_t *)(dp + ent_bytes);
+        A.out = (int32_t *)(dp + in_bytes);
+        A.n_ent = ne;
+        A.max_samples = s->max_samples;
+        A.mask_words = s->mask_words;
+        stream_append_kernel<<<(ne + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg);
+        CUDA_TRY(cudaGetLastError());
+        stream_search_kernel<<<ne, ADB_VAL_THREADS, 0, st>>>(A, s->cfg);
+        CUDA_TRY(cudaGetLastError());
+        s->ctx->launches += 2;
+        CUDA_TRY(cudaMemcpyAsync(hp + in_bytes, A.out, sizeof(int32_t) * 2 * (size_t)ne, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        const int32_t *res = (const int32_t *)(hp + in_bytes);
+        for (int q = 0; q < ne; q++) {
+            const int sl = ent[q].slot;
+            s->n[sl] = (ent[q].reset ? 0 : s->n[sl]) + ent[q].len;
+            s->live[sl] = 1;
+            s->result[sl] = res[2 * q];
+            s->settled[sl] = res[2 * q + 1] ? 1 : 0;
+        }
+    }
+    for (int k = 0; k < n; k++) {
+        polya_start[k] = s->result[slots[k]];
+        settled[k] = s->settled[slots[k]];
+    }
     return ADB_OK;
 }
 

@@ -1,0 +1,202 @@
+// Read-until sessions of the streaming poly(A) detector (SURVEY.md row f4): mean_var_shift_polyA_detect,
+// adapted/detect/mvs.py:341-426, asked again every time a channel's cache grows by a chunk.
+//
+// A session keeps per slot (one per sequencer channel) the int16 cache of the read on it and everything the
+// stateless mvs_stream_kernel (adb_stream.cuh) would recompute from the start:
+//   - the state of the two bottleneck recurrences over signal[min_obs_adapter:] (running sum of the mean; amean /
+//     assqdm of the variance; tail samples consumed).  Both are trailing windows evaluated by sequential float32
+//     recurrences, so continuing them over the appended samples reproduces the stateless series bit for bit;
+//   - the match mask "moving mean and variance in range", which is therefore prefix-stable: only bits for the new
+//     positions are appended;
+//   - the running min / max ADC code, which replaces the whole-window scan that bounds the order statistics;
+//   - the resume offset of the search loop.  A hit at idx is judged on [idx, idx + polyA_window),
+//     [idx, idx + median_shift_window) and [idx - median_shift_window, idx), each clipped at n, and on the
+//     n - idx < min_obs_post_loc exit.  Once n - idx >= max(min_obs_post_loc, polyA_window, median_shift_window)
+//     no further sample changes that decision, and the hit itself (the first mask bit at or after the offset) is
+//     final as soon as it is found.  A final rejection advances the resume offset as the reference advances
+//     `offset`; a final acceptance settles the slot.  Decisions on clipped windows are taken again on the next push.
+// The early return n < min_obs_adapter + max(windows) is tested on every push.  A slot also settles when its cache
+// is full (max_samples): later samples of that read are dropped.
+//
+// Two launches per push: stream_append_kernel (one warp per pushed slot copies the chunk into the cache and updates
+// the code bounds; its lane 0 advances the recurrences and the mask) and stream_search_kernel (one CTA per pushed
+// slot resumes the search loop with seg_stats reading the cache in global memory, so a cache is not bounded by
+// shared memory).
+#pragma once
+#include "adb_stream.cuh"
+
+struct SessSlot {  // device state of one slot
+    int32_t n;        // samples in the cache
+    int32_t t;        // tail samples (positions >= min_obs_adapter) the recurrences have consumed
+    int32_t roff;     // resume offset of the search loop (tail index)
+    int32_t result;   // last answer
+    int32_t settled;  // the answer is final
+    uint32_t kmin, kmax;  // ADC code bounds of the cache, as keys code + 32768 (kmin > kmax: empty)
+    float coff, cscale;
+    float amean, assqdm, asum;
+};
+
+struct SessEntry {  // one pushed slot, host -> device
+    int32_t slot, reset, len, _pad;
+    int64_t src;      // first sample of the chunk in the staged blob
+    float coff, cscale;
+};
+
+struct SessArgs {
+    SessSlot *slots;
+    int16_t *cache;        // [n_slots][max_samples]
+    uint32_t *mask;        // [n_slots][mask_words]
+    const SessEntry *ent;  // [n_ent]
+    const int16_t *blob;   // staged chunks
+    int32_t *out;          // [n_ent][2]: polya_start, settled
+    int n_ent, max_samples, mask_words;
+};
+
+#define SESS_APPEND_WARPS 4
+
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(SessArgs A, adb_stream_config P) {
+    const int e = blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (e >= A.n_ent) return;
+    const SessEntry E = A.ent[e];
+    SessSlot &S = A.slots[E.slot];
+    const int wm = P.pA_mean_window, wv = P.pA_var_window, moa = P.min_obs_adapter;
+    if (E.reset) {
+        if (lane == 0) {
+            S.n = 0; S.t = 0; S.roff = max(wm, wv); S.result = 0; S.settled = 0;
+            S.kmin = 0xffffffffu; S.kmax = 0u;
+            S.coff = E.coff; S.cscale = E.cscale;
+            S.amean = 0.f; S.assqdm = 0.f; S.asum = 0.f;
+        }
+        __syncwarp();
+    }
+    if (S.settled || E.len <= 0) return;
+    const int n0 = S.n, n1 = n0 + E.len;
+    int16_t *cache = A.cache + (size_t)E.slot * A.max_samples;
+    uint32_t lo = 0xffffffffu, hi = 0u;
+    for (int j = lane; j < E.len; j += 32) {
+        const int16_t v = A.blob[E.src + j];
+        cache[n0 + j] = v;
+        const uint32_t k = (uint32_t)((int)v + 32768);
+        lo = min(lo, k);
+        hi = max(hi, k);
+    }
+    lo = warp_min_u(lo);
+    hi = warp_max_u(hi);
+    __syncwarp();  // the chunk is in the cache for lane 0 (warp-level memory ordering)
+    if (lane != 0) return;
+    S.kmin = min(S.kmin, lo);
+    S.kmax = max(S.kmax, hi);
+    S.n = n1;
+    const int L = n1 - moa;
+    int i = S.t;
+    if (L <= i) return;
+    const float coff = S.coff, cscale = S.cscale;
+    auto pa = [&](int j) { return __fmul_rn(__fadd_rn((float)cache[j], coff), cscale); };
+    float amean = S.amean, assqdm = S.assqdm, asum = S.asum, mv = 0.f, mm = 0.f;
+    const float vinv = (float)(1.0 / (double)wv), minv = (float)(1.0 / (double)wm);
+    const int i0 = max(wv, wm) - 1;
+    uint32_t *mask = A.mask + (size_t)E.slot * A.mask_words;
+    uint32_t bits = (i & 31) ? (mask[i >> 5] & ((1u << (i & 31)) - 1u)) : 0u;
+    for (; i < L; i++) {
+        const float ai = pa(moa + i);
+        if (i < wv) {
+            mv_var_warm(amean, assqdm, ai, i);
+            if (i == wv - 1) mv = mv_var_first(assqdm, wv);
+        } else {
+            mv_var_step(amean, assqdm, ai, pa(moa + i - wv), vinv);
+            mv = __fmul_rn(assqdm, vinv);
+        }
+        if (i < wm) {
+            asum = __fadd_rn(asum, ai);
+            if (i == wm - 1) mm = __fdiv_rn(asum, (float)wm);
+        } else {
+            asum = mv_mean_step(asum, ai, pa(moa + i - wm));
+            mm = __fmul_rn(asum, minv);
+        }
+        if (i >= i0 && in_range_f32w(mm, P.pA_mean_range) && in_range_f32w(mv, P.pA_var_range)) bits |= 1u << (i & 31);
+        if ((i & 31) == 31) { mask[i >> 5] = bits; bits = 0u; }
+    }
+    if (L & 31) mask[L >> 5] = bits;
+    S.t = L;
+    S.amean = amean; S.assqdm = assqdm; S.asum = asum;
+}
+
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs A, adb_stream_config P) {
+    __shared__ __align__(16) unsigned char scratch[((size_t)ADB_SEL_SMEM_BYTES + 64 + 15) & ~(size_t)15];
+    __shared__ uint32_t kbuf[8];
+    __shared__ int itmp[8];
+    __shared__ double dtmp[8];
+    const int e = blockIdx.x;
+    const SessEntry E = A.ent[e];
+    SessSlot &S = A.slots[E.slot];
+    if (S.settled) {
+        if (threadIdx.x == 0) { A.out[2 * e] = S.result; A.out[2 * e + 1] = 1; }
+        return;
+    }
+    const int wm = P.pA_mean_window, wv = P.pA_var_window, moa = P.min_obs_adapter;
+    const int n = S.n;
+    const bool full = n >= A.max_samples;
+    int result = 0, settled = full ? 1 : 0, roff = S.roff;
+    if (n >= moa + max(max(wm, wv), max(P.min_obs_post_loc, P.polyA_window))) {  // mvs.py:352-363
+        ValCtx C;
+        C.cfg = nullptr;
+        C.S = sel_scratch_from(scratch);
+        C.kbuf = kbuf;
+        C.itmp = itmp;
+        C.dtmp = dtmp;
+        C.series_a = C.series_b = nullptr;
+        C.pre_var = C.pre_mean = nullptr;
+        C.pre_ae = C.pre_pe = -1;
+        C.src.f32 = nullptr;
+        C.src.i16 = A.cache + (size_t)E.slot * A.max_samples;
+        C.src.n = n;
+        C.src.coff = S.coff;
+        C.src.cscale = S.cscale;
+        C.int_keys = true;  // the session only takes scale > 0
+        C.wkmin = S.kmin;
+        C.wkmax = S.kmax;
+        const PaVal V{C.src, true};
+        C.wvmin = V(C.wkmin);
+        C.wvmax = V(C.wkmax);
+        const uint32_t *mask = A.mask + (size_t)E.slot * A.mask_words;
+        const int L = n - moa, nwords = (L + 31) >> 5;
+        const int need = max(P.min_obs_post_loc, max(P.polyA_window, P.median_shift_window));
+        int offset = roff;
+        while (offset < L) {  // mvs.py:381-425 from the first decision that was not final
+            if (threadIdx.x == 0) itmp[7] = 0x7fffffff;
+            __syncthreads();
+            for (int w = (offset >> 5) + threadIdx.x; w < nwords; w += blockDim.x) {
+                uint32_t bits = mask[w];
+                if (w == (offset >> 5)) bits &= 0xffffffffu << (offset & 31);
+                if (w == nwords - 1 && (L & 31)) bits &= (1u << (L & 31)) - 1u;  // the word holds no later bit
+                if (bits) { atomicMin(&itmp[7], w * 32 + __ffs(bits) - 1); break; }
+            }
+            __syncthreads();
+            const int hit = itmp[7];
+            __syncthreads();
+            if (hit == 0x7fffffff) break;                     // no match yet
+            const int idx = moa + hit;
+            if (n - idx < P.min_obs_post_loc) break;          // not enough signal after the hit yet
+            const bool final_ = n - idx >= need;
+            const SegStats Q = seg_stats(C, idx, min(idx + P.polyA_window, n), SS_MED | SS_LR);
+            const float m_after = seg_stats(C, idx, min(idx + P.median_shift_window, n), SS_MED).med;
+            const float m_before = seg_stats(C, max(idx - P.median_shift_window, 0), idx, SS_MED).med;
+            const double shift = (double)__fsub_rn(m_after, m_before);
+            if (in_range_f32w(Q.med, P.polyA_med_range) && in_range_d(Q.lr, P.polyA_local_range) &&
+                in_range_d(shift, P.median_shift_range)) {
+                result = idx;
+                if (final_) settled = 1;
+                break;
+            }
+            offset = idx - moa + P.search_increment_step;
+            if (final_) roff = offset;  // every earlier decision was final too: resume here next time
+        }
+    }
+    if (threadIdx.x == 0) {
+        S.roff = roff;
+        S.result = result;
+        S.settled = settled;
+        A.out[2 * e] = result;
+        A.out[2 * e + 1] = settled;
+    }
+}

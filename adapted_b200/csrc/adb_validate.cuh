@@ -381,6 +381,30 @@ __device__ void seg_mean_std(ValCtx &C, int a, int b, double &mean_out, double &
 // NaN-free segments (the only case real ADC data produces) take a branch-free loop whose only loop-carried
 // dependencies are the float32 accumulators themselves; segments with NaN take the general path with bottleneck's
 // count bookkeeping.  CTA-wide.
+// NaN-free steps of the two recurrences, shared with the streaming session (adb_stream_session.cuh), which carries
+// (amean, assqdm) and asum across pushes.  Warm-up of the variance: sample i < window enters Welford's update with a
+// divide by i + 1; the first output clamps the running state and divides by the window.
+__device__ __forceinline__ void mv_var_warm(float &amean, float &assqdm, float ai, int i) {
+    const float delta = __fsub_rn(ai, amean);
+    amean = __fadd_rn(amean, __fdiv_rn(delta, (float)(i + 1)));
+    assqdm = __fadd_rn(assqdm, __fmul_rn(delta, __fsub_rn(ai, amean)));
+}
+__device__ __forceinline__ float mv_var_first(float &assqdm, int wv) {
+    if (assqdm < 0) assqdm = 0;
+    return __fdiv_rn(assqdm, (float)wv);
+}
+// sample ai enters, aold (window samples back) leaves; the output is assqdm * count_inv
+__device__ __forceinline__ void mv_var_step(float &amean, float &assqdm, float ai, float aold, float count_inv) {
+    const float delta = __fsub_rn(ai, aold);
+    aold = __fsub_rn(aold, amean);
+    amean = __fadd_rn(amean, __fmul_rn(delta, count_inv));
+    ai = __fsub_rn(ai, amean);
+    assqdm = __fadd_rn(assqdm, __fmul_rn(__fadd_rn(ai, aold), delta));
+    if (assqdm < 0) assqdm = 0;
+}
+// running sum of the moving mean past its first window; the output is asum * count_inv
+__device__ __forceinline__ float mv_mean_step(float asum, float ai, float aold) { return __fadd_rn(asum, __fsub_rn(ai, aold)); }
+
 __device__ void seg_moving_stats(ValCtx &C, int a, int L, int wv, int wm, bool do_var, bool do_mean) {
     const ReadSrc &src = C.src;
     // any NaN in the segment?
@@ -398,24 +422,12 @@ __device__ void seg_moving_stats(ValCtx &C, int a, int L, int wv, int wm, bool d
         float *y = C.series_a;
         if (!has_nan) {
             float amean = 0.f, assqdm = 0.f;
-            for (int i = 0; i < wv; i++) {  // Welford accumulation of the first window
-                const float ai = src.pa(a + i);
-                const float delta = __fsub_rn(ai, amean);
-                amean = __fadd_rn(amean, __fdiv_rn(delta, (float)(i + 1)));
-                assqdm = __fadd_rn(assqdm, __fmul_rn(delta, __fsub_rn(ai, amean)));
-            }
-            if (assqdm < 0) assqdm = 0;
-            y[0] = __fdiv_rn(assqdm, (float)wv);
+            for (int i = 0; i < wv; i++) mv_var_warm(amean, assqdm, src.pa(a + i), i);
+            y[0] = mv_var_first(assqdm, wv);
             const float count_inv = (float)(1.0 / (double)wv);
 #pragma unroll 4
             for (int i = wv; i < L; i++) {
-                float ai = src.pa(a + i), aold = src.pa(a + i - wv);
-                const float delta = __fsub_rn(ai, aold);
-                aold = __fsub_rn(aold, amean);
-                amean = __fadd_rn(amean, __fmul_rn(delta, count_inv));
-                ai = __fsub_rn(ai, amean);
-                assqdm = __fadd_rn(assqdm, __fmul_rn(__fadd_rn(ai, aold), delta));
-                if (assqdm < 0) assqdm = 0;
+                mv_var_step(amean, assqdm, src.pa(a + i), src.pa(a + i - wv), count_inv);
                 y[i - (wv - 1)] = __fmul_rn(assqdm, count_inv);
             }
         } else {
@@ -480,7 +492,7 @@ __device__ void seg_moving_stats(ValCtx &C, int a, int L, int wv, int wm, bool d
             const float count_inv = (float)(1.0 / (double)wm);
 #pragma unroll 8
             for (int i = wm; i < L; i++) {
-                asum = __fadd_rn(asum, __fsub_rn(src.pa(a + i), src.pa(a + i - wm)));
+                asum = mv_mean_step(asum, src.pa(a + i), src.pa(a + i - wm));
                 y[i - (wm - 1)] = __fmul_rn(asum, count_inv);
             }
         } else {

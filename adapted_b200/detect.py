@@ -274,11 +274,10 @@ def mean_var_shift_polyA_detect_batch(batch_of_signals: np.ndarray, signal_lens:
                                       device: int = 0) -> np.ndarray:
     """mean_var_shift_polyA_detect for every row of a dense float32 [N, m] matrix (row i = its first signal_lens[i]
     samples): poly(A) start per read, 0 where the reference returns 0."""
-    from .config import StreamingConfig, flatten_streaming_config
+    from .config import flatten_streaming_config
+    from .stream import resolve_stream_params
 
-    if hasattr(params, "streaming"):  # a whole SigProcConfig: its optional [streaming] section
-        params = params.streaming
-    params = StreamingConfig() if params is None else params
+    params = resolve_stream_params(params)
     b, keep = _dense_batch(batch_of_signals, signal_lens)
     out = np.zeros(b.n_reads, dtype=np.int32)
     if b.n_reads == 0:
@@ -303,11 +302,10 @@ def mean_var_shift_polyA_detect_i16(adc: np.ndarray, offsets: np.ndarray, calib_
                                     device: int = 0) -> np.ndarray:
     """Ragged int16 form (what a read-until cache holds): read i = adc[offsets[i]:offsets[i+1]], calibrated on the
     device; `window` bounds the samples looked at per read (default: the longest read)."""
-    from .config import StreamingConfig, flatten_streaming_config
+    from .config import flatten_streaming_config
+    from .stream import resolve_stream_params
 
-    if hasattr(params, "streaming"):  # a whole SigProcConfig: its optional [streaming] section
-        params = params.streaming
-    params = StreamingConfig() if params is None else params
+    params = resolve_stream_params(params)
     adc = np.ascontiguousarray(adc, dtype=np.int16)
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
     lens = np.ascontiguousarray(np.diff(offsets), dtype=np.int32)

@@ -269,6 +269,37 @@ typedef struct adb_stream_config {
  */
 int adb_mvs_stream_detect_host(adb_ctx *ctx, const adb_batch *batch, const adb_stream_config *cfg, int32_t *polya_start);
 
+/*
+ * Read-until sessions of the same detector: the caller keeps asking "where does the poly(A) start in what this
+ * channel has delivered so far?" while the cache grows chunk by chunk.  A session holds `n_slots` slots (one per
+ * channel), each the int16 ADC cache (at most `max_samples` samples) of the read on it plus that read's calibration,
+ * on the context's device; pushes run on the context's stream.  The cache is never staged in shared memory, so
+ * max_samples is not bounded by the stateless call's window.
+ *
+ * After a push, every pushed slot k returns
+ *   polya_start[k]  exactly what mean_var_shift_polyA_detect(calibrate(cache), cfg) returns on the slot's whole cache
+ *                   (adb_mvs_stream_detect_host on the same samples), pA = (float32(adc) + offset) * scale;
+ *   settled[k]      1 when no later sample can change that answer: an acceptance whose windows are complete, or a full
+ *                   cache (samples beyond max_samples are dropped).  Chunks for a settled read are ignored.
+ * Per push, only the appended samples enter the moving statistics, and the search loop resumes after its last final
+ * decision (adb_stream_session.cuh).
+ */
+typedef struct adb_stream_session adb_stream_session;
+/* ADB_ERR_ARG for n_slots < 1 or max_samples < 1, ADB_ERR_UNSUPPORTED for the configurations that
+ * adb_mvs_stream_detect_host refuses.  The context must outlive the session. */
+int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots, int32_t max_samples,
+                              adb_stream_session **out);
+void adb_stream_session_destroy(adb_stream_session *s);
+/* entry k: reset[k] != 0 starts a new read on slots[k] (cache emptied, calibration taken from calib_offset[k] /
+ * calib_scale[k]), then adc[chunk_offsets[k] .. chunk_offsets[k+1]) is appended.  HOST buffers, synchronous.
+ * reset == NULL: no entry resets (calib_* may then be NULL).  Zero-length chunks are legal and return the current
+ * answer.  ADB_ERR_ARG, with the session unchanged, for a slot out of range or twice in one push, decreasing offsets,
+ * an append to a slot that was never reset, or a reset with a non-finite offset or a non-finite or non-positive
+ * scale. */
+int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                            const int16_t *adc, const uint8_t *reset, const float *calib_offset,
+                            const float *calib_scale, int32_t *polya_start, uint8_t *settled);
+
 /* ---- result tables (SURVEY.md row f2) ---------------------------------------------------------------------- */
 /*
  * Drop-in for save_detected_boundaries(processing_results, filename, save_fail_reasons)   adapted/output.py:26-51
