@@ -881,6 +881,7 @@ extern "C" int adb_mvs_stream_detect_host(adb_ctx *ctx, const adb_batch *batch, 
 struct adb_stream_session {
     adb_ctx *ctx = nullptr;
     adb_stream_config cfg;
+    bool f32 = false;  // the caches hold calibrated float32 pA (else int16 ADC codes)
     int n_slots = 0, max_samples = 0, mask_words = 0;
     DevBuf slots, cache, mask, stage;  // stage: one push's entries, chunks and answers
     void *pin = nullptr;               // pinned mirror of `stage`
@@ -891,8 +892,8 @@ struct adb_stream_session {
     int32_t push_id = 0;
 };
 
-extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
-                                         int32_t max_samples, adb_stream_session **out) {
+static int session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots, int32_t max_samples, bool f32,
+                          adb_stream_session **out) {
     if (!ctx || !cfg || !out) { set_err("null argument"); return ADB_ERR_ARG; }
     *out = nullptr;
     if (n_slots < 1 || max_samples < 1) { set_err("n_slots and max_samples must be positive"); return ADB_ERR_ARG; }
@@ -902,6 +903,7 @@ extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *
     adb_stream_session *s = new adb_stream_session();
     s->ctx = ctx;
     s->cfg = *cfg;
+    s->f32 = f32;
     s->n_slots = n_slots;
     s->max_samples = max_samples;
     s->mask_words = (max_samples + 31) / 32;
@@ -910,7 +912,7 @@ extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *
     s->stamp.assign(n_slots, 0);
     s->live.assign(n_slots, 0);
     s->settled.assign(n_slots, 0);
-    if (s->slots.ensure(sizeof(SessSlot) * (size_t)n_slots) || s->cache.ensure(sizeof(int16_t) * (size_t)n_slots * max_samples) ||
+    if (s->slots.ensure(sizeof(SessSlot) * (size_t)n_slots) || s->cache.ensure((f32 ? sizeof(float) : sizeof(int16_t)) * (size_t)n_slots * max_samples) ||
         s->mask.ensure(sizeof(uint32_t) * (size_t)n_slots * s->mask_words)) {
         adb_stream_session_destroy(s);
         set_err("cudaMalloc stream session arena");
@@ -926,6 +928,16 @@ extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *
     return ADB_OK;
 }
 
+extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
+                                         int32_t max_samples, adb_stream_session **out) {
+    return session_create(ctx, cfg, n_slots, max_samples, false, out);
+}
+
+extern "C" int adb_stream_session_create_f32(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
+                                             int32_t max_samples, adb_stream_session **out) {
+    return session_create(ctx, cfg, n_slots, max_samples, true, out);
+}
+
 extern "C" void adb_stream_session_destroy(adb_stream_session *s) {
     if (!s) return;
     cudaSetDevice(s->ctx->device);
@@ -937,16 +949,33 @@ extern "C" void adb_stream_session_destroy(adb_stream_session *s) {
     delete s;
 }
 
-extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
-                                       const int16_t *adc, const uint8_t *reset, const float *calib_offset,
-                                       const float *calib_scale, int32_t *polya_start, uint8_t *settled) {
-    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+// true when no sample of src[0, n) is infinite or NaN (exponent bits all ones); copies them to dst unless it is null
+static bool copy_finite(float *dst, const float *src, int64_t n) {
+    uint32_t bad = 0;
+    for (int64_t j = 0; j < n; j++) {
+        uint32_t b;
+        memcpy(&b, src + j, 4);
+        if (dst) memcpy(dst + j, &b, 4);
+        bad |= (b & 0x7f800000u) == 0x7f800000u;
+    }
+    return !bad;
+}
+
+// one push of either kind: `samples` is int16 ADC (with calibration on reset) or float32 pA, as the session holds
+static int session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                        const void *samples, const uint8_t *reset, const float *calib_offset, const float *calib_scale,
+                        int32_t *polya_start, uint8_t *settled) {
+    const bool f32 = s->f32;
+    const size_t esz = f32 ? sizeof(float) : sizeof(int16_t);
     if (n == 0) return ADB_OK;
     if (!slots || !chunk_offsets || !polya_start || !settled) { set_err("null argument"); return ADB_ERR_ARG; }
     if (chunk_offsets[0] < 0) { set_err("chunk_offsets must be non-negative"); return ADB_ERR_ARG; }
     for (int k = 0; k < n; k++)
         if (chunk_offsets[k + 1] < chunk_offsets[k]) { set_err("chunk_offsets must be non-decreasing"); return ADB_ERR_ARG; }
-    if (chunk_offsets[n] > chunk_offsets[0] && !adc) { set_err("null adc with non-empty chunks"); return ADB_ERR_ARG; }
+    if (chunk_offsets[n] > chunk_offsets[0] && !samples) {
+        set_err(f32 ? "null pa with non-empty chunks" : "null adc with non-empty chunks");
+        return ADB_ERR_ARG;
+    }
     // validate the whole push before any state changes: a refused push leaves the session as it was
     if (++s->push_id == 0x7fffffff) { std::fill(s->stamp.begin(), s->stamp.end(), 0); s->push_id = 1; }
     for (int k = 0; k < n; k++) {
@@ -955,6 +984,7 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
         if (s->stamp[sl] == s->push_id) { set_err("the same slot twice in one push"); return ADB_ERR_ARG; }
         s->stamp[sl] = s->push_id;
         if (reset && reset[k]) {
+            if (f32) continue;  // float32 reads carry no calibration
             if (!calib_offset || !calib_scale) { set_err("a reset needs calib_offset and calib_scale"); return ADB_ERR_ARG; }
             if (!std::isfinite(calib_scale[k]) || !(calib_scale[k] > 0.f) || !std::isfinite(calib_offset[k])) {
                 set_err("calibration scale must be finite and positive, offset finite");
@@ -965,7 +995,10 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
             return ADB_ERR_ARG;
         }
     }
-    // entries that reach the device: resets and slots whose answer is not final; chunks are clipped at max_samples
+    // entries that reach the device: resets and slots whose answer is not final; chunks are clipped at max_samples.
+    // Float32 samples that do not reach the device (settled slot, beyond max_samples) are checked for finiteness here,
+    // the others while they are staged.
+    const float *pa = (const float *)samples;
     std::vector<SessEntry> ent;
     std::vector<int> ent_k;
     ent.reserve(n);
@@ -973,16 +1006,21 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
     for (int k = 0; k < n; k++) {
         const int sl = slots[k];
         const bool rs = reset && reset[k];
-        if (!rs && s->settled[sl]) continue;
+        const int64_t clen = chunk_offsets[k + 1] - chunk_offsets[k];
+        if (!rs && s->settled[sl]) {
+            if (f32 && !copy_finite(nullptr, pa + chunk_offsets[k], clen)) { set_err("non-finite pA sample"); return ADB_ERR_ARG; }
+            continue;
+        }
         SessEntry E;
         E.slot = sl;
         E.reset = rs ? 1 : 0;
         const int64_t have = rs ? 0 : s->n[sl];
-        E.len = (int32_t)std::min<int64_t>(chunk_offsets[k + 1] - chunk_offsets[k], s->max_samples - have);
+        E.len = (int32_t)std::min<int64_t>(clen, s->max_samples - have);
         E._pad = 0;
         E.src = total;
-        E.coff = rs ? calib_offset[k] : 0.f;
-        E.cscale = rs ? calib_scale[k] : 0.f;
+        E.coff = rs && !f32 ? calib_offset[k] : 0.f;
+        E.cscale = rs && !f32 ? calib_scale[k] : 0.f;
+        if (f32 && !copy_finite(nullptr, pa + chunk_offsets[k] + E.len, clen - E.len)) { set_err("non-finite pA sample"); return ADB_ERR_ARG; }
         total += E.len;
         ent.push_back(E);
         ent_k.push_back(k);
@@ -990,7 +1028,7 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
     const int ne = (int)ent.size();
     if (ne > 0) {
         const size_t ent_bytes = (sizeof(SessEntry) * (size_t)ne + 15) & ~(size_t)15;
-        const size_t blob_bytes = ((size_t)total * sizeof(int16_t) + 15) & ~(size_t)15;
+        const size_t blob_bytes = ((size_t)total * esz + 15) & ~(size_t)15;
         const size_t in_bytes = ent_bytes + blob_bytes, bytes = in_bytes + sizeof(int32_t) * 2 * (size_t)ne;
         CUDA_TRY(cudaSetDevice(s->ctx->device));
         if (bytes > s->pin_cap) {
@@ -1004,28 +1042,53 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
         if (s->stage.ensure(bytes)) { set_err("cudaMalloc stream session staging"); return ADB_ERR_CUDA; }
         unsigned char *hp = (unsigned char *)s->pin;
         memcpy(hp, ent.data(), sizeof(SessEntry) * (size_t)ne);
-        int16_t *hb = (int16_t *)(hp + ent_bytes);
-        for (int q = 0; q < ne; q++)
-            if (ent[q].len > 0) memcpy(hb + ent[q].src, adc + chunk_offsets[ent_k[q]], sizeof(int16_t) * (size_t)ent[q].len);
+        unsigned char *hb = hp + ent_bytes;
+        for (int q = 0; q < ne; q++) {
+            if (ent[q].len <= 0) continue;
+            const int64_t o = chunk_offsets[ent_k[q]];
+            if (!f32) {
+                memcpy((int16_t *)hb + ent[q].src, (const int16_t *)samples + o, sizeof(int16_t) * (size_t)ent[q].len);
+            } else if (!copy_finite((float *)hb + ent[q].src, pa + o, ent[q].len)) {
+                set_err("non-finite pA sample");
+                return ADB_ERR_ARG;
+            }
+        }
         cudaStream_t st = s->ctx->stream;
         CUDA_TRY(cudaMemcpyAsync(s->stage.p, hp, in_bytes, cudaMemcpyHostToDevice, st));
         unsigned char *dp = (unsigned char *)s->stage.p;
-        SessArgs A;
-        A.slots = (SessSlot *)s->slots.p;
-        A.cache = (int16_t *)s->cache.p;
-        A.mask = (uint32_t *)s->mask.p;
-        A.ent = (const SessEntry *)dp;
-        A.blob = (const int16_t *)(dp + ent_bytes);
-        A.out = (int32_t *)(dp + in_bytes);
-        A.n_ent = ne;
-        A.max_samples = s->max_samples;
-        A.mask_words = s->mask_words;
-        stream_append_kernel<<<(ne + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg);
-        CUDA_TRY(cudaGetLastError());
-        stream_search_kernel<<<ne, ADB_VAL_THREADS, 0, st>>>(A, s->cfg);
+        const int ablocks = (ne + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS;
+        if (!f32) {
+            SessArgs A;
+            A.slots = (SessSlot *)s->slots.p;
+            A.cache = (int16_t *)s->cache.p;
+            A.mask = (uint32_t *)s->mask.p;
+            A.ent = (const SessEntry *)dp;
+            A.blob = (const int16_t *)(dp + ent_bytes);
+            A.out = (int32_t *)(dp + in_bytes);
+            A.n_ent = ne;
+            A.max_samples = s->max_samples;
+            A.mask_words = s->mask_words;
+            stream_append_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg);
+            CUDA_TRY(cudaGetLastError());
+            stream_search_kernel<<<ne, ADB_VAL_THREADS, 0, st>>>(A, s->cfg);
+        } else {
+            SessArgsF32 A;
+            A.slots = (SessSlot *)s->slots.p;
+            A.cache = (float *)s->cache.p;
+            A.mask = (uint32_t *)s->mask.p;
+            A.ent = (const SessEntry *)dp;
+            A.blob = (const float *)(dp + ent_bytes);
+            A.out = (int32_t *)(dp + in_bytes);
+            A.n_ent = ne;
+            A.max_samples = s->max_samples;
+            A.mask_words = s->mask_words;
+            stream_append_f32_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg);
+            CUDA_TRY(cudaGetLastError());
+            stream_search_f32_kernel<<<ne, ADB_VAL_THREADS, 0, st>>>(A, s->cfg);
+        }
         CUDA_TRY(cudaGetLastError());
         s->ctx->launches += 2;
-        CUDA_TRY(cudaMemcpyAsync(hp + in_bytes, A.out, sizeof(int32_t) * 2 * (size_t)ne, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(hp + in_bytes, dp + in_bytes, sizeof(int32_t) * 2 * (size_t)ne, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         const int32_t *res = (const int32_t *)(hp + in_bytes);
         for (int q = 0; q < ne; q++) {
@@ -1041,6 +1104,22 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
         settled[k] = s->settled[slots[k]];
     }
     return ADB_OK;
+}
+
+extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                                       const int16_t *adc, const uint8_t *reset, const float *calib_offset,
+                                       const float *calib_scale, int32_t *polya_start, uint8_t *settled) {
+    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (s->f32) { set_err("int16 push on a float32 session"); return ADB_ERR_ARG; }
+    return session_push(s, n, slots, chunk_offsets, adc, reset, calib_offset, calib_scale, polya_start, settled);
+}
+
+extern "C" int adb_stream_session_push_f32(adb_stream_session *s, int32_t n, const int32_t *slots,
+                                           const int64_t *chunk_offsets, const float *pa, const uint8_t *reset,
+                                           int32_t *polya_start, uint8_t *settled) {
+    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (!s->f32) { set_err("float32 push on an int16 session"); return ADB_ERR_ARG; }
+    return session_push(s, n, slots, chunk_offsets, pa, reset, nullptr, nullptr, polya_start, settled);
 }
 
 // ---- CNN scores (kernel-level test entry) ------------------------------------------------------------------------

@@ -1,14 +1,16 @@
 // Read-until sessions of the streaming poly(A) detector (SURVEY.md row f4): mean_var_shift_polyA_detect,
 // adapted/detect/mvs.py:341-426, asked again every time a channel's cache grows by a chunk.
 //
-// A session keeps per slot (one per sequencer channel) the int16 cache of the read on it and everything the
-// stateless mvs_stream_kernel (adb_stream.cuh) would recompute from the start:
+// A session keeps per slot (one per sequencer channel) the cache of the read on it -- int16 ADC codes with the read's
+// calibration, or calibrated float32 pA -- and everything the stateless mvs_stream_kernel (adb_stream.cuh) would
+// recompute from the start:
 //   - the state of the two bottleneck recurrences over signal[min_obs_adapter:] (running sum of the mean; amean /
 //     assqdm of the variance; tail samples consumed).  Both are trailing windows evaluated by sequential float32
 //     recurrences, so continuing them over the appended samples reproduces the stateless series bit for bit;
 //   - the match mask "moving mean and variance in range", which is therefore prefix-stable: only bits for the new
 //     positions are appended;
-//   - the running min / max ADC code, which replaces the whole-window scan that bounds the order statistics;
+//   - the running min / max sample key (ADC code + 32768, or f32_key of the pA value), which replaces the whole-window
+//     scan that bounds the order statistics;
 //   - the resume offset of the search loop.  A hit at idx is judged on [idx, idx + polyA_window),
 //     [idx, idx + median_shift_window) and [idx - median_shift_window, idx), each clipped at n, and on the
 //     n - idx < min_obs_post_loc exit.  Once n - idx >= max(min_obs_post_loc, polyA_window, median_shift_window)
@@ -19,9 +21,11 @@
 // is full (max_samples): later samples of that read are dropped.
 //
 // Two launches per push: stream_append_kernel (one warp per pushed slot copies the chunk into the cache and updates
-// the code bounds; its lane 0 advances the recurrences and the mask) and stream_search_kernel (one CTA per pushed
+// the key bounds; its lane 0 advances the recurrences and the mask) and stream_search_kernel (one CTA per pushed
 // slot resumes the search loop with seg_stats reading the cache in global memory, so a cache is not bounded by
-// shared memory).
+// shared memory).  Float32 sessions run stream_append_f32_kernel / stream_search_f32_kernel: the same code
+// (sess_append / sess_search) with the samples taken as they are, and order statistics on float keys through the
+// generic multi-level select instead of the one-pass code histogram.
 #pragma once
 #include "adb_stream.cuh"
 
@@ -31,8 +35,8 @@ struct SessSlot {  // device state of one slot
     int32_t roff;     // resume offset of the search loop (tail index)
     int32_t result;   // last answer
     int32_t settled;  // the answer is final
-    uint32_t kmin, kmax;  // ADC code bounds of the cache, as keys code + 32768 (kmin > kmax: empty)
-    float coff, cscale;
+    uint32_t kmin, kmax;  // key bounds of the cache (kmin > kmax: empty)
+    float coff, cscale;   // calibration of an int16 read (unused by float32 slots)
     float amean, assqdm, asum;
 };
 
@@ -42,20 +46,46 @@ struct SessEntry {  // one pushed slot, host -> device
     float coff, cscale;
 };
 
-struct SessArgs {
+template <class T>
+struct SessArgsT {
     SessSlot *slots;
-    int16_t *cache;        // [n_slots][max_samples]
+    T *cache;              // [n_slots][max_samples]
     uint32_t *mask;        // [n_slots][mask_words]
     const SessEntry *ent;  // [n_ent]
-    const int16_t *blob;   // staged chunks
+    const T *blob;         // staged chunks
     int32_t *out;          // [n_ent][2]: polya_start, settled
     int n_ent, max_samples, mask_words;
+};
+struct SessArgs : SessArgsT<int16_t> {};   // int16 ADC caches
+struct SessArgsF32 : SessArgsT<float> {};  // calibrated float32 pA caches
+
+// what differs between the two cache types: the order-preserving key of a sample, its pA value, and how seg_stats
+// reads the cache
+template <class T>
+struct SessSample;
+template <>
+struct SessSample<int16_t> {
+    static constexpr bool int_keys = true;  // the session only takes scale > 0
+    static __device__ __forceinline__ uint32_t key(int16_t v) { return (uint32_t)((int)v + 32768); }
+    static __device__ __forceinline__ float pa(int16_t v, float coff, float cscale) {
+        return __fmul_rn(__fadd_rn((float)v, coff), cscale);
+    }
+    static __device__ __forceinline__ void src(ReadSrc &s, const int16_t *cache) { s.f32 = nullptr; s.i16 = cache; }
+};
+template <>
+struct SessSample<float> {
+    static constexpr bool int_keys = false;
+    static __device__ __forceinline__ uint32_t key(float v) { return f32_key(v); }
+    static __device__ __forceinline__ float pa(float v, float, float) { return v; }
+    static __device__ __forceinline__ void src(ReadSrc &s, const float *cache) { s.f32 = cache; s.i16 = nullptr; }
 };
 
 #define SESS_APPEND_WARPS 4
 
-__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(SessArgs A, adb_stream_config P) {
-    const int e = blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+// warp of entry e; the kernels compute e and lane, where the compiler knows the bounds of threadIdx.x
+template <class T>
+__device__ __forceinline__ void sess_append(SessArgsT<T> A, adb_stream_config P, int e, int lane) {
+    using X = SessSample<T>;
     if (e >= A.n_ent) return;
     const SessEntry E = A.ent[e];
     SessSlot &S = A.slots[E.slot];
@@ -71,12 +101,12 @@ __global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(S
     }
     if (S.settled || E.len <= 0) return;
     const int n0 = S.n, n1 = n0 + E.len;
-    int16_t *cache = A.cache + (size_t)E.slot * A.max_samples;
+    T *cache = A.cache + (size_t)E.slot * A.max_samples;
     uint32_t lo = 0xffffffffu, hi = 0u;
     for (int j = lane; j < E.len; j += 32) {
-        const int16_t v = A.blob[E.src + j];
+        const T v = A.blob[E.src + j];
         cache[n0 + j] = v;
-        const uint32_t k = (uint32_t)((int)v + 32768);
+        const uint32_t k = X::key(v);
         lo = min(lo, k);
         hi = max(hi, k);
     }
@@ -91,7 +121,7 @@ __global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(S
     int i = S.t;
     if (L <= i) return;
     const float coff = S.coff, cscale = S.cscale;
-    auto pa = [&](int j) { return __fmul_rn(__fadd_rn((float)cache[j], coff), cscale); };
+    auto pa = [&](int j) { return X::pa(cache[j], coff, cscale); };
     float amean = S.amean, assqdm = S.assqdm, asum = S.asum, mv = 0.f, mm = 0.f;
     const float vinv = (float)(1.0 / (double)wv), minv = (float)(1.0 / (double)wm);
     const int i0 = max(wv, wm) - 1;
@@ -121,7 +151,16 @@ __global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(S
     S.amean = amean; S.assqdm = assqdm; S.asum = asum;
 }
 
-__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs A, adb_stream_config P) {
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(SessArgs A, adb_stream_config P) {
+    sess_append(A, P, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_f32_kernel(SessArgsF32 A, adb_stream_config P) {
+    sess_append(A, P, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+
+template <class T>
+__device__ __forceinline__ void sess_search(SessArgsT<T> A, adb_stream_config P) {
+    using X = SessSample<T>;
     __shared__ __align__(16) unsigned char scratch[((size_t)ADB_SEL_SMEM_BYTES + 64 + 15) & ~(size_t)15];
     __shared__ uint32_t kbuf[8];
     __shared__ int itmp[8];
@@ -147,15 +186,14 @@ __global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs
         C.series_a = C.series_b = nullptr;
         C.pre_var = C.pre_mean = nullptr;
         C.pre_ae = C.pre_pe = -1;
-        C.src.f32 = nullptr;
-        C.src.i16 = A.cache + (size_t)E.slot * A.max_samples;
+        X::src(C.src, A.cache + (size_t)E.slot * A.max_samples);
         C.src.n = n;
         C.src.coff = S.coff;
         C.src.cscale = S.cscale;
-        C.int_keys = true;  // the session only takes scale > 0
+        C.int_keys = X::int_keys;
         C.wkmin = S.kmin;
         C.wkmax = S.kmax;
-        const PaVal V{C.src, true};
+        const PaVal V{C.src, X::int_keys};
         C.wvmin = V(C.wkmin);
         C.wvmax = V(C.wkmax);
         const uint32_t *mask = A.mask + (size_t)E.slot * A.mask_words;
@@ -199,4 +237,9 @@ __global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs
         A.out[2 * e] = result;
         A.out[2 * e + 1] = settled;
     }
+}
+
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs A, adb_stream_config P) { sess_search(A, P); }
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_f32_kernel(SessArgsF32 A, adb_stream_config P) {
+    sess_search(A, P);
 }

@@ -1,14 +1,17 @@
 """Read-until sessions of the streaming poly(A) detector (mean_var_shift_polyA_detect, adapted/detect/mvs.py:341-426).
 
 A read-until client asks the detector again every time a channel delivers a chunk.  :class:`StreamSession` keeps the
-int16 cache of every channel on the GPU together with the detector's running state, so a push costs work for the
-appended samples, not for the whole cache, and its answers are exactly those of
-:func:`adapted_b200.detect.mean_var_shift_polyA_detect_i16` on the caches (include/adapted_b200.h,
-adapted_b200/csrc/adb_stream_session.cuh).
+cache of every channel on the GPU together with the detector's running state, so a push costs work for the appended
+samples, not for the whole cache.  The caches hold int16 ADC codes, calibrated per read, and the answers are exactly
+those of :func:`adapted_b200.detect.mean_var_shift_polyA_detect_i16` on them; or, with ``dtype=np.float32``,
+calibrated float32 pA, and the answers are exactly those of :func:`adapted_b200.detect.mean_var_shift_polyA_detect`
+(include/adapted_b200.h, adapted_b200/csrc/adb_stream_session.cuh).
 
     with StreamSession(StreamingConfig(), n_slots=512, max_samples=100_000) as s:
         start, settled = s.push([3, 7], [chunk3, chunk7], reset=[True, False], calib_offset=[-221.0, 0.0],
                                 calib_scale=[0.1755, 0.0])
+    with StreamSession(StreamingConfig(), n_slots=512, max_samples=100_000, dtype=np.float32) as s:
+        start, settled = s.push([3, 7], [pa3, pa7], reset=[True, False])
 """
 from __future__ import annotations
 
@@ -30,31 +33,47 @@ def resolve_stream_params(params: Any = None) -> Any:
     return StreamingConfig() if params is None else params
 
 
-def pack_chunks(slots: Sequence[int], chunks: Any) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
-    """(slots, chunks) -> (slots int32 [n], adc int16 [total], offsets int64 [n + 1]).
+SESSION_DTYPES = (np.dtype(np.int16), np.dtype(np.float32))
 
-    `chunks` is either a list of per-slot int16 arrays or an ``(adc, offsets)`` tuple with chunk k at
-    adc[offsets[k]:offsets[k + 1]].  Offsets must lie inside `adc`; their order is checked by the library."""
+
+def session_dtype(dtype: Any) -> np.dtype:
+    """np.int16 or np.float32 (any spelling numpy accepts) -> that dtype; anything else raises ValueError"""
+    try:
+        dt = np.dtype(dtype)
+    except TypeError:
+        dt = None
+    if dt not in SESSION_DTYPES:
+        raise ValueError(f"a session holds int16 ADC or float32 pA samples, not {dtype!r}")
+    return dt
+
+
+def pack_chunks(slots: Sequence[int], chunks: Any, dtype: Any = np.int16) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """(slots, chunks) -> (slots int32 [n], samples `dtype` [total], offsets int64 [n + 1]).
+
+    `chunks` is either a list of per-slot arrays or an ``(samples, offsets)`` tuple with chunk k at
+    samples[offsets[k]:offsets[k + 1]]; samples are cast to `dtype` (int16 ADC or float32 pA).  Offsets must lie
+    inside `samples`; their order is checked by the library."""
+    dt = session_dtype(dtype)
     sl = np.ascontiguousarray(np.asarray(slots).reshape(-1), dtype=np.int32)
     n = sl.size
     if isinstance(chunks, tuple):
         if len(chunks) != 2:
-            raise ValueError("chunks given as a tuple must be the pair (adc, offsets)")
-        adc = np.ascontiguousarray(np.asarray(chunks[0]).reshape(-1), dtype=np.int16)
+            raise ValueError("chunks given as a tuple must be the pair (samples, offsets)")
+        adc = np.ascontiguousarray(np.asarray(chunks[0]).reshape(-1), dtype=dt)
         offsets = np.ascontiguousarray(np.asarray(chunks[1]).reshape(-1), dtype=np.int64)
         if offsets.size != n + 1:
             raise ValueError(f"offsets must hold len(slots) + 1 = {n + 1} entries, got {offsets.size}")
         if n and (offsets.min() < 0 or offsets.max() > adc.size):
-            raise ValueError("chunk offsets must lie inside adc")
+            raise ValueError("chunk offsets must lie inside the samples")
         return sl, adc, offsets
-    parts = [np.ascontiguousarray(np.asarray(c).reshape(-1), dtype=np.int16) for c in chunks]
+    parts = [np.ascontiguousarray(np.asarray(c).reshape(-1), dtype=dt) for c in chunks]
     if len(parts) != n:
         raise ValueError(f"one chunk per slot: {n} slots, {len(parts)} chunks")
     offsets = np.zeros(n + 1, dtype=np.int64)
     if n:
         offsets[1:] = np.cumsum([p.size for p in parts])
-    adc = np.concatenate(parts) if n else np.zeros(0, np.int16)
-    return sl, np.ascontiguousarray(adc, dtype=np.int16), offsets
+    adc = np.concatenate(parts) if n else np.zeros(0, dt)
+    return sl, np.ascontiguousarray(adc, dtype=dt), offsets
 
 
 def _per_entry(values: Optional[Sequence], n: int, dtype) -> Optional[np.ndarray]:
@@ -65,41 +84,56 @@ def _per_entry(values: Optional[Sequence], n: int, dtype) -> Optional[np.ndarray
 
 
 class StreamSession:
-    """`n_slots` channels, each caching at most `max_samples` int16 samples of the read on it, on GPU `device`.
+    """`n_slots` channels, each caching at most `max_samples` samples of the read on it, on GPU `device`: int16 ADC
+    codes (`dtype` np.int16) or calibrated float32 pA (np.float32).
 
-    :meth:`push` appends one chunk to each of the given slots (after starting a new read on those marked in `reset`,
-    with that read's calibration pA = (float32(adc) + offset) * scale) and returns per slot the poly(A) start on its
-    whole cache (0: none yet) and whether that answer is final."""
+    :meth:`push` appends one chunk to each of the given slots (after starting a new read on those marked in `reset`;
+    an int16 read comes with its calibration pA = (float32(adc) + offset) * scale) and returns per slot the poly(A)
+    start on its whole cache (0: none yet) and whether that answer is final."""
 
-    def __init__(self, params: Any = None, n_slots: int = 512, max_samples: int = 100_000, device: int = 0):
+    def __init__(self, params: Any = None, n_slots: int = 512, max_samples: int = 100_000, device: int = 0,
+                 dtype: Any = np.int16):
         from .config import flatten_streaming_config
 
+        self._h = None
+        self.dtype = session_dtype(dtype)
         self.params = resolve_stream_params(params)
         self.n_slots, self.max_samples = int(n_slots), int(max_samples)
         self._cfg = _lib.fill_stream_config(flatten_streaming_config(self.params))
         self._ctx = _lib.default_context(device)
-        self._h = C.c_void_p()
-        _lib.check(_lib.load().adb_stream_session_create(self._ctx.handle, C.byref(self._cfg), self.n_slots,
-                                                         self.max_samples, C.byref(self._h)))
+        h = C.c_void_p()
+        lib = _lib.load()
+        create = lib.adb_stream_session_create_f32 if self.dtype == np.float32 else lib.adb_stream_session_create
+        _lib.check(create(self._ctx.handle, C.byref(self._cfg), self.n_slots, self.max_samples, C.byref(h)))
+        self._h = h
 
     def push(self, slots: Sequence[int], chunks: Any, reset: Optional[Sequence[bool]] = None,
              calib_offset: Optional[Sequence[float]] = None,
              calib_scale: Optional[Sequence[float]] = None) -> Tuple[np.ndarray, np.ndarray]:
         """-> (polya_start int32 [n], settled bool [n]) for the n pushed slots, in the order given.  A zero-length
         chunk returns the current answer.  Raises AdbError (the session stays usable) for a slot out of range or
-        twice in one push, decreasing offsets, an append to a slot never reset, or a bad calibration."""
+        twice in one push, decreasing offsets, an append to a slot never reset, a bad calibration, or a float32 sample
+        that is not finite.  A float32 session casts the chunks to float32 and takes no calibration (ValueError)."""
         if not self._h:
             raise ValueError("the session is closed")
-        sl, adc, offsets = pack_chunks(slots, chunks)
+        f32 = self.dtype == np.float32
+        if f32 and (calib_offset is not None or calib_scale is not None):
+            raise ValueError("a float32 session holds calibrated pA: calib_offset / calib_scale do not apply")
+        sl, samples, offsets = pack_chunks(slots, chunks, self.dtype)
         n = sl.size
         out = np.zeros(n, dtype=np.int32)
         done = np.zeros(n, dtype=np.uint8)
         rs = _per_entry(reset, n, np.uint8)
-        co = _per_entry(calib_offset, n, np.float32)
-        cs = _per_entry(calib_scale, n, np.float32)
         ptr = lambda a: None if a is None else a.ctypes.data  # noqa: E731
-        _lib.check(_lib.load().adb_stream_session_push(self._h, n, ptr(sl), ptr(offsets), ptr(adc), ptr(rs), ptr(co),
-                                                       ptr(cs), ptr(out), ptr(done)))
+        lib = _lib.load()
+        if f32:
+            _lib.check(lib.adb_stream_session_push_f32(self._h, n, ptr(sl), ptr(offsets), ptr(samples), ptr(rs),
+                                                       ptr(out), ptr(done)))
+        else:
+            co = _per_entry(calib_offset, n, np.float32)
+            cs = _per_entry(calib_scale, n, np.float32)
+            _lib.check(lib.adb_stream_session_push(self._h, n, ptr(sl), ptr(offsets), ptr(samples), ptr(rs), ptr(co),
+                                                   ptr(cs), ptr(out), ptr(done)))
         return out, done.astype(bool)
 
     def close(self) -> None:

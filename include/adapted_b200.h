@@ -299,6 +299,22 @@ void adb_stream_session_destroy(adb_stream_session *s);
 int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
                             const int16_t *adc, const uint8_t *reset, const float *calib_offset,
                             const float *calib_scale, int32_t *polya_start, uint8_t *settled);
+/*
+ * Float32 sessions: the same detector on caches of calibrated float32 pA, the input of mean_var_shift_polyA_detect
+ * itself (read-until clients that receive calibrated chunks).  polya_start[k] is exactly what
+ * adb_mvs_stream_detect_host returns on the slot's whole cache as ADB_SIG_F32; `settled` and the handling of settled
+ * reads and of max_samples are those of the int16 session.  adb_stream_session_destroy frees either kind.
+ */
+/* as adb_stream_session_create; the cache takes n_slots * max_samples * 4 bytes of device memory */
+int adb_stream_session_create_f32(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots, int32_t max_samples,
+                                  adb_stream_session **out);
+/* entry k: reset[k] != 0 starts a new read on slots[k] (cache emptied; no calibration), then
+ * pa[chunk_offsets[k] .. chunk_offsets[k+1]) is appended.  HOST buffers, synchronous.  ADB_ERR_ARG, with the session
+ * unchanged, for the errors of adb_stream_session_push, for a non-finite sample (NaN, +-inf) anywhere in the pushed
+ * chunks (also in chunks that are ignored or clipped), and for a float32 push on an int16 session;
+ * adb_stream_session_push refuses an int16 push on a float32 session the same way. */
+int adb_stream_session_push_f32(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                                const float *pa, const uint8_t *reset, int32_t *polya_start, uint8_t *settled);
 
 /* ---- result tables (SURVEY.md row f2) ---------------------------------------------------------------------- */
 /*
