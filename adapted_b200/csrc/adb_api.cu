@@ -98,7 +98,7 @@ extern "C" void adb_ctx_destroy(adb_ctx *c) {
     DevBuf *all[] = {&c->states, &c->hist, &c->series, &c->given, &c->status, &c->cnn_x, &c->cnn_act0,
                      &c->cnn_act1, &c->cnn_scores, &c->cnn_w, &c->cnn_aux, &c->cnn_post, &c->sp_rows, &c->h_signal, &c->h_offsets,
                      &c->h_lens, &c->h_coff, &c->h_cscale, &c->h_records, &c->h_misc, &c->h_misc2, &c->h_misc3,
-                     &c->gsb_plan, &c->gsb_hist, &c->gsb_tab, &c->gsb_bases, &c->gsb_active, &c->vf_done, &c->mvs_perm, &c->cnn_wtc, &c->cnn_a0t, &c->cnn_ct, &c->llr_cc};
+                     &c->gsb_plan, &c->gsb_hist, &c->gsb_tab, &c->gsb_bases, &c->gsb_active, &c->vf_done, &c->mvs_perm, &c->cnn_wtc, &c->cnn_a0t, &c->cnn_ct, &c->llr_cc, &c->val_cc};
     for (DevBuf *b : all) b->release();
     for (int k = 0; k < 2; k++) {
         DevBuf *pb[] = {&c->p_signal[k], &c->p_offsets[k], &c->p_lens[k], &c->p_coff[k], &c->p_cscale[k], &c->p_records[k], &c->p_status[k],
@@ -328,7 +328,10 @@ static int launch_llr_primary(adb_ctx *ctx, const BatchDev &B, const adb_config 
     A.ntopk = ntopk;
     A.batch_status = batch_status;
     size_t smem = trace_smem_bytes(A.nds_max, A.peak_cap, true);
-    if ((int)smem > ctx->max_smem_optin) { set_err("downscaled trace does not fit in shared memory"); return ADB_ERR_UNSUPPORTED; }
+    if ((int)smem > ctx->max_smem_optin) {
+        set_err("downscaled LLR trace of llr_primary_kernel does not fit in shared memory (max_obs_trace / downscale_factor too large)");
+        return ADB_ERR_UNSUPPORTED;
+    }
     CUDA_TRY(cudaFuncSetAttribute(llr_primary_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, llr_primary_kernel, ADB_TRACE_THREADS, smem));
@@ -362,9 +365,16 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
     if (mode == ADB_METHOD_CNN && cfg.fallback_to_llr_short_reads) trace_dims(cfg, B.m, &A.nds_max, &A.peak_cap);
     A.out = out;
     A.batch_status = batch_status;
-    size_t smem = validate_smem_bytes(A.win_bytes, A.nds_max, A.peak_cap);
-    if ((int)smem > ctx->max_smem_optin) {
-        set_err("preload window does not fit in shared memory (sig_preload_size too large for this build)");
+    A.hm_cc = nullptr;
+    // the read's window staged in shared memory where it fits next to the scratch; longer windows are read from global
+    // memory (win_bytes = 0), and the hail-mary trace keeps its prefix sums in global memory (a third of the
+    // trace's shared memory, so that several CTAs share an SM)
+    const bool staged = validate_smem_bytes(A.win_bytes, A.nds_max, A.peak_cap) <= (size_t)ctx->max_smem_optin;
+    if (!staged) A.win_bytes = 0;
+    const bool hm_ext = !staged && A.nds_max > 0;
+    const size_t smem = validate_smem_bytes(A.win_bytes, A.nds_max, A.peak_cap, hm_ext);
+    if (smem > (size_t)ctx->max_smem_optin) {
+        set_err("hail-mary trace of validate_kernel does not fit in shared memory (sig_preload_size / downscale_factor too large)");
         return ADB_ERR_UNSUPPORTED;
     }
     CUDA_TRY(cudaFuncSetAttribute(validate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -396,6 +406,10 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
     const size_t row = (size_t)B.m * sizeof(float);
     if (ctx->series.ensure((size_t)grid_max * 2 * row)) { set_err("cudaMalloc series"); return ADB_ERR_CUDA; }
     A.series = (float *)ctx->series.p;
+    if (hm_ext) {
+        if (ctx->val_cc.ensure(sizeof(double) * 2 * (size_t)A.nds_max * (size_t)grid_max)) { set_err("cudaMalloc hail-mary prefix sums"); return ADB_ERR_CUDA; }
+        A.hm_cc = (double *)ctx->val_cc.p;
+    }
     A.pre_var = A.pre_mean = nullptr;
     A.pre_off = nullptr;
     A.pre_meta = nullptr;
@@ -461,14 +475,18 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
     A.work_counter = nullptr;
     ctx->vf_last_reads = 0;
     if (B.sig_type == ADB_SIG_I16 && !ctx->opt_no_fast_validate && !overwrite) {
-        // int16 sources: counting-based validation (adb_vfast.cuh); what it leaves is picked up by validate_kernel
-        const size_t fsm = vfast_smem_bytes(A.win_bytes);
-        if ((int)fsm <= ctx->max_smem_optin) {
+        // int16 sources: counting-based validation (adb_vfast.cuh); what it leaves is picked up by validate_kernel.
+        // It stages the window (dynamic shared memory) next to its static scratch: both count against the limit.
+        const size_t fsm = vfast_smem_bytes(B.m * 2);
+        cudaFuncAttributes fa, ca;
+        CUDA_TRY(cudaFuncGetAttributes(&fa, validate_fast_kernel));
+        CUDA_TRY(cudaFuncGetAttributes(&ca, validate_cand_kernel));
+        if (fsm + std::max(fa.sharedSizeBytes, ca.sharedSizeBytes) <= (size_t)ctx->max_smem_optin) {
             if (ctx->vf_done.ensure((size_t)B.n_reads + 16)) { set_err("cudaMalloc done flags"); return ADB_ERR_CUDA; }
             CUDA_TRY(cudaMemsetAsync(ctx->vf_done.p, 0, (size_t)B.n_reads + 16, st));
             VfastArgs F;
             F.B = B; F.given = given; F.given_stride = given_stride; F.given_ntopk = given_ntopk; F.ntopk_per_read = ntopk_per_read;
-            F.mode = mode; F.win_bytes = A.win_bytes; F.out = out; F.batch_status = batch_status;
+            F.mode = mode; F.win_bytes = B.m * 2; F.out = out; F.batch_status = batch_status;
             F.pre_var = A.pre_var; F.pre_mean = A.pre_mean; F.pre_off = A.pre_off; F.pre_meta = A.pre_meta;
             F.series_med = series_med;
             F.done = (unsigned char *)ctx->vf_done.p;

@@ -464,13 +464,16 @@ struct FlatView {
     __device__ __forceinline__ long long size() const { return (long long)nr * Lout; }
 };
 
-#define CNN_PK_CAP 832  // >= Lout / 2 local maxima per row
+// Capacity of one row's peak list.  A local maximum's left edge i needs x[i-1] < x[i] and its plateau ends at
+// ia > i with x[ia] < x[i]; no left edge lies in (i, ia], so consecutive left edges are at least two apart and a row
+// of Lout scores lists at most ceil(Lout / 2) peaks.
+__host__ __device__ inline int cnn_peak_cap(int Lout) { return Lout / 2 + 8; }
 
 // pass A/B: local maxima (scipy _local_maxima_1d on the flattened minibatch array) whose LEFT EDGE lies in this row;
 // midpoints are flattened indices and may fall into a later row when a plateau crosses row boundaries.
-// One CTA (128 threads) per read.  pk_pos[r][CNN_PK_CAP] (flattened midpoint), pk_cnt[r].
+// One CTA (128 threads) per read.  pk_pos[r][pk_cap] (flattened midpoint), pk_cnt[r]; pk_cap = cnn_peak_cap(Lout).
 __global__ void __launch_bounds__(128) cnn_peaks_kernel(const float *scores, int Lout, int batch_size, int n_reads,
-                                                        long long *pk_pos, int *pk_cnt) {
+                                                        int pk_cap, long long *pk_pos, int *pk_cnt) {
     __shared__ int wcount[4];
     __shared__ int base_sh;
     const int r = blockIdx.x;
@@ -505,13 +508,13 @@ __global__ void __launch_bounds__(128) cnn_peaks_kernel(const float *scores, int
         for (int w = 0; w < (int)(threadIdx.x >> 5); w++) off += wcount[w];
         if (mid >= 0) {
             const int pos = off + __popc(m & ((1u << (threadIdx.x & 31)) - 1u));
-            if (pos < CNN_PK_CAP) pk_pos[(size_t)r * CNN_PK_CAP + pos] = mid;
+            pk_pos[(size_t)r * pk_cap + pos] = mid;
         }
         __syncthreads();
         if (threadIdx.x == 0) base_sh += wcount[0] + wcount[1] + wcount[2] + wcount[3];
         __syncthreads();
     }
-    if (threadIdx.x == 0) pk_cnt[r] = min(base_sh, CNN_PK_CAP);
+    if (threadIdx.x == 0) pk_cnt[r] = base_sh;
 }
 
 // distance filter + per-read top-k.  One CTA (128 threads) per read: gathers the peaks listed under rows r-1, r, r+1 of
@@ -519,126 +522,132 @@ __global__ void __launch_bounds__(128) cnn_peaks_kernel(const float *scores, int
 // spanning more than the neighbouring row do not occur), orders them by priority, runs scipy's greedy
 // _select_by_peak_distance, keeps the survivors whose midpoint lies in row r, sorts those by (-height, position)
 // and writes the first k positions (row-local).  cand[r][k] (0-padded), ncand[r].
-#define CNN_WS_CAP 2560
-#define CNN_WS_SORT 4096  // power of two >= CNN_WS_CAP
+// The working set holds up to three lists of pk_cap peaks: ws_cap = cnn_topk_ws_cap(pk_cap) entries of position,
+// height, compaction slot and state (CNN_WS_BYTES_PER_PEAK bytes each).  It lives in dynamic shared memory
+// (ws_glob == nullptr, one CTA per read) or, for windows whose working set does not fit there, in a slice of
+// ws_glob per CTA, the CTAs then striding over the reads.
+#define CNN_WS_BYTES_PER_PEAK 15
+__host__ __device__ inline int cnn_topk_ws_cap(int pk_cap) { return (3 * pk_cap + 15) & ~15; }
+__host__ __device__ inline size_t cnn_topk_ws_bytes(int ws_cap) { return (size_t)ws_cap * CNN_WS_BYTES_PER_PEAK; }
 __global__ void __launch_bounds__(128) cnn_topk_kernel(const float *scores, int Lout, int batch_size, int n_reads, int k,
-                                                       int dist, const long long *pk_pos, const int *pk_cnt, int *cand,
-                                                       int *ncand) {
-    __shared__ long long pos[CNN_WS_CAP];   // flattened positions, ascending
-    __shared__ float hgt[CNN_WS_CAP];
-    __shared__ unsigned short ord[CNN_WS_CAP];   // survivors of this row (compaction scratch)
-    __shared__ unsigned char keep[CNN_WS_CAP];   // 2 undecided, 1 kept, 0 removed
+                                                       int dist, int pk_cap, int ws_cap, unsigned char *ws_glob,
+                                                       const long long *pk_pos, const int *pk_cnt, int *cand, int *ncand) {
+    extern __shared__ __align__(16) unsigned char ws_smem[];
+    unsigned char *ws = ws_glob ? ws_glob + cnn_topk_ws_bytes(ws_cap) * blockIdx.x : ws_smem;
+    long long *pos = (long long *)ws;                                   // flattened positions, ascending
+    float *hgt = (float *)(pos + ws_cap);
+    unsigned short *ord = (unsigned short *)(hgt + ws_cap);             // survivors of this row (compaction scratch)
+    unsigned char *keep = (unsigned char *)(ord + ws_cap);              // 2 undecided, 1 kept, 0 removed
     __shared__ int n_sh;
-    const int r = blockIdx.x;
-    const int mb = r / batch_size;
-    FlatView V{scores, Lout, mb * batch_size, min(batch_size, n_reads - mb * batch_size)};
-    const int rl = r - V.r0;
-    // gather: the peaks of this row plus those of the neighbouring rows that can interact with them.  The distance
-    // suppression only propagates through consecutive peaks closer than `dist`, so from either end of the row the
-    // neighbour's list is followed only while its gaps stay below `dist` (usually not a single peak: the head of every
-    // row is the masked stretch in front of the adapter end).  Lists are ascending and rows consecutive, so the
-    // concatenation is ascending.
     __shared__ int take_sh[2];
-    const int c_mid = pk_cnt[r];
-    const long long lo = (long long)rl * Lout, hi = lo + Lout;
-    if (threadIdx.x == 0) {
-        int tl = 0, tr = 0;
-        const long long *pm = pk_pos + (size_t)r * CNN_PK_CAP;
-        long long first_pos = (c_mid > 0) ? pm[0] : 0x7fffffffffffffffLL, last_pos = (c_mid > 0) ? pm[c_mid - 1] : -1;
-        if (rl > 0) {
-            // trailing peaks of the previous row's list: a plateau that starts there can have its midpoint in this row
-            // (always taken); further back only while the gaps stay below dist
-            const long long *pl = pk_pos + (size_t)(r - 1) * CNN_PK_CAP;
-            const int cl = pk_cnt[r - 1];
-            long long nxt = first_pos;
-            while (tl < cl) {
-                const long long p = pl[cl - 1 - tl];
-                if (!(p >= lo || (dist > 0 && nxt != 0x7fffffffffffffffLL && nxt - p < dist))) break;
-                nxt = p; tl++;
-                if (last_pos < 0) last_pos = p;
+    for (int r = blockIdx.x; r < n_reads; r += gridDim.x) {
+        __syncthreads();  // the previous read's working set is consumed
+        const int mb = r / batch_size;
+        FlatView V{scores, Lout, mb * batch_size, min(batch_size, n_reads - mb * batch_size)};
+        const int rl = r - V.r0;
+        // gather: the peaks of this row plus those of the neighbouring rows that can interact with them.  The distance
+        // suppression only propagates through consecutive peaks closer than `dist`, so from either end of the row the
+        // neighbour's list is followed only while its gaps stay below `dist` (usually not a single peak: the head of every
+        // row is the masked stretch in front of the adapter end).  Lists are ascending and rows consecutive, so the
+        // concatenation is ascending.  Each part is at most one list: n <= 3 * pk_cap <= ws_cap.
+        const int c_mid = pk_cnt[r];
+        const long long lo = (long long)rl * Lout, hi = lo + Lout;
+        if (threadIdx.x == 0) {
+            int tl = 0, tr = 0;
+            const long long *pm = pk_pos + (size_t)r * pk_cap;
+            long long first_pos = (c_mid > 0) ? pm[0] : 0x7fffffffffffffffLL, last_pos = (c_mid > 0) ? pm[c_mid - 1] : -1;
+            if (rl > 0) {
+                // trailing peaks of the previous row's list: a plateau that starts there can have its midpoint in this row
+                // (always taken); further back only while the gaps stay below dist
+                const long long *pl = pk_pos + (size_t)(r - 1) * pk_cap;
+                const int cl = pk_cnt[r - 1];
+                long long nxt = first_pos;
+                while (tl < cl) {
+                    const long long p = pl[cl - 1 - tl];
+                    if (!(p >= lo || (dist > 0 && nxt != 0x7fffffffffffffffLL && nxt - p < dist))) break;
+                    nxt = p; tl++;
+                    if (last_pos < 0) last_pos = p;
+                }
             }
+            if (rl + 1 < V.nr && dist > 0 && last_pos >= 0) {
+                const long long *pr = pk_pos + (size_t)(r + 1) * pk_cap;
+                const int cr = pk_cnt[r + 1];
+                long long prv = last_pos;
+                while (tr < cr && pr[tr] - prv < dist) { prv = pr[tr]; tr++; }
+            }
+            take_sh[0] = tl; take_sh[1] = tr;
         }
-        if (rl + 1 < V.nr && dist > 0 && last_pos >= 0) {
-            const long long *pr = pk_pos + (size_t)(r + 1) * CNN_PK_CAP;
-            const int cr = pk_cnt[r + 1];
-            long long prv = last_pos;
-            while (tr < cr && pr[tr] - prv < dist) { prv = pr[tr]; tr++; }
-        }
-        take_sh[0] = tl; take_sh[1] = tr;
-    }
-    __syncthreads();
-    int n = 0;
-    for (int part = 0; part < 3; part++) {
-        const int rr = r - 1 + part;
-        int c, first;
-        if (part == 0) { c = take_sh[0]; first = (c > 0) ? pk_cnt[r - 1] - c : 0; }
-        else if (part == 1) { c = c_mid; first = 0; }
-        else { c = take_sh[1]; first = 0; }
-        for (int i = threadIdx.x; i < c; i += blockDim.x) {
-            if (n + i < CNN_WS_CAP) {
-                const long long p = pk_pos[(size_t)rr * CNN_PK_CAP + first + i];
+        __syncthreads();
+        int n = 0;
+        for (int part = 0; part < 3; part++) {
+            const int rr = r - 1 + part;
+            int c, first;
+            if (part == 0) { c = take_sh[0]; first = (c > 0) ? pk_cnt[r - 1] - c : 0; }
+            else if (part == 1) { c = c_mid; first = 0; }
+            else { c = take_sh[1]; first = 0; }
+            for (int i = threadIdx.x; i < c; i += blockDim.x) {
+                const long long p = pk_pos[(size_t)rr * pk_cap + first + i];
                 pos[n + i] = p;
                 hgt[n + i] = V.at(p);
                 keep[n + i] = 2;
             }
+            n += c;
         }
-        n = min(n + c, CNN_WS_CAP);
-    }
-    // priority order (np.argsort of the heights, stable: ties keep the lower index first; scipy walks it from the back):
-    // peak t has priority over peak i iff (height, index) of t is the larger pair.  Only peaks closer than `dist` are
-    // ever compared, so no sorted order is materialised.
-    auto over = [&](int t, int i) { const float ht = hgt[t], hi_ = hgt[i]; return (ht > hi_) || (ht == hi_ && t > i); };
-    __syncthreads();
-    // _select_by_peak_distance: in priority order a kept peak removes everything closer than `dist`; equivalently a peak
-    // is kept iff no KEPT peak of higher priority lies within the distance.  Resolved in parallel rounds: a peak
-    // decides once all its higher-priority neighbours have decided (the highest of every neighbourhood at once).
-    if (dist > 0) {
-        bool pending = true;
-        while (__syncthreads_or(pending)) {
-            pending = false;
-            unsigned char newst[(CNN_WS_CAP + 127) / 128];
-            int cnt = 0;
-            for (int i = threadIdx.x; i < n; i += blockDim.x, cnt++) {
-                unsigned char st = keep[i];
-                if (st == 2) {
-                    bool killed = false, wait = false;
-                    for (int t = i - 1; t >= 0 && pos[i] - pos[t] < dist; t--)
-                        if (over(t, i)) { const unsigned char s2 = keep[t]; killed |= (s2 == 1); wait |= (s2 == 2); }
-                    for (int t = i + 1; t < n && pos[t] - pos[i] < dist; t++)
-                        if (over(t, i)) { const unsigned char s2 = keep[t]; killed |= (s2 == 1); wait |= (s2 == 2); }
-                    if (killed) st = 0;
-                    else if (!wait) st = 1;
-                    else pending = true;
+        // priority order (np.argsort of the heights, stable: ties keep the lower index first; scipy walks it from the back):
+        // peak t has priority over peak i iff (height, index) of t is the larger pair.  Only peaks closer than `dist` are
+        // ever compared, so no sorted order is materialised.
+        auto over = [&](int t, int i) { const float ht = hgt[t], hi_ = hgt[i]; return (ht > hi_) || (ht == hi_ && t > i); };
+        __syncthreads();
+        // _select_by_peak_distance: in priority order a kept peak removes everything closer than `dist`; equivalently a peak
+        // is kept iff no KEPT peak of higher priority lies within the distance.  Resolved in parallel rounds: a peak
+        // decides once all its higher-priority neighbours have decided (the highest of every neighbourhood at once).
+        // A round reads the states in bits 0-1 and writes the new state of its own peaks into bits 2-3 (a peak's byte has
+        // one writer; readers mask), which become the state after the barrier.
+        if (dist > 0) {
+            bool pending = true;
+            while (__syncthreads_or(pending)) {
+                pending = false;
+                for (int i = threadIdx.x; i < n; i += blockDim.x) {
+                    unsigned char st = keep[i] & 3;
+                    if (st == 2) {
+                        bool killed = false, wait = false;
+                        for (int t = i - 1; t >= 0 && pos[i] - pos[t] < dist; t--)
+                            if (over(t, i)) { const unsigned char s2 = keep[t] & 3; killed |= (s2 == 1); wait |= (s2 == 2); }
+                        for (int t = i + 1; t < n && pos[t] - pos[i] < dist; t++)
+                            if (over(t, i)) { const unsigned char s2 = keep[t] & 3; killed |= (s2 == 1); wait |= (s2 == 2); }
+                        if (killed) st = 0;
+                        else if (!wait) st = 1;
+                        else pending = true;
+                    }
+                    keep[i] = (unsigned char)((keep[i] & 3) | (st << 2));
                 }
-                newst[cnt] = st;
+                __syncthreads();
+                for (int i = threadIdx.x; i < n; i += blockDim.x) keep[i] = keep[i] >> 2;
             }
-            __syncthreads();
-            cnt = 0;
-            for (int i = threadIdx.x; i < n; i += blockDim.x, cnt++) keep[i] = newst[cnt];
+        } else {
+            for (int i = threadIdx.x; i < n; i += blockDim.x) keep[i] = 1;
         }
-    } else {
-        for (int i = threadIdx.x; i < n; i += blockDim.x) keep[i] = 1;
-    }
-    __syncthreads();
-    // survivors in row r, best first: (-height, position); compacted, then ranked by counting among themselves
-    if (threadIdx.x == 0) n_sh = 0;
-    __syncthreads();
-    for (int i = threadIdx.x; i < n; i += blockDim.x)
-        if (keep[i] == 1 && pos[i] >= lo && pos[i] < hi) ord[atomicAdd(&n_sh, 1)] = (unsigned short)i;
-    __syncthreads();
-    const int ns = n_sh;
-    for (int a = threadIdx.x; a < ns; a += blockDim.x) {
-        const int i = ord[a];
-        const float h = hgt[i];
-        int rank = 0;
-        for (int b = 0; b < ns; b++) {
-            const int j = ord[b];
-            const float hj = hgt[j];
-            rank += (hj > h) || (hj == h && j < i);
+        __syncthreads();
+        // survivors in row r, best first: (-height, position); compacted, then ranked by counting among themselves
+        if (threadIdx.x == 0) n_sh = 0;
+        __syncthreads();
+        for (int i = threadIdx.x; i < n; i += blockDim.x)
+            if (keep[i] == 1 && pos[i] >= lo && pos[i] < hi) ord[atomicAdd(&n_sh, 1)] = (unsigned short)i;
+        __syncthreads();
+        const int ns = n_sh;
+        for (int a = threadIdx.x; a < ns; a += blockDim.x) {
+            const int i = ord[a];
+            const float h = hgt[i];
+            int rank = 0;
+            for (int b = 0; b < ns; b++) {
+                const int j = ord[b];
+                const float hj = hgt[j];
+                rank += (hj > h) || (hj == h && j < i);
+            }
+            if (rank < k) cand[(size_t)r * k + rank] = (int)(pos[i] - lo);
         }
-        if (rank < k) cand[(size_t)r * k + rank] = (int)(pos[i] - lo);
+        if (threadIdx.x == 0) ncand[r] = ns;
     }
-    if (threadIdx.x == 0) ncand[r] = ns;
 }
 
 // groups of candidates are assigned to rows in order of appearance (cnn.py:149-158): read r's candidates land in row
@@ -839,8 +848,15 @@ static int cnn_forward_dev(adb_ctx *ctx, const float *x, int n, const CnnDims &D
 static int cnn_primary_boundaries(adb_ctx *ctx, const BatchDev &B, const adb_config &cfg, const float *w_dev, int *given,
                                   cudaStream_t st) {
     const CnnDims D = cnn_dims(B.m, cfg.min_obs_adapter, cfg.downscale_factor);
-    if (D.Lx < CNN_K || D.Lout < 3 || D.Lout / 2 + 8 > CNN_PK_CAP) {
+    if (D.Lx < CNN_K || D.Lout < 3) {
         set_err("preload window outside the range supported by the CNN kernels");
+        return ADB_ERR_UNSUPPORTED;
+    }
+    const int pk_cap = cnn_peak_cap(D.Lout), ws_cap = cnn_topk_ws_cap(pk_cap);
+    if (ws_cap > 65536) {
+        // cnn_topk_kernel compacts the survivors by 16-bit working-set index (windows up to about 437 000 samples at
+        // downscale factor 10)
+        set_err("preload window too long for the 16-bit working-set indices of cnn_topk_kernel");
         return ADB_ERR_UNSUPPORTED;
     }
     const int n = B.n_reads, k = cfg.polya_cand_k;
@@ -868,15 +884,23 @@ static int cnn_primary_boundaries(adb_ctx *ctx, const BatchDev &B, const adb_con
     }
     int rc = cnn_forward_dev(ctx, x, n, D, w_dev, scores, st);
     if (rc) return rc;
-    // post-processing scratch: apos, ppos, pk_cnt, ncand [n] ints; cand [n][k]; pk_pos [n][CNN_PK_CAP] int64
+    // cnn_topk_kernel's working set: dynamic shared memory (one CTA per read) where it fits, else a slice of global
+    // scratch per CTA of a grid striding over the reads
+    const size_t ws_bytes = cnn_topk_ws_bytes(ws_cap);
+    const bool ws_in_smem = (int)(ws_bytes + 64) <= ctx->max_smem_optin;
+    const int topk_grid = ws_in_smem ? n : std::max(1, std::min(n, ctx->sm_count * 8));
+    // post-processing scratch: pk_pos [n][pk_cap] int64; apos, ppos, pk_cnt, ncand [n] ints; cand [n][k];
+    // [topk_grid] working sets (global variant only)
     const size_t ints = (size_t)n * (4 + std::max(k, 1));
-    if (ctx->cnn_post.ensure(sizeof(long long) * (size_t)n * CNN_PK_CAP + sizeof(int) * ints + 64)) {
+    const size_t ws_off = (sizeof(long long) * (size_t)n * pk_cap + sizeof(int) * ints + 15) & ~(size_t)15;
+    if (ctx->cnn_post.ensure(ws_off + (ws_in_smem ? 0 : ws_bytes * (size_t)topk_grid) + 64)) {
         set_err("cudaMalloc cnn post-processing");
         return ADB_ERR_CUDA;
     }
     long long *pk_pos = (long long *)ctx->cnn_post.p;
-    int *apos = (int *)(pk_pos + (size_t)n * CNN_PK_CAP), *ppos = apos + n, *pk_cnt = ppos + n, *ncand = pk_cnt + n;
+    int *apos = (int *)(pk_pos + (size_t)n * pk_cap), *ppos = apos + n, *pk_cnt = ppos + n, *ncand = pk_cnt + n;
     int *cand = ncand + n;
+    unsigned char *ws_glob = ws_in_smem ? nullptr : (unsigned char *)ctx->cnn_post.p + ws_off;
     const int nadp = (cfg.max_obs_adapter - cfg.min_obs_adapter) / cfg.downscale_factor;
     const int n_batches = (n + B.batch_size - 1) / B.batch_size;
     {
@@ -888,11 +912,14 @@ static int cnn_primary_boundaries(adb_ctx *ctx, const BatchDev &B, const adb_con
         CUDA_TRY(cudaMemsetAsync(cand, 0, sizeof(int) * (size_t)n * k, st));
         {
             KernelTimer t(ctx, 6, st);
-            cnn_peaks_kernel<<<n, 128, 0, st>>>(scores, D.Lout, B.batch_size, n, pk_pos, pk_cnt);
+            cnn_peaks_kernel<<<n, 128, 0, st>>>(scores, D.Lout, B.batch_size, n, pk_cap, pk_pos, pk_cnt);
         }
         {
             KernelTimer t(ctx, 6, st);
-            cnn_topk_kernel<<<n, 128, 0, st>>>(scores, D.Lout, B.batch_size, n, k, 5, pk_pos, pk_cnt, cand, ncand);
+            const size_t sm = ws_in_smem ? ws_bytes : 0;
+            if (ws_in_smem) CUDA_TRY(cudaFuncSetAttribute(cnn_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+            cnn_topk_kernel<<<topk_grid, 128, sm, st>>>(scores, D.Lout, B.batch_size, n, k, 5, pk_cap, ws_cap, ws_glob,
+                                                         pk_pos, pk_cnt, cand, ncand);
         }
         ctx->launches += 2;
     }

@@ -86,6 +86,7 @@ struct adb_ctx {
     int gsb_last_batches = 0;
     int opt_exact_gsel = 0;  // adb_ctx_set_option("exact_global_select"): always use the multi-pass select
     DevBuf cnn_x, cnn_act0, cnn_act1, cnn_scores, cnn_w, cnn_aux, cnn_post, sp_rows, cnn_wtc, cnn_a0t, cnn_ct;
+    DevBuf val_cc;  // hail-mary prefix sums of the unstaged validate_kernel: [grid][2][nds_max] doubles
     // staging for the *_host entry points
     DevBuf h_signal, h_offsets, h_lens, h_coff, h_cscale, h_records, h_misc, h_misc2, h_misc3;
 };

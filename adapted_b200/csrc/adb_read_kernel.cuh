@@ -10,7 +10,9 @@
 //                        a device array (LLR / CNN / start-peak primaries alike), plus the CNN path's "hail mary"
 //                        LLR fallback (combined.py:251-301).  The read's preload window is staged ONCE in shared
 //                        memory by the TMA bulk engine (cp.async.bulk + mbarrier) and every order statistic, moving
-//                        statistic and sum is computed from there.
+//                        statistic and sum is computed from there.  Windows too long for that (win_bytes == 0) are
+//                        read straight from global memory; shared memory then holds only the scratch, and the
+//                        hail-mary trace keeps its prefix sums in global memory.
 //
 // Primary boundaries travel between the two as int[n_reads][stride]: adapter_end, polya_end, top-k...,
 // with n_topk == -1 encoded as polya_end_topk = None.
@@ -255,8 +257,9 @@ struct ValidateArgs {
     int given_ntopk;      // entries per read when ntopk_per_read == nullptr (-1: None)
     const int *ntopk_per_read;  // optional per-read override (LLR: -1 / 1)
     int mode;             // ADB_METHOD_*
-    int win_bytes;        // capacity of the staged window (bytes)
+    int win_bytes;        // capacity of the staged window (bytes); 0: the window is read from global memory
     int nds_max, peak_cap;// hail-mary trace buffers (CNN mode only; 0 otherwise)
+    double *hm_cc;        // [gridDim.x][2][nds_max] hail-mary prefix sums in global memory (nullptr: in shared memory)
     adb_record *out;
     float *series;        // [gridDim.x][2][m]
     const int *batch_status;
@@ -271,26 +274,31 @@ struct ValidateArgs {
     int *work_counter;
 };
 
-__host__ __device__ inline size_t validate_smem_bytes(int win_bytes, int nds_max, int peak_cap) {
+// shared memory of validate_kernel: [window (+48)][scratch: select histogram | hail-mary trace buffers][small].
+// win_bytes == 0: no staged window; c_ext: the trace's prefix sums live in global memory.
+__host__ __device__ inline size_t validate_win_cap(int win_bytes) {
+    return win_bytes > 0 ? (((size_t)win_bytes + 48 + 15) & ~(size_t)15) : 0;
+}
+__host__ __device__ inline size_t validate_scratch_bytes(int nds_max, int peak_cap, bool c_ext) {
     size_t scratch = ADB_SEL_SMEM_BYTES + 64;
-    size_t tr = nds_max > 0 ? trace_smem_bytes(nds_max, peak_cap) : 0;
+    size_t tr = nds_max > 0 ? trace_smem_bytes(nds_max, peak_cap, c_ext) : 0;
     if (tr > scratch) scratch = tr;
-    scratch = (scratch + 15) & ~(size_t)15;
-    return (((size_t)win_bytes + 48 + 15) & ~(size_t)15) + scratch + 256;
+    return (scratch + 15) & ~(size_t)15;
+}
+__host__ __device__ inline size_t validate_smem_bytes(int win_bytes, int nds_max, int peak_cap, bool c_ext = false) {
+    return validate_win_cap(win_bytes) + validate_scratch_bytes(nds_max, peak_cap, c_ext) + 256;
 }
 
+// A.win_bytes > 0: the read's window is copied to shared memory first; 0: every reader works on the read in global
+// memory (the same plain loads; the staged copy keeps the source's 16-byte phase and nobody reads past the read's
+// samples, so the readers see the same data either way).  One kernel for both: a second instantiation would give the
+// large device functions two call sites and change how they are inlined.
 __global__ void __launch_bounds__(ADB_VAL_THREADS, 3) validate_kernel(ValidateArgs A, adb_config cfg) {
     extern __shared__ __align__(128) unsigned char smem[];
-    // layout: [window (+48)][scratch: select histogram | hail-mary trace buffers][small]
     unsigned char *winbuf = smem;
-    const size_t win_cap = (((size_t)A.win_bytes + 48 + 15) & ~(size_t)15);
-    unsigned char *scratch = smem + win_cap;
-    size_t scratch_sz = ADB_SEL_SMEM_BYTES + 64;
-    {
-        size_t tr = A.nds_max > 0 ? trace_smem_bytes(A.nds_max, A.peak_cap) : 0;
-        if (tr > scratch_sz) scratch_sz = tr;
-        scratch_sz = (scratch_sz + 15) & ~(size_t)15;
-    }
+    unsigned char *scratch = smem + validate_win_cap(A.win_bytes);
+    const bool c_ext = A.hm_cc != nullptr;
+    const size_t scratch_sz = validate_scratch_bytes(A.nds_max, A.peak_cap, c_ext);
     unsigned char *small = scratch + scratch_sz;
     uint32_t *kbuf = (uint32_t *)small;          // 8 words
     int *itmp = (int *)(small + 32);             // 8 ints
@@ -343,7 +351,7 @@ __global__ void __launch_bounds__(ADB_VAL_THREADS, 3) validate_kernel(ValidateAr
         const int full_len = A.B.full_lens[r];
         // ---- stage the preload window in shared memory (TMA bulk copy) ----
         ReadSrc src = gsrc;
-        {
+        if (A.win_bytes > 0) {
             const int esz = gsrc.f32 ? 4 : 2;
             const unsigned char *g = gsrc.f32 ? (const unsigned char *)gsrc.f32 : (const unsigned char *)gsrc.i16;
             unsigned char *w = cta_stage_window(winbuf, g, gsrc.n * esz, bar, phase);
@@ -403,7 +411,8 @@ __global__ void __launch_bounds__(ADB_VAL_THREADS, 3) validate_kernel(ValidateAr
                     continue;
                 }
                 __syncthreads();
-                const TraceScratch T = trace_scratch_from(scratch, A.nds_max, A.peak_cap);
+                const TraceScratch T = trace_scratch_from(scratch, A.nds_max, A.peak_cap,
+                                                          c_ext ? A.hm_cc + (size_t)blockIdx.x * 2 * A.nds_max : nullptr);
                 float *ds = (float *)T.trace;
                 for (int b = threadIdx.x; b < nds; b += blockDim.x) {
                     const int j0 = sa + b * f;

@@ -14,7 +14,7 @@
 #define ADB_MAX_MEAN_WINDOW 65536
 
 struct ValCtx {
-    ReadSrc src;         // the read's preload window, STAGED IN SHARED MEMORY (pointers address smem)
+    ReadSrc src;         // the read's preload window: staged in shared memory, or the read in global memory
     const adb_config *cfg;
     SelScratch S;
     uint32_t *kbuf;      // shared: 4 keys + 4 ranks

@@ -180,6 +180,13 @@ typedef struct adb_batch {
  * 0.weight[64,1,7] 0.bias[64] 2.weight[64,64,7] 2.bias[64] 4.weight[64,64,7] 4.bias[64] 6.weight[64,2,7] 6.bias[2]
  * (58 882 floats, adapted/detect/cnn.py:16-52).  `batch_status` (optional, [n_batches]) receives the per-minibatch
  * adb_status (where the reference raises outside its per-read try and loses the minibatch).
+ * Supported preload windows (batch->m = sig_preload_size): any m up to 131 072 samples, for ADB_SIG_I16 and
+ * ADB_SIG_F32 alike, here and in adb_detect_dev, adb_detect_pipelined_host, adb_detect_pipelined_svb_host and
+ * adb_detect_files.  Windows too long for a kernel's shared-memory layout take a variant that reads the signal from
+ * global memory (same records).  Ceilings that remain return ADB_ERR_UNSUPPORTED with adb_last_error() naming them:
+ * the 16-bit working-set indices of the CNN top-k (about 437 000 samples at downscale factor 10), the CNN path's
+ * hail-mary LLR trace and the LLR primary trace in shared memory (both above about 21 000 downscaled points, i.e.
+ * m / downscale_factor; far above 131 072 samples at the shipped downscale factors).
  */
 int adb_detect_host(adb_ctx *ctx, const adb_batch *batch, const adb_config *cfg, const float *cnn_weights,
                     adb_record *out_records, int32_t *batch_status);
