@@ -164,6 +164,13 @@ def load() -> C.CDLL:
     L.adb_stream_session_create_f32.restype = ip
     L.adb_stream_session_push_f32.argtypes = [vp, C.c_int32, vp, vp, vp, vp, vp, vp]
     L.adb_stream_session_push_f32.restype = ip
+    L.adb_stream_session_create_dev.argtypes = [vp, C.POINTER(AdbStreamConfig), C.c_int32, C.c_int32, C.c_int32,
+                                                C.POINTER(vp)]
+    L.adb_stream_session_create_dev.restype = ip
+    L.adb_stream_session_push_dev.argtypes = [vp, C.c_int32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.adb_stream_session_push_dev.restype = ip
+    L.adb_stream_session_reason.argtypes = [C.c_int32]
+    L.adb_stream_session_reason.restype = C.c_char_p
     L.adb_format_csv.argtypes = [vp, vp, C.c_int32, vp, C.c_int32, C.c_char_p, C.c_int32, vp, C.c_int64]
     L.adb_format_csv.restype = C.c_int64
     L.adb_format_csv_ex.argtypes = [vp, vp, C.c_int32, vp, C.c_int32, C.c_char_p, C.c_int32, vp, vp, vp, vp, C.c_int64]

@@ -900,8 +900,12 @@ struct adb_stream_session {
     adb_ctx *ctx = nullptr;
     adb_stream_config cfg;
     bool f32 = false;  // the caches hold calibrated float32 pA (else int16 ADC codes)
+    bool dev = false;  // pushes come from device memory (adb_stream_session_push_dev)
     int n_slots = 0, max_samples = 0, mask_words = 0;
     DevBuf slots, cache, mask, stage;  // stage: one push's entries, chunks and answers
+    DevBuf dstate;                     // device pushes: SessDev arrays and the answers of sess_search
+    SessDev D{};
+    int32_t *dout = nullptr;
     void *pin = nullptr;               // pinned mirror of `stage`
     size_t pin_cap = 0;
     // host mirror per slot: samples cached, a read was started, last answer, settled; stamp: duplicate check of a push
@@ -911,7 +915,7 @@ struct adb_stream_session {
 };
 
 static int session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots, int32_t max_samples, bool f32,
-                          adb_stream_session **out) {
+                          bool dev, adb_stream_session **out) {
     if (!ctx || !cfg || !out) { set_err("null argument"); return ADB_ERR_ARG; }
     *out = nullptr;
     if (n_slots < 1 || max_samples < 1) { set_err("n_slots and max_samples must be positive"); return ADB_ERR_ARG; }
@@ -942,18 +946,52 @@ static int session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_
         set_err("cudaMemset stream session state");
         return ADB_ERR_CUDA;
     }
+    if (dev) {  // everything a device push needs, so that a push allocates nothing
+        s->dev = true;
+        const size_t ns = (size_t)n_slots;
+        const size_t o_out = sizeof(SessEntry) * ns, o_err = o_out + sizeof(int32_t) * 2 * ns,
+                     o_stamp = o_err + sizeof(unsigned long long), o_started = o_stamp + sizeof(uint32_t) * ns;
+        if (s->dstate.ensure(o_started + ns)) {
+            adb_stream_session_destroy(s);
+            set_err("cudaMalloc stream session arena");
+            return ADB_ERR_CUDA;
+        }
+        unsigned char *p = (unsigned char *)s->dstate.p;
+        s->D.ent = (SessEntry *)p;
+        s->dout = (int32_t *)(p + o_out);
+        s->D.err = (unsigned long long *)(p + o_err);
+        s->D.stamp = (uint32_t *)(p + o_stamp);
+        s->D.started = p + o_started;
+        s->D.n_slots = n_slots;
+        if (cudaMemsetAsync(s->D.stamp, 0xff, sizeof(uint32_t) * ns, ctx->stream) != cudaSuccess ||
+            cudaMemsetAsync(s->D.started, 0, ns, ctx->stream) != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+            adb_stream_session_destroy(s);
+            set_err("cudaMemset stream session state");
+            return ADB_ERR_CUDA;
+        }
+    }
     *out = s;
     return ADB_OK;
 }
 
 extern "C" int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
                                          int32_t max_samples, adb_stream_session **out) {
-    return session_create(ctx, cfg, n_slots, max_samples, false, out);
+    return session_create(ctx, cfg, n_slots, max_samples, false, false, out);
 }
 
 extern "C" int adb_stream_session_create_f32(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
                                              int32_t max_samples, adb_stream_session **out) {
-    return session_create(ctx, cfg, n_slots, max_samples, true, out);
+    return session_create(ctx, cfg, n_slots, max_samples, true, false, out);
+}
+
+extern "C" int adb_stream_session_create_dev(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots,
+                                             int32_t max_samples, int32_t sig_type, adb_stream_session **out) {
+    if (sig_type != ADB_SIG_I16 && sig_type != ADB_SIG_F32) {
+        if (out) *out = nullptr;
+        set_err("sig_type must be ADB_SIG_I16 or ADB_SIG_F32");
+        return ADB_ERR_ARG;
+    }
+    return session_create(ctx, cfg, n_slots, max_samples, sig_type == ADB_SIG_F32, true, out);
 }
 
 extern "C" void adb_stream_session_destroy(adb_stream_session *s) {
@@ -963,6 +1001,7 @@ extern "C" void adb_stream_session_destroy(adb_stream_session *s) {
     s->cache.release();
     s->mask.release();
     s->stage.release();
+    s->dstate.release();
     if (s->pin) cudaFreeHost(s->pin);
     delete s;
 }
@@ -1128,6 +1167,7 @@ extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const i
                                        const int16_t *adc, const uint8_t *reset, const float *calib_offset,
                                        const float *calib_scale, int32_t *polya_start, uint8_t *settled) {
     if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (s->dev) { set_err("host push on a device-push session"); return ADB_ERR_ARG; }
     if (s->f32) { set_err("int16 push on a float32 session"); return ADB_ERR_ARG; }
     return session_push(s, n, slots, chunk_offsets, adc, reset, calib_offset, calib_scale, polya_start, settled);
 }
@@ -1136,8 +1176,98 @@ extern "C" int adb_stream_session_push_f32(adb_stream_session *s, int32_t n, con
                                            const int64_t *chunk_offsets, const float *pa, const uint8_t *reset,
                                            int32_t *polya_start, uint8_t *settled) {
     if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (s->dev) { set_err("host push on a device-push session"); return ADB_ERR_ARG; }
     if (!s->f32) { set_err("float32 push on an int16 session"); return ADB_ERR_ARG; }
     return session_push(s, n, slots, chunk_offsets, pa, reset, nullptr, nullptr, polya_start, settled);
+}
+
+// the adb_last_error() text of each refusal of session_push, by SessReason
+static const char *const kSessReasonText[SESS_R_COUNT] = {
+    nullptr,
+    "chunk_offsets must be non-negative",
+    "chunk_offsets must be non-decreasing",
+    "null adc with non-empty chunks",
+    "null pa with non-empty chunks",
+    "slot out of range",
+    "the same slot twice in one push",
+    "a reset needs calib_offset and calib_scale",
+    "calibration scale must be finite and positive, offset finite",
+    "append to a slot that was never reset",
+    "non-finite pA sample",
+};
+
+extern "C" const char *adb_stream_session_reason(int32_t reason) {
+    return reason > SESS_R_NONE && reason < SESS_R_COUNT ? kSessReasonText[reason] : nullptr;
+}
+
+extern "C" int adb_stream_session_push_dev(adb_stream_session *s, int32_t n, const int32_t *slots,
+                                           const int64_t *chunk_offsets, const void *samples, const uint8_t *reset,
+                                           const float *calib_offset, const float *calib_scale, int32_t *polya_start,
+                                           uint8_t *settled, int32_t *status, void *cuda_stream) {
+    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (!s->dev) { set_err("device push on a host-push session"); return ADB_ERR_ARG; }
+    if (n > s->n_slots) { set_err("more entries than slots: a push names each slot at most once"); return ADB_ERR_ARG; }
+    if (!status || !chunk_offsets || (n > 0 && (!slots || !polya_start || !settled))) { set_err("null argument"); return ADB_ERR_ARG; }
+    if (s->f32 && (calib_offset || calib_scale)) { set_err("a float32 session takes no calibration"); return ADB_ERR_ARG; }
+    CUDA_TRY(cudaSetDevice(s->ctx->device));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    if (n == 0) {
+        CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(int32_t) * 2, st));
+        return ADB_OK;
+    }
+    SessPush Q;
+    Q.slots = slots;
+    Q.offs = chunk_offsets;
+    Q.samples = samples;
+    Q.reset = reset;
+    Q.coff = calib_offset;
+    Q.cscale = calib_scale;
+    Q.polya_start = polya_start;
+    Q.settled = settled;
+    Q.status = status;
+    Q.n = n;
+    const int eblocks = (n + SESS_DEV_THREADS - 1) / SESS_DEV_THREADS;
+    // float32: enough CTAs for the finiteness scan, whose length only the device knows
+    const int cblocks = s->f32 ? std::max(eblocks, 4 * s->ctx->sm_count) : eblocks;
+    const int ablocks = (n + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS;
+    stream_dev_stamp_kernel<<<eblocks, SESS_DEV_THREADS, 0, st>>>(Q, s->D);
+    CUDA_TRY(cudaGetLastError());
+    if (!s->f32) {
+        SessArgs A;
+        A.slots = (SessSlot *)s->slots.p;
+        A.cache = (int16_t *)s->cache.p;
+        A.mask = (uint32_t *)s->mask.p;
+        A.ent = s->D.ent;
+        A.blob = (const int16_t *)samples;
+        A.out = s->dout;
+        A.n_ent = n;
+        A.max_samples = s->max_samples;
+        A.mask_words = s->mask_words;
+        stream_dev_check_kernel<<<cblocks, SESS_DEV_THREADS, 0, st>>>(A, Q, s->D);
+        CUDA_TRY(cudaGetLastError());
+        stream_append_dev_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg, s->D);
+        CUDA_TRY(cudaGetLastError());
+        stream_search_dev_kernel<<<n, ADB_VAL_THREADS, 0, st>>>(A, s->cfg, s->D, Q);
+    } else {
+        SessArgsF32 A;
+        A.slots = (SessSlot *)s->slots.p;
+        A.cache = (float *)s->cache.p;
+        A.mask = (uint32_t *)s->mask.p;
+        A.ent = s->D.ent;
+        A.blob = (const float *)samples;
+        A.out = s->dout;
+        A.n_ent = n;
+        A.max_samples = s->max_samples;
+        A.mask_words = s->mask_words;
+        stream_dev_check_f32_kernel<<<cblocks, SESS_DEV_THREADS, 0, st>>>(A, Q, s->D);
+        CUDA_TRY(cudaGetLastError());
+        stream_append_dev_f32_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg, s->D);
+        CUDA_TRY(cudaGetLastError());
+        stream_search_dev_f32_kernel<<<n, ADB_VAL_THREADS, 0, st>>>(A, s->cfg, s->D, Q);
+    }
+    CUDA_TRY(cudaGetLastError());
+    s->ctx->launches += 4;
+    return ADB_OK;
 }
 
 // ---- CNN scores (kernel-level test entry) ------------------------------------------------------------------------

@@ -26,6 +26,11 @@
 // shared memory).  Float32 sessions run stream_append_f32_kernel / stream_search_f32_kernel: the same code
 // (sess_append / sess_search) with the samples taken as they are, and order statistics on float keys through the
 // generic multi-level select instead of the one-pass code histogram.
+//
+// Device pushes (adb_stream_session_push_dev) take entries and chunks in device memory and run on the caller's stream
+// with no host synchronise: stream_dev_stamp_kernel and stream_dev_check_kernel validate the whole push and build the
+// entries before any state changes, then stream_append_dev_kernel / stream_search_dev_kernel run sess_append /
+// sess_search on the caller's buffer unless the push was refused, and write the answers and the status.
 #pragma once
 #include "adb_stream.cuh"
 
@@ -40,9 +45,9 @@ struct SessSlot {  // device state of one slot
     float amean, assqdm, asum;
 };
 
-struct SessEntry {  // one pushed slot, host -> device
+struct SessEntry {  // one pushed slot, host -> device (device pushes: built by stream_dev_check_kernel)
     int32_t slot, reset, len, _pad;
-    int64_t src;      // first sample of the chunk in the staged blob
+    int64_t src;      // first sample of the chunk in the staged blob (device pushes: in the caller's buffer)
     float coff, cscale;
 };
 
@@ -242,4 +247,167 @@ __device__ __forceinline__ void sess_search(SessArgsT<T> A, adb_stream_config P)
 __global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs A, adb_stream_config P) { sess_search(A, P); }
 __global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_f32_kernel(SessArgsF32 A, adb_stream_config P) {
     sess_search(A, P);
+}
+
+// ---- device pushes ----------------------------------------------------------------------------------------------
+// Refusals of a push, in the order the host push (session_push, adb_api.cu) checks them.  A refusal is recorded as the
+// key (phase << 40) | (entry << 8) | reason and the push keeps the smallest key, so the device reports the refusal the
+// host push would report first: the phase orders the host's passes, the entry its per-entry loop.
+enum SessReason : int32_t {
+    SESS_R_NONE = 0,
+    SESS_R_NEG_OFFSET,    // phase 0
+    SESS_R_DECREASING,    // phase 1, per entry
+    SESS_R_NULL_ADC,      // phase 2
+    SESS_R_NULL_PA,       // phase 2
+    SESS_R_SLOT_RANGE,    // phase 3, per entry, in this order
+    SESS_R_DUPLICATE,
+    SESS_R_NO_CALIB,
+    SESS_R_BAD_CALIB,
+    SESS_R_NOT_STARTED,
+    SESS_R_NON_FINITE,    // phase 4
+    SESS_R_COUNT
+};
+#define SESS_DEV_OK 0xffffffffffffffffull
+#define SESS_DEV_THREADS 256
+
+struct SessPush {  // the caller's arrays of one device push (device pointers)
+    const int32_t *slots;     // [n]
+    const int64_t *offs;      // [n + 1] chunk offsets into `samples`
+    const void *samples;      // int16 ADC or float32 pA, as the session holds
+    const uint8_t *reset;     // [n] or null
+    const float *coff, *cscale;  // [n] or null (int16 only)
+    int32_t *polya_start;     // [n]
+    uint8_t *settled;         // [n]
+    int32_t *status;          // [2]: adb_status, SessReason
+    int n;
+};
+
+struct SessDev {  // state of a device-push session next to SessSlot, and the scratch of one push
+    uint32_t *stamp;    // [n_slots] first entry of the running push that names the slot; 0xffffffff between pushes
+    uint8_t *started;   // [n_slots] a read was started on the slot by an accepted push
+    SessEntry *ent;     // [n_slots] entries of the running push
+    unsigned long long *err;  // smallest refusal key of the running push, SESS_DEV_OK if none
+    int n_slots;
+};
+
+__device__ __forceinline__ void sess_refuse(SessDev D, int phase, int k, int reason) {
+    atomicMin(D.err, ((unsigned long long)phase << 40) | ((unsigned long long)(uint32_t)k << 8) | (unsigned)reason);
+}
+__device__ __forceinline__ bool non_finite_f32(float v) { return (__float_as_uint(v) & 0x7f800000u) == 0x7f800000u; }
+
+// opens the push: clears its refusal key and stamps every slot named with the first entry naming it
+__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_stamp_kernel(SessPush Q, SessDev D) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) *D.err = SESS_DEV_OK;
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < Q.n; k += gridDim.x * blockDim.x) {
+        const int sl = Q.slots[k];
+        if (sl >= 0 && sl < D.n_slots) atomicMin(&D.stamp[sl], (uint32_t)k);
+    }
+}
+
+// Every check of the host push, and the entries from device state: entry k appends chunk k straight from the
+// caller's buffer (src = chunk_offsets[k]), clipped at max_samples; a settled slot that is not reset gets a
+// zero-length entry, for which sess_search returns the final answer.  Float32 sessions also scan every sample of
+// [chunk_offsets[0], chunk_offsets[n]) for NaN / inf, chunks of settled slots and clipped samples included.
+template <class T>
+__device__ __forceinline__ void sess_dev_check(SessArgsT<T> A, SessPush Q, SessDev D) {
+    constexpr bool f32 = !SessSample<T>::int_keys;
+    const int stride = gridDim.x * blockDim.x, tid = blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t o0 = Q.offs[0], o1 = Q.offs[Q.n];
+    if (tid == 0) {
+        if (o0 < 0) sess_refuse(D, 0, 0, SESS_R_NEG_OFFSET);
+        if (o1 > o0 && !Q.samples) sess_refuse(D, 2, 0, f32 ? SESS_R_NULL_PA : SESS_R_NULL_ADC);
+    }
+    for (int k = tid; k < Q.n; k += stride) {
+        const int64_t a = Q.offs[k], b = Q.offs[k + 1];
+        if (b < a) sess_refuse(D, 1, k, SESS_R_DECREASING);
+        const int sl = Q.slots[k];
+        const bool rs = Q.reset && Q.reset[k];
+        int r = SESS_R_NONE;
+        if (sl < 0 || sl >= D.n_slots) {
+            r = SESS_R_SLOT_RANGE;
+        } else if (D.stamp[sl] != (uint32_t)k) {  // reads k' < k, or the cleared stamp once entry k' is through
+            r = SESS_R_DUPLICATE;
+        } else {
+            D.stamp[sl] = 0xffffffffu;
+            if (rs) {
+                if (!f32) {
+                    if (!Q.coff || !Q.cscale) r = SESS_R_NO_CALIB;
+                    else if (!isfinite(Q.cscale[k]) || !(Q.cscale[k] > 0.f) || !isfinite(Q.coff[k])) r = SESS_R_BAD_CALIB;
+                }
+            } else if (!D.started[sl]) {
+                r = SESS_R_NOT_STARTED;
+            }
+        }
+        if (r != SESS_R_NONE) { sess_refuse(D, 3, k, r); continue; }
+        const SessSlot &S = A.slots[sl];
+        SessEntry E;
+        E.slot = sl;
+        E.reset = rs ? 1 : 0;
+        E._pad = 0;
+        E.src = a;
+        E.len = !rs && S.settled ? 0 : (int32_t)min(b - a, (int64_t)(A.max_samples - (rs ? 0 : S.n)));
+        E.coff = rs && !f32 ? Q.coff[k] : 0.f;
+        E.cscale = rs && !f32 ? Q.cscale[k] : 0.f;
+        D.ent[k] = E;
+    }
+    if (f32 && Q.samples && o0 >= 0 && o1 > o0) {  // block-uniform
+        const float *x = (const float *)Q.samples + o0;
+        const int64_t cnt = o1 - o0;
+        const int64_t head = min(cnt, (int64_t)(((16u - ((uint32_t)(uintptr_t)x & 15u)) & 15u) >> 2));
+        const int64_t nv = (cnt - head) >> 2;
+        const float4 *v = (const float4 *)(x + head);
+        bool bad = false;
+        for (int64_t j = tid; j < head; j += stride) bad |= non_finite_f32(x[j]);
+        for (int64_t j = tid; j < nv; j += stride) {
+            const float4 q = __ldg(v + j);
+            bad |= non_finite_f32(q.x) | non_finite_f32(q.y) | non_finite_f32(q.z) | non_finite_f32(q.w);
+        }
+        for (int64_t j = head + 4 * nv + tid; j < cnt; j += stride) bad |= non_finite_f32(x[j]);
+        if (__syncthreads_or(bad) && threadIdx.x == 0) sess_refuse(D, 4, 0, SESS_R_NON_FINITE);
+    }
+}
+
+__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_check_kernel(SessArgs A, SessPush Q, SessDev D) {
+    sess_dev_check(A, Q, D);
+}
+__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_check_f32_kernel(SessArgsF32 A, SessPush Q, SessDev D) {
+    sess_dev_check(A, Q, D);
+}
+
+template <class T>
+__device__ __forceinline__ void sess_append_dev(SessArgsT<T> A, adb_stream_config P, SessDev D, int e, int lane) {
+    if (*D.err != SESS_DEV_OK) return;  // refused: nothing changes
+    if (lane == 0 && e < A.n_ent && A.ent[e].reset) D.started[A.ent[e].slot] = 1;
+    sess_append(A, P, e, lane);
+}
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_dev_kernel(SessArgs A, adb_stream_config P, SessDev D) {
+    sess_append_dev(A, P, D, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_dev_f32_kernel(SessArgsF32 A, adb_stream_config P,
+                                                                                      SessDev D) {
+    sess_append_dev(A, P, D, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+}
+
+// closes the push: the status always, the answers only for an accepted push (a refused one leaves them untouched)
+template <class T>
+__device__ __forceinline__ void sess_search_dev(SessArgsT<T> A, adb_stream_config P, SessDev D, SessPush Q) {
+    const unsigned long long err = *D.err;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        Q.status[0] = err == SESS_DEV_OK ? ADB_OK : ADB_ERR_ARG;
+        Q.status[1] = err == SESS_DEV_OK ? SESS_R_NONE : (int32_t)(err & 0xffu);
+    }
+    if (err != SESS_DEV_OK) return;
+    sess_search(A, P);
+    if (threadIdx.x == 0) {  // sess_search wrote them from this thread
+        Q.polya_start[blockIdx.x] = A.out[2 * blockIdx.x];
+        Q.settled[blockIdx.x] = A.out[2 * blockIdx.x + 1] ? 1 : 0;
+    }
+}
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_dev_kernel(SessArgs A, adb_stream_config P, SessDev D,
+                                                                            SessPush Q) {
+    sess_search_dev(A, P, D, Q);
+}
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_dev_f32_kernel(SessArgsF32 A, adb_stream_config P,
+                                                                                SessDev D, SessPush Q) {
+    sess_search_dev(A, P, D, Q);
 }

@@ -12,6 +12,9 @@ calibrated float32 pA, and the answers are exactly those of :func:`adapted_b200.
                                 calib_scale=[0.1755, 0.0])
     with StreamSession(StreamingConfig(), n_slots=512, max_samples=100_000, dtype=np.float32) as s:
         start, settled = s.push([3, 7], [pa3, pa7], reset=[True, False])
+
+A session created with ``device_push=True`` takes its pushes from CUDA tensors instead and enqueues them on a stream,
+without a host synchronise (:meth:`StreamSession.push_device`).
 """
 from __future__ import annotations
 
@@ -89,22 +92,33 @@ class StreamSession:
 
     :meth:`push` appends one chunk to each of the given slots (after starting a new read on those marked in `reset`;
     an int16 read comes with its calibration pA = (float32(adc) + offset) * scale) and returns per slot the poly(A)
-    start on its whole cache (0: none yet) and whether that answer is final."""
+    start on its whole cache (0: none yet) and whether that answer is final.
+
+    With `device_push` the session takes :meth:`push_device` instead: the same pushes from CUDA tensors, enqueued on a
+    stream, answers in CUDA tensors."""
 
     def __init__(self, params: Any = None, n_slots: int = 512, max_samples: int = 100_000, device: int = 0,
-                 dtype: Any = np.int16):
+                 dtype: Any = np.int16, device_push: bool = False):
         from .config import flatten_streaming_config
 
         self._h = None
         self.dtype = session_dtype(dtype)
+        self.device_push = bool(device_push)
+        self.device = int(device)
         self.params = resolve_stream_params(params)
         self.n_slots, self.max_samples = int(n_slots), int(max_samples)
         self._cfg = _lib.fill_stream_config(flatten_streaming_config(self.params))
         self._ctx = _lib.default_context(device)
         h = C.c_void_p()
         lib = _lib.load()
-        create = lib.adb_stream_session_create_f32 if self.dtype == np.float32 else lib.adb_stream_session_create
-        _lib.check(create(self._ctx.handle, C.byref(self._cfg), self.n_slots, self.max_samples, C.byref(h)))
+        f32 = self.dtype == np.float32
+        if self.device_push:
+            _lib.check(lib.adb_stream_session_create_dev(self._ctx.handle, C.byref(self._cfg), self.n_slots,
+                                                         self.max_samples, _lib.SIG_F32 if f32 else _lib.SIG_I16,
+                                                         C.byref(h)))
+        else:
+            create = lib.adb_stream_session_create_f32 if f32 else lib.adb_stream_session_create
+            _lib.check(create(self._ctx.handle, C.byref(self._cfg), self.n_slots, self.max_samples, C.byref(h)))
         self._h = h
 
     def push(self, slots: Sequence[int], chunks: Any, reset: Optional[Sequence[bool]] = None,
@@ -116,6 +130,8 @@ class StreamSession:
         that is not finite.  A float32 session casts the chunks to float32 and takes no calibration (ValueError)."""
         if not self._h:
             raise ValueError("the session is closed")
+        if self.device_push:
+            raise ValueError("a device-push session takes push_device(), not push()")
         f32 = self.dtype == np.float32
         if f32 and (calib_offset is not None or calib_scale is not None):
             raise ValueError("a float32 session holds calibrated pA: calib_offset / calib_scale do not apply")
@@ -135,6 +151,90 @@ class StreamSession:
             _lib.check(lib.adb_stream_session_push(self._h, n, ptr(sl), ptr(offsets), ptr(samples), ptr(rs), ptr(co),
                                                    ptr(cs), ptr(out), ptr(done)))
         return out, done.astype(bool)
+
+    def push_device(self, slots: Any, chunk_offsets: Any, samples: Any, reset: Any = None, calib_offset: Any = None,
+                    calib_scale: Any = None, stream: Any = None, out: Any = None) -> Tuple[Any, Any, Any]:
+        """:meth:`push` from CUDA tensors on the session's device, enqueued on `stream` (torch's current stream by
+        default) with no host synchronise -> (polya_start int32 [n], settled bool [n], status int32 [2]), CUDA tensors
+        written in stream order.
+
+        slots int32 [n]; chunk_offsets int64 [n + 1], chunk k is samples[chunk_offsets[k]:chunk_offsets[k + 1]];
+        samples int16 ADC or float32 pA as the session holds, 1-D; reset bool or uint8 [n] (None: no entry resets);
+        calib_offset / calib_scale float32 [n] (int16 sessions only).  All contiguous.  `out` optionally gives the
+        three output tensors to write instead of new ones.
+
+        The data is checked on the device: status is {0, 0} for an accepted push, {-2, reason} for one the host push
+        would refuse, which then changes neither the session nor polya_start / settled (see
+        :meth:`raise_for_status`).  Arguments of the wrong dtype, device, layout or shape raise ValueError before
+        anything is enqueued."""
+        import torch
+
+        if not self._h:
+            raise ValueError("the session is closed")
+        if not self.device_push:
+            raise ValueError("push_device() needs a session created with device_push=True")
+        f32 = self.dtype == np.float32
+        if f32 and (calib_offset is not None or calib_scale is not None):
+            raise ValueError("a float32 session holds calibrated pA: calib_offset / calib_scale do not apply")
+        dev = torch.device("cuda", self.device)
+        given = []
+
+        def arg(t, name, dtypes, size=None):
+            if t is None:
+                return
+            if not isinstance(t, torch.Tensor):
+                raise ValueError(f"{name} must be a torch tensor, got {type(t).__name__}")
+            if t.dtype not in dtypes:
+                raise ValueError(f"{name} must be {' or '.join(str(d) for d in dtypes)}, got {t.dtype}")
+            if t.dim() != 1 or (size is not None and t.numel() != size):
+                want = f"[{size}]" if size is not None else "1-D"
+                raise ValueError(f"{name} must have shape {want}, got {list(t.shape)}")
+            if not t.is_contiguous():
+                raise ValueError(f"{name} must be contiguous")
+            given.append((name, t))
+
+        if slots is None or chunk_offsets is None or samples is None:
+            raise ValueError("slots, chunk_offsets and samples are required")
+        arg(slots, "slots", (torch.int32,))
+        n = slots.numel()
+        if n > self.n_slots:
+            raise ValueError(f"{n} entries for {self.n_slots} slots: a push names each slot at most once")
+        arg(chunk_offsets, "chunk_offsets", (torch.int64,), n + 1)
+        arg(samples, "samples", (torch.float32,) if f32 else (torch.int16,))
+        arg(reset, "reset", (torch.uint8, torch.bool), n)
+        arg(calib_offset, "calib_offset", (torch.float32,), n)
+        arg(calib_scale, "calib_scale", (torch.float32,), n)
+        if out is not None:
+            if len(out) != 3:
+                raise ValueError("out must be the three tensors (polya_start, settled, status)")
+            arg(out[0], "polya_start", (torch.int32,), n)
+            arg(out[1], "settled", (torch.bool, torch.uint8), n)
+            arg(out[2], "status", (torch.int32,), 2)
+        for name, t in given:
+            if t.device != dev:
+                raise ValueError(f"{name} must be on {dev}, got {t.device}")
+        if out is None:
+            out = (torch.empty(n, dtype=torch.int32, device=dev), torch.empty(n, dtype=torch.bool, device=dev),
+                   torch.empty(2, dtype=torch.int32, device=dev))
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        ptr = lambda t: None if t is None or t.numel() == 0 else t.data_ptr()  # noqa: E731
+        _lib.check(_lib.load().adb_stream_session_push_dev(
+            self._h, n, ptr(slots), ptr(chunk_offsets), ptr(samples), ptr(reset), ptr(calib_offset), ptr(calib_scale),
+            ptr(out[0]), ptr(out[1]), ptr(out[2]), stream.cuda_stream))
+        return tuple(out)
+
+    @staticmethod
+    def raise_for_status(status: Any) -> None:
+        """Waits for the push that writes `status` (push_device's third result) and raises ValueError with the host
+        push's message if it was refused."""
+        import torch
+
+        torch.cuda.synchronize(status.device)  # the push may have run on any stream
+        code, reason = (int(v) for v in status.cpu())
+        if code != 0:
+            text = _lib.load().adb_stream_session_reason(reason)
+            raise ValueError(text.decode() if text else f"push refused (status {code}, reason {reason})")
 
     def close(self) -> None:
         if getattr(self, "_h", None):

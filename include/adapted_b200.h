@@ -322,6 +322,37 @@ int adb_stream_session_create_f32(adb_ctx *ctx, const adb_stream_config *cfg, in
  * adb_stream_session_push refuses an int16 push on a float32 session the same way. */
 int adb_stream_session_push_f32(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
                                 const float *pa, const uint8_t *reset, int32_t *polya_start, uint8_t *settled);
+/*
+ * Device-push sessions: the same sessions for clients that hold their chunks on the GPU.  A push reads its entries and
+ * chunks from device memory and writes its answers to device memory; all its work is enqueued on the caller's stream,
+ * with no host synchronise and no allocation, so pushes overlap the caller's own kernels and can be captured in a
+ * CUDA graph.  Answers and refusals are exactly those of the host push.  Host pushes (adb_stream_session_push /
+ * _push_f32) refuse a device-push session, and adb_stream_session_push_dev refuses the other sessions.
+ */
+/* as adb_stream_session_create / _create_f32 with sig_type ADB_SIG_I16 / ADB_SIG_F32 (anything else: ADB_ERR_ARG).
+ * Allocates everything a push needs (cache, mask, slot state, and entry and validation scratch for n_slots entries);
+ * adb_stream_session_destroy frees it. */
+int adb_stream_session_create_dev(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots, int32_t max_samples,
+                                  int32_t sig_type, adb_stream_session **out);
+/*
+ * One push, every pointer a DEVICE pointer, asynchronous on `cuda_stream` (a cudaStream_t; NULL is CUDA's default
+ * stream).  The arguments mean what they mean for adb_stream_session_push / _push_f32: `samples` holds int16 ADC or
+ * float32 pA as the session does, at least chunk_offsets[n] of them; calib_offset / calib_scale are NULL for float32.
+ * polya_start (int32 [n]) and settled (uint8 [n]) receive what the host push returns, including the final answer of a
+ * settled slot.  status (int32 [2]) receives {adb_status, reason}: {ADB_OK, 0} for an accepted push, {ADB_ERR_ARG,
+ * reason} for a refused one, which changes neither the session nor polya_start / settled.
+ * adb_stream_session_reason(reason) is the text adb_last_error() gives for the same refusal of the host push.
+ * Everything that depends on the data is checked on the device, in stream order, before any state changes; the call
+ * itself returns ADB_ERR_ARG, enqueueing nothing, only for a null handle, status or array pointer, a session that is
+ * not a device-push session, n > n_slots (a valid push names each slot at most once), or a calibration given to a
+ * float32 session.  Pushes to one session must be ordered on the device (one stream, or events between streams).
+ */
+int adb_stream_session_push_dev(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                                const void *samples, const uint8_t *reset, const float *calib_offset,
+                                const float *calib_scale, int32_t *polya_start, uint8_t *settled, int32_t *status,
+                                void *cuda_stream);
+/* the text of a refusal reason of adb_stream_session_push_dev's status[1]; NULL for 0 and unknown codes */
+const char *adb_stream_session_reason(int32_t reason);
 
 /* ---- result tables (SURVEY.md row f2) ---------------------------------------------------------------------- */
 /*
