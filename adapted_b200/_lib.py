@@ -183,6 +183,10 @@ def load() -> C.CDLL:
     L.adb_svb16_decode_host.restype = ip
     L.adb_detect_pipelined_svb_host.argtypes = [vp, C.POINTER(AdbSvbBatch), C.POINTER(AdbConfig), vp, vp, vp, C.c_int32]
     L.adb_detect_pipelined_svb_host.restype = ip
+    L.adb_zstd_decompress_host.argtypes = [vp, vp, vp, C.c_int32, vp, vp, vp]
+    L.adb_zstd_decompress_host.restype = ip
+    L.adb_detect_pipelined_vbz_host.argtypes = [vp, C.POINTER(AdbSvbBatch), C.POINTER(AdbConfig), vp, vp, vp, C.c_int32]
+    L.adb_detect_pipelined_vbz_host.restype = ip
     L.adb_detect_files.argtypes = [vp, C.POINTER(AdbFileJob), C.POINTER(AdbConfig), vp, C.POINTER(AdbFileStats)]
     L.adb_detect_files.restype = ip
     for f in ("adb_detect_pipelined_host", "adb_ctx_set_timing", "adb_ctx_get_timing", "adb_ctx_create", "adb_detect_host", "adb_detect_dev", "adb_llr_trace_host",

@@ -98,11 +98,11 @@ extern "C" void adb_ctx_destroy(adb_ctx *c) {
     DevBuf *all[] = {&c->states, &c->hist, &c->series, &c->given, &c->status, &c->cnn_x, &c->cnn_act0,
                      &c->cnn_act1, &c->cnn_scores, &c->cnn_w, &c->cnn_aux, &c->cnn_post, &c->sp_rows, &c->h_signal, &c->h_offsets,
                      &c->h_lens, &c->h_coff, &c->h_cscale, &c->h_records, &c->h_misc, &c->h_misc2, &c->h_misc3,
-                     &c->gsb_plan, &c->gsb_hist, &c->gsb_tab, &c->gsb_bases, &c->gsb_active, &c->vf_done, &c->mvs_perm, &c->cnn_wtc, &c->cnn_a0t, &c->cnn_ct, &c->llr_cc, &c->val_cc};
+                     &c->gsb_plan, &c->gsb_hist, &c->gsb_tab, &c->gsb_bases, &c->gsb_active, &c->vf_done, &c->mvs_perm, &c->cnn_wtc, &c->cnn_a0t, &c->cnn_ct, &c->llr_cc, &c->val_cc, &c->z_fail};
     for (DevBuf *b : all) b->release();
     for (int k = 0; k < 2; k++) {
         DevBuf *pb[] = {&c->p_signal[k], &c->p_offsets[k], &c->p_lens[k], &c->p_coff[k], &c->p_cscale[k], &c->p_records[k], &c->p_status[k],
-                        &c->p_comp[k], &c->p_coffs[k], &c->p_nsamp[k]};
+                        &c->p_comp[k], &c->p_coffs[k], &c->p_nsamp[k], &c->p_frames[k], &c->p_foffs[k], &c->p_zstat[k]};
         for (DevBuf *b : pb) b->release();
         if (c->p_done[k]) cudaEventDestroy(c->p_done[k]);
         if (c->p_copied[k]) cudaEventDestroy(c->p_copied[k]);
@@ -123,6 +123,7 @@ extern "C" int adb_ctx_set_option(adb_ctx *c, const char *name, int value) {
     if (!strcmp(name, "cnn_fp32_pipe")) { c->opt_cnn_fp32 = value; return ADB_OK; }
     if (!strcmp(name, "pipeline_copy_only")) { c->opt_copy_only = value; return ADB_OK; }
     if (!strcmp(name, "no_cand_followup")) { c->opt_no_cand_followup = value; return ADB_OK; }
+    if (!strcmp(name, "host_zstd")) { c->opt_host_zstd = value; return ADB_OK; }
     set_err(std::string("unknown option: ") + name);
     return ADB_ERR_ARG;
 }
@@ -150,6 +151,7 @@ extern "C" int64_t adb_ctx_query(adb_ctx *c, const char *name) {
         for (unsigned char v : h) n += (v == 0);
         return n;
     }
+    if (!strcmp(name, "zstd_host_frames")) return c->zstd_host_frames;
     return -1;
 }
 

@@ -65,6 +65,8 @@ struct adb_ctx {
     // double-buffered staging for the pipelined host entry point
     DevBuf p_signal[2], p_offsets[2], p_lens[2], p_coff[2], p_cscale[2], p_records[2], p_status[2];
     DevBuf p_comp[2], p_coffs[2], p_nsamp[2];  // compressed ingest: svb16 streams, their offsets, samples per read
+    DevBuf p_frames[2], p_foffs[2], p_zstat[2];  // VBZ ingest: zstd frames, their offsets, per-frame status
+    DevBuf z_fail;                                 // VBZ ingest: frames the device refused (one counter per call)
     int opt_copy_only = 0;     // adb_ctx_set_option("pipeline_copy_only"): pipelined entry points skip the kernels
     // pinned slot ring of adb_detect_files, kept between calls (pinning gigabytes costs seconds)
     void *file_ring = nullptr;
@@ -84,7 +86,9 @@ struct adb_ctx {
     int opt_cnn_fp32 = 0;      // adb_ctx_set_option("cnn_fp32_pipe"): 64->64 convolutions on the FP32 pipe instead of tcgen05
     int vf_last_reads = 0;
     int gsb_last_batches = 0;
-    int opt_exact_gsel = 0;  // adb_ctx_set_option("exact_global_select"): always use the multi-pass select
+    int opt_exact_gsel = 0;
+    int opt_host_zstd = 0;        // adb_ctx_set_option("host_zstd"): adb_detect_files decompresses zstd frames on the host (A/B)
+    int64_t zstd_host_frames = 0;  // adb_ctx_query("zstd_host_frames"): frames the last call decompressed on the host  // adb_ctx_set_option("exact_global_select"): always use the multi-pass select
     DevBuf cnn_x, cnn_act0, cnn_act1, cnn_scores, cnn_w, cnn_aux, cnn_post, sp_rows, cnn_wtc, cnn_a0t, cnn_ct;
     DevBuf val_cc;  // hail-mary prefix sums of the unstaged validate_kernel: [grid][2][nds_max] doubles
     // staging for the *_host entry points

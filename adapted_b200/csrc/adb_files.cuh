@@ -142,14 +142,15 @@ struct Slot {
     // pinned host memory
     uint8_t *comp = nullptr;
     size_t comp_cap = 0;
-    int64_t *coffs = nullptr;
+    int64_t *coffs = nullptr, *foffs = nullptr;  // foffs: zstd frames of a device-decoded chunk
+    int32_t *zfail = nullptr;                     // frames of the chunk the device refused
     int32_t *nsamp = nullptr, *lens = nullptr, *src_file = nullptr, *src_read = nullptr, *status = nullptr;
     float *coff = nullptr, *cscale = nullptr;
     char *ids = nullptr;
     adb_record *recs = nullptr;
     int nr = 0, nb = 0;
-    size_t comp_bytes = 0;
-    int svb = 1;
+    size_t comp_bytes = 0, dec_bytes = 0;
+    int svb = 1;  // 0: raw int16, 1: svb16 streams, 2: zstd frames of svb16 streams (decoded on the device)
     bool last = false;
     int error = 0;
     cudaEvent_t done = nullptr;
@@ -175,7 +176,7 @@ static void file_ring_free(void *p) {
     FileRing *ring = (FileRing *)p;
     if (!ring) return;
     for (auto &s : ring->slots) {
-        void *ps[] = {s.comp, s.coffs, s.nsamp, s.lens, s.src_file, s.src_read, s.status, s.coff, s.cscale, s.ids, s.recs};
+        void *ps[] = {s.comp, s.coffs, s.foffs, s.zfail, s.nsamp, s.lens, s.src_file, s.src_read, s.status, s.coff, s.cscale, s.ids, s.recs};
         for (void *q : ps) if (q) cudaFreeHost(q);
         if (s.done) cudaEventDestroy(s.done);
     }
@@ -253,6 +254,8 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
             s.comp_cap = ring->comp_cap;
             if (cudaHostAlloc((void **)&s.comp, s.comp_cap, cudaHostAllocDefault) != cudaSuccess ||
                 cudaHostAlloc((void **)&s.coffs, sizeof(int64_t) * ((size_t)chunk_reads + 1), cudaHostAllocDefault) != cudaSuccess ||
+                cudaHostAlloc((void **)&s.foffs, sizeof(int64_t) * ((size_t)chunk_reads + 1), cudaHostAllocDefault) != cudaSuccess ||
+                cudaHostAlloc((void **)&s.zfail, sizeof(int32_t) * 4, cudaHostAllocDefault) != cudaSuccess ||
                 cudaHostAlloc((void **)&s.nsamp, sizeof(int32_t) * (size_t)chunk_reads, cudaHostAllocDefault) != cudaSuccess ||
                 cudaHostAlloc((void **)&s.lens, sizeof(int32_t) * (size_t)chunk_reads, cudaHostAllocDefault) != cudaSuccess ||
                 cudaHostAlloc((void **)&s.src_file, sizeof(int32_t) * (size_t)chunk_reads, cudaHostAllocDefault) != cudaSuccess ||
@@ -282,13 +285,14 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
         if (!failed.load()) { fail_msg = msg; failed.store(code); }
     };
     double read_s = 0.0, write_s = 0.0, gpu_wait_s = 0.0;
-    std::atomic<long long> comp_total{0};
+    std::atomic<long long> comp_total{0}, host_frames{0};
+    const bool device_zstd = !ctx->opt_host_zstd;
 
     // ---- reader ----
     std::thread reader([&]() {
         std::vector<CopyJob> jobs;
         Slot *s = q_free.pop();
-        s->nr = 0; s->comp_bytes = 0; s->last = false; s->error = 0;
+        s->nr = 0; s->comp_bytes = 0; s->dec_bytes = 0; s->last = false; s->error = 0;
         s->svb = 1;
         auto flush = [&](bool last) {
             const double t0 = now_s();
@@ -308,6 +312,7 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
                     if (k >= cut.size()) break;
                     const CopyJob &j = cut[k];
                     if (j.zstd) {
+                        host_frames++;
                         const size_t got = zstd.decompress(j.dst, j.dst_cap, j.src, j.bytes);
                         if (zstd.is_error(got) || got != j.dst_cap) fail(ADB_ERR_ARG, "zstd frame of a read does not decompress to its stated size");
                     } else {
@@ -321,13 +326,13 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
             work();
             for (auto &t : pool) t.join();
             jobs.clear();
-            if (s->svb) memset(s->comp + s->comp_bytes, 0, 16);  // the slack behind the last stream
+            if (s->svb == 1) memset(s->comp + s->comp_bytes, 0, 16);  // the slack behind the last stream
             comp_total += (long long)s->comp_bytes;
             read_s += now_s() - t0;
             q_filled.push(s);
             if (!last) {
                 s = q_free.pop();
-                s->nr = 0; s->comp_bytes = 0; s->last = false; s->error = 0; s->svb = 1;
+                s->nr = 0; s->comp_bytes = 0; s->dec_bytes = 0; s->last = false; s->error = 0; s->svb = 1;
             }
         };
         for (int fi = 0; fi < (int)files.size() && !failed.load(); fi++) {
@@ -337,14 +342,33 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
             const int idw = (int)f.h.id_width;
             for (int64_t r = 0; r < (int64_t)f.h.n_reads && !failed.load(); r++) {
                 if (keep && !keep[r]) continue;
-                if (s->nr > 0 && s->svb != (svb ? 1 : 0)) flush(false);  // a chunk holds one representation
-                s->svb = svb ? 1 : 0;
-                const int k = s->nr;
                 const int64_t o0 = f.coffs[r], o1 = f.coffs[r + 1];
+                if (o0 < 0 || o1 < o0 || (uint64_t)o1 > f.h.blob_bytes) { fail(ADB_ERR_ARG, "stream offsets outside the container blob"); break; }
                 int ns = std::min(f.nsamp[r], m);
                 size_t bytes = (size_t)(o1 - o0), dst_bytes = bytes;
                 const uint8_t *src = f.blob + o0;
-                if (o0 < 0 || o1 < o0 || (uint64_t)o1 > f.h.blob_bytes) { fail(ADB_ERR_ARG, "stream offsets outside the container blob"); break; }
+                // an svb16 stream in one zstd frame that the device takes travels as it is (no host decompression)
+                uint64_t zcs = 0;
+                const bool zdev = zs && svb && device_zstd && zstd_screen(src, bytes, per_read_cap * 4, &zcs);
+                const int rep = zdev ? 2 : (svb ? 1 : 0);
+                if (s->nr > 0 && s->svb != rep) flush(false);  // a chunk holds one representation
+                s->svb = rep;
+                const int k = s->nr;
+                if (zdev) {
+                    if (f.nsamp[r] > m) { fail(ADB_ERR_UNSUPPORTED, "compressed read longer than sig_preload_size in the container"); break; }
+                    const size_t dst_off = s->comp_bytes, dec_off = s->dec_bytes;
+                    if (dst_off + bytes + 32 > s->comp_cap) { fail(ADB_ERR_ARG, "a read's stream exceeds the worst-case size for its sample count"); break; }
+                    const bool extend = !jobs.empty() && !jobs.back().zstd && jobs.back().src + jobs.back().bytes == src &&
+                                        jobs.back().dst + jobs.back().bytes == s->comp + dst_off;
+                    if (extend) jobs.back().bytes += bytes;
+                    else jobs.push_back({src, s->comp + dst_off, bytes, bytes, false});
+                    s->foffs[k] = (int64_t)dst_off;
+                    s->comp_bytes = dst_off + bytes;
+                    s->foffs[k + 1] = (int64_t)s->comp_bytes;
+                    s->coffs[k] = (int64_t)dec_off;
+                    s->dec_bytes = dec_off + (size_t)((zcs + 15) & ~(uint64_t)15);
+                    s->coffs[k + 1] = (int64_t)s->dec_bytes;
+                } else {
                 if (zs) {
                     const unsigned long long cs = zstd.content_size(src, bytes);
                     if (cs == (unsigned long long)-1 || cs == (unsigned long long)-2 || cs > per_read_cap * 4) { fail(ADB_ERR_ARG, "zstd frame without a usable content size"); break; }
@@ -370,6 +394,7 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
                 s->coffs[k] = svb ? (int64_t)dst_off : (int64_t)(dst_off / 2);
                 s->comp_bytes = dst_off + dst_bytes;
                 s->coffs[k + 1] = svb ? (int64_t)((s->comp_bytes + 15) & ~(size_t)15) : (int64_t)(s->comp_bytes / 2);
+                }
                 s->nsamp[k] = ns;
                 s->lens[k] = f.lens[r];
                 s->coff[k] = f.coff[r];
@@ -469,6 +494,8 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
             if (s->nr > 0 && !s->error && cudaEventSynchronize(s->done) != cudaSuccess) fail(ADB_ERR_CUDA, "cudaEventSynchronize failed in the writer");
             gpu_wait_s += now_s() - t0;
             const double t1 = now_s();
+            if (!s->error && s->nr > 0 && s->svb == 2 && *s->zfail != 0)
+                fail(ADB_ERR_ARG, "zstd frame of a read does not decompress to its stated size");
             if (!s->error && !failed.load()) {
                 for (int b = 0; b < s->nb; b++) {
                     const int a = b * mbs, e = std::min(s->nr, a + mbs);
@@ -569,6 +596,7 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
                 if (ch >= 2) CUDA_TRY(cudaEventSynchronize(c->p_done[0]));
                 const size_t cbytes = s->comp_bytes + 16;
                 size_t dec_samples = 0;
+                // (the svb16 streams of a zstd chunk are laid out in p_comp after the zstd decode)
                 for (int i = 0; i < nr; i++) dec_samples += (size_t)s->nsamp[i];
                 if (c->p_comp[0].ensure(cbytes + 64) || c->p_coffs[0].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
                     c->p_nsamp[0].ensure(sizeof(int32_t) * (size_t)nr + 16) || c->p_signal[0].ensure(dec_samples * 2 + 64) ||
@@ -578,16 +606,38 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
                     set_err("cudaMalloc pipeline staging");
                     return ADB_ERR_CUDA;
                 }
-                void *sig_dst = s->svb ? c->p_comp[0].p : c->p_signal[0].p;
-                CUDA_TRY(cudaMemcpyAsync(sig_dst, s->comp, s->svb ? cbytes : s->comp_bytes, cudaMemcpyHostToDevice, cs));
-                CUDA_TRY(cudaMemcpyAsync(s->svb ? c->p_coffs[0].p : c->p_offsets[0].p, s->coffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
+                if (s->svb == 2) {  // zstd frames -> zstd_decode_kernel -> svb16 streams in p_comp
+                    if (c->p_frames[0].ensure(s->comp_bytes + 16) || c->p_foffs[0].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
+                        c->p_comp[0].ensure(s->dec_bytes + 64) || c->p_zstat[0].ensure(sizeof(int32_t) * (size_t)nr + 16) ||
+                        c->z_fail.ensure(16)) {
+                        set_err("cudaMalloc pipeline staging");
+                        return ADB_ERR_CUDA;
+                    }
+                    CUDA_TRY(cudaMemcpyAsync(c->p_frames[0].p, s->comp, s->comp_bytes, cudaMemcpyHostToDevice, cs));
+                    CUDA_TRY(cudaMemcpyAsync(c->p_foffs[0].p, s->foffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
+                    CUDA_TRY(cudaMemcpyAsync(c->p_coffs[0].p, s->coffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
+                    h2d_bytes += (long long)(s->comp_bytes + (size_t)nr * 8);
+                } else {
+                    void *sig_dst = s->svb ? c->p_comp[0].p : c->p_signal[0].p;
+                    CUDA_TRY(cudaMemcpyAsync(sig_dst, s->comp, s->svb ? cbytes : s->comp_bytes, cudaMemcpyHostToDevice, cs));
+                    CUDA_TRY(cudaMemcpyAsync(s->svb ? c->p_coffs[0].p : c->p_offsets[0].p, s->coffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
+                    h2d_bytes += (long long)cbytes;
+                }
                 CUDA_TRY(cudaMemcpyAsync(c->p_nsamp[0].p, s->nsamp, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
                 CUDA_TRY(cudaMemcpyAsync(c->p_lens[0].p, s->lens, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
                 CUDA_TRY(cudaMemcpyAsync(c->p_coff[0].p, s->coff, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
                 CUDA_TRY(cudaMemcpyAsync(c->p_cscale[0].p, s->cscale, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
                 CUDA_TRY(cudaEventRecord(c->p_copied[0], cs));
                 CUDA_TRY(cudaStreamWaitEvent(ks, c->p_copied[0], 0));
-                h2d_bytes += (long long)(cbytes + (size_t)nr * 28);
+                h2d_bytes += (long long)((size_t)nr * 28);
+                if (s->svb == 2) {
+                    CUDA_TRY(cudaMemsetAsync(c->z_fail.p, 0, sizeof(int32_t), ks));
+                    CUDA_TRY(cudaMemsetAsync((uint8_t *)c->p_comp[0].p + s->dec_bytes, 0, 16, ks));  // the slack behind the last stream
+                    int r1 = launch_zstd_decode(c, (const uint8_t *)c->p_frames[0].p, (const int64_t *)c->p_foffs[0].p, (uint8_t *)c->p_comp[0].p,
+                                                (const int64_t *)c->p_coffs[0].p, (int32_t *)c->p_zstat[0].p, (int32_t *)c->z_fail.p, nr, ks);
+                    if (r1) return r1;
+                    CUDA_TRY(cudaMemcpyAsync(s->zfail, c->z_fail.p, sizeof(int32_t), cudaMemcpyDeviceToHost, ks));
+                }
                 if (s->svb) {
                     int r2 = launch_svb_decode(c, (const uint8_t *)c->p_comp[0].p, (const int64_t *)c->p_coffs[0].p,
                                                (const int32_t *)c->p_nsamp[0].p, nr, (int64_t *)c->p_offsets[0].p,
@@ -626,6 +676,7 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
     stats->files = n_files.load();
     stats->comp_bytes = comp_total.load();
     stats->h2d_bytes = h2d_bytes;
+    ctx->zstd_host_frames = host_frames.load();
     stats->seconds = now_s() - t_start;
     stats->read_s = read_s;
     stats->gpu_wait_s = gpu_wait_s;

@@ -233,9 +233,42 @@ def svb16_decode(comp: np.ndarray, comp_offsets: np.ndarray, n_samples: np.ndarr
     return out, off
 
 
-def detect_reads_svb(comp: np.ndarray, comp_offsets: np.ndarray, n_samples: np.ndarray, full_lens: np.ndarray,
+def zstd_decompress(frames: np.ndarray, frame_offsets: np.ndarray, capacities: np.ndarray, device: int = 0):
+    """zstd decode on the GPU (adb_zstd_decompress_host): frame i = frames[frame_offsets[i]: frame_offsets[i + 1]]
+    decodes into a slot of capacities[i] bytes.  Returns (out uint8, status int32 [n]): slot i is
+    out[o[i]: o[i] + capacities[i]] with o the exclusive prefix sum of the capacities; status[i] is the decoded size or
+    a negative ADB_ZSTD_E_* code."""
+    frames = np.ascontiguousarray(frames, dtype=np.uint8)
+    foff = np.ascontiguousarray(frame_offsets, dtype=np.int64)
+    cap = np.ascontiguousarray(capacities, dtype=np.int64)
+    n = cap.size
+    if foff.size != n + 1 or (n and (foff[0] < 0 or np.any(foff[1:] < foff[:-1]) or foff[-1] > frames.size)) or np.any(cap < 0):
+        raise ValueError("frame_offsets must hold n + 1 non-decreasing offsets inside `frames`; capacities >= 0")
+    doff = np.zeros(n + 1, dtype=np.int64)
+    np.cumsum(cap, out=doff[1:])
+    out = np.zeros(int(doff[-1]), dtype=np.uint8)
+    status = np.zeros(n, dtype=np.int32)
+    if n == 0:
+        return out, status
+    ctx = _lib.default_context(device)
+    _lib.check(_lib.load().adb_zstd_decompress_host(ctx.handle, frames.ctypes.data, foff.ctypes.data, n, out.ctypes.data,
+                                                    doff.ctypes.data, status.ctypes.data))
+    return out, status
+
+
+def detect_reads_vbz(frames: np.ndarray, frame_offsets: np.ndarray, n_samples: np.ndarray, full_lens: np.ndarray,
                      calib_offset: np.ndarray, calib_scale: np.ndarray, spc: Any, model: Any = None,
                      minibatch_size: int = 1000, chunk_minibatches: int = 16, device: int = 0):
+    """VBZ ingest: one zstd frame per read over its svb16 stream (adapted_b200.svb16.vbz_encode_reads) travels to the
+    GPU as it is, is decoded there (zstd, then svb16) and detected (adb_detect_pipelined_vbz_host).  Returns
+    (records, batch_status), as detect_reads_svb does for the same reads."""
+    return detect_reads_svb(frames, frame_offsets, n_samples, full_lens, calib_offset, calib_scale, spc, model,
+                            minibatch_size, chunk_minibatches, device, _vbz=True)
+
+
+def detect_reads_svb(comp: np.ndarray, comp_offsets: np.ndarray, n_samples: np.ndarray, full_lens: np.ndarray,
+                     calib_offset: np.ndarray, calib_scale: np.ndarray, spc: Any, model: Any = None,
+                     minibatch_size: int = 1000, chunk_minibatches: int = 16, device: int = 0, _vbz: bool = False):
     """Compressed ingest: svb16 streams (adapted_b200.svb16) travel to the GPU compressed, are decoded there and
     detected (adb_detect_pipelined_svb_host).  Returns (records, batch_status)."""
     comp = np.ascontiguousarray(comp, dtype=np.uint8)
@@ -248,7 +281,8 @@ def detect_reads_svb(comp: np.ndarray, comp_offsets: np.ndarray, n_samples: np.n
     flat = flatten_config(spc)
     m = int(flat["sig_preload_size"])
     if ns.size != n or co.size != n or cs.size != n or (n and (coff.size != n + 1 or np.any(coff[1:] < coff[:-1]) or coff[0] < 0
-                                                              or coff[-1] + 16 > comp.size or np.any(coff % 16))):
+                                                              or coff[-1] + (0 if _vbz else 16) > comp.size
+                                                              or (not _vbz and np.any(coff % 16)))):
         raise ValueError("inconsistent compressed batch description")
     if n and (ns.min() < 0 or ns.max() > m):
         raise ValueError("n_samples must lie in [0, sig_preload_size]")
@@ -263,8 +297,9 @@ def detect_reads_svb(comp: np.ndarray, comp_offsets: np.ndarray, n_samples: np.n
                          calib_scale=cs.ctypes.data)
     cfg = _lib.fill_config(flat)
     ctx = _lib.default_context(device)
-    _lib.check(_lib.load().adb_detect_pipelined_svb_host(ctx.handle, C.byref(b), C.byref(cfg), w.ctypes.data if w is not None else None,
-                                                         recs.ctypes.data, status.ctypes.data, int(chunk_minibatches)))
+    entry = _lib.load().adb_detect_pipelined_vbz_host if _vbz else _lib.load().adb_detect_pipelined_svb_host
+    _lib.check(entry(ctx.handle, C.byref(b), C.byref(cfg), w.ctypes.data if w is not None else None,
+                     recs.ctypes.data, status.ctypes.data, int(chunk_minibatches)))
     return recs, status
 
 

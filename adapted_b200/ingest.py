@@ -110,18 +110,7 @@ def write_container_v2(path: str, adc: np.ndarray, offsets: np.ndarray, full_len
             ns = np.diff(offsets).astype(np.int32)
             flags = 0
     if zstd:
-        z = _zstd()
-        frames, zoff = [], [0]
-        for i in range(n):
-            src = np.ascontiguousarray(blob[coffs[i]: coffs[i + 1]])
-            dst = np.empty(int(z.ZSTD_compressBound(src.size)), np.uint8)
-            got = z.ZSTD_compress(dst.ctypes.data, dst.size, src.ctypes.data, src.size, 1)
-            if z.ZSTD_isError(got):
-                raise RuntimeError("ZSTD_compress failed")
-            frames.append(dst[:got])
-            zoff.append(zoff[-1] + int(got))
-        blob = np.concatenate(frames + [np.zeros(16, np.uint8)]) if frames else np.zeros(16, np.uint8)
-        coffs = np.asarray(zoff, np.int64)
+        blob, coffs = svb16.zstd_frames(blob, coffs, 1)
         flags |= F_ZSTD
     ids = np.asarray([str(i).encode() for i in read_ids], dtype="S") if len(read_ids) else np.zeros(0, "S1")
     ids = ids.astype(f"S{ids.dtype.itemsize + 1}")  # NUL terminated

@@ -64,6 +64,35 @@ def encode_reads(adc: np.ndarray, offsets: np.ndarray) -> Tuple[np.ndarray, np.n
     return comp, coff, ns
 
 
+def zstd_frames(blob: np.ndarray, offsets: np.ndarray, level: int = 1) -> Tuple[np.ndarray, np.ndarray]:
+    """One zstd frame (libzstd ``ZSTD_compress``) per slice ``blob[offsets[i]: offsets[i + 1]]`` -> (frames uint8 blob
+    with 16 zero bytes behind the last frame, frame_offsets int64 [n + 1])."""
+    from .ingest import _zstd
+
+    z = _zstd()
+    offsets = np.asarray(offsets, np.int64)
+    frames, zoff = [], [0]
+    for i in range(offsets.size - 1):
+        src = np.ascontiguousarray(blob[offsets[i]: offsets[i + 1]])
+        dst = np.empty(int(z.ZSTD_compressBound(src.size)), np.uint8)
+        got = z.ZSTD_compress(dst.ctypes.data, dst.size, src.ctypes.data, src.size, int(level))
+        if z.ZSTD_isError(got):
+            raise RuntimeError("ZSTD_compress failed")
+        frames.append(dst[:got])
+        zoff.append(zoff[-1] + int(got))
+    out = np.concatenate(frames + [np.zeros(SLACK, np.uint8)])
+    return out, np.asarray(zoff, np.int64)
+
+
+def vbz_encode_reads(adc: np.ndarray, offsets: np.ndarray, level: int = 1) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """pod5's VBZ, one zstd frame per read: ragged int16 reads -> (frames uint8 blob, frame_offsets int64 [n + 1],
+    n_samples int32 [n]).  Frame i decompresses to read i's svb16 stream as ``encode_reads`` lays it out (zero padded
+    to a multiple of 16 bytes), so its content size is a multiple of 16."""
+    comp, coff, ns = encode_reads(adc, offsets)
+    frames, foff = zstd_frames(comp, coff, level)
+    return frames, foff, ns
+
+
 def decode_reads(comp: np.ndarray, comp_offsets: np.ndarray, n_samples: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
     """Plain numpy decoder (the restated pod5 svb16 scalar decoder) -> (adc int16, offsets int64 [n + 1])."""
     n = n_samples.size

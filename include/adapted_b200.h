@@ -146,11 +146,14 @@ void adb_ctx_destroy(adb_ctx *ctx);
 int64_t adb_ctx_launch_count(const adb_ctx *ctx);
 /* Tuning switches that never change results.  "exact_global_select" = 1: always take the multi-pass radix select
  * for the minibatch-global median / MAD (normalize.py:15-22) instead of the sampled one-pass select.
- * "no_fast_validate" = 1: int16 reads go through the histogram-based validate kernel only (A/B testing). */
+ * "no_fast_validate" = 1: int16 reads go through the histogram-based validate kernel only (A/B testing).
+ * "host_zstd" = 1: adb_detect_files decompresses the zstd frames of VBZ containers on the host (libzstd) instead of
+ * on the GPU (A/B testing; the reference of the device path). */
 int adb_ctx_set_option(adb_ctx *ctx, const char *name, int value);
 /* Diagnostics of the most recent call (synchronises the device).  "global_select_fallbacks": minibatches the sampled
  * select handed to the exact multi-pass select; "validate_handovers": reads the counting-based validate kernel left
- * to the histogram-based one (both for the last pass of at most 256 minibatches).  -1: unknown name / error. */
+ * to the histogram-based one (both for the last pass of at most 256 minibatches); "zstd_host_frames": zstd frames
+ * the last adb_detect_files call decompressed on the host.  -1: unknown name / error. */
 int64_t adb_ctx_query(adb_ctx *ctx, const char *name);
 
 /* ---- minibatch detection ---------------------------------------------------------------------------- */
@@ -417,6 +420,36 @@ int adb_svb16_decode_host(adb_ctx *ctx, const adb_svb_batch *batch, int16_t *out
  * ctx option "pipeline_copy_only" = 1 skips the kernels (bench.py: the box's host -> device ceiling for these chunks).
  */
 int adb_detect_pipelined_svb_host(adb_ctx *ctx, const adb_svb_batch *batch, const adb_config *cfg, const float *cnn_weights,
+                                  adb_record *out_records, int32_t *batch_status, int32_t chunk_batches);
+
+/* ---- VBZ ingest: the zstd stage on the GPU (adb_zstd.cuh) ------------------------------------------------------ */
+/*
+ * zstd decode on the GPU (RFC 8878 frames without dictionaries), HOST buffers (kernel-level test entry): frame i =
+ * src[src_offsets[i] .. src_offsets[i + 1]) decodes into the slot dst[dst_offsets[i] .. dst_offsets[i + 1]).
+ * status[i] = the decoded size, or a negative ADB_ZSTD_E_* code; a refused frame leaves everything outside its slot
+ * untouched.  Bytes of a slot past the decoded size are unspecified (the decoder parks literals there).  Every frame
+ * is decoded on the device, including the ones adb_detect_files would leave to the host.
+ */
+#define ADB_ZSTD_E_TRUNCATED (-1) /* frame ends before its last block, or a section runs past its block      */
+#define ADB_ZSTD_E_MAGIC (-2)     /* not a zstd frame (skippable frames included)                             */
+#define ADB_ZSTD_E_RESERVED (-3)  /* reserved bit, block type or sequence mode bits set                       */
+#define ADB_ZSTD_E_DICT (-4)      /* dictionary ID other than 0                                               */
+#define ADB_ZSTD_E_DST_SIZE (-5)  /* output past the slot, or a block past the block maximum                  */
+#define ADB_ZSTD_E_OFFSET (-6)    /* match offset beyond the bytes produced or the window                     */
+#define ADB_ZSTD_E_SIZE (-7)      /* decoded size differs from the frame's content size                       */
+#define ADB_ZSTD_E_CHECKSUM (-8)  /* XXH64 content checksum mismatch                                          */
+#define ADB_ZSTD_E_CORRUPT (-9)   /* a table description or bitstream RFC 8878 declares corrupt               */
+#define ADB_ZSTD_E_TRAILING (-10) /* bytes left over behind the frame                                         */
+int adb_zstd_decompress_host(adb_ctx *ctx, const uint8_t *src, const int64_t *src_offsets, int32_t n, uint8_t *dst,
+                             const int64_t *dst_offsets, int32_t *status);
+/*
+ * adb_detect_pipelined_svb_host for VBZ reads (pod5's signal form): batch->comp holds one zstd frame per read
+ * (comp_offsets delimit the frames; no alignment or slack needed).  Frames travel host -> device as they are and go
+ * through zstd_decode_kernel, svb16_decode_kernel and detection.  Every frame must hold a content size of at most the
+ * worst-case stream of m samples and no dictionary (ADB_ERR_UNSUPPORTED otherwise); a frame the device refuses fails
+ * the call with ADB_ERR_ARG.  "pipeline_copy_only" skips the kernels.
+ */
+int adb_detect_pipelined_vbz_host(adb_ctx *ctx, const adb_svb_batch *batch, const adb_config *cfg, const float *cnn_weights,
                                   adb_record *out_records, int32_t *batch_status, int32_t chunk_batches);
 
 /* ---- file level (SURVEY.md row f1): containers -> GPU -> boundary tables, all stages overlapped ------------- */
