@@ -902,18 +902,18 @@ struct adb_stream_session {
     adb_ctx *ctx = nullptr;
     adb_stream_config cfg;
     bool f32 = false;  // the caches hold calibrated float32 pA (else int16 ADC codes)
-    bool dev = false;  // pushes come from device memory (adb_stream_session_push_dev)
+    bool dev = false;  // pushes come from device memory (adb_stream_session_push_dev), else from host memory
     int n_slots = 0, max_samples = 0, mask_words = 0;
-    DevBuf slots, cache, mask, stage;  // stage: one push's entries, chunks and answers
-    DevBuf dstate;                     // device pushes: SessDev arrays and the answers of sess_search
+    DevBuf slots, cache, mask;
+    DevBuf dstate;                     // SessDev arrays, and the entries and answers of a device push
     SessDev D{};
     int32_t *dout = nullptr;
-    void *pin = nullptr;               // pinned mirror of `stage`
+    DevBuf stage;                      // a host push's arrays, chunks, answers and entries
+    void *pin = nullptr;               // pinned mirror of the front of `stage`
     size_t pin_cap = 0;
-    // host mirror per slot: samples cached, a read was started, last answer, settled; stamp: duplicate check of a push
-    std::vector<int32_t> n, result, stamp;
-    std::vector<uint8_t> live, settled;
-    int32_t push_id = 0;
+    // host pushes: the `settled` answer last returned per slot.  A chunk for such a slot that is not reset is not
+    // uploaded (the device gives it no samples either); settled only clears on a reset, so the byte stays exact.
+    std::vector<uint8_t> settled;
 };
 
 static int session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_slots, int32_t max_samples, bool f32,
@@ -928,49 +928,33 @@ static int session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_t n_
     s->ctx = ctx;
     s->cfg = *cfg;
     s->f32 = f32;
+    s->dev = dev;
     s->n_slots = n_slots;
     s->max_samples = max_samples;
     s->mask_words = (max_samples + 31) / 32;
-    s->n.assign(n_slots, 0);
-    s->result.assign(n_slots, 0);
-    s->stamp.assign(n_slots, 0);
-    s->live.assign(n_slots, 0);
     s->settled.assign(n_slots, 0);
-    if (s->slots.ensure(sizeof(SessSlot) * (size_t)n_slots) || s->cache.ensure((f32 ? sizeof(float) : sizeof(int16_t)) * (size_t)n_slots * max_samples) ||
-        s->mask.ensure(sizeof(uint32_t) * (size_t)n_slots * s->mask_words)) {
+    const size_t ns = (size_t)n_slots;
+    const size_t o_out = sizeof(SessEntry) * ns, o_err = o_out + sizeof(int32_t) * 2 * ns,
+                 o_stamp = o_err + sizeof(unsigned long long), o_started = o_stamp + sizeof(uint32_t) * ns;
+    if (s->slots.ensure(sizeof(SessSlot) * ns) || s->cache.ensure((f32 ? sizeof(float) : sizeof(int16_t)) * ns * max_samples) ||
+        s->mask.ensure(sizeof(uint32_t) * ns * s->mask_words) || s->dstate.ensure(o_started + ns)) {
         adb_stream_session_destroy(s);
         set_err("cudaMalloc stream session arena");
         return ADB_ERR_CUDA;
     }
-    if (cudaMemsetAsync(s->slots.p, 0, sizeof(SessSlot) * (size_t)n_slots, ctx->stream) != cudaSuccess ||
-        cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+    unsigned char *p = (unsigned char *)s->dstate.p;
+    s->D.ent = (SessEntry *)p;
+    s->dout = (int32_t *)(p + o_out);
+    s->D.err = (unsigned long long *)(p + o_err);
+    s->D.stamp = (uint32_t *)(p + o_stamp);
+    s->D.started = p + o_started;
+    s->D.n_slots = n_slots;
+    if (cudaMemsetAsync(s->slots.p, 0, sizeof(SessSlot) * ns, ctx->stream) != cudaSuccess ||
+        cudaMemsetAsync(s->D.stamp, 0xff, sizeof(uint32_t) * ns, ctx->stream) != cudaSuccess ||
+        cudaMemsetAsync(s->D.started, 0, ns, ctx->stream) != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
         adb_stream_session_destroy(s);
         set_err("cudaMemset stream session state");
         return ADB_ERR_CUDA;
-    }
-    if (dev) {  // everything a device push needs, so that a push allocates nothing
-        s->dev = true;
-        const size_t ns = (size_t)n_slots;
-        const size_t o_out = sizeof(SessEntry) * ns, o_err = o_out + sizeof(int32_t) * 2 * ns,
-                     o_stamp = o_err + sizeof(unsigned long long), o_started = o_stamp + sizeof(uint32_t) * ns;
-        if (s->dstate.ensure(o_started + ns)) {
-            adb_stream_session_destroy(s);
-            set_err("cudaMalloc stream session arena");
-            return ADB_ERR_CUDA;
-        }
-        unsigned char *p = (unsigned char *)s->dstate.p;
-        s->D.ent = (SessEntry *)p;
-        s->dout = (int32_t *)(p + o_out);
-        s->D.err = (unsigned long long *)(p + o_err);
-        s->D.stamp = (uint32_t *)(p + o_stamp);
-        s->D.started = p + o_started;
-        s->D.n_slots = n_slots;
-        if (cudaMemsetAsync(s->D.stamp, 0xff, sizeof(uint32_t) * ns, ctx->stream) != cudaSuccess ||
-            cudaMemsetAsync(s->D.started, 0, ns, ctx->stream) != cudaSuccess || cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
-            adb_stream_session_destroy(s);
-            set_err("cudaMemset stream session state");
-            return ADB_ERR_CUDA;
-        }
     }
     *out = s;
     return ADB_OK;
@@ -1008,182 +992,7 @@ extern "C" void adb_stream_session_destroy(adb_stream_session *s) {
     delete s;
 }
 
-// true when no sample of src[0, n) is infinite or NaN (exponent bits all ones); copies them to dst unless it is null
-static bool copy_finite(float *dst, const float *src, int64_t n) {
-    uint32_t bad = 0;
-    for (int64_t j = 0; j < n; j++) {
-        uint32_t b;
-        memcpy(&b, src + j, 4);
-        if (dst) memcpy(dst + j, &b, 4);
-        bad |= (b & 0x7f800000u) == 0x7f800000u;
-    }
-    return !bad;
-}
-
-// one push of either kind: `samples` is int16 ADC (with calibration on reset) or float32 pA, as the session holds
-static int session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
-                        const void *samples, const uint8_t *reset, const float *calib_offset, const float *calib_scale,
-                        int32_t *polya_start, uint8_t *settled) {
-    const bool f32 = s->f32;
-    const size_t esz = f32 ? sizeof(float) : sizeof(int16_t);
-    if (n == 0) return ADB_OK;
-    if (!slots || !chunk_offsets || !polya_start || !settled) { set_err("null argument"); return ADB_ERR_ARG; }
-    if (chunk_offsets[0] < 0) { set_err("chunk_offsets must be non-negative"); return ADB_ERR_ARG; }
-    for (int k = 0; k < n; k++)
-        if (chunk_offsets[k + 1] < chunk_offsets[k]) { set_err("chunk_offsets must be non-decreasing"); return ADB_ERR_ARG; }
-    if (chunk_offsets[n] > chunk_offsets[0] && !samples) {
-        set_err(f32 ? "null pa with non-empty chunks" : "null adc with non-empty chunks");
-        return ADB_ERR_ARG;
-    }
-    // validate the whole push before any state changes: a refused push leaves the session as it was
-    if (++s->push_id == 0x7fffffff) { std::fill(s->stamp.begin(), s->stamp.end(), 0); s->push_id = 1; }
-    for (int k = 0; k < n; k++) {
-        const int sl = slots[k];
-        if (sl < 0 || sl >= s->n_slots) { set_err("slot out of range"); return ADB_ERR_ARG; }
-        if (s->stamp[sl] == s->push_id) { set_err("the same slot twice in one push"); return ADB_ERR_ARG; }
-        s->stamp[sl] = s->push_id;
-        if (reset && reset[k]) {
-            if (f32) continue;  // float32 reads carry no calibration
-            if (!calib_offset || !calib_scale) { set_err("a reset needs calib_offset and calib_scale"); return ADB_ERR_ARG; }
-            if (!std::isfinite(calib_scale[k]) || !(calib_scale[k] > 0.f) || !std::isfinite(calib_offset[k])) {
-                set_err("calibration scale must be finite and positive, offset finite");
-                return ADB_ERR_ARG;
-            }
-        } else if (!s->live[sl]) {
-            set_err("append to a slot that was never reset");
-            return ADB_ERR_ARG;
-        }
-    }
-    // entries that reach the device: resets and slots whose answer is not final; chunks are clipped at max_samples.
-    // Float32 samples that do not reach the device (settled slot, beyond max_samples) are checked for finiteness here,
-    // the others while they are staged.
-    const float *pa = (const float *)samples;
-    std::vector<SessEntry> ent;
-    std::vector<int> ent_k;
-    ent.reserve(n);
-    int64_t total = 0;
-    for (int k = 0; k < n; k++) {
-        const int sl = slots[k];
-        const bool rs = reset && reset[k];
-        const int64_t clen = chunk_offsets[k + 1] - chunk_offsets[k];
-        if (!rs && s->settled[sl]) {
-            if (f32 && !copy_finite(nullptr, pa + chunk_offsets[k], clen)) { set_err("non-finite pA sample"); return ADB_ERR_ARG; }
-            continue;
-        }
-        SessEntry E;
-        E.slot = sl;
-        E.reset = rs ? 1 : 0;
-        const int64_t have = rs ? 0 : s->n[sl];
-        E.len = (int32_t)std::min<int64_t>(clen, s->max_samples - have);
-        E._pad = 0;
-        E.src = total;
-        E.coff = rs && !f32 ? calib_offset[k] : 0.f;
-        E.cscale = rs && !f32 ? calib_scale[k] : 0.f;
-        if (f32 && !copy_finite(nullptr, pa + chunk_offsets[k] + E.len, clen - E.len)) { set_err("non-finite pA sample"); return ADB_ERR_ARG; }
-        total += E.len;
-        ent.push_back(E);
-        ent_k.push_back(k);
-    }
-    const int ne = (int)ent.size();
-    if (ne > 0) {
-        const size_t ent_bytes = (sizeof(SessEntry) * (size_t)ne + 15) & ~(size_t)15;
-        const size_t blob_bytes = ((size_t)total * esz + 15) & ~(size_t)15;
-        const size_t in_bytes = ent_bytes + blob_bytes, bytes = in_bytes + sizeof(int32_t) * 2 * (size_t)ne;
-        CUDA_TRY(cudaSetDevice(s->ctx->device));
-        if (bytes > s->pin_cap) {
-            if (s->pin) cudaFreeHost(s->pin);
-            s->pin = nullptr;
-            s->pin_cap = 0;
-            const size_t want = bytes + bytes / 4;
-            CUDA_TRY(cudaHostAlloc(&s->pin, want, cudaHostAllocDefault));
-            s->pin_cap = want;
-        }
-        if (s->stage.ensure(bytes)) { set_err("cudaMalloc stream session staging"); return ADB_ERR_CUDA; }
-        unsigned char *hp = (unsigned char *)s->pin;
-        memcpy(hp, ent.data(), sizeof(SessEntry) * (size_t)ne);
-        unsigned char *hb = hp + ent_bytes;
-        for (int q = 0; q < ne; q++) {
-            if (ent[q].len <= 0) continue;
-            const int64_t o = chunk_offsets[ent_k[q]];
-            if (!f32) {
-                memcpy((int16_t *)hb + ent[q].src, (const int16_t *)samples + o, sizeof(int16_t) * (size_t)ent[q].len);
-            } else if (!copy_finite((float *)hb + ent[q].src, pa + o, ent[q].len)) {
-                set_err("non-finite pA sample");
-                return ADB_ERR_ARG;
-            }
-        }
-        cudaStream_t st = s->ctx->stream;
-        CUDA_TRY(cudaMemcpyAsync(s->stage.p, hp, in_bytes, cudaMemcpyHostToDevice, st));
-        unsigned char *dp = (unsigned char *)s->stage.p;
-        const int ablocks = (ne + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS;
-        if (!f32) {
-            SessArgs A;
-            A.slots = (SessSlot *)s->slots.p;
-            A.cache = (int16_t *)s->cache.p;
-            A.mask = (uint32_t *)s->mask.p;
-            A.ent = (const SessEntry *)dp;
-            A.blob = (const int16_t *)(dp + ent_bytes);
-            A.out = (int32_t *)(dp + in_bytes);
-            A.n_ent = ne;
-            A.max_samples = s->max_samples;
-            A.mask_words = s->mask_words;
-            stream_append_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg);
-            CUDA_TRY(cudaGetLastError());
-            stream_search_kernel<<<ne, ADB_VAL_THREADS, 0, st>>>(A, s->cfg);
-        } else {
-            SessArgsF32 A;
-            A.slots = (SessSlot *)s->slots.p;
-            A.cache = (float *)s->cache.p;
-            A.mask = (uint32_t *)s->mask.p;
-            A.ent = (const SessEntry *)dp;
-            A.blob = (const float *)(dp + ent_bytes);
-            A.out = (int32_t *)(dp + in_bytes);
-            A.n_ent = ne;
-            A.max_samples = s->max_samples;
-            A.mask_words = s->mask_words;
-            stream_append_f32_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg);
-            CUDA_TRY(cudaGetLastError());
-            stream_search_f32_kernel<<<ne, ADB_VAL_THREADS, 0, st>>>(A, s->cfg);
-        }
-        CUDA_TRY(cudaGetLastError());
-        s->ctx->launches += 2;
-        CUDA_TRY(cudaMemcpyAsync(hp + in_bytes, dp + in_bytes, sizeof(int32_t) * 2 * (size_t)ne, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        const int32_t *res = (const int32_t *)(hp + in_bytes);
-        for (int q = 0; q < ne; q++) {
-            const int sl = ent[q].slot;
-            s->n[sl] = (ent[q].reset ? 0 : s->n[sl]) + ent[q].len;
-            s->live[sl] = 1;
-            s->result[sl] = res[2 * q];
-            s->settled[sl] = res[2 * q + 1] ? 1 : 0;
-        }
-    }
-    for (int k = 0; k < n; k++) {
-        polya_start[k] = s->result[slots[k]];
-        settled[k] = s->settled[slots[k]];
-    }
-    return ADB_OK;
-}
-
-extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
-                                       const int16_t *adc, const uint8_t *reset, const float *calib_offset,
-                                       const float *calib_scale, int32_t *polya_start, uint8_t *settled) {
-    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
-    if (s->dev) { set_err("host push on a device-push session"); return ADB_ERR_ARG; }
-    if (s->f32) { set_err("int16 push on a float32 session"); return ADB_ERR_ARG; }
-    return session_push(s, n, slots, chunk_offsets, adc, reset, calib_offset, calib_scale, polya_start, settled);
-}
-
-extern "C" int adb_stream_session_push_f32(adb_stream_session *s, int32_t n, const int32_t *slots,
-                                           const int64_t *chunk_offsets, const float *pa, const uint8_t *reset,
-                                           int32_t *polya_start, uint8_t *settled) {
-    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
-    if (s->dev) { set_err("host push on a device-push session"); return ADB_ERR_ARG; }
-    if (!s->f32) { set_err("float32 push on an int16 session"); return ADB_ERR_ARG; }
-    return session_push(s, n, slots, chunk_offsets, pa, reset, nullptr, nullptr, polya_start, settled);
-}
-
-// the adb_last_error() text of each refusal of session_push, by SessReason
+// the adb_last_error() text of each refusal of a push, by SessReason
 static const char *const kSessReasonText[SESS_R_COUNT] = {
     nullptr,
     "chunk_offsets must be non-negative",
@@ -1202,6 +1011,158 @@ extern "C" const char *adb_stream_session_reason(int32_t reason) {
     return reason > SESS_R_NONE && reason < SESS_R_COUNT ? kSessReasonText[reason] : nullptr;
 }
 
+// enqueues one push on `st` (adb_stream_session.cuh): the arrays of Q, the entries D.ent and the answers `out` are
+// device memory for Q.n entries
+template <class Args>
+static int session_enqueue(adb_stream_session *s, const SessPush &Q, const SessDev &D, int32_t *out, cudaStream_t st,
+                           void (*check)(Args, SessPush, SessDev), void (*append)(Args, adb_stream_config, SessDev),
+                           void (*search)(Args, adb_stream_config, SessDev, SessPush)) {
+    Args A;
+    A.slots = (SessSlot *)s->slots.p;
+    A.cache = (decltype(A.cache))s->cache.p;
+    A.mask = (uint32_t *)s->mask.p;
+    A.ent = D.ent;
+    A.blob = (decltype(A.blob))Q.samples;
+    A.out = out;
+    A.n_ent = Q.n;
+    A.max_samples = s->max_samples;
+    A.mask_words = s->mask_words;
+    const int eblocks = (Q.n + SESS_DEV_THREADS - 1) / SESS_DEV_THREADS;
+    // float32: enough CTAs for the finiteness scan, whose length only the device knows
+    const int cblocks = s->f32 ? std::max(eblocks, 4 * s->ctx->sm_count) : eblocks;
+    stream_stamp_kernel<<<eblocks, SESS_DEV_THREADS, 0, st>>>(Q, D);
+    CUDA_TRY(cudaGetLastError());
+    check<<<cblocks, SESS_DEV_THREADS, 0, st>>>(A, Q, D);
+    CUDA_TRY(cudaGetLastError());
+    append<<<(Q.n + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg, D);
+    CUDA_TRY(cudaGetLastError());
+    search<<<Q.n, ADB_VAL_THREADS, 0, st>>>(A, s->cfg, D, Q);
+    CUDA_TRY(cudaGetLastError());
+    s->ctx->launches += 4;
+    return ADB_OK;
+}
+
+static int session_enqueue(adb_stream_session *s, const SessPush &Q, const SessDev &D, int32_t *out, cudaStream_t st) {
+    if (s->f32)
+        return session_enqueue<SessArgsF32>(s, Q, D, out, st, stream_check_f32_kernel, stream_append_f32_kernel,
+                                            stream_search_f32_kernel);
+    return session_enqueue<SessArgs>(s, Q, D, out, st, stream_check_kernel, stream_append_kernel, stream_search_kernel);
+}
+
+// true when no sample of x[0, n) is infinite or NaN (exponent bits all ones)
+static bool all_finite(const float *x, int64_t n) {
+    uint32_t bad = 0;
+    for (int64_t j = 0; j < n; j++) {
+        uint32_t b;
+        memcpy(&b, x + j, 4);
+        bad |= (b & 0x7f800000u) == 0x7f800000u;
+    }
+    return !bad;
+}
+
+// A host push is a device push from a stage: the caller's arrays and chunks go up in one copy, the launches run on
+// the context's stream, and the status and the answers come back in one copy.  The device checks everything.
+static int host_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                     const void *samples, const uint8_t *reset, const float *calib_offset, const float *calib_scale,
+                     int32_t *polya_start, uint8_t *settled) {
+    if (n == 0) return ADB_OK;
+    if (!slots || !chunk_offsets || !polya_start || !settled) { set_err("null argument"); return ADB_ERR_ARG; }
+    const size_t esz = s->f32 ? sizeof(float) : sizeof(int16_t);
+    // The chunks are read only where valid offsets delimit them.  Otherwise the caller's offsets go up unchanged with
+    // null samples, and the device refuses the push for its offsets or for the null samples.
+    bool stage_samples = samples && chunk_offsets[0] >= 0;
+    for (int k = 0; stage_samples && k < n; k++) stage_samples = chunk_offsets[k + 1] >= chunk_offsets[k];
+    std::vector<int64_t> offs(chunk_offsets, chunk_offsets + n + 1);
+    if (stage_samples) {  // rebased into the staged chunks; a settled slot's chunk stays behind unless it holds a NaN / inf
+        offs[0] = 0;
+        for (int k = 0; k < n; k++) {
+            const int sl = slots[k];
+            int64_t len = chunk_offsets[k + 1] - chunk_offsets[k];
+            if (!(reset && reset[k]) && sl >= 0 && sl < s->n_slots && s->settled[sl] &&
+                (!s->f32 || all_finite((const float *)samples + chunk_offsets[k], len)))
+                len = 0;
+            offs[k + 1] = offs[k] + len;
+        }
+    }
+    size_t bytes = 0;
+    auto take = [&](size_t size, size_t align) {
+        const size_t o = (bytes + align - 1) / align * align;
+        bytes = o + size;
+        return o;
+    };
+    const size_t nn = (size_t)n;
+    const size_t o_slots = take(sizeof(int32_t) * nn, 4), o_offs = take(sizeof(int64_t) * (nn + 1), 8),
+                 o_reset = take(reset ? nn : 0, 1), o_coff = take(calib_offset ? 4 * nn : 0, 4),
+                 o_cscale = take(calib_scale ? 4 * nn : 0, 4), o_blob = take(stage_samples ? esz * (size_t)offs[n] : 0, 16),
+                 in_bytes = bytes;
+    const size_t o_status = take(sizeof(int32_t) * 2, 16), o_pa = take(sizeof(int32_t) * nn, 4), o_done = take(nn, 1),
+                 io_bytes = bytes;
+    const size_t o_ent = take(sizeof(SessEntry) * nn, 16), o_out = take(sizeof(int32_t) * 2 * nn, 4);
+    CUDA_TRY(cudaSetDevice(s->ctx->device));
+    if (io_bytes > s->pin_cap) {
+        if (s->pin) cudaFreeHost(s->pin);
+        s->pin = nullptr;
+        s->pin_cap = 0;
+        const size_t want = io_bytes + io_bytes / 4;
+        CUDA_TRY(cudaHostAlloc(&s->pin, want, cudaHostAllocDefault));
+        s->pin_cap = want;
+    }
+    if (s->stage.ensure(bytes)) { set_err("cudaMalloc stream session staging"); return ADB_ERR_CUDA; }
+    unsigned char *hp = (unsigned char *)s->pin, *dp = (unsigned char *)s->stage.p;
+    memcpy(hp + o_slots, slots, sizeof(int32_t) * nn);
+    memcpy(hp + o_offs, offs.data(), sizeof(int64_t) * (nn + 1));
+    if (reset) memcpy(hp + o_reset, reset, nn);
+    if (calib_offset) memcpy(hp + o_coff, calib_offset, 4 * nn);
+    if (calib_scale) memcpy(hp + o_cscale, calib_scale, 4 * nn);
+    if (stage_samples)
+        for (int k = 0; k < n; k++)
+            memcpy(hp + o_blob + esz * offs[k], (const unsigned char *)samples + esz * chunk_offsets[k],
+                   esz * (offs[k + 1] - offs[k]));
+    cudaStream_t st = s->ctx->stream;
+    CUDA_TRY(cudaMemcpyAsync(dp, hp, in_bytes, cudaMemcpyHostToDevice, st));
+    SessPush Q;
+    Q.slots = (const int32_t *)(dp + o_slots);
+    Q.offs = (const int64_t *)(dp + o_offs);
+    Q.samples = stage_samples ? dp + o_blob : nullptr;
+    Q.reset = reset ? dp + o_reset : nullptr;
+    Q.coff = calib_offset ? (const float *)(dp + o_coff) : nullptr;
+    Q.cscale = calib_scale ? (const float *)(dp + o_cscale) : nullptr;
+    Q.polya_start = (int32_t *)(dp + o_pa);
+    Q.settled = dp + o_done;
+    Q.status = (int32_t *)(dp + o_status);
+    Q.n = n;
+    SessDev D = s->D;
+    D.ent = (SessEntry *)(dp + o_ent);
+    int rc = session_enqueue(s, Q, D, (int32_t *)(dp + o_out), st);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(hp + o_status, dp + o_status, io_bytes - o_status, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const int32_t *status = (const int32_t *)(hp + o_status);
+    if (status[0] != ADB_OK) { set_err(kSessReasonText[status[1]]); return ADB_ERR_ARG; }
+    memcpy(polya_start, hp + o_pa, sizeof(int32_t) * nn);
+    memcpy(settled, hp + o_done, nn);
+    for (int k = 0; k < n; k++) s->settled[slots[k]] = settled[k];
+    return ADB_OK;
+}
+
+extern "C" int adb_stream_session_push(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
+                                       const int16_t *adc, const uint8_t *reset, const float *calib_offset,
+                                       const float *calib_scale, int32_t *polya_start, uint8_t *settled) {
+    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (s->dev) { set_err("host push on a device-push session"); return ADB_ERR_ARG; }
+    if (s->f32) { set_err("int16 push on a float32 session"); return ADB_ERR_ARG; }
+    return host_push(s, n, slots, chunk_offsets, adc, reset, calib_offset, calib_scale, polya_start, settled);
+}
+
+extern "C" int adb_stream_session_push_f32(adb_stream_session *s, int32_t n, const int32_t *slots,
+                                           const int64_t *chunk_offsets, const float *pa, const uint8_t *reset,
+                                           int32_t *polya_start, uint8_t *settled) {
+    if (!s || n < 0) { set_err("invalid argument"); return ADB_ERR_ARG; }
+    if (s->dev) { set_err("host push on a device-push session"); return ADB_ERR_ARG; }
+    if (!s->f32) { set_err("float32 push on an int16 session"); return ADB_ERR_ARG; }
+    return host_push(s, n, slots, chunk_offsets, pa, reset, nullptr, nullptr, polya_start, settled);
+}
+
 extern "C" int adb_stream_session_push_dev(adb_stream_session *s, int32_t n, const int32_t *slots,
                                            const int64_t *chunk_offsets, const void *samples, const uint8_t *reset,
                                            const float *calib_offset, const float *calib_scale, int32_t *polya_start,
@@ -1217,59 +1178,8 @@ extern "C" int adb_stream_session_push_dev(adb_stream_session *s, int32_t n, con
         CUDA_TRY(cudaMemsetAsync(status, 0, sizeof(int32_t) * 2, st));
         return ADB_OK;
     }
-    SessPush Q;
-    Q.slots = slots;
-    Q.offs = chunk_offsets;
-    Q.samples = samples;
-    Q.reset = reset;
-    Q.coff = calib_offset;
-    Q.cscale = calib_scale;
-    Q.polya_start = polya_start;
-    Q.settled = settled;
-    Q.status = status;
-    Q.n = n;
-    const int eblocks = (n + SESS_DEV_THREADS - 1) / SESS_DEV_THREADS;
-    // float32: enough CTAs for the finiteness scan, whose length only the device knows
-    const int cblocks = s->f32 ? std::max(eblocks, 4 * s->ctx->sm_count) : eblocks;
-    const int ablocks = (n + SESS_APPEND_WARPS - 1) / SESS_APPEND_WARPS;
-    stream_dev_stamp_kernel<<<eblocks, SESS_DEV_THREADS, 0, st>>>(Q, s->D);
-    CUDA_TRY(cudaGetLastError());
-    if (!s->f32) {
-        SessArgs A;
-        A.slots = (SessSlot *)s->slots.p;
-        A.cache = (int16_t *)s->cache.p;
-        A.mask = (uint32_t *)s->mask.p;
-        A.ent = s->D.ent;
-        A.blob = (const int16_t *)samples;
-        A.out = s->dout;
-        A.n_ent = n;
-        A.max_samples = s->max_samples;
-        A.mask_words = s->mask_words;
-        stream_dev_check_kernel<<<cblocks, SESS_DEV_THREADS, 0, st>>>(A, Q, s->D);
-        CUDA_TRY(cudaGetLastError());
-        stream_append_dev_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg, s->D);
-        CUDA_TRY(cudaGetLastError());
-        stream_search_dev_kernel<<<n, ADB_VAL_THREADS, 0, st>>>(A, s->cfg, s->D, Q);
-    } else {
-        SessArgsF32 A;
-        A.slots = (SessSlot *)s->slots.p;
-        A.cache = (float *)s->cache.p;
-        A.mask = (uint32_t *)s->mask.p;
-        A.ent = s->D.ent;
-        A.blob = (const float *)samples;
-        A.out = s->dout;
-        A.n_ent = n;
-        A.max_samples = s->max_samples;
-        A.mask_words = s->mask_words;
-        stream_dev_check_f32_kernel<<<cblocks, SESS_DEV_THREADS, 0, st>>>(A, Q, s->D);
-        CUDA_TRY(cudaGetLastError());
-        stream_append_dev_f32_kernel<<<ablocks, SESS_APPEND_WARPS * 32, 0, st>>>(A, s->cfg, s->D);
-        CUDA_TRY(cudaGetLastError());
-        stream_search_dev_f32_kernel<<<n, ADB_VAL_THREADS, 0, st>>>(A, s->cfg, s->D, Q);
-    }
-    CUDA_TRY(cudaGetLastError());
-    s->ctx->launches += 4;
-    return ADB_OK;
+    const SessPush Q{slots, chunk_offsets, samples, reset, calib_offset, calib_scale, polya_start, settled, status, n};
+    return session_enqueue(s, Q, s->D, s->dout, st);
 }
 
 // ---- CNN scores (kernel-level test entry) ------------------------------------------------------------------------

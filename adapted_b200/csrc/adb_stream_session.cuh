@@ -20,17 +20,16 @@
 // The early return n < min_obs_adapter + max(windows) is tested on every push.  A slot also settles when its cache
 // is full (max_samples): later samples of that read are dropped.
 //
-// Two launches per push: stream_append_kernel (one warp per pushed slot copies the chunk into the cache and updates
-// the key bounds; its lane 0 advances the recurrences and the mask) and stream_search_kernel (one CTA per pushed
-// slot resumes the search loop with seg_stats reading the cache in global memory, so a cache is not bounded by
-// shared memory).  Float32 sessions run stream_append_f32_kernel / stream_search_f32_kernel: the same code
-// (sess_append / sess_search) with the samples taken as they are, and order statistics on float keys through the
-// generic multi-level select instead of the one-pass code histogram.
-//
-// Device pushes (adb_stream_session_push_dev) take entries and chunks in device memory and run on the caller's stream
-// with no host synchronise: stream_dev_stamp_kernel and stream_dev_check_kernel validate the whole push and build the
-// entries before any state changes, then stream_append_dev_kernel / stream_search_dev_kernel run sess_append /
-// sess_search on the caller's buffer unless the push was refused, and write the answers and the status.
+// Four launches per push, all reading the push's arrays from device memory: the caller's for a device push
+// (adb_stream_session_push_dev, on the caller's stream), a stage uploaded in one copy for a host push
+// (adb_stream_session_push / _push_f32, on the context's stream, which then downloads the status and the answers).
+// stream_stamp_kernel and stream_check_kernel validate the whole push and build the entries before any state
+// changes.  stream_append_kernel (one warp per pushed slot copies the chunk into the cache and updates the key bounds;
+// its lane 0 advances the recurrences and the mask) and stream_search_kernel (one CTA per pushed slot resumes the
+// search loop with seg_stats reading the cache in global memory, so a cache is not bounded by shared memory) return
+// at once for a refused push; the search writes the status and the answers.  Float32 sessions run the _f32 kernels:
+// the same code (sess_check / sess_append / sess_search) with the samples taken as they are, and order statistics on
+// float keys through the generic multi-level select instead of the one-pass code histogram.
 #pragma once
 #include "adb_stream.cuh"
 
@@ -45,9 +44,9 @@ struct SessSlot {  // device state of one slot
     float amean, assqdm, asum;
 };
 
-struct SessEntry {  // one pushed slot, host -> device (device pushes: built by stream_dev_check_kernel)
+struct SessEntry {  // one pushed slot, built by stream_check_kernel
     int32_t slot, reset, len, _pad;
-    int64_t src;      // first sample of the chunk in the staged blob (device pushes: in the caller's buffer)
+    int64_t src;      // first sample of the chunk in `blob`
     float coff, cscale;
 };
 
@@ -57,7 +56,7 @@ struct SessArgsT {
     T *cache;              // [n_slots][max_samples]
     uint32_t *mask;        // [n_slots][mask_words]
     const SessEntry *ent;  // [n_ent]
-    const T *blob;         // staged chunks
+    const T *blob;         // the push's samples
     int32_t *out;          // [n_ent][2]: polya_start, settled
     int n_ent, max_samples, mask_words;
 };
@@ -156,13 +155,6 @@ __device__ __forceinline__ void sess_append(SessArgsT<T> A, adb_stream_config P,
     S.amean = amean; S.assqdm = assqdm; S.asum = asum;
 }
 
-__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(SessArgs A, adb_stream_config P) {
-    sess_append(A, P, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
-}
-__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_f32_kernel(SessArgsF32 A, adb_stream_config P) {
-    sess_append(A, P, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
-}
-
 template <class T>
 __device__ __forceinline__ void sess_search(SessArgsT<T> A, adb_stream_config P) {
     using X = SessSample<T>;
@@ -244,15 +236,12 @@ __device__ __forceinline__ void sess_search(SessArgsT<T> A, adb_stream_config P)
     }
 }
 
-__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs A, adb_stream_config P) { sess_search(A, P); }
-__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_f32_kernel(SessArgsF32 A, adb_stream_config P) {
-    sess_search(A, P);
-}
-
-// ---- device pushes ----------------------------------------------------------------------------------------------
-// Refusals of a push, in the order the host push (session_push, adb_api.cu) checks them.  A refusal is recorded as the
-// key (phase << 40) | (entry << 8) | reason and the push keeps the smallest key, so the device reports the refusal the
-// host push would report first: the phase orders the host's passes, the entry its per-entry loop.
+// ---- validation and the kernels of a push -----------------------------------------------------------------------
+// Refusals of a push.  A push is refused for the first check it fails, in this order: phase 0, a negative first
+// offset; phase 1, the first entry whose offsets decrease; phase 2, null samples with non-empty chunks; phase 3, entry
+// by entry, the first of that entry's checks below to fail; phase 4, a non-finite float32 sample.  A refusal is
+// recorded as the key (phase << 40) | (entry << 8) | reason and the push keeps the smallest key, which is that first
+// refusal.
 enum SessReason : int32_t {
     SESS_R_NONE = 0,
     SESS_R_NEG_OFFSET,    // phase 0
@@ -270,7 +259,7 @@ enum SessReason : int32_t {
 #define SESS_DEV_OK 0xffffffffffffffffull
 #define SESS_DEV_THREADS 256
 
-struct SessPush {  // the caller's arrays of one device push (device pointers)
+struct SessPush {  // the arrays of one push, in device memory
     const int32_t *slots;     // [n]
     const int64_t *offs;      // [n + 1] chunk offsets into `samples`
     const void *samples;      // int16 ADC or float32 pA, as the session holds
@@ -282,10 +271,10 @@ struct SessPush {  // the caller's arrays of one device push (device pointers)
     int n;
 };
 
-struct SessDev {  // state of a device-push session next to SessSlot, and the scratch of one push
+struct SessDev {  // state of a session next to SessSlot, and the scratch of one push
     uint32_t *stamp;    // [n_slots] first entry of the running push that names the slot; 0xffffffff between pushes
     uint8_t *started;   // [n_slots] a read was started on the slot by an accepted push
-    SessEntry *ent;     // [n_slots] entries of the running push
+    SessEntry *ent;     // [n] entries of the running push
     unsigned long long *err;  // smallest refusal key of the running push, SESS_DEV_OK if none
     int n_slots;
 };
@@ -296,7 +285,7 @@ __device__ __forceinline__ void sess_refuse(SessDev D, int phase, int k, int rea
 __device__ __forceinline__ bool non_finite_f32(float v) { return (__float_as_uint(v) & 0x7f800000u) == 0x7f800000u; }
 
 // opens the push: clears its refusal key and stamps every slot named with the first entry naming it
-__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_stamp_kernel(SessPush Q, SessDev D) {
+__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_stamp_kernel(SessPush Q, SessDev D) {
     if (blockIdx.x == 0 && threadIdx.x == 0) *D.err = SESS_DEV_OK;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < Q.n; k += gridDim.x * blockDim.x) {
         const int sl = Q.slots[k];
@@ -304,12 +293,12 @@ __global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_stamp_kernel(Sess
     }
 }
 
-// Every check of the host push, and the entries from device state: entry k appends chunk k straight from the
-// caller's buffer (src = chunk_offsets[k]), clipped at max_samples; a settled slot that is not reset gets a
+// Every check of the push, and the entries from device state: entry k appends chunk k straight from `samples`
+// (src = chunk_offsets[k]), clipped at max_samples; a settled slot that is not reset gets a
 // zero-length entry, for which sess_search returns the final answer.  Float32 sessions also scan every sample of
 // [chunk_offsets[0], chunk_offsets[n]) for NaN / inf, chunks of settled slots and clipped samples included.
 template <class T>
-__device__ __forceinline__ void sess_dev_check(SessArgsT<T> A, SessPush Q, SessDev D) {
+__device__ __forceinline__ void sess_check(SessArgsT<T> A, SessPush Q, SessDev D) {
     constexpr bool f32 = !SessSample<T>::int_keys;
     const int stride = gridDim.x * blockDim.x, tid = blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t o0 = Q.offs[0], o1 = Q.offs[Q.n];
@@ -367,30 +356,31 @@ __device__ __forceinline__ void sess_dev_check(SessArgsT<T> A, SessPush Q, SessD
     }
 }
 
-__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_check_kernel(SessArgs A, SessPush Q, SessDev D) {
-    sess_dev_check(A, Q, D);
+__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_check_kernel(SessArgs A, SessPush Q, SessDev D) {
+    sess_check(A, Q, D);
 }
-__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_dev_check_f32_kernel(SessArgsF32 A, SessPush Q, SessDev D) {
-    sess_dev_check(A, Q, D);
+__global__ void __launch_bounds__(SESS_DEV_THREADS) stream_check_f32_kernel(SessArgsF32 A, SessPush Q, SessDev D) {
+    sess_check(A, Q, D);
 }
 
+// a refused push changes nothing; an accepted reset starts a read on its slot
 template <class T>
-__device__ __forceinline__ void sess_append_dev(SessArgsT<T> A, adb_stream_config P, SessDev D, int e, int lane) {
-    if (*D.err != SESS_DEV_OK) return;  // refused: nothing changes
+__device__ __forceinline__ void sess_append_checked(SessArgsT<T> A, adb_stream_config P, SessDev D, int e, int lane) {
+    if (*D.err != SESS_DEV_OK) return;
     if (lane == 0 && e < A.n_ent && A.ent[e].reset) D.started[A.ent[e].slot] = 1;
     sess_append(A, P, e, lane);
 }
-__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_dev_kernel(SessArgs A, adb_stream_config P, SessDev D) {
-    sess_append_dev(A, P, D, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_kernel(SessArgs A, adb_stream_config P, SessDev D) {
+    sess_append_checked(A, P, D, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
-__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_dev_f32_kernel(SessArgsF32 A, adb_stream_config P,
-                                                                                      SessDev D) {
-    sess_append_dev(A, P, D, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
+__global__ void __launch_bounds__(SESS_APPEND_WARPS * 32) stream_append_f32_kernel(SessArgsF32 A, adb_stream_config P,
+                                                                                  SessDev D) {
+    sess_append_checked(A, P, D, blockIdx.x * SESS_APPEND_WARPS + (threadIdx.x >> 5), threadIdx.x & 31);
 }
 
 // closes the push: the status always, the answers only for an accepted push (a refused one leaves them untouched)
 template <class T>
-__device__ __forceinline__ void sess_search_dev(SessArgsT<T> A, adb_stream_config P, SessDev D, SessPush Q) {
+__device__ __forceinline__ void sess_search_checked(SessArgsT<T> A, adb_stream_config P, SessDev D, SessPush Q) {
     const unsigned long long err = *D.err;
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         Q.status[0] = err == SESS_DEV_OK ? ADB_OK : ADB_ERR_ARG;
@@ -403,11 +393,11 @@ __device__ __forceinline__ void sess_search_dev(SessArgsT<T> A, adb_stream_confi
         Q.settled[blockIdx.x] = A.out[2 * blockIdx.x + 1] ? 1 : 0;
     }
 }
-__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_dev_kernel(SessArgs A, adb_stream_config P, SessDev D,
-                                                                            SessPush Q) {
-    sess_search_dev(A, P, D, Q);
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_kernel(SessArgs A, adb_stream_config P, SessDev D,
+                                                                        SessPush Q) {
+    sess_search_checked(A, P, D, Q);
 }
-__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_dev_f32_kernel(SessArgsF32 A, adb_stream_config P,
-                                                                                SessDev D, SessPush Q) {
-    sess_search_dev(A, P, D, Q);
+__global__ void __launch_bounds__(ADB_VAL_THREADS) stream_search_f32_kernel(SessArgsF32 A, adb_stream_config P, SessDev D,
+                                                                            SessPush Q) {
+    sess_search_checked(A, P, D, Q);
 }

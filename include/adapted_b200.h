@@ -301,7 +301,9 @@ int adb_stream_session_create(adb_ctx *ctx, const adb_stream_config *cfg, int32_
                               adb_stream_session **out);
 void adb_stream_session_destroy(adb_stream_session *s);
 /* entry k: reset[k] != 0 starts a new read on slots[k] (cache emptied, calibration taken from calib_offset[k] /
- * calib_scale[k]), then adc[chunk_offsets[k] .. chunk_offsets[k+1]) is appended.  HOST buffers, synchronous.
+ * calib_scale[k]), then adc[chunk_offsets[k] .. chunk_offsets[k+1]) is appended.  HOST buffers, synchronous: the
+ * push goes to the device in one copy (chunks for settled reads that are not reset stay behind) and runs the kernels
+ * of adb_stream_session_push_dev on the context's stream, which check it before any state changes.
  * reset == NULL: no entry resets (calib_* may then be NULL).  Zero-length chunks are legal and return the current
  * answer.  ADB_ERR_ARG, with the session unchanged, for a slot out of range or twice in one push, decreasing offsets,
  * an append to a slot that was never reset, or a reset with a non-finite offset or a non-finite or non-positive
@@ -347,8 +349,9 @@ int adb_stream_session_create_dev(adb_ctx *ctx, const adb_stream_config *cfg, in
  * adb_stream_session_reason(reason) is the text adb_last_error() gives for the same refusal of the host push.
  * Everything that depends on the data is checked on the device, in stream order, before any state changes; the call
  * itself returns ADB_ERR_ARG, enqueueing nothing, only for a null handle, status or array pointer, a session that is
- * not a device-push session, n > n_slots (a valid push names each slot at most once), or a calibration given to a
- * float32 session.  Pushes to one session must be ordered on the device (one stream, or events between streams).
+ * not a device-push session, n > n_slots (a valid push names each slot at most once; a host push reports the
+ * refusal it meets first instead), or a calibration given to a float32 session.  Pushes to one session must be
+ * ordered on the device (one stream, or events between streams).
  */
 int adb_stream_session_push_dev(adb_stream_session *s, int32_t n, const int32_t *slots, const int64_t *chunk_offsets,
                                 const void *samples, const uint8_t *reset, const float *calib_offset,

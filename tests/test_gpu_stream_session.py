@@ -240,6 +240,17 @@ def test_session_argument_errors_leave_it_usable():
             with pytest.raises(AdbError) as e:
                 s.push(kw["slots"], kw["chunks"], reset=kw.get("reset"), calib_offset=co, calib_scale=scale)
             assert e.value.status == -2, kw
+        # more entries than slots: the first refusal in check order
+        many = [
+            (dict(slots=[1] * 5, chunks=[r0[:10]] * 5), "the same slot twice in one push"),
+            (dict(slots=[1] * 5, chunks=(r0, np.array([0, 10, 20, 15, 30, 40]))),
+             "chunk_offsets must be non-decreasing"),
+            (dict(slots=[4, 1, 1, 1, 1], chunks=[r0[:10]] * 5), "slot out of range"),
+        ]
+        for kw, msg in many:
+            with pytest.raises(AdbError) as e:
+                s.push(kw["slots"], kw["chunks"], calib_offset=co, calib_scale=cs)
+            assert e.value.status == -2 and str(e.value).endswith(": " + msg), (kw, str(e.value))
         # nothing of the refused pushes reached the session: slot 1 still holds r0[:9000]
         again, _ = s.push([1], [r0[:0]])
         assert again[0] == got[0] == _oracle(r0[:9000], co, cs, p)

@@ -317,6 +317,17 @@ def test_f32_session_argument_errors_leave_it_usable():
             with pytest.raises(AdbError) as e:
                 s.push(kw["slots"], kw["chunks"], reset=kw.get("reset"))
             assert e.value.status == -2, kw
+        # more entries than slots: the first refusal in check order
+        many = [
+            (dict(slots=[1] * 7, chunks=[r0[9000:9010]] * 7), "the same slot twice in one push"),
+            (dict(slots=[1] * 7, chunks=(r0, np.array([0, 10, 20, 15, 30, 40, 50, 60]))),
+             "chunk_offsets must be non-decreasing"),
+            (dict(slots=[6] + [1] * 6, chunks=[r0[9000:9010]] * 7), "slot out of range"),
+        ]
+        for kw, msg in many:
+            with pytest.raises(AdbError) as e:
+                s.push(kw["slots"], kw["chunks"])
+            assert e.value.status == -2 and str(e.value).endswith(": " + msg), (kw, str(e.value))
         # calibration belongs to int16 sessions
         for kw in (dict(calib_offset=co, calib_scale=cs), dict(calib_offset=[co]), dict(calib_scale=[cs])):
             with pytest.raises(ValueError):
