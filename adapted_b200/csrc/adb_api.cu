@@ -75,13 +75,13 @@ extern "C" int adb_ctx_create(int device, adb_ctx **out) {
     CUDA_TRY(cudaGetDeviceProperties(&prop, device));
     c->sm_count = prop.multiProcessorCount;
     c->max_smem_optin = (int)prop.sharedMemPerBlockOptin;
-    if (const char *e = getenv("ADB_HIST_VALIDATE")) c->opt_hist_validate = atoi(e);  // A/B switch of the validation kernel
+    if (const char *e = getenv("ADB_HIST_VALIDATE")) c->opt.hist_validate = atoi(e);  // A/B switch of the validation kernel
     c->ct_slot = ct_slot_take(device);
     CUDA_TRY(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     CUDA_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    for (int k = 0; k < 2; k++) {
-        CUDA_TRY(cudaEventCreateWithFlags(&c->p_done[k], cudaEventDisableTiming));
-        CUDA_TRY(cudaEventCreateWithFlags(&c->p_copied[k], cudaEventDisableTiming));
+    for (ChunkBufs &b : c->p) {
+        CUDA_TRY(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&b.copied, cudaEventDisableTiming));
     }
     *out = c;
     return ADB_OK;
@@ -100,12 +100,12 @@ extern "C" void adb_ctx_destroy(adb_ctx *c) {
                      &c->h_lens, &c->h_coff, &c->h_cscale, &c->h_records, &c->h_misc, &c->h_misc2, &c->h_misc3,
                      &c->gsb_plan, &c->gsb_hist, &c->gsb_tab, &c->gsb_bases, &c->gsb_active, &c->vf_done, &c->mvs_perm, &c->cnn_wtc, &c->cnn_a0t, &c->cnn_ct, &c->llr_cc, &c->val_cc, &c->z_fail};
     for (DevBuf *b : all) b->release();
-    for (int k = 0; k < 2; k++) {
-        DevBuf *pb[] = {&c->p_signal[k], &c->p_offsets[k], &c->p_lens[k], &c->p_coff[k], &c->p_cscale[k], &c->p_records[k], &c->p_status[k],
-                        &c->p_comp[k], &c->p_coffs[k], &c->p_nsamp[k], &c->p_frames[k], &c->p_foffs[k], &c->p_zstat[k]};
-        for (DevBuf *b : pb) b->release();
-        if (c->p_done[k]) cudaEventDestroy(c->p_done[k]);
-        if (c->p_copied[k]) cudaEventDestroy(c->p_copied[k]);
+    for (ChunkBufs &b : c->p) {
+        DevBuf *pb[] = {&b.signal, &b.offsets, &b.lens, &b.coff, &b.cscale, &b.records, &b.status,
+                        &b.comp, &b.coffs, &b.nsamp, &b.frames, &b.foffs, &b.zstat};
+        for (DevBuf *d : pb) d->release();
+        if (b.done) cudaEventDestroy(b.done);
+        if (b.copied) cudaEventDestroy(b.copied);
     }
     adb_ctx_set_timing(c, 0);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
@@ -117,13 +117,13 @@ extern "C" int64_t adb_ctx_launch_count(const adb_ctx *c) { return c ? c->launch
 
 extern "C" int adb_ctx_set_option(adb_ctx *c, const char *name, int value) {
     if (!c || !name) return ADB_ERR_ARG;
-    if (!strcmp(name, "exact_global_select")) { c->opt_exact_gsel = value; return ADB_OK; }
-    if (!strcmp(name, "no_fast_validate")) { c->opt_no_fast_validate = value; return ADB_OK; }
-    if (!strcmp(name, "hist_validate")) { c->opt_hist_validate = value; return ADB_OK; }
-    if (!strcmp(name, "cnn_fp32_pipe")) { c->opt_cnn_fp32 = value; return ADB_OK; }
-    if (!strcmp(name, "pipeline_copy_only")) { c->opt_copy_only = value; return ADB_OK; }
-    if (!strcmp(name, "no_cand_followup")) { c->opt_no_cand_followup = value; return ADB_OK; }
-    if (!strcmp(name, "host_zstd")) { c->opt_host_zstd = value; return ADB_OK; }
+    if (!strcmp(name, "exact_global_select")) { c->opt.exact_gsel = value; return ADB_OK; }
+    if (!strcmp(name, "no_fast_validate")) { c->opt.no_fast_validate = value; return ADB_OK; }
+    if (!strcmp(name, "hist_validate")) { c->opt.hist_validate = value; return ADB_OK; }
+    if (!strcmp(name, "cnn_fp32_pipe")) { c->opt.cnn_fp32 = value; return ADB_OK; }
+    if (!strcmp(name, "pipeline_copy_only")) { c->opt.copy_only = value; return ADB_OK; }
+    if (!strcmp(name, "no_cand_followup")) { c->opt.no_cand_followup = value; return ADB_OK; }
+    if (!strcmp(name, "host_zstd")) { c->opt.host_zstd = value; return ADB_OK; }
     set_err(std::string("unknown option: ") + name);
     return ADB_ERR_ARG;
 }
@@ -253,7 +253,7 @@ static int run_global_med_mad(adb_ctx *ctx, const BatchDev &B, int n_batches, in
     const int gx = std::max(1, std::min(B.batch_size, (ctx->sm_count * 8 + n_batches - 1) / n_batches));
     const int *active = nullptr;
     ctx->gsb_last_batches = 0;
-    if (B.sig_type == ADB_SIG_I16 && !ctx->opt_exact_gsel) {
+    if (B.sig_type == ADB_SIG_I16 && !ctx->opt.exact_gsel) {
         if (ctx->gsb_plan.ensure(sizeof(GsbPlan) * (size_t)n_batches) || ctx->gsb_hist.ensure(sizeof(unsigned) * GSB_BINS * (size_t)n_batches) ||
             ctx->gsb_tab.ensure(sizeof(unsigned) * GSB_TAB * (size_t)B.n_reads) || ctx->gsb_bases.ensure(sizeof(GsbRead) * (size_t)B.n_reads) ||
             ctx->gsb_active.ensure(sizeof(int) * (size_t)n_batches)) { set_err("cudaMalloc sampled select"); return ADB_ERR_CUDA; }
@@ -447,7 +447,7 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
                 M.perm = perm;
                 CUDA_TRY(cudaFuncSetAttribute(mvs_series_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mvs_smem_bytes()));
                 mvs_series_kernel<<<(B.n_reads + MVS_LANES - 1) / MVS_LANES, MVS_LANES, mvs_smem_bytes(), st>>>(M, cfg);
-                if (!ctx->opt_no_fast_validate) {
+                if (!ctx->opt.no_fast_validate) {
                     // medians of the two series of every row, one warp per series (consumed by validate_fast_kernel)
                     SeriesMedianArgs SM;
                     SM.B = B; SM.pre_var = M.var_pool; SM.pre_mean = M.mean_pool; SM.pre_off = M.row_off; SM.pre_meta = M.meta;
@@ -476,7 +476,7 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
     A.pending = A.n_pending = nullptr;
     A.work_counter = nullptr;
     ctx->vf_last_reads = 0;
-    if (B.sig_type == ADB_SIG_I16 && !ctx->opt_no_fast_validate && !overwrite) {
+    if (B.sig_type == ADB_SIG_I16 && !ctx->opt.no_fast_validate && !overwrite) {
         // int16 sources: counting-based validation (adb_vfast.cuh); what it leaves is picked up by validate_kernel.
         // It stages the window (dynamic shared memory) next to its static scratch: both count against the limit.
         const size_t fsm = vfast_smem_bytes(B.m * 2);
@@ -492,7 +492,7 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
             F.pre_var = A.pre_var; F.pre_mean = A.pre_mean; F.pre_off = A.pre_off; F.pre_meta = A.pre_meta;
             F.series_med = series_med;
             F.done = (unsigned char *)ctx->vf_done.p;
-            F.cand_followup = (pre && mode == ADB_METHOD_CNN && (ntopk_per_read || given_ntopk > 1) && !ctx->opt_no_cand_followup) ? 1 : 0;
+            F.cand_followup = (pre && mode == ADB_METHOD_CNN && (ntopk_per_read || given_ntopk > 1) && !ctx->opt.no_cand_followup) ? 1 : 0;
             CUDA_TRY(cudaFuncSetAttribute(validate_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsm));
             int focc = 0;
             CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&focc, validate_fast_kernel, VF_THREADS, fsm));
@@ -500,7 +500,7 @@ static int launch_validate(adb_ctx *ctx, const BatchDev &B, const adb_config &cf
             const int fgrid = std::max(1, std::min(B.n_reads, ctx->sm_count * focc));
             // the tensor-core histogram variant needs an accumulator per piece of the window: the ranges of the MVS check
             // and of the median-shift check together can cut a read into more pieces than it has
-            const bool use_hist = ctx->opt_hist_validate && B.m <= 65535 && !(cfg.mvs_detect_check && cfg.detect_med_shift);
+            const bool use_hist = ctx->opt.hist_validate && B.m <= 65535 && !(cfg.mvs_detect_check && cfg.detect_med_shift);
             if (use_hist) {
                 const size_t hsm = vhist_smem_bytes();
                 CUDA_TRY(cudaFuncSetAttribute(validate_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hsm));
@@ -654,6 +654,14 @@ struct StreamDrain {
     }
 };
 
+// the CNN weights of a host-buffer call, copied into the context's h_misc2 on its stream
+static int upload_cnn_weights(adb_ctx *ctx, const float *cnn_weights, const float **w_dev) {
+    if (ctx->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc weights"); return ADB_ERR_CUDA; }
+    CUDA_TRY(cudaMemcpyAsync(ctx->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, ctx->stream));
+    *w_dev = (const float *)ctx->h_misc2.p;
+    return ADB_OK;
+}
+
 struct StagedBatch {
     adb_batch dev;
     size_t signal_bytes;
@@ -708,9 +716,8 @@ extern "C" int adb_detect_host(adb_ctx *ctx, const adb_batch *batch, const adb_c
     if (ctx->h_misc.ensure(sizeof(int) * (size_t)n_batches + 16)) { set_err("cudaMalloc status"); return ADB_ERR_CUDA; }
     const float *w_dev = nullptr;
     if (cnn_weights && cfg->primary_method == ADB_METHOD_CNN) {
-        if (ctx->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc weights"); return ADB_ERR_CUDA; }
-        CUDA_TRY(cudaMemcpyAsync(ctx->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, st));
-        w_dev = (const float *)ctx->h_misc2.p;
+        rc = upload_cnn_weights(ctx, cnn_weights, &w_dev);
+        if (rc) return rc;
     }
     rc = adb_detect_dev(ctx, &sb.dev, cfg, w_dev, (adb_record *)ctx->h_records.p, (int *)ctx->h_misc.p, st);
     if (rc) return rc;
@@ -718,117 +725,6 @@ extern "C" int adb_detect_host(adb_ctx *ctx, const adb_batch *batch, const adb_c
     if (batch_status)
         CUDA_TRY(cudaMemcpyAsync(batch_status, ctx->h_misc.p, sizeof(int) * (size_t)n_batches, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    return ADB_OK;
-}
-
-// Pipelined ingest for long jobs: the reads are cut into chunks of `chunk_batches` minibatches; the H2D copy of
-// chunk i+1 (copy stream) overlaps the kernels of chunk i (compute stream), records return per chunk.  Host buffers
-// should be pinned (cudaHostAlloc / torch pin_memory) for the copies to be asynchronous.  I16 ragged input only.
-extern "C" int adb_detect_pipelined_host(adb_ctx *ctx, const adb_batch *batch, const adb_config *cfg,
-                                         const float *cnn_weights, adb_record *out_records, int32_t *batch_status,
-                                         int32_t chunk_batches) {
-    if (!ctx || !out_records) { set_err("null argument"); return ADB_ERR_ARG; }
-    int rc = check_batch(batch);
-    if (rc) return rc;
-    rc = check_config(cfg);
-    if (rc) return rc;
-    if (batch->sig_type != ADB_SIG_I16) { set_err("pipelined ingest takes ragged int16 input"); return ADB_ERR_ARG; }
-    if (chunk_batches < 1) chunk_batches = 1;
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    if (batch->n_reads == 0) return ADB_OK;
-    const float *w_dev = nullptr;
-    if (cfg->primary_method == ADB_METHOD_CNN) {
-        if (!cnn_weights) { set_err("cnn_weights required"); return ADB_ERR_ARG; }
-        if (ctx->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc weights"); return ADB_ERR_CUDA; }
-        CUDA_TRY(cudaMemcpyAsync(ctx->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, ctx->stream));
-        w_dev = (const float *)ctx->h_misc2.p;
-    }
-    const int n_batches = (batch->n_reads + batch->batch_size - 1) / batch->batch_size;
-    // Chunk schedule (in minibatches).  The first copy and the last chunk's kernels cannot overlap anything, so the
-    // job starts and ends with small chunks (chunk_batches / 4, / 2) and runs full-size chunks in between, where the
-    // per-chunk launch overheads and kernel tails matter.
-    std::vector<int> sched;
-    {
-        const int q = std::max(1, chunk_batches / 4), h = std::max(1, chunk_batches / 2);
-        int left = n_batches;
-        std::vector<int> tail;
-        if (n_batches >= 2 * (q + h) + chunk_batches) {
-            sched.push_back(q); sched.push_back(h);
-            tail.push_back(h); tail.push_back(q);
-            left -= 2 * (q + h);
-        }
-        while (left > 0) { const int c = std::min(left, chunk_batches); sched.push_back(c); left -= c; }
-        sched.insert(sched.end(), tail.begin(), tail.end());
-    }
-    // consecutive chunks alternate between this context and its twin: each has its own compute stream and scratch arena,
-    // the copies of all chunks go through one copy stream in order
-    if (!ctx->twin && sched.size() >= 3) {
-        rc = adb_ctx_create(ctx->device, &ctx->twin);
-        if (rc) return rc;
-    }
-    if (ctx->twin) {
-        ctx->twin->opt_no_fast_validate = ctx->opt_no_fast_validate;
-        ctx->twin->opt_hist_validate = ctx->opt_hist_validate;
-        ctx->twin->opt_cnn_fp32 = ctx->opt_cnn_fp32;
-        ctx->twin->opt_exact_gsel = ctx->opt_exact_gsel;
-        ctx->twin->opt_no_cand_followup = ctx->opt_no_cand_followup;
-    }
-    adb_ctx *cc[2] = {ctx, ctx->twin ? ctx->twin : ctx};
-    const float *w_devs[2] = {w_dev, w_dev};
-    if (w_dev && ctx->twin) {
-        if (ctx->twin->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc weights"); return ADB_ERR_CUDA; }
-        CUDA_TRY(cudaMemcpyAsync(ctx->twin->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, ctx->twin->stream));
-        w_devs[1] = (const float *)ctx->twin->h_misc2.p;
-    }
-    cudaStream_t cs = ctx->copy_stream;
-    StreamDrain drain;
-    drain.add(cs);
-    drain.add(ctx->stream);
-    if (ctx->twin) drain.add(ctx->twin->stream);
-    int b0 = 0;  // first minibatch of the chunk
-    for (int ch = 0; ch < (int)sched.size(); ch++) {
-        adb_ctx *c = cc[ch & 1];
-        const int slot = ctx->twin ? 0 : (ch & 1);
-        cudaStream_t ks = c->stream;
-        const int r0 = b0 * batch->batch_size;
-        const int r1 = (int)std::min<long long>((long long)batch->n_reads, (long long)(b0 + sched[ch]) * batch->batch_size), nr = r1 - r0;
-        const int nb = (nr + batch->batch_size - 1) / batch->batch_size;
-        const int64_t e0 = batch->offsets[r0], e1 = batch->offsets[r1];
-        // the slot is free once the D2H of the chunk that used it two iterations ago has finished
-        if (ch >= 2) CUDA_TRY(cudaEventSynchronize(c->p_done[slot]));
-        if (c->p_signal[slot].ensure((size_t)(e1 - e0) * 2 + 64) || c->p_offsets[slot].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
-            c->p_lens[slot].ensure(sizeof(int32_t) * (size_t)nr + 16) || c->p_coff[slot].ensure(sizeof(float) * (size_t)nr + 16) ||
-            c->p_cscale[slot].ensure(sizeof(float) * (size_t)nr + 16) || c->p_records[slot].ensure(sizeof(adb_record) * (size_t)nr) ||
-            c->p_status[slot].ensure(sizeof(int) * (size_t)nb + 16)) { set_err("cudaMalloc pipeline staging"); return ADB_ERR_CUDA; }
-        CUDA_TRY(cudaMemcpyAsync(c->p_signal[slot].p, (const int16_t *)batch->signal + e0, (size_t)(e1 - e0) * 2, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_offsets[slot].p, batch->offsets + r0, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_lens[slot].p, batch->full_lens + r0, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_coff[slot].p, batch->calib_offset + r0, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_cscale[slot].p, batch->calib_scale + r0, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaEventRecord(c->p_copied[slot], cs));
-        CUDA_TRY(cudaStreamWaitEvent(ks, c->p_copied[slot], 0));
-        adb_batch d = *batch;
-        // offsets stay absolute: rebase the blob pointer so that blob[offsets[i]] is the staged copy
-        d.signal = (const int16_t *)c->p_signal[slot].p - e0;
-        d.offsets = (const int64_t *)c->p_offsets[slot].p;
-        d.full_lens = (const int32_t *)c->p_lens[slot].p;
-        d.calib_offset = (const float *)c->p_coff[slot].p;
-        d.calib_scale = (const float *)c->p_cscale[slot].p;
-        d.n_reads = nr;
-        if (!ctx->opt_copy_only) {
-            rc = adb_detect_dev(c, &d, cfg, w_devs[ch & 1], (adb_record *)c->p_records[slot].p, (int *)c->p_status[slot].p, ks);
-            if (rc) return rc;
-        }
-        CUDA_TRY(cudaMemcpyAsync(out_records + r0, c->p_records[slot].p, sizeof(adb_record) * (size_t)nr, cudaMemcpyDeviceToHost, ks));
-        if (batch_status)
-            CUDA_TRY(cudaMemcpyAsync(batch_status + b0, c->p_status[slot].p, sizeof(int) * (size_t)nb, cudaMemcpyDeviceToHost, ks));
-        CUDA_TRY(cudaEventRecord(c->p_done[slot], ks));
-        b0 += sched[ch];
-    }
-    if (ctx->twin) CUDA_TRY(cudaStreamSynchronize(ctx->twin->stream));
-    cudaStream_t ks = ctx->stream;
-    CUDA_TRY(cudaStreamSynchronize(ks));
-    CUDA_TRY(cudaStreamSynchronize(cs));
     return ADB_OK;
 }
 
@@ -1193,11 +1089,13 @@ extern "C" int adb_cnn_scores_host(adb_ctx *ctx, const float *x, int32_t n, int3
     D.L1 = (L + 2 * 3 - CNN_K) / 3 + 1;
     D.LP = (D.L1 + 3) & ~3;
     D.Lout = (D.L1 - 1) * 3 - 2 * 3 + CNN_K;
-    if (ctx->cnn_x.ensure(sizeof(float) * (size_t)n * L) || ctx->cnn_scores.ensure(sizeof(float) * (size_t)n * 2 * D.Lout) ||
-        ctx->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc cnn buffers"); return ADB_ERR_CUDA; }
+    if (ctx->cnn_x.ensure(sizeof(float) * (size_t)n * L) || ctx->cnn_scores.ensure(sizeof(float) * (size_t)n * 2 * D.Lout))
+        { set_err("cudaMalloc cnn buffers"); return ADB_ERR_CUDA; }
     CUDA_TRY(cudaMemcpyAsync(ctx->cnn_x.p, x, sizeof(float) * (size_t)n * L, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, st));
-    int rc = cnn_forward_dev(ctx, (const float *)ctx->cnn_x.p, n, D, (const float *)ctx->h_misc2.p, (float *)ctx->cnn_scores.p, st);
+    const float *w_dev = nullptr;
+    int rc = upload_cnn_weights(ctx, cnn_weights, &w_dev);
+    if (rc) return rc;
+    rc = cnn_forward_dev(ctx, (const float *)ctx->cnn_x.p, n, D, w_dev, (float *)ctx->cnn_scores.p, st);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(scores, ctx->cnn_scores.p, sizeof(float) * (size_t)n * 2 * D.Lout, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));

@@ -753,7 +753,7 @@ static int cnn_forward_dev(adb_ctx *ctx, const float *x, int n, const CnnDims &D
     CUDA_TRY(cudaFuncSetAttribute(cnn_conv64_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_TRY(cudaFuncSetAttribute(cnn_conv64_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     float *a0 = (float *)ctx->cnn_act0.p, *a1 = (float *)ctx->cnn_act1.p;
-    const bool use_tc = !ctx->opt_cnn_fp32;
+    const bool use_tc = !ctx->opt.cnn_fp32;
     __half *wtc = nullptr;
     unsigned char *a0t = nullptr;
     int *redo = nullptr;

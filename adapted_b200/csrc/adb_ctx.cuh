@@ -46,6 +46,25 @@ struct DevBuf {
     }
 };
 
+// adb_ctx_set_option switches; the pipelined entry points copy them onto the twin in one assignment
+struct AdbOptions {
+    int copy_only = 0;           // "pipeline_copy_only": pipelined entry points skip the kernels
+    int no_fast_validate = 0;    // "no_fast_validate"
+    int hist_validate = 1;       // "hist_validate" 0: counting passes (validate_fast_kernel) instead of the tensor-core histograms (adb_vhist.cuh)
+    int no_cand_followup = 0;    // "no_cand_followup": further poly(A) candidates go to validate_kernel (A/B)
+    int cnn_fp32 = 0;            // "cnn_fp32_pipe": 64->64 convolutions on the FP32 pipe instead of tcgen05
+    int exact_gsel = 0;          // "exact_global_select": always use the multi-pass select
+    int host_zstd = 0;           // "host_zstd": adb_detect_files decompresses zstd frames on the host (A/B)
+};
+
+// device staging of one chunk of the pipelined entry points (adb_ingest.cuh)
+struct ChunkBufs {
+    DevBuf signal, offsets, lens, coff, cscale, records, status;
+    DevBuf comp, coffs, nsamp;  // svb16 streams, their offsets, samples per read
+    DevBuf frames, foffs, zstat;  // zstd frames, their offsets, per-frame status
+    cudaEvent_t copied = nullptr, done = nullptr;  // the chunk's H2D copies / its D2H copies have finished
+};
+
 struct adb_ctx {
     int device = 0;
     int sm_count = 0;
@@ -62,16 +81,12 @@ struct adb_ctx {
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[8];  // see ADB_TC_* in adb_api.cu
     double timing_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     int64_t timing_n[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    // double-buffered staging for the pipelined host entry point
-    DevBuf p_signal[2], p_offsets[2], p_lens[2], p_coff[2], p_cscale[2], p_records[2], p_status[2];
-    DevBuf p_comp[2], p_coffs[2], p_nsamp[2];  // compressed ingest: svb16 streams, their offsets, samples per read
-    DevBuf p_frames[2], p_foffs[2], p_zstat[2];  // VBZ ingest: zstd frames, their offsets, per-frame status
-    DevBuf z_fail;                                 // VBZ ingest: frames the device refused (one counter per call)
-    int opt_copy_only = 0;     // adb_ctx_set_option("pipeline_copy_only"): pipelined entry points skip the kernels
+    AdbOptions opt;
+    ChunkBufs p[2];  // double-buffered staging for the pipelined entry points
+    DevBuf z_fail;   // VBZ ingest: frames the device refused
     // pinned slot ring of adb_detect_files, kept between calls (pinning gigabytes costs seconds)
     void *file_ring = nullptr;
     void (*file_ring_free)(void *) = nullptr;
-    cudaEvent_t p_done[2] = {nullptr, nullptr}, p_copied[2] = {nullptr, nullptr};
     // scratch (device)
     DevBuf states, hist, series, given, status;
     DevBuf gsb_plan, gsb_hist, gsb_tab, gsb_bases, gsb_active;  // sampled one-pass global select
@@ -79,16 +94,10 @@ struct adb_ctx {
     DevBuf llr_cc;             // prefix sums of llr_primary_kernel (per resident CTA)
     DevBuf vf_done;            // per-read flags of validate_fast_kernel
     int ct_slot = -1;          // this context's slot of the constant bank adb_c_convT (adb_cnn_tc.cuh), -1: none left
-    int opt_no_fast_validate = 0;
-    int opt_hist_validate = 1;  // adb_ctx_set_option("hist_validate", 0): counting passes (validate_fast_kernel) instead of the tensor-core histograms (adb_vhist.cuh)
-    int opt_no_cand_followup = 0;  // adb_ctx_set_option("no_cand_followup"): further poly(A) candidates go to validate_kernel (A/B)
     int cnn_a0t_l1 = -1;       // L1 the tile-layout activation buffer was last zeroed for
-    int opt_cnn_fp32 = 0;      // adb_ctx_set_option("cnn_fp32_pipe"): 64->64 convolutions on the FP32 pipe instead of tcgen05
     int vf_last_reads = 0;
     int gsb_last_batches = 0;
-    int opt_exact_gsel = 0;
-    int opt_host_zstd = 0;        // adb_ctx_set_option("host_zstd"): adb_detect_files decompresses zstd frames on the host (A/B)
-    int64_t zstd_host_frames = 0;  // adb_ctx_query("zstd_host_frames"): frames the last call decompressed on the host  // adb_ctx_set_option("exact_global_select"): always use the multi-pass select
+    int64_t zstd_host_frames = 0;  // adb_ctx_query("zstd_host_frames"): frames the last call decompressed on the host
     DevBuf cnn_x, cnn_act0, cnn_act1, cnn_scores, cnn_w, cnn_aux, cnn_post, sp_rows, cnn_wtc, cnn_a0t, cnn_ct;
     DevBuf val_cc;  // hail-mary prefix sums of the unstaged validate_kernel: [grid][2][nds_max] doubles
     // staging for the *_host entry points

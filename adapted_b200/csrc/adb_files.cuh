@@ -150,7 +150,7 @@ struct Slot {
     adb_record *recs = nullptr;
     int nr = 0, nb = 0;
     size_t comp_bytes = 0, dec_bytes = 0;
-    int svb = 1;  // 0: raw int16, 1: svb16 streams, 2: zstd frames of svb16 streams (decoded on the device)
+    int rep = CHUNK_SVB16;  // CHUNK_RAW, CHUNK_SVB16 or CHUNK_ZSTD (zstd frames of svb16 streams, decoded on the device)
     bool last = false;
     int error = 0;
     cudaEvent_t done = nullptr;
@@ -222,20 +222,10 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
     if (any_zstd && !zstd.load()) { set_err("container is zstd-compressed and libzstd.so.1 cannot be loaded"); return ADB_ERR_UNSUPPORTED; }
 
     CUDA_TRY(cudaSetDevice(ctx->device));
-    if (!ctx->twin) { rc = adb_ctx_create(ctx->device, &ctx->twin); if (rc) return rc; }
-    ctx->twin->opt_no_fast_validate = ctx->opt_no_fast_validate;
-        ctx->twin->opt_hist_validate = ctx->opt_hist_validate;
-    ctx->twin->opt_cnn_fp32 = ctx->opt_cnn_fp32;
-    ctx->twin->opt_exact_gsel = ctx->opt_exact_gsel;
-        ctx->twin->opt_no_cand_followup = ctx->opt_no_cand_followup;
-    adb_ctx *cc[2] = {ctx, ctx->twin};
-    const float *w_devs[2] = {nullptr, nullptr};
-    if (cfg->primary_method == ADB_METHOD_CNN)
-        for (int k = 0; k < 2; k++) {
-            if (cc[k]->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc weights"); return ADB_ERR_CUDA; }
-            CUDA_TRY(cudaMemcpyAsync(cc[k]->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, cc[k]->stream));
-            w_devs[k] = (const float *)cc[k]->h_misc2.p;
-        }
+    adb_ctx *cc[2];
+    const float *w_devs[2];
+    rc = pair_setup(ctx, true, cfg, cnn_weights, cc, w_devs);
+    if (rc) return rc;
 
     // ---- the pinned ring (kept in the context between calls) ----
     const int n_slots = 4;
@@ -286,14 +276,14 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
     };
     double read_s = 0.0, write_s = 0.0, gpu_wait_s = 0.0;
     std::atomic<long long> comp_total{0}, host_frames{0};
-    const bool device_zstd = !ctx->opt_host_zstd;
+    const bool device_zstd = !ctx->opt.host_zstd;
 
     // ---- reader ----
     std::thread reader([&]() {
         std::vector<CopyJob> jobs;
         Slot *s = q_free.pop();
         s->nr = 0; s->comp_bytes = 0; s->dec_bytes = 0; s->last = false; s->error = 0;
-        s->svb = 1;
+        s->rep = CHUNK_SVB16;
         auto flush = [&](bool last) {
             const double t0 = now_s();
             s->nb = (s->nr + mbs - 1) / mbs;
@@ -326,13 +316,13 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
             work();
             for (auto &t : pool) t.join();
             jobs.clear();
-            if (s->svb == 1) memset(s->comp + s->comp_bytes, 0, 16);  // the slack behind the last stream
+            if (s->rep == CHUNK_SVB16) memset(s->comp + s->comp_bytes, 0, 16);  // the slack behind the last stream
             comp_total += (long long)s->comp_bytes;
             read_s += now_s() - t0;
             q_filled.push(s);
             if (!last) {
                 s = q_free.pop();
-                s->nr = 0; s->comp_bytes = 0; s->dec_bytes = 0; s->last = false; s->error = 0; s->svb = 1;
+                s->nr = 0; s->comp_bytes = 0; s->dec_bytes = 0; s->last = false; s->error = 0; s->rep = CHUNK_SVB16;
             }
         };
         for (int fi = 0; fi < (int)files.size() && !failed.load(); fi++) {
@@ -350,9 +340,9 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
                 // an svb16 stream in one zstd frame that the device takes travels as it is (no host decompression)
                 uint64_t zcs = 0;
                 const bool zdev = zs && svb && device_zstd && zstd_screen(src, bytes, per_read_cap * 4, &zcs);
-                const int rep = zdev ? 2 : (svb ? 1 : 0);
-                if (s->nr > 0 && s->svb != rep) flush(false);  // a chunk holds one representation
-                s->svb = rep;
+                const int rep = zdev ? CHUNK_ZSTD : (svb ? CHUNK_SVB16 : CHUNK_RAW);
+                if (s->nr > 0 && s->rep != rep) flush(false);  // a chunk holds one representation
+                s->rep = rep;
                 const int k = s->nr;
                 if (zdev) {
                     if (f.nsamp[r] > m) { fail(ADB_ERR_UNSUPPORTED, "compressed read longer than sig_preload_size in the container"); break; }
@@ -494,7 +484,7 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
             if (s->nr > 0 && !s->error && cudaEventSynchronize(s->done) != cudaSuccess) fail(ADB_ERR_CUDA, "cudaEventSynchronize failed in the writer");
             gpu_wait_s += now_s() - t0;
             const double t1 = now_s();
-            if (!s->error && s->nr > 0 && s->svb == 2 && *s->zfail != 0)
+            if (!s->error && s->nr > 0 && s->rep == CHUNK_ZSTD && *s->zfail != 0)
                 fail(ADB_ERR_ARG, "zstd frame of a read does not decompress to its stated size");
             if (!s->error && !failed.load()) {
                 for (int b = 0; b < s->nb; b++) {
@@ -590,74 +580,31 @@ extern "C" int adb_detect_files(adb_ctx *ctx, const adb_file_job *job, const adb
         cudaStream_t ks = c->stream;
         const int nr = s->nr;
         if (nr > 0 && !s->error && !failed.load()) {
-            int e = ADB_OK;
+            ChunkDesc k;
+            k.rep = s->rep;
+            k.payload = s->comp;
+            k.payload_bytes = s->comp_bytes + (s->rep == CHUNK_SVB16 ? 16 : 0);  // svb16: the slack behind the last stream
+            k.offsets = s->rep == CHUNK_ZSTD ? s->foffs : s->coffs;
+            k.dec_offsets = s->coffs;
+            k.n_samples = s->nsamp; k.full_lens = s->lens; k.calib_offset = s->coff; k.calib_scale = s->cscale;
+            k.nr = nr; k.nb = s->nb; k.m = m; k.batch_size = mbs;
             auto step = [&]() -> int {
-                // the device buffers of this context are free once its previous chunk has finished
-                if (ch >= 2) CUDA_TRY(cudaEventSynchronize(c->p_done[0]));
-                const size_t cbytes = s->comp_bytes + 16;
-                size_t dec_samples = 0;
-                // (the svb16 streams of a zstd chunk are laid out in p_comp after the zstd decode)
-                for (int i = 0; i < nr; i++) dec_samples += (size_t)s->nsamp[i];
-                if (c->p_comp[0].ensure(cbytes + 64) || c->p_coffs[0].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
-                    c->p_nsamp[0].ensure(sizeof(int32_t) * (size_t)nr + 16) || c->p_signal[0].ensure(dec_samples * 2 + 64) ||
-                    c->p_offsets[0].ensure(sizeof(int64_t) * ((size_t)nr + 1)) || c->p_lens[0].ensure(sizeof(int32_t) * (size_t)nr + 16) ||
-                    c->p_coff[0].ensure(sizeof(float) * (size_t)nr + 16) || c->p_cscale[0].ensure(sizeof(float) * (size_t)nr + 16) ||
-                    c->p_records[0].ensure(sizeof(adb_record) * (size_t)nr) || c->p_status[0].ensure(sizeof(int) * (size_t)s->nb + 16)) {
-                    set_err("cudaMalloc pipeline staging");
-                    return ADB_ERR_CUDA;
+                // zstd: the frames the device refuses, counted per chunk and read by the writer with the records
+                int32_t *z_fail = nullptr;
+                if (s->rep == CHUNK_ZSTD) {
+                    if (c->z_fail.ensure(16)) { set_err("cudaMalloc pipeline staging"); return ADB_ERR_CUDA; }
+                    z_fail = (int32_t *)c->z_fail.p;
+                    CUDA_TRY(cudaMemsetAsync(z_fail, 0, sizeof(int32_t), ks));
                 }
-                if (s->svb == 2) {  // zstd frames -> zstd_decode_kernel -> svb16 streams in p_comp
-                    if (c->p_frames[0].ensure(s->comp_bytes + 16) || c->p_foffs[0].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
-                        c->p_comp[0].ensure(s->dec_bytes + 64) || c->p_zstat[0].ensure(sizeof(int32_t) * (size_t)nr + 16) ||
-                        c->z_fail.ensure(16)) {
-                        set_err("cudaMalloc pipeline staging");
-                        return ADB_ERR_CUDA;
-                    }
-                    CUDA_TRY(cudaMemcpyAsync(c->p_frames[0].p, s->comp, s->comp_bytes, cudaMemcpyHostToDevice, cs));
-                    CUDA_TRY(cudaMemcpyAsync(c->p_foffs[0].p, s->foffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-                    CUDA_TRY(cudaMemcpyAsync(c->p_coffs[0].p, s->coffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-                    h2d_bytes += (long long)(s->comp_bytes + (size_t)nr * 8);
-                } else {
-                    void *sig_dst = s->svb ? c->p_comp[0].p : c->p_signal[0].p;
-                    CUDA_TRY(cudaMemcpyAsync(sig_dst, s->comp, s->svb ? cbytes : s->comp_bytes, cudaMemcpyHostToDevice, cs));
-                    CUDA_TRY(cudaMemcpyAsync(s->svb ? c->p_coffs[0].p : c->p_offsets[0].p, s->coffs, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-                    h2d_bytes += (long long)cbytes;
-                }
-                CUDA_TRY(cudaMemcpyAsync(c->p_nsamp[0].p, s->nsamp, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-                CUDA_TRY(cudaMemcpyAsync(c->p_lens[0].p, s->lens, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-                CUDA_TRY(cudaMemcpyAsync(c->p_coff[0].p, s->coff, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-                CUDA_TRY(cudaMemcpyAsync(c->p_cscale[0].p, s->cscale, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-                CUDA_TRY(cudaEventRecord(c->p_copied[0], cs));
-                CUDA_TRY(cudaStreamWaitEvent(ks, c->p_copied[0], 0));
-                h2d_bytes += (long long)((size_t)nr * 28);
-                if (s->svb == 2) {
-                    CUDA_TRY(cudaMemsetAsync(c->z_fail.p, 0, sizeof(int32_t), ks));
-                    CUDA_TRY(cudaMemsetAsync((uint8_t *)c->p_comp[0].p + s->dec_bytes, 0, 16, ks));  // the slack behind the last stream
-                    int r1 = launch_zstd_decode(c, (const uint8_t *)c->p_frames[0].p, (const int64_t *)c->p_foffs[0].p, (uint8_t *)c->p_comp[0].p,
-                                                (const int64_t *)c->p_coffs[0].p, (int32_t *)c->p_zstat[0].p, (int32_t *)c->z_fail.p, nr, ks);
-                    if (r1) return r1;
-                    CUDA_TRY(cudaMemcpyAsync(s->zfail, c->z_fail.p, sizeof(int32_t), cudaMemcpyDeviceToHost, ks));
-                }
-                if (s->svb) {
-                    int r2 = launch_svb_decode(c, (const uint8_t *)c->p_comp[0].p, (const int64_t *)c->p_coffs[0].p,
-                                               (const int32_t *)c->p_nsamp[0].p, nr, (int64_t *)c->p_offsets[0].p,
-                                               (int16_t *)c->p_signal[0].p, ks);
-                    if (r2) return r2;
-                }
-                adb_batch d;
-                d.signal = c->p_signal[0].p; d.sig_type = ADB_SIG_I16; d.n_reads = nr; d.m = m; d.batch_size = mbs;
-                d.offsets = (const int64_t *)c->p_offsets[0].p; d.full_lens = (const int32_t *)c->p_lens[0].p;
-                d.calib_offset = (const float *)c->p_coff[0].p; d.calib_scale = (const float *)c->p_cscale[0].p;
-                int r3 = adb_detect_dev(c, &d, cfg, w_devs[ch & 1], (adb_record *)c->p_records[0].p, (int *)c->p_status[0].p, ks);
-                if (r3) return r3;
-                CUDA_TRY(cudaMemcpyAsync(s->recs, c->p_records[0].p, sizeof(adb_record) * (size_t)nr, cudaMemcpyDeviceToHost, ks));
-                CUDA_TRY(cudaMemcpyAsync(s->status, c->p_status[0].p, sizeof(int) * (size_t)s->nb, cudaMemcpyDeviceToHost, ks));
-                CUDA_TRY(cudaEventRecord(c->p_done[0], ks));
+                int rc2 = enqueue_chunk(c, 0, cs, k, cfg, w_devs[ch & 1], z_fail, true, s->recs, s->status);
+                if (rc2) return rc2;
+                if (z_fail) CUDA_TRY(cudaMemcpyAsync(s->zfail, z_fail, sizeof(int32_t), cudaMemcpyDeviceToHost, ks));
                 CUDA_TRY(cudaEventRecord(s->done, ks));
                 return ADB_OK;
             };
-            e = step();
+            const int e = step();
             if (e) { fail(e, adb_err_string()); s->error = 1; }
+            else h2d_bytes += (long long)(s->comp_bytes + (s->rep == CHUNK_ZSTD ? (size_t)nr * 8 : 16) + (size_t)nr * 28);
         } else if (failed.load()) {
             s->error = 1;
         }

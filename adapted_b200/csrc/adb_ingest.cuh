@@ -38,6 +38,10 @@ static int check_svb_batch(const adb_svb_batch *b) {
         set_err("invalid adb_svb_batch");
         return ADB_ERR_ARG;
     }
+    // one branch-free pass (it vectorizes): the pipelined calls run it before their first copy
+    int outside = 0;
+    for (int i = 0; i < b->n_reads; i++) outside |= (uint32_t)b->n_samples[i] > (uint32_t)b->m;
+    if (outside) { set_err("n_samples outside [0, m]"); return ADB_ERR_ARG; }
     return ADB_OK;
 }
 
@@ -87,22 +91,23 @@ extern "C" int adb_zstd_decompress_host(adb_ctx *ctx, const uint8_t *src, const 
     cudaStream_t st = ctx->stream;
     StreamDrain drain;
     drain.add(st);
+    ChunkBufs &b = ctx->p[0];
     const int64_t s0 = src_offsets[0], d0 = dst_offsets[0];
     const size_t sbytes = (size_t)(src_offsets[n] - s0), dbytes = (size_t)(dst_offsets[n] - d0);
-    if (ctx->p_frames[0].ensure(sbytes + 16) || ctx->p_foffs[0].ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
-        ctx->p_comp[0].ensure(dbytes + 16) || ctx->p_coffs[0].ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
-        ctx->p_zstat[0].ensure(sizeof(int32_t) * (size_t)n + 16)) { set_err("cudaMalloc zstd staging"); return ADB_ERR_CUDA; }
-    if (sbytes) CUDA_TRY(cudaMemcpyAsync(ctx->p_frames[0].p, src + s0, sbytes, cudaMemcpyHostToDevice, st));
+    if (b.frames.ensure(sbytes + 16) || b.foffs.ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
+        b.comp.ensure(dbytes + 16) || b.coffs.ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
+        b.zstat.ensure(sizeof(int32_t) * (size_t)n + 16)) { set_err("cudaMalloc zstd staging"); return ADB_ERR_CUDA; }
+    if (sbytes) CUDA_TRY(cudaMemcpyAsync(b.frames.p, src + s0, sbytes, cudaMemcpyHostToDevice, st));
     // the slots start as the caller left them: bytes the decoder does not write come back unchanged
-    if (dbytes) CUDA_TRY(cudaMemcpyAsync(ctx->p_comp[0].p, dst + d0, dbytes, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->p_foffs[0].p, src_offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->p_coffs[0].p, dst_offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, st));
-    int rc = launch_zstd_decode(ctx, (const uint8_t *)ctx->p_frames[0].p - s0, (const int64_t *)ctx->p_foffs[0].p,
-                                (uint8_t *)ctx->p_comp[0].p - d0, (const int64_t *)ctx->p_coffs[0].p, (int32_t *)ctx->p_zstat[0].p,
+    if (dbytes) CUDA_TRY(cudaMemcpyAsync(b.comp.p, dst + d0, dbytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b.foffs.p, src_offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b.coffs.p, dst_offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, st));
+    int rc = launch_zstd_decode(ctx, (const uint8_t *)b.frames.p - s0, (const int64_t *)b.foffs.p,
+                                (uint8_t *)b.comp.p - d0, (const int64_t *)b.coffs.p, (int32_t *)b.zstat.p,
                                 nullptr, n, st);
     if (rc) return rc;
-    if (dbytes) CUDA_TRY(cudaMemcpyAsync(dst + d0, ctx->p_comp[0].p, dbytes, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(status, ctx->p_zstat[0].p, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
+    if (dbytes) CUDA_TRY(cudaMemcpyAsync(dst + d0, b.comp.p, dbytes, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(status, b.zstat.p, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     drain.armed = false;
     return ADB_OK;
@@ -115,26 +120,24 @@ extern "C" int adb_svb16_decode_host(adb_ctx *ctx, const adb_svb_batch *batch, i
     const int n = batch->n_reads;
     if (n == 0) return ADB_OK;
     int64_t total = 0;
-    for (int i = 0; i < n; i++) {
-        if (batch->n_samples[i] < 0 || batch->n_samples[i] > batch->m) { set_err("n_samples outside [0, m]"); return ADB_ERR_ARG; }
-        total += batch->n_samples[i];
-    }
+    for (int i = 0; i < n; i++) total += batch->n_samples[i];
     CUDA_TRY(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     StreamDrain drain;
     drain.add(st);
+    ChunkBufs &b = ctx->p[0];
     const int64_t c0 = batch->comp_offsets[0], c1 = batch->comp_offsets[n];
     const size_t cbytes = (size_t)(c1 - c0) + 16;
-    if (ctx->p_comp[0].ensure(cbytes + 64) || ctx->p_coffs[0].ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
-        ctx->p_nsamp[0].ensure(sizeof(int32_t) * (size_t)n + 16) || ctx->p_offsets[0].ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
-        ctx->p_signal[0].ensure((size_t)total * 2 + 64)) { set_err("cudaMalloc svb16 staging"); return ADB_ERR_CUDA; }
-    CUDA_TRY(cudaMemcpyAsync(ctx->p_comp[0].p, batch->comp + c0, cbytes, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->p_coffs[0].p, batch->comp_offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(ctx->p_nsamp[0].p, batch->n_samples, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-    rc = launch_svb_decode(ctx, (const uint8_t *)ctx->p_comp[0].p - c0, (const int64_t *)ctx->p_coffs[0].p,
-                           (const int32_t *)ctx->p_nsamp[0].p, n, (int64_t *)ctx->p_offsets[0].p, (int16_t *)ctx->p_signal[0].p, st);
+    if (b.comp.ensure(cbytes + 64) || b.coffs.ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
+        b.nsamp.ensure(sizeof(int32_t) * (size_t)n + 16) || b.offsets.ensure(sizeof(int64_t) * ((size_t)n + 1)) ||
+        b.signal.ensure((size_t)total * 2 + 64)) { set_err("cudaMalloc svb16 staging"); return ADB_ERR_CUDA; }
+    CUDA_TRY(cudaMemcpyAsync(b.comp.p, batch->comp + c0, cbytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b.coffs.p, batch->comp_offsets, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(b.nsamp.p, batch->n_samples, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
+    rc = launch_svb_decode(ctx, (const uint8_t *)b.comp.p - c0, (const int64_t *)b.coffs.p,
+                           (const int32_t *)b.nsamp.p, n, (int64_t *)b.offsets.p, (int16_t *)b.signal.p, st);
     if (rc) return rc;
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(out_adc, ctx->p_signal[0].p, (size_t)total * 2, cudaMemcpyDeviceToHost, st));
+    if (total > 0) CUDA_TRY(cudaMemcpyAsync(out_adc, b.signal.p, (size_t)total * 2, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     drain.armed = false;
     return ADB_OK;
@@ -156,6 +159,178 @@ static std::vector<int> pipeline_schedule(int n_batches, int chunk_batches) {
     return sched;
 }
 
+// Before the first chunk of a pipelined call: create the twin when `want_twin` asks for it (consecutive chunks
+// alternate between ctx and its twin: own compute stream, own scratch), give the twin the options of ctx, and upload
+// the CNN weights to every context in use.  Without a twin, cc[1] and w_devs[1] repeat cc[0] and w_devs[0].
+static int pair_setup(adb_ctx *ctx, bool want_twin, const adb_config *cfg, const float *cnn_weights, adb_ctx *cc[2],
+                      const float *w_devs[2]) {
+    if (cfg->primary_method == ADB_METHOD_CNN && !cnn_weights) { set_err("cnn_weights required"); return ADB_ERR_ARG; }
+    if (want_twin && !ctx->twin) {
+        int rc = adb_ctx_create(ctx->device, &ctx->twin);
+        if (rc) return rc;
+    }
+    if (ctx->twin) ctx->twin->opt = ctx->opt;
+    cc[0] = ctx;
+    cc[1] = ctx->twin ? ctx->twin : ctx;
+    w_devs[0] = w_devs[1] = nullptr;
+    if (cfg->primary_method != ADB_METHOD_CNN) return ADB_OK;
+    for (int k = 0; k < (ctx->twin ? 2 : 1); k++) {
+        int rc = upload_cnn_weights(cc[k], cnn_weights, &w_devs[k]);
+        if (rc) return rc;
+    }
+    if (!ctx->twin) w_devs[1] = w_devs[0];
+    return ADB_OK;
+}
+
+enum { CHUNK_RAW = 0, CHUNK_SVB16 = 1, CHUNK_ZSTD = 2 };
+
+// One chunk of reads in host memory.  The offsets may index a larger buffer: the chunk's payload starts at offsets[0]
+// (dec_offsets[0] for the decoded streams), and the staged copies are addressed through pointers rebased by it.
+struct ChunkDesc {
+    int rep = CHUNK_RAW;  // raw int16 samples, svb16 streams, or one zstd frame per read over its svb16 stream
+    const void *payload = nullptr;
+    size_t payload_bytes = 0;              // svb16: with the 16 bytes of slack behind the last stream
+    const int64_t *offsets = nullptr;      // [nr + 1] samples (raw), streams (svb16) or frames (zstd)
+    const int64_t *dec_offsets = nullptr;  // zstd: [nr + 1] 16-byte aligned slots of the decoded svb16 streams
+    const int32_t *n_samples = nullptr;    // [nr] samples per read; raw chunks may leave it null
+    const int32_t *full_lens = nullptr;
+    const float *calib_offset = nullptr, *calib_scale = nullptr;
+    int nr = 0, nb = 0, m = 0, batch_size = 0;
+};
+
+// Stages chunk k in slot `slot` of context c and enqueues all of its work.  The H2D copies go on the copy stream cs;
+// on c's stream follow the zstd decode (refused frames counted in z_fail) and the svb16 decode that k.rep needs,
+// detection (skipped when !run), and the D2H copies of the records and, when out_status is given, the minibatch status.
+static int enqueue_chunk(adb_ctx *c, int slot, cudaStream_t cs, const ChunkDesc &k, const adb_config *cfg, const float *w_dev,
+                         int32_t *z_fail, bool run, adb_record *out_records, int32_t *out_status) {
+    ChunkBufs &b = c->p[slot];
+    const cudaStream_t ks = c->stream;
+    const int nr = k.nr;
+    const size_t n8 = sizeof(int64_t) * ((size_t)nr + 1), n4 = sizeof(int32_t) * (size_t)nr;
+    // the decoded reads: the raw payload, or n_samples in total (counted while the slot's previous chunk still runs)
+    size_t sig_bytes = k.payload_bytes;
+    if (k.rep != CHUNK_RAW) {
+        int64_t samples = 0;
+        for (int i = 0; i < nr; i++) samples += k.n_samples[i];
+        sig_bytes = 2 * (size_t)samples;
+    }
+    // the slot is free once the chunk that used it last has been copied back
+    CUDA_TRY(cudaEventSynchronize(b.done));
+    const int64_t dec0 = k.rep == CHUNK_ZSTD ? k.dec_offsets[0] : 0, dec_bytes = k.rep == CHUNK_ZSTD ? k.dec_offsets[nr] - dec0 : 0;
+    DevBuf &in = k.rep == CHUNK_ZSTD ? b.frames : k.rep == CHUNK_SVB16 ? b.comp : b.signal;
+    DevBuf &in_off = k.rep == CHUNK_ZSTD ? b.foffs : k.rep == CHUNK_SVB16 ? b.coffs : b.offsets;
+    if (b.signal.ensure(sig_bytes + 64) || b.offsets.ensure(n8) || b.lens.ensure(n4 + 16) || b.coff.ensure(n4 + 16) ||
+        b.cscale.ensure(n4 + 16) || b.records.ensure(sizeof(adb_record) * (size_t)nr) || b.status.ensure(sizeof(int) * (size_t)k.nb + 16) ||
+        (k.n_samples && b.nsamp.ensure(n4 + 16)) ||
+        (k.rep != CHUNK_RAW && (b.coffs.ensure(n8) || b.comp.ensure((k.rep == CHUNK_ZSTD ? (size_t)dec_bytes : k.payload_bytes) + 64))) ||
+        (k.rep == CHUNK_ZSTD && (b.frames.ensure(k.payload_bytes + 16) || b.foffs.ensure(n8) || b.zstat.ensure(n4 + 16)))) {
+        set_err("cudaMalloc pipeline staging");
+        return ADB_ERR_CUDA;
+    }
+    CUDA_TRY(cudaMemcpyAsync(in.p, k.payload, k.payload_bytes, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaMemcpyAsync(in_off.p, k.offsets, n8, cudaMemcpyHostToDevice, cs));
+    if (k.rep == CHUNK_ZSTD) CUDA_TRY(cudaMemcpyAsync(b.coffs.p, k.dec_offsets, n8, cudaMemcpyHostToDevice, cs));
+    if (k.n_samples) CUDA_TRY(cudaMemcpyAsync(b.nsamp.p, k.n_samples, n4, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaMemcpyAsync(b.lens.p, k.full_lens, n4, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaMemcpyAsync(b.coff.p, k.calib_offset, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaMemcpyAsync(b.cscale.p, k.calib_scale, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
+    CUDA_TRY(cudaEventRecord(b.copied, cs));
+    CUDA_TRY(cudaStreamWaitEvent(ks, b.copied, 0));
+    if (run) {
+        const int64_t base = k.offsets[0];
+        const int16_t *signal = (const int16_t *)b.signal.p;
+        int rc = ADB_OK;
+        if (k.rep == CHUNK_RAW) {
+            signal -= base;  // the offsets stay as given
+        } else {
+            const uint8_t *streams = (const uint8_t *)b.comp.p - base;
+            if (k.rep == CHUNK_ZSTD) {
+                uint8_t *dec = (uint8_t *)b.comp.p - dec0;
+                CUDA_TRY(cudaMemsetAsync((uint8_t *)b.comp.p + dec_bytes, 0, 16, ks));  // the slack behind the last stream
+                rc = launch_zstd_decode(c, (const uint8_t *)b.frames.p - base, (const int64_t *)b.foffs.p, dec,
+                                        (const int64_t *)b.coffs.p, (int32_t *)b.zstat.p, z_fail, nr, ks);
+                if (rc) return rc;
+                streams = dec;
+            }
+            rc = launch_svb_decode(c, streams, (const int64_t *)b.coffs.p, (const int32_t *)b.nsamp.p, nr, (int64_t *)b.offsets.p,
+                                   (int16_t *)b.signal.p, ks);
+            if (rc) return rc;
+        }
+        adb_batch d;
+        d.signal = signal; d.sig_type = ADB_SIG_I16; d.n_reads = nr; d.m = k.m; d.batch_size = k.batch_size;
+        d.offsets = (const int64_t *)b.offsets.p; d.full_lens = (const int32_t *)b.lens.p;
+        d.calib_offset = (const float *)b.coff.p; d.calib_scale = (const float *)b.cscale.p;
+        rc = adb_detect_dev(c, &d, cfg, w_dev, (adb_record *)b.records.p, (int *)b.status.p, ks);
+        if (rc) return rc;
+    }
+    CUDA_TRY(cudaMemcpyAsync(out_records, b.records.p, sizeof(adb_record) * (size_t)nr, cudaMemcpyDeviceToHost, ks));
+    if (out_status) CUDA_TRY(cudaMemcpyAsync(out_status, b.status.p, sizeof(int) * (size_t)k.nb, cudaMemcpyDeviceToHost, ks));
+    CUDA_TRY(cudaEventRecord(b.done, ks));
+    return ADB_OK;
+}
+
+// The chunk loop of the pipelined host entry points.  Reads [r0, r1) of each scheduled chunk go through enqueue_chunk;
+// set_payload(k, r0, r1) fills in what depends on the input form.  All copies go through ctx's copy stream in order;
+// with a twin, every chunk of a context uses its slot 0, otherwise consecutive chunks alternate between ctx's slots.
+template <class Batch, class SetPayload>
+static int detect_pipelined(adb_ctx *ctx, const Batch &batch, const adb_config *cfg, const float *cnn_weights,
+                            adb_record *out_records, int32_t *batch_status, int32_t chunk_batches, int32_t *z_fail,
+                            SetPayload set_payload) {
+    const int bs = batch.batch_size;
+    const std::vector<int> sched = pipeline_schedule((batch.n_reads + bs - 1) / bs, std::max(1, chunk_batches));
+    adb_ctx *cc[2];
+    const float *w_devs[2];
+    int rc = pair_setup(ctx, sched.size() >= 3, cfg, cnn_weights, cc, w_devs);
+    if (rc) return rc;
+    cudaStream_t cs = ctx->copy_stream;
+    StreamDrain drain;
+    drain.add(cs);
+    drain.add(ctx->stream);
+    if (ctx->twin) drain.add(ctx->twin->stream);
+    for (int ch = 0, b0 = 0; ch < (int)sched.size(); b0 += sched[ch++]) {
+        const int r0 = b0 * bs, r1 = (int)std::min<long long>((long long)batch.n_reads, (long long)(b0 + sched[ch]) * bs);
+        ChunkDesc k;
+        k.nr = r1 - r0;
+        k.nb = (k.nr + bs - 1) / bs;
+        k.m = batch.m;
+        k.batch_size = bs;
+        k.full_lens = batch.full_lens + r0;
+        k.calib_offset = batch.calib_offset + r0;
+        k.calib_scale = batch.calib_scale + r0;
+        set_payload(k, r0, r1);
+        rc = enqueue_chunk(cc[ch & 1], ctx->twin ? 0 : (ch & 1), cs, k, cfg, w_devs[ch & 1], z_fail, !ctx->opt.copy_only,
+                           out_records + r0, batch_status ? batch_status + b0 : nullptr);
+        if (rc) return rc;
+    }
+    if (ctx->twin) CUDA_TRY(cudaStreamSynchronize(ctx->twin->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(cs));
+    drain.armed = false;
+    return ADB_OK;
+}
+
+// Pipelined ingest for long jobs: the reads are cut into chunks of `chunk_batches` minibatches; the H2D copy of
+// chunk i+1 (copy stream) overlaps the kernels of chunk i (compute stream), records return per chunk.  Host buffers
+// should be pinned (cudaHostAlloc / torch pin_memory) for the copies to be asynchronous.  I16 ragged input only.
+extern "C" int adb_detect_pipelined_host(adb_ctx *ctx, const adb_batch *batch, const adb_config *cfg,
+                                         const float *cnn_weights, adb_record *out_records, int32_t *batch_status,
+                                         int32_t chunk_batches) {
+    if (!ctx || !out_records) { set_err("null argument"); return ADB_ERR_ARG; }
+    int rc = check_batch(batch);
+    if (rc) return rc;
+    rc = check_config(cfg);
+    if (rc) return rc;
+    if (batch->sig_type != ADB_SIG_I16) { set_err("pipelined ingest takes ragged int16 input"); return ADB_ERR_ARG; }
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    if (batch->n_reads == 0) return ADB_OK;
+    return detect_pipelined(ctx, *batch, cfg, cnn_weights, out_records, batch_status, chunk_batches, nullptr,
+                            [&](ChunkDesc &k, int r0, int r1) {
+                                k.payload = (const int16_t *)batch->signal + batch->offsets[r0];
+                                k.payload_bytes = (size_t)(batch->offsets[r1] - batch->offsets[r0]) * 2;
+                                k.offsets = batch->offsets + r0;
+                            });
+}
+
 // adb_detect_pipelined_svb_host (vbz = false) and adb_detect_pipelined_vbz_host (vbz = true: batch->comp holds one
 // zstd frame per read, decoded on the device into the svb16 layout before svb16_decode_kernel)
 static int detect_pipelined_comp(adb_ctx *ctx, const adb_svb_batch *batch, const adb_config *cfg, const float *cnn_weights,
@@ -165,7 +340,6 @@ static int detect_pipelined_comp(adb_ctx *ctx, const adb_svb_batch *batch, const
     if (rc) return rc;
     rc = check_config(cfg);
     if (rc) return rc;
-    if (chunk_batches < 1) chunk_batches = 1;
     CUDA_TRY(cudaSetDevice(ctx->device));
     if (batch->n_reads == 0) return ADB_OK;
     // VBZ: every frame is screened on the host (content size -> layout of the decoded streams: 16-byte aligned, 16 bytes
@@ -184,120 +358,22 @@ static int detect_pipelined_comp(adb_ctx *ctx, const adb_svb_batch *batch, const
             }
             dec_off[i + 1] = dec_off[i] + (int64_t)((cs + 15) & ~(uint64_t)15);
         }
+        // one counter for the call and both contexts, cleared on the copy stream: every chunk's kernels wait for its copies
+        if (ctx->z_fail.ensure(16)) { set_err("cudaMalloc zstd counter"); return ADB_ERR_CUDA; }
+        CUDA_TRY(cudaMemsetAsync(ctx->z_fail.p, 0, sizeof(int32_t), ctx->copy_stream));
     }
-    if (vbz && ctx->z_fail.ensure(16)) { set_err("cudaMalloc zstd counter"); return ADB_ERR_CUDA; }
-    // (on the copy stream: every chunk's kernels wait for its copies)
-    if (vbz) CUDA_TRY(cudaMemsetAsync(ctx->z_fail.p, 0, sizeof(int32_t), ctx->copy_stream));
-    const int n_batches = (batch->n_reads + batch->batch_size - 1) / batch->batch_size;
-    const std::vector<int> sched = pipeline_schedule(n_batches, chunk_batches);
-    if (!ctx->twin && sched.size() >= 3) {
-        rc = adb_ctx_create(ctx->device, &ctx->twin);
-        if (rc) return rc;
-    }
-    if (ctx->twin) {
-        ctx->twin->opt_no_fast_validate = ctx->opt_no_fast_validate;
-        ctx->twin->opt_hist_validate = ctx->opt_hist_validate;
-        ctx->twin->opt_cnn_fp32 = ctx->opt_cnn_fp32;
-        ctx->twin->opt_exact_gsel = ctx->opt_exact_gsel;
-        ctx->twin->opt_no_cand_followup = ctx->opt_no_cand_followup;
-    }
-    adb_ctx *cc[2] = {ctx, ctx->twin ? ctx->twin : ctx};
-    const float *w_devs[2] = {nullptr, nullptr};
-    if (cfg->primary_method == ADB_METHOD_CNN) {
-        if (!cnn_weights) { set_err("cnn_weights required"); return ADB_ERR_ARG; }
-        for (int k = 0; k < (ctx->twin ? 2 : 1); k++) {
-            if (cc[k]->h_misc2.ensure(sizeof(float) * ADB_CNN_NPARAMS)) { set_err("cudaMalloc weights"); return ADB_ERR_CUDA; }
-            CUDA_TRY(cudaMemcpyAsync(cc[k]->h_misc2.p, cnn_weights, sizeof(float) * ADB_CNN_NPARAMS, cudaMemcpyHostToDevice, cc[k]->stream));
-            w_devs[k] = (const float *)cc[k]->h_misc2.p;
-        }
-        if (!ctx->twin) w_devs[1] = w_devs[0];
-    }
-    cudaStream_t cs = ctx->copy_stream;
-    StreamDrain drain;
-    drain.add(cs);
-    drain.add(ctx->stream);
-    if (ctx->twin) drain.add(ctx->twin->stream);
-    int b0 = 0;
-    for (int ch = 0; ch < (int)sched.size(); ch++) {
-        adb_ctx *c = cc[ch & 1];
-        const int slot = ctx->twin ? 0 : (ch & 1);
-        cudaStream_t ks = c->stream;
-        const int r0 = b0 * batch->batch_size;
-        const int r1 = (int)std::min<long long>((long long)batch->n_reads, (long long)(b0 + sched[ch]) * batch->batch_size), nr = r1 - r0;
-        const int nb = (nr + batch->batch_size - 1) / batch->batch_size;
-        const int64_t c0 = batch->comp_offsets[r0], c1 = batch->comp_offsets[r1];
-        const size_t cbytes = (size_t)(c1 - c0) + 16;  // the slack behind the last stream travels along
-        // the decoded reads of the chunk: at most nr * m samples; the exact size follows from the compressed size
-        // (a stream holds at least one byte per sample)
-        const size_t dec_cap = std::min<size_t>((size_t)nr * (size_t)batch->m, (size_t)(c1 - c0));
-        if (ch >= 2) CUDA_TRY(cudaEventSynchronize(c->p_done[slot]));
-        if (c->p_comp[slot].ensure(cbytes + 64) || c->p_coffs[slot].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
-            c->p_nsamp[slot].ensure(sizeof(int32_t) * (size_t)nr + 16) || c->p_signal[slot].ensure(dec_cap * 2 + 64) ||
-            c->p_offsets[slot].ensure(sizeof(int64_t) * ((size_t)nr + 1)) || c->p_lens[slot].ensure(sizeof(int32_t) * (size_t)nr + 16) ||
-            c->p_coff[slot].ensure(sizeof(float) * (size_t)nr + 16) || c->p_cscale[slot].ensure(sizeof(float) * (size_t)nr + 16) ||
-            c->p_records[slot].ensure(sizeof(adb_record) * (size_t)nr) || c->p_status[slot].ensure(sizeof(int) * (size_t)nb + 16)) {
-            set_err("cudaMalloc pipeline staging");
-            return ADB_ERR_CUDA;
-        }
-        if (vbz) {  // frames travel; the decoded streams are laid out from dec_off rebased to the chunk
-            const int64_t d0 = dec_off[r0], dbytes = dec_off[r1] - d0;
-            if (c->p_frames[slot].ensure((size_t)(c1 - c0) + 16) || c->p_foffs[slot].ensure(sizeof(int64_t) * ((size_t)nr + 1)) ||
-                c->p_comp[slot].ensure((size_t)dbytes + 64) || c->p_zstat[slot].ensure(sizeof(int32_t) * (size_t)nr + 16) ||
-                c->p_signal[slot].ensure(std::min<size_t>((size_t)nr * (size_t)batch->m, (size_t)dbytes) * 2 + 64)) {
-                set_err("cudaMalloc pipeline staging");
-                return ADB_ERR_CUDA;
-            }
-            CUDA_TRY(cudaMemcpyAsync(c->p_frames[slot].p, batch->comp + c0, (size_t)(c1 - c0), cudaMemcpyHostToDevice, cs));
-            CUDA_TRY(cudaMemcpyAsync(c->p_foffs[slot].p, batch->comp_offsets + r0, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-            CUDA_TRY(cudaMemcpyAsync(c->p_coffs[slot].p, dec_off.data() + r0, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-        } else {
-            CUDA_TRY(cudaMemcpyAsync(c->p_comp[slot].p, batch->comp + c0, cbytes, cudaMemcpyHostToDevice, cs));
-            CUDA_TRY(cudaMemcpyAsync(c->p_coffs[slot].p, batch->comp_offsets + r0, sizeof(int64_t) * ((size_t)nr + 1), cudaMemcpyHostToDevice, cs));
-        }
-        CUDA_TRY(cudaMemcpyAsync(c->p_nsamp[slot].p, batch->n_samples + r0, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_lens[slot].p, batch->full_lens + r0, sizeof(int32_t) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_coff[slot].p, batch->calib_offset + r0, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaMemcpyAsync(c->p_cscale[slot].p, batch->calib_scale + r0, sizeof(float) * (size_t)nr, cudaMemcpyHostToDevice, cs));
-        CUDA_TRY(cudaEventRecord(c->p_copied[slot], cs));
-        CUDA_TRY(cudaStreamWaitEvent(ks, c->p_copied[slot], 0));
-        if (!ctx->opt_copy_only) {
-            int64_t sbase = c0;
-            if (vbz) {
-                sbase = dec_off[r0];
-                uint8_t *dec = (uint8_t *)c->p_comp[slot].p - sbase;
-                CUDA_TRY(cudaMemsetAsync(dec + dec_off[r1], 0, 16, ks));
-                rc = launch_zstd_decode(c, (const uint8_t *)c->p_frames[slot].p - c0, (const int64_t *)c->p_foffs[slot].p, dec,
-                                        (const int64_t *)c->p_coffs[slot].p, (int32_t *)c->p_zstat[slot].p, (int32_t *)ctx->z_fail.p, nr, ks);
-                if (rc) return rc;
-            }
-            rc = launch_svb_decode(c, (const uint8_t *)c->p_comp[slot].p - sbase, (const int64_t *)c->p_coffs[slot].p,
-                                   (const int32_t *)c->p_nsamp[slot].p, nr, (int64_t *)c->p_offsets[slot].p,
-                                   (int16_t *)c->p_signal[slot].p, ks);
-            if (rc) return rc;
-            adb_batch d;
-            d.signal = c->p_signal[slot].p;
-            d.sig_type = ADB_SIG_I16;
-            d.n_reads = nr;
-            d.m = batch->m;
-            d.batch_size = batch->batch_size;
-            d.offsets = (const int64_t *)c->p_offsets[slot].p;
-            d.full_lens = (const int32_t *)c->p_lens[slot].p;
-            d.calib_offset = (const float *)c->p_coff[slot].p;
-            d.calib_scale = (const float *)c->p_cscale[slot].p;
-            rc = adb_detect_dev(c, &d, cfg, w_devs[ch & 1], (adb_record *)c->p_records[slot].p, (int *)c->p_status[slot].p, ks);
-            if (rc) return rc;
-        }
-        CUDA_TRY(cudaMemcpyAsync(out_records + r0, c->p_records[slot].p, sizeof(adb_record) * (size_t)nr, cudaMemcpyDeviceToHost, ks));
-        if (batch_status)
-            CUDA_TRY(cudaMemcpyAsync(batch_status + b0, c->p_status[slot].p, sizeof(int) * (size_t)nb, cudaMemcpyDeviceToHost, ks));
-        CUDA_TRY(cudaEventRecord(c->p_done[slot], ks));
-        b0 += sched[ch];
-    }
-    if (ctx->twin) CUDA_TRY(cudaStreamSynchronize(ctx->twin->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(cs));
-    drain.armed = false;
-    if (vbz && !ctx->opt_copy_only) {
+    rc = detect_pipelined(ctx, *batch, cfg, cnn_weights, out_records, batch_status, chunk_batches,
+                          vbz ? (int32_t *)ctx->z_fail.p : nullptr, [&](ChunkDesc &k, int r0, int r1) {
+                              const int64_t c0 = batch->comp_offsets[r0], c1 = batch->comp_offsets[r1];
+                              k.rep = vbz ? CHUNK_ZSTD : CHUNK_SVB16;
+                              k.payload = batch->comp + c0;
+                              k.payload_bytes = (size_t)(c1 - c0) + (vbz ? 0 : 16);  // svb16: the slack travels along
+                              k.offsets = batch->comp_offsets + r0;
+                              k.dec_offsets = vbz ? dec_off.data() + r0 : nullptr;
+                              k.n_samples = batch->n_samples + r0;
+                          });
+    if (rc) return rc;
+    if (vbz && !ctx->opt.copy_only) {
         int32_t n_failed = 0;
         CUDA_TRY(cudaMemcpy(&n_failed, ctx->z_fail.p, sizeof(int32_t), cudaMemcpyDeviceToHost));
         if (n_failed) {

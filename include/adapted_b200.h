@@ -402,7 +402,8 @@ int adb_open_pores_host(adb_ctx *ctx, const adb_batch *batch, const int32_t *sel
  * yield_signals_from_pod5 calls, adapted/file_proc.py:165-175).  Read i's stream starts at comp[comp_offsets[i]]
  * (16-byte aligned): ceil(n / 8) key bytes (bit j % 8 of byte j / 8: 0 = one data byte, 1 = two, little endian), zero
  * padded to a multiple of 4, then the data bytes of the n = n_samples[i] <= m values; 16 bytes of slack follow the
- * last stream.  About 1.15 bytes per sample on nanopore signal instead of 2.
+ * last stream.  About 1.15 bytes per sample on nanopore signal instead of 2.  Every entry point that takes an
+ * adb_svb_batch refuses n_samples outside [0, m] with ADB_ERR_ARG.
  */
 typedef struct adb_svb_batch {
     const uint8_t *comp;

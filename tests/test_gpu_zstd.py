@@ -71,7 +71,9 @@ def test_refusals():
 
 @pytest.mark.parametrize("chem", ["rna002", "rna004"])
 def test_detect_reads_vbz_equals_svb(chem):
+    from adapted_b200 import _lib
     from adapted_b200.detect import detect_reads_svb, detect_reads_vbz
+    from tests.test_svb16 import _pipelined
 
     spc = get_chemistry_specific_config(chem)
     m = int(spc.sig_preload_size)
@@ -82,12 +84,23 @@ def test_detect_reads_vbz_equals_svb(chem):
     assert foff[-1] < coff[-1]
     args = (b.full_lens, b.calib_offset, b.calib_scale, spc, w)
     r1, s1 = detect_reads_svb(comp, coff, ns, *args, minibatch_size=100, chunk_minibatches=2)
-    r2, s2 = detect_reads_vbz(frames, foff, ns2, *args, minibatch_size=100, chunk_minibatches=2)
-    assert np.array_equal(s1, s2)
-    assert r1.tobytes() == r2.tobytes()
+    for chunk in (1, 2):
+        r2, s2 = detect_reads_vbz(frames, foff, ns2, *args, minibatch_size=100, chunk_minibatches=chunk)
+        assert np.array_equal(s1, s2), chunk
+        assert r1.tobytes() == r2.tobytes(), chunk
+    ctx = _lib.Context(0)  # one chunk on a context without a twin
+    try:
+        rc, r2, s2 = _pipelined(ctx, frames, foff, ns2, b, spc, w, 100, 64, vbz=True)
+        assert rc == 0, _lib.load().adb_last_error()
+        assert np.array_equal(s1, s2)
+        assert r1.tobytes() == r2.tobytes()
+    finally:
+        ctx.close()
 
 
 def test_detect_reads_vbz_refuses_a_corrupt_frame():
+    """in the call's one chunk, and in the second of five one-minibatch chunks: the twin context runs that one and
+    counts the refused frame in the counter of the call"""
     from adapted_b200 import _lib
     from adapted_b200.detect import detect_reads_vbz
 
@@ -98,8 +111,11 @@ def test_detect_reads_vbz_refuses_a_corrupt_frame():
     h = int(foff[10])
     assert frames[h + 4] == 0x60  # single segment, 2-byte content size (value - 256)
     frames[h + 6] += 1  # read 10 claims 256 bytes more than it decodes to
-    with pytest.raises(_lib.AdbError):
-        detect_reads_vbz(frames, foff, ns, b.full_lens, b.calib_offset, b.calib_scale, spc, minibatch_size=25)
+    for mbs, chunk in ((25, 16), (10, 1)):
+        with pytest.raises(_lib.AdbError) as e:
+            detect_reads_vbz(frames, foff, ns, b.full_lens, b.calib_offset, b.calib_scale, spc, minibatch_size=mbs,
+                             chunk_minibatches=chunk)
+        assert e.value.status == -2, chunk
 
 
 def _native(paths, out, spc, w, host_zstd=False):

@@ -63,11 +63,40 @@ def test_cuda_decode_round_trip(name):
     assert np.array_equal(dec, adc)
 
 
+def _pipelined(ctx, comp, coff, ns, b, spc, w, minibatch_size, chunk_minibatches, vbz=False):
+    """adb_detect_pipelined_svb_host / _vbz_host called on `ctx` directly, without the checks of detect_reads_svb ->
+    (status code, records, batch status)"""
+    import ctypes as C
+
+    from adapted_b200 import _lib
+    from adapted_b200.config import flatten_config
+    from adapted_b200.detect import flatten_cnn_weights
+
+    flat = flatten_config(spc)
+    comp, coff, ns = np.ascontiguousarray(comp, np.uint8), np.ascontiguousarray(coff, np.int64), np.ascontiguousarray(ns, np.int32)
+    lens, co, cs = (np.ascontiguousarray(x, t) for x, t in ((b.full_lens, np.int32), (b.calib_offset, np.float32), (b.calib_scale, np.float32)))
+    wf = flatten_cnn_weights(w) if flat["primary_method"] == 1 else None
+    recs = np.zeros(lens.size, _lib.RECORD_DTYPE)
+    status = np.zeros((lens.size + minibatch_size - 1) // minibatch_size, np.int32)
+    sb = _lib.AdbSvbBatch(comp=comp.ctypes.data, comp_offsets=coff.ctypes.data, n_samples=ns.ctypes.data, n_reads=lens.size,
+                          m=int(flat["sig_preload_size"]), batch_size=minibatch_size, full_lens=lens.ctypes.data,
+                          calib_offset=co.ctypes.data, calib_scale=cs.ctypes.data)
+    cfg = _lib.fill_config(flat)
+    L = _lib.load()
+    entry = L.adb_detect_pipelined_vbz_host if vbz else L.adb_detect_pipelined_svb_host
+    rc = entry(ctx.handle, C.byref(sb), C.byref(cfg), wf.ctypes.data if wf is not None else None, recs.ctypes.data,
+               status.ctypes.data, chunk_minibatches)
+    return rc, recs, status
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("chem,kw", [("rna002", {}), ("rna004", {"short_frac": 0.2}), ("rna004", {"stress": True})])
 def test_compressed_ingest_equals_plain_ingest(chem, kw):
     """records of the compressed pipelined ingest (H2D of svb16 streams, device decode) == records of the plain int16
-    call, byte for byte, over several chunks incl. a short last minibatch"""
+    call, byte for byte, incl. a short last minibatch: with every minibatch a chunk and with small chunks at both ends
+    (the default context and its twin), and on a context without a twin, in one chunk and in two chunks that alternate
+    between its staging slots"""
+    from adapted_b200 import _lib
     from adapted_b200.detect import detect_reads, detect_reads_svb
     from tests.golden_io import load_cnn_weights
 
@@ -77,10 +106,49 @@ def test_compressed_ingest_equals_plain_ingest(chem, kw):
     want, st_want = detect_reads(b.adc, b.offsets, b.full_lens, b.calib_offset, b.calib_scale, spc, model=w, minibatch_size=100,
                                  return_records=True)
     comp, coff, ns = svb16.encode_reads(b.adc, b.offsets)
-    got, st_got = detect_reads_svb(comp, coff, ns, b.full_lens, b.calib_offset, b.calib_scale, spc, model=w, minibatch_size=100,
-                                   chunk_minibatches=3)
-    assert np.array_equal(st_got, st_want)
-    assert got.tobytes() == want.tobytes()
+    for chunk in (1, 3):
+        got, st_got = detect_reads_svb(comp, coff, ns, b.full_lens, b.calib_offset, b.calib_scale, spc, model=w, minibatch_size=100,
+                                       chunk_minibatches=chunk)
+        assert np.array_equal(st_got, st_want), chunk
+        assert got.tobytes() == want.tobytes(), chunk
+    ctx = _lib.Context(0)
+    try:
+        for chunk in (64, 8):  # 12 minibatches: one chunk, then chunks of 8 and 4
+            rc, got, st_got = _pipelined(ctx, comp, coff, ns, b, spc, w, 100, chunk)
+            assert rc == 0, _lib.load().adb_last_error()
+            assert np.array_equal(st_got, st_want), chunk
+            assert got.tobytes() == want.tobytes(), chunk
+    finally:
+        ctx.close()
+
+
+@pytest.mark.gpu
+def test_compressed_entry_points_refuse_n_samples_above_m():
+    """a C caller's n_samples outside [0, m] is refused by every compressed entry point before anything is decoded"""
+    import ctypes as C
+
+    from adapted_b200 import _lib
+
+    spc = get_chemistry_specific_config("rna002")
+    m = int(spc.sig_preload_size)
+    b = make_reads(30, "rna002", m, seed=4)
+    comp, coff, ns = svb16.encode_reads(b.adc, b.offsets)
+    frames, foff, _ = svb16.vbz_encode_reads(b.adc, b.offsets)
+    ns = ns.copy()
+    ns[7] = m + 1
+    ctx = _lib.Context(0)
+    try:
+        for vbz, data, offs in ((False, comp, coff), (True, frames, foff)):
+            rc, _, _ = _pipelined(ctx, data, offs, ns, b, spc, None, 10, 1, vbz=vbz)
+            assert rc == -2 and _lib.load().adb_last_error() == b"n_samples outside [0, m]", (vbz, rc)
+        sb = _lib.AdbSvbBatch(comp=comp.ctypes.data, comp_offsets=coff.ctypes.data, n_samples=ns.ctypes.data, n_reads=ns.size, m=m,
+                              batch_size=10, full_lens=b.full_lens.ctypes.data, calib_offset=b.calib_offset.ctypes.data,
+                              calib_scale=b.calib_scale.ctypes.data)
+        out = np.zeros(int(ns.astype(np.int64).sum()), np.int16)
+        assert _lib.load().adb_svb16_decode_host(ctx.handle, C.byref(sb), out.ctypes.data) == -2
+        assert _lib.load().adb_last_error() == b"n_samples outside [0, m]"
+    finally:
+        ctx.close()
 
 
 @pytest.mark.parametrize("zstd", [False, True])
