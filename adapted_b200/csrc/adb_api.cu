@@ -121,6 +121,7 @@ extern "C" int adb_ctx_set_option(adb_ctx *c, const char *name, int value) {
     if (!strcmp(name, "no_fast_validate")) { c->opt.no_fast_validate = value; return ADB_OK; }
     if (!strcmp(name, "hist_validate")) { c->opt.hist_validate = value; return ADB_OK; }
     if (!strcmp(name, "cnn_fp32_pipe")) { c->opt.cnn_fp32 = value; return ADB_OK; }
+    if (!strcmp(name, "cnn_tc_per_read_tiles")) { c->opt.cnn_tc_per_read = value; return ADB_OK; }
     if (!strcmp(name, "pipeline_copy_only")) { c->opt.copy_only = value; return ADB_OK; }
     if (!strcmp(name, "no_cand_followup")) { c->opt.no_cand_followup = value; return ADB_OK; }
     if (!strcmp(name, "host_zstd")) { c->opt.host_zstd = value; return ADB_OK; }
@@ -1089,9 +1090,13 @@ extern "C" int adb_cnn_scores_host(adb_ctx *ctx, const float *x, int32_t n, int3
     D.L1 = (L + 2 * 3 - CNN_K) / 3 + 1;
     D.LP = (D.L1 + 3) & ~3;
     D.Lout = (D.L1 - 1) * 3 - 2 * 3 + CNN_K;
-    if (ctx->cnn_x.ensure(sizeof(float) * (size_t)n * L) || ctx->cnn_scores.ensure(sizeof(float) * (size_t)n * 2 * D.Lout))
+    D.XS = 3 * (D.L1 + 3);
+    if (ctx->cnn_x.ensure(sizeof(float) * (size_t)n * D.XS) || ctx->cnn_scores.ensure(sizeof(float) * (size_t)n * 2 * D.Lout))
         { set_err("cudaMalloc cnn buffers"); return ADB_ERR_CUDA; }
-    CUDA_TRY(cudaMemcpyAsync(ctx->cnn_x.p, x, sizeof(float) * (size_t)n * L, cudaMemcpyHostToDevice, st));
+    // rows of XS samples: the reads' samples, then zeros (the padding between reads of the convolutions)
+    CUDA_TRY(cudaMemcpy2DAsync(ctx->cnn_x.p, sizeof(float) * D.XS, x, sizeof(float) * L, sizeof(float) * L, n,
+                               cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemset2DAsync((float *)ctx->cnn_x.p + L, sizeof(float) * D.XS, 0, sizeof(float) * (D.XS - L), n, st));
     const float *w_dev = nullptr;
     int rc = upload_cnn_weights(ctx, cnn_weights, &w_dev);
     if (rc) return rc;

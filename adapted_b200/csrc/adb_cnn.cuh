@@ -64,8 +64,10 @@ __device__ __forceinline__ float cnn_block_mean(F f, int factor) {
     return __fdiv_rn(np_sum_f32_leaf(f, factor), (float)factor);
 }
 
-// x[r][0..L) ; L = ceil((m - A0) / f).  One CTA (256 threads) per read; dynamic smem = L floats + select scratch.
-__global__ void __launch_bounds__(256) cnn_prep_kernel(BatchDev B, int A0, int f, int L, float *x) {
+// x[r][0..L) ; L = ceil((m - A0) / f), row stride xs >= L: x[r][L..xs) are written as zeros on every call (the tensor-core
+// convolutions read them as the zero padding between reads, adb_cnn_tc.cuh).  One CTA (256 threads) per read; dynamic
+// smem = L floats + select scratch.
+__global__ void __launch_bounds__(256) cnn_prep_kernel(BatchDev B, int A0, int f, int L, int xs, float *x) {
     extern __shared__ __align__(16) unsigned char smem[];
     float *ds = (float *)smem;
     unsigned char *scr = smem + (((size_t)L * 4 + 15) & ~(size_t)15);
@@ -97,9 +99,9 @@ __global__ void __launch_bounds__(256) cnn_prep_kernel(BatchDev B, int A0, int f
         const float dmax = fmaxf(fabsf(__fsub_rn(key_f32(kmax), med)), fabsf(__fsub_rn(key_f32(kmin), med)));
         mad = cta_median_keys(D, KeyF32Id(), nv, f32_key(0.0f), f32_key(dmax), S, kbuf);
     }
-    float *xr = x + (size_t)r * L;
-    for (int b = threadIdx.x; b < L; b += blockDim.x) {
-        float v = CNN_SCORE_EXCL;
+    float *xr = x + (size_t)r * xs;
+    for (int b = threadIdx.x; b < xs; b += blockDim.x) {
+        float v = b < L ? CNN_SCORE_EXCL : 0.0f;
         if (b < nv) {
             v = __fdiv_rn(__fsub_rn(ds[b], med), mad);
             if (!(v == v)) v = CNN_SCORE_EXCL;          // torch.nan_to_num(nan=-5)
@@ -117,7 +119,7 @@ __global__ void __launch_bounds__(256) cnn_prep_kernel(BatchDev B, int A0, int f
 #define PREP_WARPS 4
 #define PREP_CHUNK_BINS 320   // bins per staged chunk: 320 x downscale factor 10 x 2 B = 6400 B <= the warp's key area
 __host__ __device__ inline size_t cnn_prep_warp_smem(int L) { return (size_t)PREP_WARPS * (2 * ((L + 3) & ~3) + SM_NCAND + 4) * 4; }
-__global__ void __launch_bounds__(PREP_WARPS * 32) cnn_prep_warp_kernel(BatchDev B, int A0, int f, int L, float *x) {
+__global__ void __launch_bounds__(PREP_WARPS * 32) cnn_prep_warp_kernel(BatchDev B, int A0, int f, int L, int xs, float *x) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int Lp = (L + 3) & ~3;
@@ -213,9 +215,9 @@ __global__ void __launch_bounds__(PREP_WARPS * 32) cnn_prep_warp_kernel(BatchDev
             warp_select2(K, nvp >> 2, 0u, false, nvp, rank, mn, mx, cand, a, b2, hb);
             mad = (nv & 1) ? key_f32(a) : __fdiv_rn(__fadd_rn(key_f32(a), key_f32(b2)), 2.0f);
         }
-        float *xr = x + (size_t)r * L;
-        for (int b = lane; b < L; b += 32) {
-            float v = CNN_SCORE_EXCL;
+        float *xr = x + (size_t)r * xs;
+        for (int b = lane; b < xs; b += 32) {  // (the zeros of x[r][L..xs) included)
+            float v = b < L ? CNN_SCORE_EXCL : 0.0f;
             if (b < nv) {
                 v = __fdiv_rn(__fsub_rn(ds[b], med), mad);
                 if (!(v == v)) v = CNN_SCORE_EXCL;          // torch.nan_to_num(nan=-5)
@@ -240,14 +242,15 @@ __global__ void cnn_pack_weights_kernel(const float *w, float *packed /* 2 x [64
 }
 
 // ---- Conv1d(64 -> 64, k = 7, pad 3) + ReLU ------------------------------------------------------------------------------
-// in  : FUSE_L1 ? x [N][Lx] : act [N][64][LP]        out : act [N][64][LP]   (LP = padded row length, multiple of 4)
+// in  : FUSE_L1 ? x [N][Lx] (row stride xs) : act [N][64][LP]        out : act [N][64][LP]   (LP = padded row length,
+// multiple of 4)
 // Persistent CTAs; the 114.7 KB of packed weights stay in shared memory for the CTA's whole life.
 // `only` (optional, [n_reads]): process just the reads flagged there (the reads the tensor-core kernel could not
 // represent in its fp16 split, adb_cnn_tc.cuh).
 template <bool FUSE_L1>
 __global__ void __launch_bounds__(CNN_THREADS, 1) cnn_conv64_kernel(const float *in, float *out, const float *packed_w,
                                                                    const float *bias, const float *w1, const float *b1,
-                                                                   int n_reads, int Lx, int L1, int LP, const int *only) {
+                                                                   int n_reads, int Lx, int xs, int L1, int LP, const int *only) {
     if (only) {  // nothing flagged (only[-1] == 0) or nothing flagged for this CTA: leave before the weights are loaded
         if (only[-1] == 0) return;
         const int tiles_per_read = (L1 + CNN_TILE - 1) / CNN_TILE, n_tiles = n_reads * tiles_per_read;
@@ -279,7 +282,7 @@ __global__ void __launch_bounds__(CNN_THREADS, 1) cnn_conv64_kernel(const float 
         __syncthreads();
         if (FUSE_L1) {
             // x window needed by act1 positions [t0-3, t0+CNN_TILE+3): x[3p-3 .. 3p+3]
-            const float *xr = in + (size_t)r * Lx;
+            const float *xr = in + (size_t)r * xs;
             const int x0 = 3 * (t0 - 3) - 3, nx = 3 * (CNN_TILE + 6) + 6;
             for (int i = threadIdx.x; i < nx; i += blockDim.x) {
                 const int j = x0 + i;
@@ -359,44 +362,47 @@ __host__ __device__ inline size_t cnn_conv_smem_bytes() {
 // out[3u+2] = x[u+1] w2 + x[u] w5  (three coalesced loads and 14 FMAs per input channel; the per-output summation
 // order -- channels ascending, taps ascending -- is unchanged).
 #define CNN_CONVT_THREADS 192  // 3 CTAs cover the 550 positions of an RNA004 read with 4 % idle threads
-// `only` (optional): just the reads flagged there (tensor-core path: reads recomputed on the FP32 pipe).
+// blockIdx.y strides over the reads.  `only` (optional): just the reads flagged there (tensor-core path: reads recomputed
+// on the FP32 pipe; only[-1] == 0, nothing flagged, is the common case: a small grid leaves at once).
 __global__ void __launch_bounds__(CNN_CONVT_THREADS) cnn_convT_kernel(const float *act, const float *w4, const float *b4, int L1, int LP,
-                                                        int Lout, float *scores, const int *only) {
-    if (only && (only[-1] == 0 || only[blockIdx.y] == 0)) return;
+                                                        int Lout, int n_reads, float *scores, const int *only) {
+    if (only && only[-1] == 0) return;
     __shared__ __align__(16) float ws[CNN_C * 16];  // per ci: co0 k0..6, pad, co1 k0..6, pad
     for (int i = threadIdx.x; i < CNN_C * 16; i += blockDim.x) {
         const int ci = i >> 4, e = i & 15, co = e >> 3, k = e & 7;
         ws[i] = (k < CNN_K) ? w4[(ci * 2 + co) * CNN_K + k] : 0.0f;
     }
     __syncthreads();
-    const int r = blockIdx.y;
     const int u = blockIdx.x * blockDim.x + threadIdx.x;
     if (3 * u >= Lout) return;
-    const float *ar = act + (size_t)r * CNN_C * LP;
-    const float bias0 = b4[0], bias1 = b4[1];
-    float o[2][3] = {{bias0, bias0, bias0}, {bias1, bias1, bias1}};
-    const bool has_m = (u - 1 >= 0) && (u - 1 < L1), has_c = u < L1, has_p = u + 1 < L1;
+    for (int r = blockIdx.y; r < n_reads; r += gridDim.y) {
+        if (only && only[r] == 0) continue;
+        const float *ar = act + (size_t)r * CNN_C * LP;
+        const float bias0 = b4[0], bias1 = b4[1];
+        float o[2][3] = {{bias0, bias0, bias0}, {bias1, bias1, bias1}};
+        const bool has_m = (u - 1 >= 0) && (u - 1 < L1), has_c = u < L1, has_p = u + 1 < L1;
 #pragma unroll 8
-    for (int ci = 0; ci < CNN_C; ci++) {
-        const float *ap = ar + (size_t)ci * LP;
-        const float xm = has_m ? ap[u - 1] : 0.0f, xc = has_c ? ap[u] : 0.0f, xp = has_p ? ap[u + 1] : 0.0f;
-        const float4 wa = *reinterpret_cast<const float4 *>(ws + ci * 16), wb = *reinterpret_cast<const float4 *>(ws + ci * 16 + 4);
-        const float4 wc = *reinterpret_cast<const float4 *>(ws + ci * 16 + 8), wd = *reinterpret_cast<const float4 *>(ws + ci * 16 + 12);
-        // taps in ascending k: k = j%3 pairs with x[u+1], k+3 with x[u], k+6 with x[u-1]
-        if (has_p) { o[0][0] = fmaf(xp, wa.x, o[0][0]); o[1][0] = fmaf(xp, wc.x, o[1][0]); }
-        if (has_c) { o[0][0] = fmaf(xc, wa.w, o[0][0]); o[1][0] = fmaf(xc, wc.w, o[1][0]); }
-        if (has_m) { o[0][0] = fmaf(xm, wb.z, o[0][0]); o[1][0] = fmaf(xm, wd.z, o[1][0]); }
-        if (has_p) { o[0][1] = fmaf(xp, wa.y, o[0][1]); o[1][1] = fmaf(xp, wc.y, o[1][1]); }
-        if (has_c) { o[0][1] = fmaf(xc, wb.x, o[0][1]); o[1][1] = fmaf(xc, wd.x, o[1][1]); }
-        if (has_p) { o[0][2] = fmaf(xp, wa.z, o[0][2]); o[1][2] = fmaf(xp, wc.z, o[1][2]); }
-        if (has_c) { o[0][2] = fmaf(xc, wb.y, o[0][2]); o[1][2] = fmaf(xc, wd.y, o[1][2]); }
-    }
+        for (int ci = 0; ci < CNN_C; ci++) {
+            const float *ap = ar + (size_t)ci * LP;
+            const float xm = has_m ? ap[u - 1] : 0.0f, xc = has_c ? ap[u] : 0.0f, xp = has_p ? ap[u + 1] : 0.0f;
+            const float4 wa = *reinterpret_cast<const float4 *>(ws + ci * 16), wb = *reinterpret_cast<const float4 *>(ws + ci * 16 + 4);
+            const float4 wc = *reinterpret_cast<const float4 *>(ws + ci * 16 + 8), wd = *reinterpret_cast<const float4 *>(ws + ci * 16 + 12);
+            // taps in ascending k: k = j%3 pairs with x[u+1], k+3 with x[u], k+6 with x[u-1]
+            if (has_p) { o[0][0] = fmaf(xp, wa.x, o[0][0]); o[1][0] = fmaf(xp, wc.x, o[1][0]); }
+            if (has_c) { o[0][0] = fmaf(xc, wa.w, o[0][0]); o[1][0] = fmaf(xc, wc.w, o[1][0]); }
+            if (has_m) { o[0][0] = fmaf(xm, wb.z, o[0][0]); o[1][0] = fmaf(xm, wd.z, o[1][0]); }
+            if (has_p) { o[0][1] = fmaf(xp, wa.y, o[0][1]); o[1][1] = fmaf(xp, wc.y, o[1][1]); }
+            if (has_c) { o[0][1] = fmaf(xc, wb.x, o[0][1]); o[1][1] = fmaf(xc, wd.x, o[1][1]); }
+            if (has_p) { o[0][2] = fmaf(xp, wa.z, o[0][2]); o[1][2] = fmaf(xp, wc.z, o[1][2]); }
+            if (has_c) { o[0][2] = fmaf(xc, wb.y, o[0][2]); o[1][2] = fmaf(xc, wd.y, o[1][2]); }
+        }
 #pragma unroll
-    for (int c = 0; c < 3; c++) {
-        const int j = 3 * u + c;
-        if (j < Lout) {
-            scores[((size_t)r * 2 + 0) * Lout + j] = o[0][c];
-            scores[((size_t)r * 2 + 1) * Lout + j] = o[1][c];
+        for (int c = 0; c < 3; c++) {
+            const int j = 3 * u + c;
+            if (j < Lout) {
+                scores[((size_t)r * 2 + 0) * Lout + j] = o[0][c];
+                scores[((size_t)r * 2 + 1) * Lout + j] = o[1][c];
+            }
         }
     }
 }
@@ -696,6 +702,7 @@ __global__ void __launch_bounds__(256) cnn_shift_kernel(const int *apos, const i
 // ---- host orchestration -----------------------------------------------------------------------------------------------------
 struct CnnDims {
     int Lx, L1, LP, Lout;
+    int XS;  // row stride of x: 3 (L1 + 3) samples, the zeros behind a read are the padding between reads (adb_cnn_tc.cuh)
 };
 static CnnDims cnn_dims(int m, int A0, int f) {
     CnnDims d;
@@ -703,10 +710,11 @@ static CnnDims cnn_dims(int m, int A0, int f) {
     d.L1 = (d.Lx + 2 * 3 - CNN_K) / 3 + 1;
     d.LP = (d.L1 + 3) & ~3;
     d.Lout = (d.L1 - 1) * 3 - 2 * 3 + CNN_K;
+    d.XS = 3 * (d.L1 + 3);
     return d;
 }
 
-// x [n][Lx] (device) -> scores [n][2][Lout] (device); chunked over reads to bound the activation buffers
+// x [n][Lx] (device, row stride XS) -> scores [n][2][Lout] (device); chunked over reads to bound the activation buffers
 // tensor-core version of the two 64 -> 64 convolutions (adb_cnn_tc.cuh)
 __global__ void cnn_tc_pack_weights_kernel(const float *w, __half *packed);
 static int cnn_tc_launch_setup();
@@ -730,9 +738,10 @@ __global__ void cnn_ct_pack_kernel(const float *w4 /* torch layout [ci][co][k] *
 }
 
 static void cnn_tc_launch(int layer, const void *in, void *out, const __half *wp, const float *bias, const float *w1,
-                          const float *b1, int n_reads, int Lx, int L1, int LP, int *redo, int sm_count, cudaStream_t st, int cslot = -1);
-static size_t cnn_tc_a0t_bytes_per_read(int L1);
-static int cnn_tc_a0t_rows_host(int L1);
+                          const float *b1, int n_reads, int Lx, int L1, int LP, int per_read, int *redo, int sm_count,
+                          cudaStream_t st, int cslot = -1);
+static int cnn_tc_a0t_rows_host(int n_reads, int L1, int per_read);
+static int cnn_tc_read_rows_host(int L1, int per_read);
 
 static int cnn_forward_dev(adb_ctx *ctx, const float *x, int n, const CnnDims &D, const float *w_dev, float *scores,
                            cudaStream_t st) {
@@ -758,6 +767,8 @@ static int cnn_forward_dev(adb_ctx *ctx, const float *x, int n, const CnnDims &D
     unsigned char *a0t = nullptr;
     int *redo = nullptr;
     int cslot = -1;  // slot of the constant bank holding the transposed convolution's weights (-1: shared memory)
+    const int per_read = ctx->opt.cnn_tc_per_read;
+    int a0t_rows = 0;
     if (use_tc) {
         // split fp16 weights of both layers, then the per-read "outside the fp16 range" flags of one chunk
         const size_t wbytes = sizeof(__half) * 2 * CNN_K * 2 * 4096;
@@ -779,16 +790,19 @@ static int cnn_forward_dev(adb_ctx *ctx, const float *x, int n, const CnnDims &D
             cslot = ctx->ct_slot;
         }
         if (cnn_tc_launch_setup()) { set_err("cudaFuncSetAttribute cnn tc"); return ADB_ERR_CUDA; }
-        // layer 2 -> layer 3 activations in layer 3's tile layout; the padding rows are never written: zero them whenever
-        // the buffer is (re)allocated
-        const size_t a0t_bytes = cnn_tc_a0t_bytes_per_read(D.L1) * (size_t)chunk;
+        // layer 2 -> layer 3 activations in layer 3's tile layout, rows per octet sized for the full chunk (a shorter
+        // last chunk uses a prefix of every octet's run); the rows in front of the stream (and with per-read tiles the
+        // rows between the reads) are never written: zero them whenever the buffer is (re)allocated
+        a0t_rows = cnn_tc_a0t_rows_host(chunk, D.L1, per_read);
+        const size_t a0t_bytes = (size_t)2 * 8 * a0t_rows * 16;
         const void *before = ctx->cnn_a0t.p;
         const size_t cap_before = ctx->cnn_a0t.cap;
         if (ctx->cnn_a0t.ensure(a0t_bytes)) { set_err("cudaMalloc cnn a0t"); return ADB_ERR_CUDA; }
-        // (also when L1 changes: rows between the old and the new end would keep activations of the old geometry)
-        if (ctx->cnn_a0t.p != before || ctx->cnn_a0t.cap != cap_before || ctx->cnn_a0t_l1 != D.L1)
+        // (also when the geometry changes: rows that are never written would keep activations of the old one)
+        const int geom[3] = {D.L1, cnn_tc_read_rows_host(D.L1, per_read), a0t_rows};
+        if (ctx->cnn_a0t.p != before || ctx->cnn_a0t.cap != cap_before || memcmp(ctx->cnn_a0t_geom, geom, sizeof geom))
             CUDA_TRY(cudaMemsetAsync(ctx->cnn_a0t.p, 0, ctx->cnn_a0t.cap, st));
-        ctx->cnn_a0t_l1 = D.L1;
+        memcpy(ctx->cnn_a0t_geom, geom, sizeof geom);
         a0t = (unsigned char *)ctx->cnn_a0t.p;
     }
     for (int r0 = 0; r0 < n; r0 += chunk) {
@@ -799,43 +813,44 @@ static int cnn_forward_dev(adb_ctx *ctx, const float *x, int n, const CnnDims &D
             CUDA_TRY(cudaMemsetAsync(redo - 4, 0, sizeof(int) * ((size_t)nc + 4), st));
             {
                 KernelTimer t(ctx, 5, st);
-                cnn_tc_launch(2, x + (size_t)r0 * D.Lx, a0t, wtc, w_dev + CNN_B2, w_dev + CNN_W1, w_dev + CNN_B1, nc, D.Lx, D.L1,
-                              cnn_tc_a0t_rows_host(D.L1), redo, ctx->sm_count, st);
+                cnn_tc_launch(2, x + (size_t)r0 * D.XS, a0t, wtc, w_dev + CNN_B2, w_dev + CNN_W1, w_dev + CNN_B1, nc, D.XS, D.L1,
+                              a0t_rows, per_read, redo, ctx->sm_count, st);
             }
             {
                 KernelTimer t(ctx, 5, st);
                 // layer 3 + the transposed convolution: scores straight from the epilogue
                 cnn_tc_launch(3, a0t, scores + (size_t)r0 * 2 * D.Lout, wtc + (size_t)CNN_K * 2 * 4096, w_dev + CNN_B3,
-                              w_dev + CNN_W4, w_dev + CNN_B4, nc, D.Lout, D.L1, cnn_tc_a0t_rows_host(D.L1), redo,
+                              w_dev + CNN_W4, w_dev + CNN_B4, nc, D.Lout, D.L1, a0t_rows, per_read, redo,
                               ctx->sm_count, st, cslot);
             }
             {
                 // reads with a value outside the fp16 range (flagged by either layer): both layers again on the FP32 pipe
                 KernelTimer t(ctx, 7, st);
-                cnn_conv64_kernel<true><<<grid, CNN_THREADS, smem, st>>>(x + (size_t)r0 * D.Lx, a0, packed, w_dev + CNN_B2,
-                                                                          w_dev + CNN_W1, w_dev + CNN_B1, nc, D.Lx, D.L1, D.LP, redo);
+                cnn_conv64_kernel<true><<<grid, CNN_THREADS, smem, st>>>(x + (size_t)r0 * D.XS, a0, packed, w_dev + CNN_B2,
+                                                                          w_dev + CNN_W1, w_dev + CNN_B1, nc, D.Lx, D.XS, D.L1, D.LP, redo);
                 cnn_conv64_kernel<false><<<grid, CNN_THREADS, smem, st>>>(a0, a1, packed + CNN_C * CNN_K * CNN_C, w_dev + CNN_B3,
-                                                                           nullptr, nullptr, nc, D.Lx, D.L1, D.LP, redo);
+                                                                           nullptr, nullptr, nc, D.Lx, D.XS, D.L1, D.LP, redo);
             }
             ctx->launches += 2;
         } else {
         {
             KernelTimer t(ctx, 5, st);
-            cnn_conv64_kernel<true><<<grid, CNN_THREADS, smem, st>>>(x + (size_t)r0 * D.Lx, a0, packed, w_dev + CNN_B2,
-                                                                      w_dev + CNN_W1, w_dev + CNN_B1, nc, D.Lx, D.L1, D.LP, nullptr);
+            cnn_conv64_kernel<true><<<grid, CNN_THREADS, smem, st>>>(x + (size_t)r0 * D.XS, a0, packed, w_dev + CNN_B2,
+                                                                      w_dev + CNN_W1, w_dev + CNN_B1, nc, D.Lx, D.XS, D.L1, D.LP, nullptr);
         }
         {
             KernelTimer t(ctx, 5, st);
             cnn_conv64_kernel<false><<<grid, CNN_THREADS, smem, st>>>(a0, a1, packed + CNN_C * CNN_K * CNN_C, w_dev + CNN_B3,
-                                                                       nullptr, nullptr, nc, D.Lx, D.L1, D.LP, nullptr);
+                                                                       nullptr, nullptr, nc, D.Lx, D.XS, D.L1, D.LP, nullptr);
         }
         }
         {
-            // FP32 path: every read; tensor-core path: only the reads redone on the FP32 pipe (the others got their
-            // scores from layer 3's epilogue)
+            // FP32 path: every read, one CTA row per read; tensor-core path: only the reads redone on the FP32 pipe (the
+            // others got their scores from layer 3's epilogue), usually none: CTA rows striding over the reads, at most
+            // as many as the redo kernels' grid
             KernelTimer t(ctx, use_tc ? 7 : 5, st);
-            dim3 g(((D.Lout + 2) / 3 + CNN_CONVT_THREADS - 1) / CNN_CONVT_THREADS, nc);
-            cnn_convT_kernel<<<g, CNN_CONVT_THREADS, 0, st>>>(a1, w_dev + CNN_W4, w_dev + CNN_B4, D.L1, D.LP, D.Lout,
+            dim3 g(((D.Lout + 2) / 3 + CNN_CONVT_THREADS - 1) / CNN_CONVT_THREADS, use_tc ? grid : nc);
+            cnn_convT_kernel<<<g, CNN_CONVT_THREADS, 0, st>>>(a1, w_dev + CNN_W4, w_dev + CNN_B4, D.L1, D.LP, D.Lout, nc,
                                                 scores + (size_t)r0 * 2 * D.Lout, use_tc ? redo : nullptr);
         }
         ctx->launches += 3;
@@ -860,7 +875,7 @@ static int cnn_primary_boundaries(adb_ctx *ctx, const BatchDev &B, const adb_con
         return ADB_ERR_UNSUPPORTED;
     }
     const int n = B.n_reads, k = cfg.polya_cand_k;
-    if (ctx->cnn_x.ensure(sizeof(float) * (size_t)n * D.Lx) || ctx->cnn_scores.ensure(sizeof(float) * (size_t)n * 2 * D.Lout)) {
+    if (ctx->cnn_x.ensure(sizeof(float) * (size_t)n * D.XS) || ctx->cnn_scores.ensure(sizeof(float) * (size_t)n * 2 * D.Lout)) {
         set_err("cudaMalloc cnn buffers");
         return ADB_ERR_CUDA;
     }
@@ -876,9 +891,9 @@ static int cnn_primary_boundaries(adb_ctx *ctx, const BatchDev &B, const adb_con
             int occ = 0;
             CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, cnn_prep_warp_kernel, PREP_WARPS * 32, wsm));
             const int grid = std::max(1, std::min((n + PREP_WARPS - 1) / PREP_WARPS, ctx->sm_count * std::max(occ, 1)));
-            cnn_prep_warp_kernel<<<grid, PREP_WARPS * 32, wsm, st>>>(B, cfg.min_obs_adapter, cfg.downscale_factor, D.Lx, x);
+            cnn_prep_warp_kernel<<<grid, PREP_WARPS * 32, wsm, st>>>(B, cfg.min_obs_adapter, cfg.downscale_factor, D.Lx, D.XS, x);
         } else {
-            cnn_prep_kernel<<<n, 256, smem, st>>>(B, cfg.min_obs_adapter, cfg.downscale_factor, D.Lx, x);
+            cnn_prep_kernel<<<n, 256, smem, st>>>(B, cfg.min_obs_adapter, cfg.downscale_factor, D.Lx, D.XS, x);
         }
         ctx->launches += 1;
     }

@@ -140,20 +140,68 @@ __device__ __forceinline__ bool tc_split_store(unsigned char *hi_plane, unsigned
     return bad;
 }
 
+// Row stream of a chunk.  The reads of a chunk lie end to end, S rows apart: read r's position p is stream row
+// g = r S + p.  With S = L1 + 3 ("packed", the default) the three rows behind every read are exactly the zero padding a
+// k = 7, pad 3 convolution needs on both sides of a read, and the +-1-row neighbours of the fused transposed
+// convolution are zero as well, so tiles walk the stream without regard to read boundaries:
+//     layer 2: tile j covers rows 128 j ..;   layer 3: tile j covers rows 126 j - 1 .. (two rows overlap, see below)
+// A row that is not a position of a read of the chunk (a gap row, a row in front of the stream or behind its last read)
+// is zero padding.  Per-read tiling (option "cnn_tc_per_read_tiles", the previous scheme, kept as the A/B arm) is the
+// same stream with S the per-read block below and the tiles restarting at every read.
+//
 // Intermediate activations between the two layers ("A0T"): layer 2's epilogue writes its output already split into the
 // fp16 hi / lo planes and in the row order of layer 3's shared-memory tile,
-//     A0T[read][plane][ci / 8][rho = position + TC_A0T_PAD][ci % 8]      (16 B per row, `a0t_rows` rows per octet),
+//     A0T[plane][ci / 8][rho = g + TC_A0T_PAD][ci % 8]      (16 B per row, `a0t_rows` rows per octet),
 // so that the operand tile of a layer-3 job is 16 contiguous runs of 134 rows: sixteen cp.async.bulk copies per tile,
-// no thread touches the data.  Rows outside [0, L1) are layer 3's zero padding: rows >= L1 are written as zeros, the
-// three rows in front of position 0 and the tail rows are never written and stay zero from the buffer's memset.
-#define TC_A0T_PAD 4                                        // zero rows in front of position 0
+// no thread touches the data.  Layer 2 writes every row its tiles cover, gap rows as zeros; the rows in front of the
+// stream (and, with per-read tiling, the rows between a read's last tile and the next read) are never written and stay
+// zero from the buffer's memset.
+#define TC_A0T_PAD 4                                        // zero rows in front of the stream
 #define TC_L3_STRIDE (TC_ROWS - 2)                          // layer 3 tiles overlap by two rows (fused convT, see below)
-// rows per octet for a layer-1 length L1: what layer 2's tiles write (positions 0 .. 128 J2 - 1) and what layer 3's last
-// tile reads (rho up to 126 (J3 - 1) + 133), whichever is larger; the kernels get it in their `LP` argument
-__host__ __device__ inline int cnn_tc_a0t_rows(int L1) {
+#define TC_GAP 3                                            // zero rows behind every read of the packed stream
+
+struct TcTiles {
+    int S;       // rows per read
+    int stride;  // rows a tile advances: TC_ROWS (layer 2) or TC_L3_STRIDE (layer 3)
+    int jpr;     // tiles per segment: per read (per-read tiling) or the whole chunk (packed)
+    int n_jobs;
+    // first row of tile `job` (layer 3: the row in front of its first output row, as seen from rho = g + TC_A0T_PAD)
+    __host__ __device__ int row0(int job) const { return (job / jpr) * S + (job % jpr) * stride; }
+};
+__host__ __device__ inline int cnn_tc_read_rows(int L1, int per_read) {
+    if (!per_read) return L1 + TC_GAP;
+    // one block per read: what its layer 2 tiles write (rho up to 128 J2 + 3) and what its last layer 3 tile reads
+    // (rho up to 126 (J3 - 1) + 133), whichever is larger
     const int j2 = (L1 + TC_ROWS - 1) / TC_ROWS, j3 = (L1 + TC_L3_STRIDE - 1) / TC_L3_STRIDE;
     const int w = TC_ROWS * j2 + TC_A0T_PAD, rd = TC_L3_STRIDE * (j3 - 1) + TC_NQ;
     return ((w > rd ? w : rd) + 7) & ~7;
+}
+__host__ __device__ inline TcTiles cnn_tc_tiles(int layer, int n_reads, int L1, int per_read) {
+    TcTiles t;
+    t.S = cnn_tc_read_rows(L1, per_read);
+    t.stride = layer == 3 ? TC_L3_STRIDE : TC_ROWS;
+    if (per_read) {
+        t.jpr = (L1 + t.stride - 1) / t.stride;
+        t.n_jobs = n_reads * t.jpr;
+    } else {
+        t.n_jobs = (int)(((long long)n_reads * t.S + t.stride - 1) / t.stride);
+        t.jpr = t.n_jobs;
+    }
+    return t;
+}
+// rows per octet of A0T for chunks of up to n_reads reads: what layer 2's last tile writes and what layer 3's last tile
+// reads, whichever is larger; the kernels get it in their `LP` argument
+__host__ __device__ inline int cnn_tc_a0t_rows(int n_reads, int L1, int per_read) {
+    const TcTiles t2 = cnn_tc_tiles(2, n_reads, L1, per_read), t3 = cnn_tc_tiles(3, n_reads, L1, per_read);
+    const int w = t2.row0(t2.n_jobs - 1) + TC_ROWS + TC_A0T_PAD, rd = t3.row0(t3.n_jobs - 1) + TC_NQ;
+    return ((w > rd ? w : rd) + 7) & ~7;
+}
+// stream row g -> (read, position); true if it is a position of a read of the chunk.  g >= -TC_A0T_PAD > -S: the rows in
+// front of the stream give read 0 and a negative position.
+__device__ __forceinline__ bool tc_row_read(int g, int S, int L1, int n_reads, int &r, int &p) {
+    r = g / S;
+    p = g - r * S;
+    return (unsigned)p < (unsigned)L1 && r < n_reads;
 }
 #define TC_TILE_RUN (TC_NQ * 16)                            // bytes of one (plane, octet) run of a tile
 
@@ -163,25 +211,28 @@ __host__ __device__ inline size_t cnn_tc_smem_bytes_layer(int layer) {
     return (size_t)TC_WBYTES + 2 * 2 * (size_t)TC_PLANE + (size_t)(TC_NX + 10) * 4 + 64 * 8 * 4 + 64 * 4 + 160 + 1024;
 }
 
-// LAYER 2: in = x [N][Lx] (layer 1 fused into the operand build), out = A0T.
+// LAYER 2: in = x [N][Lx] with the row stride Lx = 3 S_packed samples (zeros behind each read's samples: stream row g
+//   takes its layer-1 inputs from x[3 g - 3 .. 3 g + 3] across read boundaries), layer 1 fused into the operand build;
+//   out = A0T.
 // LAYER 3: in = A0T, out = scores [N][2][Lout]: the transposed convolution (64 -> 2, k = 7, stride 3, pad 3) is fused
 //   into the epilogue, layer 3's activations never leave the SM.  out[co][3u + c] needs the activations of positions
-//   u - 1, u, u + 1; tiles of 128 rows therefore advance by 126 positions (rows t0 .. t0 + 127 with t0 = 126 j - 1
-//   produce the outputs of u = t0 + 1 .. t0 + 126) and nothing is exchanged between tiles.  Warp w (rows (w % 4) * 32 ..)
+//   u - 1, u, u + 1; tiles of 128 rows therefore advance by 126 rows (rows t0 .. t0 + 127 with t0 = 126 j - 1
+//   produce the outputs of rows t0 + 1 .. t0 + 126) and nothing is exchanged between tiles.  Warp w (rows (w % 4) * 32 ..)
 //   reads all 64 channels of its rows from TMEM and accumulates, for output channel co = w / 4, the seven per-tap
 //   partial sums P_k = sum_ci act[ci][row] * W4[ci][co][k]; then out[3u] = P0(u+1) + P3(u) + P6(u-1),
 //   out[3u+1] = P1(u+1) + P4(u), out[3u+2] = P2(u+1) + P5(u) with the neighbours' sums by shuffle (warp edges through
 //   a 256-byte shared buffer, one named barrier per tile).  `w1` / `b1` carry W4 / b4, `Lx` carries Lout.
 // wp  : packed weights of this layer, [7][2][4096] fp16 (cnn_tc_pack_weights_kernel)
 // redo: [N] set to 1 for reads with a value outside the fp16 range (recomputed on the FP32 pipe afterwards)
+// per_read: tiles restart at every read (cnn_tc_tiles)
 template <int LAYER, int CSLOT = -1>  // CSLOT >= 0 (layer 3): transposed-convolution weights from that slot of adb_c_convT
 __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_conv64_tc_kernel(const void *in, void *out, const __half *wp,
                                                                      const float *bias, const float *w1, const float *b1,
-                                                                     int n_reads, int Lx, int L1, int LP, int *redo) {
+                                                                     int n_reads, int Lx, int L1, int LP, int per_read, int *redo) {
     constexpr int NBUF = LAYER == 3 ? 3 : 2;
     constexpr int NWW = LAYER == 2 ? 2 * TC_WORKERS / 32 : TC_WORKERS / 32;  // worker warps (layer 2: builders + drainers)
     const int a0t_rows = LP;                                    // rows per octet of A0T (cnn_tc_a0t_rows)
-    const size_t a0t_read_bytes = (size_t)2 * 8 * a0t_rows * 16;
+    const TcTiles T = cnn_tc_tiles(LAYER, n_reads, L1, per_read);
     extern __shared__ __align__(1024) unsigned char tsm[];
     unsigned char *Wsm = tsm;                                   // resident weights [7][hi, lo][8][64][8] fp16
     unsigned char *Abuf = tsm + TC_WBYTES;                      // NBUF tile buffers x (hi plane, lo plane)
@@ -224,9 +275,8 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem = *tmem_slot;
 
-    // layer 2 tiles: t0 = 128 j; layer 3 tiles: t0 = 126 j - 1
-    const int jobs_per_read = LAYER == 3 ? (L1 + TC_L3_STRIDE - 1) / TC_L3_STRIDE : (L1 + TC_ROWS - 1) / TC_ROWS;
-    const int n_jobs = n_reads * jobs_per_read;
+    // layer 2 tiles: t0 = T.row0(j); layer 3 tiles: t0 = T.row0(j) - 1
+    const int n_jobs = T.n_jobs;
 
     // ---- LAYER 2 tile building by the workers: x window -> layer 1 on the FP32 pipe -> hi / lo planes of buffer b ----
     float px[2];
@@ -240,19 +290,18 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
         }
     }
     auto prefetch = [&](int job) {
-        const int r = job / jobs_per_read, t0 = (job % jobs_per_read) * TC_ROWS;
-        const float *xr = (const float *)in + (size_t)r * Lx;
-        const int x0 = 3 * (t0 - 3) - 3;
+        // x of row t0 - 3 (packed: 3 (t0 - 3) - 3 = 3 t0 - 12 in the whole chunk's x; per-read: in its read's x row).
+        // Samples of other reads that land in the window only feed rows that are not positions of this tile's reads.
+        const int x0 = (job / T.jpr) * Lx + 3 * ((job % T.jpr) * TC_ROWS) - 12, xn = n_reads * Lx;
 #pragma unroll
         for (int u = 0; u < 2; u++) {
             const int i = tid + u * TC_WORKERS, j = x0 + i;
-            px[u] = (i < TC_NX && j >= 0 && j < Lx) ? xr[j] : 0.0f;
+            px[u] = (i < TC_NX && j >= 0 && j < xn) ? ((const float *)in)[j] : 0.0f;
         }
     };
     auto build = [&](int job, int b) {
-        const int r = job / jobs_per_read, t0 = (job % jobs_per_read) * TC_ROWS;
+        const int t0 = T.row0(job);
         unsigned char *hi_plane = Abuf + (size_t)b * 2 * TC_PLANE, *lo_plane = hi_plane + TC_PLANE;
-        bool bad = false;
         asm volatile("bar.sync 1, %0;" ::"n"(TC_WORKERS) : "memory");  // every worker is done with the previous x window
 #pragma unroll
         for (int u = 0; u < 2; u++) {
@@ -262,9 +311,9 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
         asm volatile("bar.sync 1, %0;" ::"n"(TC_WORKERS) : "memory");
         // warp w builds channel octet w (its 8 x 7 layer-1 weights live in registers), lanes walk the rows
         for (int q = lane; q < TC_NQ; q += 32) {
-            const int p = t0 - 3 + q;
-            float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // zero padding of layer 2's input outside [0, L1)
-            if (p >= 0 && p < L1) {
+            int r, p;
+            float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};  // zero padding of layer 2's input outside the reads
+            if (tc_row_read(t0 - 3 + q, T.S, L1, n_reads, r, p)) {
                 float xs[CNN_K];
 #pragma unroll
                 for (int k = 0; k < CNN_K; k++) xs[k] = Xs[3 * q + k];
@@ -276,17 +325,16 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
                     v[j] = fmaxf(a, 0.0f);
                 }
             }
-            bad |= tc_split_store(hi_plane, lo_plane, warp, q, v);
+            // (only a position of a read can leave the range: r is that read)
+            if (tc_split_store(hi_plane, lo_plane, warp, q, v)) { redo[r] = 1; redo[-1] = 1; }  // redo[-1]: "any read flagged" (lets the FP32 pass leave at once)
         }
-        if (bad) { redo[r] = 1; redo[-1] = 1; }  // redo[-1]: "any read flagged" (lets the FP32 pass leave at once)
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic writes -> visible to the tensor core
         asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&afull[b])) : "memory");
     };
     // ---- LAYER 3 tile loading: sixteen bulk copies (plane x octet runs of 134 rows) completing on afull[b] ----
     auto load_tile = [&](int job, int b) {
-        // rows of positions t0 - 3 .. t0 + 130 with t0 = 126 j - 1: rho = position + 4 starts at 126 j
-        const int r = job / jobs_per_read, rho0 = (job % jobs_per_read) * TC_L3_STRIDE;
-        const unsigned char *src = (const unsigned char *)in + (size_t)r * a0t_read_bytes + (size_t)rho0 * 16;
+        // rows t0 - 3 .. t0 + 130 with t0 = row0 - 1: rho = g + 4 starts at row0
+        const unsigned char *src = (const unsigned char *)in + (size_t)T.row0(job) * 16;
         unsigned char *dst = Abuf + (size_t)b * 2 * TC_PLANE;
         mbar_expect_tx(&afull[b], 16 * TC_TILE_RUN);
 #pragma unroll 1
@@ -318,17 +366,17 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
     };
     // ---- epilogue of one tile: warp w reads TMEM lanes (w % 4) * 32.., columns (w / 4) * 32.. of accumulator tb ----
     auto epilogue = [&](int job, int tb, uint32_t phase, int eb) {
-        const int r = job / jobs_per_read;
-        const int t0 = LAYER == 3 ? (job % jobs_per_read) * TC_L3_STRIDE - 1 : (job % jobs_per_read) * TC_ROWS;
+        const int g = T.row0(job) - (LAYER == 3 ? 1 : 0) + (warp & 3) * 32 + lane;  // this thread's row
         mbar_wait(&accb[tb], phase);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const int q = (warp & 3) * 32 + lane, ch0 = ((warp >> 2) & 1) * 32;  // (layer 2: the drainers are warps 8 .. 15)
-        const int p = t0 + q;
+        int r, p;
+        // rows that are not positions of a read are zero padding: for layer 3's input and for the transposed convolution
+        const bool live = tc_row_read(g, T.S, L1, n_reads, r, p);
         uint32_t v[32];
         if (LAYER == 3) {
             const int co = warp >> 2, wq = warp & 3;
             const uint32_t taddr = tmem + ((uint32_t)(wq * 32) << 16) + (uint32_t)(tb * 128);
-            const bool live = p >= 0 && p < L1;   // rows outside the read are zero padding for the transposed convolution
             float P[CNN_K] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
             const float4 *wv = reinterpret_cast<const float4 *>(W4s + co * 512);
 #pragma unroll
@@ -381,7 +429,7 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
             if (lane == 31 && wq < 3) { up0 = eg[(wq + 1) * 4 + 0]; up1 = eg[(wq + 1) * 4 + 1]; up2 = eg[(wq + 1) * 4 + 2]; }
             if (lane == 0 && wq > 0) dn6 = eg[(wq - 1) * 4 + 3];
             const int Lout = Lx;
-            if (q >= 1 && q <= TC_L3_STRIDE && p < L1 && 3 * p < Lout) {
+            if (q >= 1 && q <= TC_L3_STRIDE && live && 3 * p < Lout) {
                 const float bco = b1[co];
                 float *orow = (float *)out + ((size_t)r * 2 + co) * Lout + 3 * p;
                 orow[0] = __fadd_rn(bco, __fadd_rn(__fadd_rn(up0, P[3]), dn6));
@@ -389,7 +437,7 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
                 if (3 * p + 2 < Lout) orow[2] = __fadd_rn(bco, __fadd_rn(up2, P[5]));
             }
         } else {
-            // bias + ReLU, split, and straight into layer 3's tile layout (rows >= L1: zeros = its padding)
+            // bias + ReLU, split, and straight into layer 3's tile layout (rows outside the reads: zeros = its padding)
             const uint32_t taddr = tmem + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(tb * 128 + ch0);
             tc_ld32(taddr, v);
             {   // + the hi * lo products (columns 64 ..)
@@ -398,7 +446,7 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
 #pragma unroll
                 for (int c = 0; c < 32; c++) v[c] = __float_as_uint(__fadd_rn(__uint_as_float(v[c]), __uint_as_float(v2[c])));
             }
-            unsigned char *base = (unsigned char *)out + (size_t)r * a0t_read_bytes + (size_t)(p + TC_A0T_PAD) * 16;
+            unsigned char *base = (unsigned char *)out + (size_t)(g + TC_A0T_PAD) * 16;
             bool bad = false;
 #pragma unroll
             for (int o = 0; o < 4; o++) {
@@ -407,7 +455,7 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
                 for (int j = 0; j < 4; j++) {
                     float f0 = fmaxf(__fadd_rn(__uint_as_float(v[8 * o + 2 * j]), Bs[ch0 + 8 * o + 2 * j]), 0.0f);
                     float f1 = fmaxf(__fadd_rn(__uint_as_float(v[8 * o + 2 * j + 1]), Bs[ch0 + 8 * o + 2 * j + 1]), 0.0f);
-                    if (p >= L1) { f0 = 0.0f; f1 = 0.0f; }
+                    if (!live) { f0 = 0.0f; f1 = 0.0f; }
                     const __half h0 = __float2half_rn(f0), h1 = __float2half_rn(f1);
                     const float g0 = __half2float(h0), g1 = __half2float(h1);
                     bad |= !(fabsf(g0) <= 65504.0f) || !(fabsf(g1) <= 65504.0f);
@@ -418,7 +466,7 @@ __global__ void __launch_bounds__(LAYER == 2 ? TC_THREADS2 : TC_THREADS, 1) cnn_
                 *reinterpret_cast<uint4 *>(base + off) = *reinterpret_cast<const uint4 *>(h);
                 *reinterpret_cast<uint4 *>(base + (size_t)8 * ((size_t)a0t_rows * 16) + off) = *reinterpret_cast<const uint4 *>(l);
             }
-            if (bad) { redo[r] = 1; redo[-1] = 1; }
+            if (bad) { redo[r] = 1; redo[-1] = 1; }  // (gap rows are zeros: a flagged row is a position of read r)
         }
     };
 
@@ -511,18 +559,18 @@ static int cnn_tc_launch_setup() {
 
 // layer 2: in = x, out = A0T;  layer 3: in = A0T, out = scores [N][2][Lout] (w1 / b1 = W4 / b4, Lx = Lout)
 static void cnn_tc_launch(int layer, const void *in, void *out, const __half *wp, const float *bias, const float *w1,
-                          const float *b1, int n_reads, int Lx, int L1, int LP, int *redo, int sm_count, cudaStream_t st,
-                          int cslot) {
-    const int jobs = n_reads * (layer == 3 ? (L1 + TC_L3_STRIDE - 1) / TC_L3_STRIDE : (L1 + TC_ROWS - 1) / TC_ROWS);
+                          const float *b1, int n_reads, int Lx, int L1, int LP, int per_read, int *redo, int sm_count,
+                          cudaStream_t st, int cslot) {
+    const int jobs = cnn_tc_tiles(layer, n_reads, L1, per_read).n_jobs;
     const int grid = std::max(1, std::min(jobs, sm_count));
     const size_t smem = cnn_tc_smem_bytes_layer(layer);
-    if (layer == 2) cnn_conv64_tc_kernel<2><<<grid, TC_THREADS2, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, redo);
-    else if (cslot == 0) cnn_conv64_tc_kernel<3, 0><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, redo);
-    else if (cslot == 1) cnn_conv64_tc_kernel<3, 1><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, redo);
-    else if (cslot == 2) cnn_conv64_tc_kernel<3, 2><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, redo);
-    else if (cslot == 3) cnn_conv64_tc_kernel<3, 3><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, redo);
-    else cnn_conv64_tc_kernel<3><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, redo);
+    if (layer == 2) cnn_conv64_tc_kernel<2><<<grid, TC_THREADS2, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, per_read, redo);
+    else if (cslot == 0) cnn_conv64_tc_kernel<3, 0><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, per_read, redo);
+    else if (cslot == 1) cnn_conv64_tc_kernel<3, 1><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, per_read, redo);
+    else if (cslot == 2) cnn_conv64_tc_kernel<3, 2><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, per_read, redo);
+    else if (cslot == 3) cnn_conv64_tc_kernel<3, 3><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, per_read, redo);
+    else cnn_conv64_tc_kernel<3><<<grid, TC_THREADS, smem, st>>>(in, out, wp, bias, w1, b1, n_reads, Lx, L1, LP, per_read, redo);
 }
 
-static size_t cnn_tc_a0t_bytes_per_read(int L1) { return (size_t)2 * 8 * cnn_tc_a0t_rows(L1) * 16; }
-static int cnn_tc_a0t_rows_host(int L1) { return cnn_tc_a0t_rows(L1); }
+static int cnn_tc_a0t_rows_host(int n_reads, int L1, int per_read) { return cnn_tc_a0t_rows(n_reads, L1, per_read); }
+static int cnn_tc_read_rows_host(int L1, int per_read) { return cnn_tc_read_rows(L1, per_read); }

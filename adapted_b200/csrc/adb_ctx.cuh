@@ -53,6 +53,7 @@ struct AdbOptions {
     int hist_validate = 1;       // "hist_validate" 0: counting passes (validate_fast_kernel) instead of the tensor-core histograms (adb_vhist.cuh)
     int no_cand_followup = 0;    // "no_cand_followup": further poly(A) candidates go to validate_kernel (A/B)
     int cnn_fp32 = 0;            // "cnn_fp32_pipe": 64->64 convolutions on the FP32 pipe instead of tcgen05
+    int cnn_tc_per_read = 0;     // "cnn_tc_per_read_tiles": tensor-core convolution tiles restart at every read instead of walking the packed row stream (A/B)
     int exact_gsel = 0;          // "exact_global_select": always use the multi-pass select
     int host_zstd = 0;           // "host_zstd": adb_detect_files decompresses zstd frames on the host (A/B)
 };
@@ -94,7 +95,7 @@ struct adb_ctx {
     DevBuf llr_cc;             // prefix sums of llr_primary_kernel (per resident CTA)
     DevBuf vf_done;            // per-read flags of validate_fast_kernel
     int ct_slot = -1;          // this context's slot of the constant bank adb_c_convT (adb_cnn_tc.cuh), -1: none left
-    int cnn_a0t_l1 = -1;       // L1 the tile-layout activation buffer was last zeroed for
+    int cnn_a0t_geom[3] = {-1, -1, -1};  // (L1, rows per read, rows per octet) the tile-layout activation buffer was last zeroed for
     int vf_last_reads = 0;
     int gsb_last_batches = 0;
     int64_t zstd_host_frames = 0;  // adb_ctx_query("zstd_host_frames"): frames the last call decompressed on the host
